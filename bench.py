@@ -15,6 +15,12 @@ accumulators.  Prints ONE JSON line on rank 0.
   --config 3   BASELINE configs[3]: x4 128->512 (infer_x4 / UC Merced shape), global batch 32 sharded (strong)
   --sweep      BASELINE configs[4]: x4 64->256 global batch 1..256 on the N ranks (device-timed images/s per
                batch size in one JSON line, next to the CPU B = 1 rate at N = 1)
+
+  --dump-outputs DIR   after the timed steps, write what the last one returned: DIR/sr.npy (float32 SR images,
+               (B,3,H,W), the whole batch for N > 1) and DIR/psnr.npy (float64 PSNR of each image vs the synthetic HR);
+               with --impl reference, DIR/sr.npy of its one image.  The inputs depend only on the arguments, so two
+               builds of the project can be compared output for output.
+  --steps K    timed steps of every loop; with --sweep, the timed batches per batch size.
 """
 import argparse
 import json
@@ -43,7 +49,12 @@ def parse():
     ap.add_argument("--hr", type=int, default=None, help="HR resolution (overrides the config)")
     ap.add_argument("--dtype", default=os.environ.get("FDSR_DTYPE", "fp16"))
     ap.add_argument("--no-cpu-baseline", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the last timed step's outputs as DIR/<name>.npy")
     a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
+    if a.dump_outputs and a.sweep:
+        ap.error("--dump-outputs writes the outputs of one timed sampling path, not of the --sweep batch sizes")
     world = int(os.environ.get("WORLD_SIZE", "1"))
     # (lr, hr, global batch or None = 16 per rank, scaling)
     lr, hr, gb, scaling = {1: (64, 256, None, "weak"), 2: (32, 256, 64, "strong"), 3: (128, 512, 32, "strong")}[a.config]
@@ -63,6 +74,24 @@ def synthetic_lr(batch, res, seed):
     a = torch.randint(0, 256, (batch, 3, res, res), generator=g).float()
     a = torch.nn.functional.avg_pool2d(torch.nn.functional.pad(a, (2, 2, 2, 2), mode="reflect"), 5, 1)
     return a.round().clamp(0, 255).to(torch.uint8).permute(0, 2, 3, 1).contiguous()
+
+
+DUMP_BYTES = 60_000_000   # --dump-outputs writes at most 64 MB, .npy headers included
+
+
+def dump_outputs(d, arrays):
+    """Each array as d/<name>.npy.  One that would take the dump past DUMP_BYTES is written as a fixed, seeded sample of
+    its rows (last axis whole): the same rows in every run with the same arguments."""
+    import numpy as np
+    os.makedirs(d, exist_ok=True)
+    room = DUMP_BYTES
+    for name, a in arrays.items():
+        a = a.cpu().numpy()
+        if a.nbytes > room:
+            rows = a.reshape(-1, a.shape[-1])
+            a = rows[np.sort(np.random.default_rng(0).choice(len(rows), room // rows[0].nbytes, replace=False))]
+        np.save(os.path.join(d, name + ".npy"), a)
+        room -= a.nbytes
 
 
 def measured_peaks():
@@ -150,8 +179,10 @@ def run_reference(args, rank):
         O.unet_forward(sd, cfg, torch.cat([cond, noises[0]], 1), torch.full((1, 1), 0.5))  # warm threads/allocator
     t0 = time.perf_counter()
     for _ in range(args.steps):
-        O.sample_loop(sd, cfg, tab, cond, noises)
+        sr = O.sample_loop(sd, cfg, tab, cond, noises)
     dt = (time.perf_counter() - t0) / args.steps
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"sr": sr})
     val = 1.0 / dt
     sample = f"T=20 sampling of 1 image {args.lr}->{args.hr} per step, fp32, torch CPU {cores} threads"
     out = {"impl": "reference", "metric": "sr_images_per_s_T20", "value": val, "unit": "images/s",
@@ -218,7 +249,7 @@ def run_ours(args, rank, world, local_rank):
             P.reduce_sums(local)                           # all-reduce of the metric sums
             del full
         acc.add_(local)
-        return sr
+        return sr, psnr
 
     sr_host = np.zeros((B, 3, H, H), dtype=np.float32)   # caller-owned result buffer, reused every step
 
@@ -238,19 +269,26 @@ def run_ours(args, rank, world, local_rank):
         e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         l0 = eng.launch_count()
         e0.record()
-        for i in range(steps):
+        for i in range(steps - 1):
             fn(warmup + i)
+        last = fn(warmup + steps - 1)      # only the last result is held: every step reuses the freed output buffer
         e1.record()
         sync()
         ms = torch.tensor([e0.elapsed_time(e1)], dtype=torch.float64, device=dev)
         if world > 1:
             dist.all_reduce(ms, op=dist.ReduceOp.MAX)
-        return ms.item() / steps, eng.launch_count() - l0
+        return ms.item() / steps, eng.launch_count() - l0, last
 
     clocks = ClockSampler(local_rank) if rank == 0 else None
     if clocks:
         clocks.start()
-    ms_dev, launches = timed(step_device, args.steps, max(args.warmup, 3))
+    ms_dev, launches, (sr_last, psnr_last) = timed(step_device, args.steps, max(args.warmup, 3))
+    if args.dump_outputs:
+        if world > 1:
+            sr_last, psnr_last = P.gather_batch(sr_last, B * world), P.gather_batch(psnr_last, B * world)
+        if rank == 0:
+            dump_outputs(args.dump_outputs, {"psnr": psnr_last, "sr": sr_last})
+    del sr_last, psnr_last
     ws_gib = eng.workspace_bytes() / 2 ** 30
     # end to end through the host-buffer API, one batch submitted ahead: the H2D / D2H copies and the host-side memcpy of
     # batch i overlap the sampling of batch i+1 (every step still copies its own input in and its own result out)
@@ -272,7 +310,7 @@ def run_ours(args, rank, world, local_rank):
             dist.all_reduce(ms, op=dist.ReduceOp.MAX)
         return ms.item() / steps
 
-    ms_e2e = timed_e2e(max(3, min(args.steps, 6)), 1)
+    ms_e2e = timed_e2e(args.steps, 1)
     clk = clocks.stop() if clocks else None
     value = B * world / (ms_dev / 1e3)
     e2e = B * world / (ms_e2e / 1e3)
@@ -384,7 +422,7 @@ def run_sweep(args, rank, world, local_rank):
         if mine > 0:
             lr = torch.from_numpy(synthetic_lr(mine, h, 1 + rank).numpy()).to(dev)
             _, cond = eng.bicubic_u8(lr, H, H, want_u8=False)
-            reps = max(2, min(8, 64 // mine))
+            reps = args.steps
             for i in range(2):
                 netG.super_resolution(cond, False, seed=i, image_offset=start)
         torch.cuda.synchronize(dev)
@@ -410,7 +448,7 @@ def run_sweep(args, rank, world, local_rank):
     if rank == 0:
         best = max(rows, key=lambda r: r["images_per_s"])
         emit({"metric": "sr_images_per_s_T20", "value": best["images_per_s"], "unit": "images/s", "n_gpus": world,
-              "steps": len(rows), "warmup": 2, "ms_per_step": best["ms_per_batch"], "higher_is_better": True,
+              "steps": args.steps, "warmup": 2, "ms_per_step": best["ms_per_batch"], "higher_is_better": True,
               "scaling": "strong", "vs_baseline": None, "dtype": args.dtype, "data": "synthetic",
               "config": {"workload": f"FastDiffSR x{H // h} {h}->{H} T={T} sampling, global batch sweep 1..256 on "
                                      f"{world} rank(s) (BASELINE configs[4]); value = best row"},

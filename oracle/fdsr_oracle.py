@@ -6,13 +6,13 @@ the CUDA path: only ``tests/``, ``__graft_entry__.smoke()`` and ``bench.py``'s C
 ``--impl reference`` legs may import it.  The product package never does (it fails loudly when
 its CUDA library is missing).
 
-Parity pinning: ``oracle/make_golden.py`` imports the real reference from ``/root/reference``
-(possible only in the build container), asserts that every function below reproduces it, and
+Parity pinning: ``oracle/make_golden.py`` imports the real reference from a checkout of the
+original FastDiffSR repository, asserts that every function below reproduces it, and
 writes ``tests/golden/*.npz``; ``tests/test_oracle_golden.py`` re-checks this file against those
 fixtures anywhere.  The bicubic restatement is additionally pinned by the reference's own
 UC-Merced fixtures (lr_128 -> sr_128_512, bit-exact).
 
-Reference locations restated here (paths relative to /root/reference/FastDiffSR):
+Reference locations restated here (paths relative to the original FastDiffSR repository):
   make_beta_schedule            model/fastdiffsr_modules/diffusion.py:21-64
   schedule tables               model/fastdiffsr_modules/diffusion.py:109-155
   p_mean_variance / p_sample    model/fastdiffsr_modules/diffusion.py:157-190
@@ -683,3 +683,23 @@ def sr3_sample_loop(sd, cfg, tables, cond, noises, image_size=256, continous=Fal
     if not continous:
         return x
     return torch.cat([torch.cat([cond[b:b + 1]] + [f[b:b + 1] for f in frames], dim=0) for b in range(B)], dim=0)
+
+
+# --------------------------------------------------------------------------------------
+# Golden fixtures (tests/golden/*.npz, written by oracle/make_golden.py)
+# --------------------------------------------------------------------------------------
+
+def golden_inputs(name):
+    """The seeded inputs of fixture `name`, in the order make_golden.py draws them.  The fixture stores the float64 sum
+    of each (`<input>_sum`) instead of the tensor; the tests regenerate the input here and check that sum."""
+    if name.startswith("unet64_"):
+        g = torch.Generator().manual_seed(11)
+        x6 = torch.randn(2, 6, 64, 64, generator=g)
+        cond = torch.rand(1, 3, 64, 64, generator=g) * 2 - 1
+        return dict(x6=x6, cond=cond, noises=torch.randn(20, 1, 3, 64, 64, generator=g))
+    if name.startswith("sr3_"):
+        H = {"sr3_256": 128, "sr3_64": 64}[name]
+        g = torch.Generator().manual_seed(21)
+        x6 = torch.randn(2, 6, H, H, generator=g).half().float()   # exactly representable in fp16
+        return dict(x6=x6, cond=torch.rand(1, 3, H, H, generator=g) * 2 - 1)
+    return {}

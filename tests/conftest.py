@@ -1,6 +1,7 @@
 import os
 import sys
 
+import numpy as np
 import pytest
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
@@ -18,6 +19,20 @@ def pytest_configure(config):
 @pytest.fixture(scope="session")
 def golden_dir():
     return GOLDEN
+
+
+@pytest.fixture(scope="session")
+def golden(oracle):
+    """load(name) -> tests/golden/<name>.npz as a dict, with the seeded inputs the fixture does not store regenerated
+    (fdsr_oracle.golden_inputs) after checking each against the float64 sum stored as `<input>_sum`."""
+    def load(name):
+        with np.load(os.path.join(GOLDEN, name + ".npz")) as z:
+            g = dict(z)
+        for k, v in oracle.golden_inputs(name).items():
+            assert abs(float(v.double().sum()) - float(g[k + "_sum"])) < 1e-6, f"{name}: {k} differs from the fixture's"
+            g[k] = v.numpy()
+        return g
+    return load
 
 
 @pytest.fixture(scope="session")

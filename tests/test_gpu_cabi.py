@@ -12,12 +12,12 @@ pytestmark = pytest.mark.gpu
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
 
-def test_plain_c_program_samples_and_matches_reference(oracle, schedule, golden_dir, tmp_path):
+def test_plain_c_program_samples_and_matches_reference(oracle, schedule, golden, tmp_path):
     from fastdiffsr_b200._lib import LIB_PATH
     cuda = os.environ.get("CUDA_HOME", "/usr/local/cuda")
     if shutil.which("gcc") is None or not os.path.exists(os.path.join(cuda, "include", "cuda_runtime_api.h")):
         pytest.skip("gcc or the CUDA runtime headers are missing")
-    g = np.load(os.path.join(golden_dir, "unet64_default.npz"))
+    g = golden("unet64_default")
     sd = oracle.make_state_dict(oracle.DEFAULT_UNET, seed=0)        # the weights the fixture was generated with
     d = tmp_path
     with open(d / "manifest.txt", "w") as mf, open(d / "weights.bin", "wb") as wf:

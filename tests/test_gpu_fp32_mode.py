@@ -2,8 +2,6 @@
 the committed reference outputs and the oracle.  BASELINE.json north_star: per-step epsilon relative
 L2 <= 1e-4 in fp32 mode.  Needs a B200: `pytest -m gpu`.
 """
-import os
-
 import numpy as np
 import pytest
 import torch
@@ -34,9 +32,9 @@ def ctx32(oracle, schedule):
 
 
 @pytest.mark.parametrize("tag", ["default", "jitter"])
-def test_fp32_unet_eps_vs_reference_golden(ctx32, golden_dir, tag):
+def test_fp32_unet_eps_vs_reference_golden(ctx32, golden, tag):
     sd, eng = ctx32[tag]
-    g = np.load(os.path.join(golden_dir, f"unet64_{tag}.npz"))
+    g = golden(f"unet64_{tag}")
     x6 = torch.from_numpy(g["x6"]).cuda()
     for i, t in enumerate((19, 7)):
         eps = eng.unet_forward(x6[:, :3].contiguous(), x6[:, 3:].contiguous(), t).cpu()
@@ -69,11 +67,11 @@ def test_fp32_every_layer_vs_oracle(ctx32, oracle, schedule):
     assert rel_l2(eps, eps_ref) <= EPS_TOL_FP32
 
 
-def test_fp32_sampler_vs_reference_golden(ctx32, oracle, golden_dir):
+def test_fp32_sampler_vs_reference_golden(ctx32, oracle, golden):
     """The whole 20-step chain with the reference's injected noise: trajectory stays within 1e-3 of the
     reference (the clamp and 20 accumulated steps amplify the per-step 1e-5), PSNR delta <= 0.05 dB."""
     sd, eng = ctx32["default"]
-    g = np.load(os.path.join(golden_dir, "unet64_default.npz"))
+    g = golden("unet64_default")
     cond = torch.from_numpy(g["cond"]).cuda()
     noises = torch.from_numpy(g["noises"]).cuda()
     ref = torch.from_numpy(g["sr"])

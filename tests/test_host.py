@@ -13,7 +13,8 @@ from fastdiffsr_b200 import _lib
 from fastdiffsr_b200.config import default_config, load_config, NoneDict
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-REF_CFG = "/root/reference/FastDiffSR/config"
+# a checkout of the original FastDiffSR repository (test_reference_DDPM_wrapper_runs_on_patched_define_G)
+REF_ROOT = os.environ.get("FASTDIFFSR_REFERENCE", "")
 
 
 def test_config_comment_stripping(tmp_path):
@@ -22,6 +23,9 @@ def test_config_comment_stripping(tmp_path):
     opt = load_config(str(p), phase="val")
     assert opt["gpu_ids"] == [0, 1] and opt["distributed"] is True
     assert isinstance(opt["model"], NoneDict) and opt["model"]["missing"] is None
+    # README names a file that does not exist; the alias resolves to infer_x4 (SURVEY F4)
+    (tmp_path / "sr_fastdiffsr_infer_x4.json").write_text('{"datasets": {"val": {"l_resolution": 128}}}\n')
+    assert load_config(str(tmp_path / "sr_fastdiffsr_infer_128_512.json"))["datasets"]["val"]["l_resolution"] == 128
 
 
 def test_default_configs_cover_reference_names():
@@ -31,19 +35,6 @@ def test_default_configs_cover_reference_names():
         assert opt["model"]["which_model_G"] == "fastdiffsr"
         assert opt["model"]["beta_schedule"]["val"]["n_timestep"] == 20
     assert default_config("sr_fastdiffsr_infer_x4")["datasets"]["val"]["r_resolution"] == 512
-
-
-@pytest.mark.skipif(not os.path.isdir(REF_CFG), reason="reference tree only exists in the build container")
-def test_default_configs_equal_reference_json():
-    for name in ("sr_fastdiffsr_test_64_256", "sr_fastdiffsr_test_32_256", "sr_fastdiffsr_infer_x4"):
-        ref = load_config(os.path.join(REF_CFG, name + ".json"))
-        mine = default_config(name)
-        for key in ("unet", "beta_schedule", "diffusion", "which_model_G"):
-            assert ref["model"][key] == mine["model"][key], (name, key)
-        assert ref["datasets"]["train"]["l_resolution"] == mine["datasets"]["train"]["l_resolution"]
-    # README names a file that does not exist; the alias resolves to infer_x4 (SURVEY F4)
-    opt = load_config(os.path.join(REF_CFG, "sr_fastdiffsr_infer_128_512.json"))
-    assert opt["datasets"]["val"]["l_resolution"] == 128
 
 
 def test_define_G_surface_and_state_dict(oracle, golden_dir):
@@ -74,16 +65,12 @@ def test_define_G_surface_and_state_dict(oracle, golden_dir):
 
 
 def test_sr3_define_G_surface_and_configs(oracle):
-    """which_model_G = 'ddpm' (the SR3 baseline): config defaults equal the reference JSONs, state_dict surface
-    equals the reference's (421 tensors incl. the time_mlp.0.inv_freq buffer), no CPU fallback."""
+    """which_model_G = 'ddpm' (the SR3 baseline): config defaults, state_dict surface equals the reference's (421
+    tensors incl. the time_mlp.0.inv_freq buffer), no CPU fallback."""
     for name in ("sr_ddpm_test_64_256", "sr_ddpm_test_32_256", "sr_ddpm_infer_x4"):
         mine = default_config(name)
         assert mine["model"]["which_model_G"] == "ddpm" and mine["model"]["beta_schedule"]["val"]["n_timestep"] == 1000
-        if os.path.isdir(REF_CFG):
-            ref = load_config(os.path.join(REF_CFG, name + ".json"))
-            for key in ("unet", "beta_schedule", "diffusion", "which_model_G"):
-                assert ref["model"][key] == mine["model"][key], (name, key)
-    opt = default_config("sr_ddpm_test_64_256")
+    opt =default_config("sr_ddpm_test_64_256")
     netG = F.define_G(opt)
     assert isinstance(netG.denoise_fn, F.SR3UNet) and netG.sr3
     keys = [(k, tuple(v.shape)) for k, v in netG.state_dict().items()]
@@ -194,10 +181,9 @@ def test_reference_checkpoint_with_schedule_buffers_loads_through_load_network(o
         evaluate.load_network(F.define_G(opt), opt)
 
 
-REF_ROOT = "/root/reference/FastDiffSR"
-
-
-@pytest.mark.skipif(not os.path.isdir(REF_ROOT), reason="reference tree only exists in the build container")
+@pytest.mark.skipif(not REF_ROOT, reason="imports and runs the original FastDiffSR's own model/ package, which is not part "
+                                          "of this repository and cannot be stored as test data; runs when "
+                                          "FASTDIFFSR_REFERENCE names a checkout of that repository")
 def test_reference_DDPM_wrapper_runs_on_patched_define_G(oracle, tmp_path):
     """INTEGRATION.md's one-line patch, exercised with the reference's OWN wrapper: `model.networks.define_G` replaced
     by fastdiffsr_b200.define_G, then the unmodified `model.model.DDPM` (model/model.py:12-42) is constructed — set_device,
