@@ -71,6 +71,9 @@ _SIGS = {
                                       C.c_int64, C.c_void_p]),
     "fdsr_sample": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint64, C.c_void_p, C.c_void_p,
                               C.c_int32, C.c_int32, C.c_int32, C.c_void_p]),
+    "fdsr_sample_tiled": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint64, C.c_void_p, C.c_void_p,
+                                    C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.c_int32,
+                                    C.c_void_p]),
     "fdsr_trace_frames": (C.c_int32, [C.c_void_p]),
     "fdsr_super_resolve_u8": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int32, C.c_int32, C.c_int32, C.c_int32,
                                         C.c_int32, C.c_void_p, C.c_uint64, C.c_void_p, C.c_void_p]),

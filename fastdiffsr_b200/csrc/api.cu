@@ -18,6 +18,7 @@
 #include "conv_kernel.cuh"
 #include "conv_f32.cuh"
 #include "attn_kernel.cuh"
+#include "tile_kernels.cuh"
 
 using namespace fdsr;
 
@@ -195,6 +196,10 @@ struct fdsr_ctx {
   }
   int64_t launches = 0;
   double flops_per_px = 0.0;  // conv FLOPs per full-resolution output pixel per image
+  // fdsr_sample_tiled: [SampleArgs | canvas x_t (B,3,H,W) fp32 | per-tile eps store [slot][3][te_y][te_x] fp32],
+  // grow-only, apart from the workspace (which only ever holds one chunk of tiles)
+  uint8_t* d_tiled = nullptr;
+  size_t tiled_cap = 0;
 };
 
 namespace {
@@ -1430,14 +1435,15 @@ int pack_input(fdsr_ctx* c, cudaStream_t st) {
 //   fused = false: cat[cond, x] is packed first and eps lands in the internal eps buffer (the fdsr_unet_forward hook);
 //   fused = true (sampler): the packed input already holds x_t (written by the previous step's epilogue) and the final
 //                  conv's epilogue turns eps into x_{t-1} in place (kOutPosterior) — no pack / posterior launches.
+//   packed = true (tiled sampler): the network input was assembled by tile_pack_kernel; eps lands in the eps buffer.
 template <typename T>
-int unet_internal(fdsr_ctx* c, int t, cudaStream_t st, bool fused) {
+int unet_internal(fdsr_ctx* c, int t, cudaStream_t st, bool fused, bool packed = false) {
   if (c->layers_dirty) {
     int rc = upload_layers(c);
     if (rc) return rc;
   }
   CUDA_TRY(c, cudaMemsetAsync(c->d_ws + c->stats_off, 0, c->stats_bytes, st));
-  if (!fused) {
+  if (!fused && !packed) {
     int rc = pack_input<T>(c, st);
     if (rc) return rc;
   }
@@ -1529,6 +1535,68 @@ int sample_enqueue(fdsr_ctx* c, bool has_trace, cudaStream_t st) {
     }
   }
   res2img_kernel<<<gb, 256, 0, st>>>(x, cond, sr, per, per, B, args, 0, sr3);
+  ++c->launches;
+  CUDA_TRY(c, cudaGetLastError());
+  return FDSR_OK;
+}
+
+// One axis of the tile grid (the rule stated in tile_kernels.cuh / include/fdsr.h)
+TileAxis make_axis(int L, int t, int overlap) {
+  TileAxis a;
+  a.L = L;
+  a.te = std::min(t, L / 8 * 8);
+  a.oe = std::min(overlap, a.te - 8);
+  a.s = a.te - a.oe;
+  a.n = L > a.te ? (L - a.te + a.s - 1) / a.s + 1 : 1;
+  return a;
+}
+
+// The T-step tiled loop.  d_tiled holds [SampleArgs | x (B,3,H,W) | eps store of n_chunks * bc tile slots]; the
+// workspace is reserved for one chunk (bc tiles of te_y x te_x).  Plain stream launches: a chunk's UNet (~5 ms at
+// bc = 16, 256^2) keeps the device well behind the host's ~0.3 ms of launch calls.
+template <typename T>
+int tiled_enqueue(fdsr_ctx* c, const float* cond, float* sr_out, bool has_trace, int B, const TileAxis& ay,
+                  const TileAxis& ax, int64_t n_tiles, int64_t n_chunks, int bc, cudaStream_t st) {
+  const SampleArgs* args = reinterpret_cast<const SampleArgs*>(c->d_tiled);
+  const uint32_t HW = uint32_t(ay.L) * uint32_t(ax.L);
+  const int64_t per = int64_t(3) * HW;
+  float* x = reinterpret_cast<float*>(c->d_tiled + 256);
+  float* eps_store = reinterpret_cast<float*>(c->d_tiled + 256 + align_up(size_t(per) * B * 4, 256));
+  const int64_t tile_floats = int64_t(3) * ay.te * ax.te;
+  const size_t chunk_bytes = size_t(bc) * tile_floats * 4;
+  const dim3 pgrid(unsigned((uint64_t(HW) + 255) / 256), unsigned(B));
+  const unsigned gb = unsigned((per * B + 255) / 256);
+  const unsigned pack_blocks = unsigned((int64_t(bc) * ay.te * ax.te + 255) / 256);
+  T* xin = reinterpret_cast<T*>(c->d_ws + c->tensors[c->t_xin].off);
+  const float* eps_chunk = reinterpret_cast<const float*>(c->d_ws + c->off_eps);
+  const int T_ = c->T, nfr = fdsr_trace_frames(c), inter = 1 | (T_ / 10);
+  noise_init_kernel<<<pgrid, 256, 0, st>>>(x, HW, args, uint32_t(T_));
+  ++c->launches;
+  int frame = 0;
+  if (has_trace) {
+    res2img_kernel<<<gb, 256, 0, st>>>(cond, cond, nullptr, per, per * nfr, B, args, 0, 0);
+    ++c->launches;
+    frame = 1;
+  }
+  for (int k = 0, t = T_ - 1; t >= 0; --t, ++k) {
+    for (int64_t ch = 0; ch < n_chunks; ++ch) {
+      tile_pack_kernel<T><<<pack_blocks, 256, 0, st>>>(cond, x, xin, ay, ax, ch * bc, n_tiles, bc);
+      CUDA_TRY(c, cudaGetLastError());
+      ++c->launches;
+      int rc = unet_internal<T>(c, t, st, false, true);
+      if (rc) return rc;
+      CUDA_TRY(c, cudaMemcpyAsync(eps_store + ch * bc * tile_floats, eps_chunk, chunk_bytes, cudaMemcpyDeviceToDevice, st));
+    }
+    tile_blend_posterior_kernel<<<pgrid, 256, 0, st>>>(x, eps_store, ay, ax, c->post[t], args, k + 1, uint32_t(t),
+                                                       t > 0 ? 1 : 0);
+    ++c->launches;
+    if (has_trace && t % inter == 0) {
+      res2img_kernel<<<gb, 256, 0, st>>>(x, cond, nullptr, per, per * nfr, B, args, per * frame, 0);
+      ++c->launches;
+      ++frame;
+    }
+  }
+  res2img_kernel<<<gb, 256, 0, st>>>(x, cond, sr_out, per, per, B, args, 0, 0);
   ++c->launches;
   CUDA_TRY(c, cudaGetLastError());
   return FDSR_OK;
@@ -1683,6 +1751,7 @@ int fdsr_destroy(fdsr_ctx* c) {
   cudaFree(c->d_prof);
   cudaFree(c->d_bic_tmp);
   cudaFree(c->d_metric);
+  cudaFree(c->d_tiled);
   for (auto& sl : c->slot) {
     cudaFree(sl.d_stage);
     if (sl.h_pin) cudaFreeHost(sl.h_pin);
@@ -1988,6 +2057,48 @@ int fdsr_sample(fdsr_ctx* c, const float* cond, const float* noise, uint64_t see
   }
   CUDA_TRY(c, cudaMemcpyAsync(sr_out, c->d_ws + c->off_sr, bytes, cudaMemcpyDeviceToDevice, st));
   return FDSR_OK;
+}
+
+int fdsr_sample_tiled(fdsr_ctx* c, const float* cond, const float* noise, uint64_t seed, float* sr_out, float* trace,
+                      int32_t B, int32_t H, int32_t W, int32_t tile_h, int32_t tile_w, int32_t overlap,
+                      int32_t tile_batch, void* stream) {
+  if (!c) return FDSR_E_INVALID;
+  if (!cond || !sr_out) return fail(c, FDSR_E_INVALID, "null argument");
+  if (c->cfg.model != FDSR_MODEL_FASTDIFFSR)
+    return fail(c, FDSR_E_INVALID, "tiled sampling is implemented for the FastDiffSR model only, not the SR3 baseline");
+  if (B < 1 || B > 65535) return fail(c, FDSR_E_INVALID, "B must be 1..65535 (got %d)", B);
+  if (H < 8 || W < 8) return fail(c, FDSR_E_INVALID, "canvas H and W must be >= 8 (got %dx%d)", H, W);
+  if (uint64_t(H) * uint64_t(W) >= (uint64_t(1) << 32))
+    return fail(c, FDSR_E_INVALID, "canvas H*W must be below 2^32 (got %dx%d)", H, W);
+  if (tile_h < 8 || tile_w < 8 || tile_h % 8 || tile_w % 8)
+    return fail(c, FDSR_E_INVALID, "tile sizes must be multiples of 8 and >= 8 (got %dx%d)", tile_h, tile_w);
+  if (overlap < 0) return fail(c, FDSR_E_INVALID, "overlap must be >= 0 (got %d)", overlap);
+  if (tile_batch < 1) return fail(c, FDSR_E_INVALID, "tile_batch must be >= 1 (got %d)", tile_batch);
+  int rc = check_ready(c);
+  if (rc) return rc;
+  const TileAxis ay = make_axis(H, tile_h, overlap), ax = make_axis(W, tile_w, overlap);
+  // equal chunks: every UNet call has the shape (bc, te_y, te_x); the last chunk repeats its last tile
+  const int64_t n_tiles = int64_t(B) * ay.n * ax.n;
+  const int64_t n_chunks = (n_tiles + tile_batch - 1) / tile_batch;
+  const int bc = int((n_tiles + n_chunks - 1) / n_chunks);
+  rc = fdsr_reserve(c, bc, ay.te, ax.te);
+  if (rc) return rc;
+  const size_t need = 256 + align_up(size_t(B) * 3 * H * W * 4, 256) + size_t(n_chunks) * bc * 3 * ay.te * ax.te * 4;
+  if (need > c->tiled_cap) {
+    cudaFree(c->d_tiled);
+    c->d_tiled = nullptr;
+    c->tiled_cap = 0;
+    CUDA_TRY(c, cudaMalloc(&c->d_tiled, need));
+    c->tiled_cap = need;
+  }
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  set_args_kernel<<<1, 1, 0, st>>>(reinterpret_cast<SampleArgs*>(c->d_tiled), SampleArgs{seed, c->image0, noise, trace});
+  ++c->launches;
+  if (c->cfg.dtype == FDSR_DTYPE_FP32)
+    return tiled_enqueue<float>(c, cond, sr_out, trace != nullptr, B, ay, ax, n_tiles, n_chunks, bc, st);
+  if (c->cfg.dtype == FDSR_DTYPE_BF16)
+    return tiled_enqueue<__nv_bfloat16>(c, cond, sr_out, trace != nullptr, B, ay, ax, n_tiles, n_chunks, bc, st);
+  return tiled_enqueue<__half>(c, cond, sr_out, trace != nullptr, B, ay, ax, n_tiles, n_chunks, bc, st);
 }
 
 int fdsr_bicubic_u8(fdsr_ctx* c, const uint8_t* lr, int32_t B, int32_t h, int32_t w, int32_t H, int32_t W,

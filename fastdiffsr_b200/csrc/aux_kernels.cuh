@@ -60,6 +60,29 @@ __device__ __forceinline__ void st_pair(T* p, float a, float b) {
 // Channel order of the packed input: [x0 x1 x2 0 | c0 c1 c2 0 | 0 ...] (x_t first, so that the fused posterior
 // epilogue of the final conv rewrites it with one aligned 8-byte store per pixel); the stem weights are packed with
 // the matching permutation of the reference's cat([cond, x]) order (kXinPerm in api.cu).
+// One pixel of the packed input from the three x / cond channels at xp[0], xp[plane], xp[2 plane] (likewise cp);
+// shared with the tiled sampler's tile_pack_kernel, whose one-tile result must equal fdsr_sample's bit for bit.
+template <typename T>
+__device__ __forceinline__ void pack_pixel(T* __restrict__ out, const float* __restrict__ xp,
+                                           const float* __restrict__ cp, int64_t plane) {
+  if constexpr (sizeof(T) == 4) {
+    float4* o = reinterpret_cast<float4*>(out);
+    o[0] = make_float4(xp[0], xp[plane], xp[2 * plane], 0.f);
+    o[1] = make_float4(cp[0], cp[plane], cp[2 * plane], 0.f);
+    o[2] = make_float4(0.f, 0.f, 0.f, 0.f);
+    o[3] = make_float4(0.f, 0.f, 0.f, 0.f);
+  } else {
+    uint4 lo, hi = make_uint4(0u, 0u, 0u, 0u);
+    lo.x = Cvt<T>::pack(xp[0], xp[plane]);
+    lo.y = Cvt<T>::pack(xp[2 * plane], 0.f);
+    lo.z = Cvt<T>::pack(cp[0], cp[plane]);
+    lo.w = Cvt<T>::pack(cp[2 * plane], 0.f);
+    uint4* o = reinterpret_cast<uint4*>(out);
+    o[0] = lo;
+    o[1] = hi;
+  }
+}
+
 template <typename T>
 __global__ void pack_input_kernel(const float* __restrict__ cond, const float* __restrict__ x,
                                   T* __restrict__ out, int B, int HW) {
@@ -67,24 +90,7 @@ __global__ void pack_input_kernel(const float* __restrict__ cond, const float* _
   if (i >= int64_t(B) * HW) return;
   const int b = int(i / HW);
   const int p = int(i - int64_t(b) * HW);
-  const float* cp = cond + int64_t(b) * 3 * HW + p;
-  const float* xp = x + int64_t(b) * 3 * HW + p;
-  if constexpr (sizeof(T) == 4) {
-    float4* o = reinterpret_cast<float4*>(out + i * 16);
-    o[0] = make_float4(xp[0], xp[HW], xp[2 * HW], 0.f);
-    o[1] = make_float4(cp[0], cp[HW], cp[2 * HW], 0.f);
-    o[2] = make_float4(0.f, 0.f, 0.f, 0.f);
-    o[3] = make_float4(0.f, 0.f, 0.f, 0.f);
-  } else {
-    uint4 lo, hi = make_uint4(0u, 0u, 0u, 0u);
-    lo.x = Cvt<T>::pack(xp[0], xp[HW]);
-    lo.y = Cvt<T>::pack(xp[2 * HW], 0.f);
-    lo.z = Cvt<T>::pack(cp[0], cp[HW]);
-    lo.w = Cvt<T>::pack(cp[2 * HW], 0.f);
-    uint4* o = reinterpret_cast<uint4*>(out + i * 16);
-    o[0] = lo;
-    o[1] = hi;
-  }
+  pack_pixel<T>(out + i * 16, x + int64_t(b) * 3 * HW + p, cond + int64_t(b) * 3 * HW + p, HW);
 }
 
 // ------------------------------------------------------------------------------------------

@@ -1,0 +1,125 @@
+// Tiled sampling of canvases of any size (fdsr_sample_tiled, include/fdsr.h; DESIGN §4.4): overlapping tiles share
+// one canvas-wide chain.  Every step, the tiles' eps predictions are blended into one canvas-wide eps and a single
+// posterior update moves the canvas-wide x_t (MultiDiffusion in eps space).
+//
+// Grid rule per axis (length L, tile t, overlap o):  t_e = min(t, 8 floor(L/8)), o_e = min(o, t_e - 8), s = t_e - o_e;
+// starts i*s for every i with i*s < L - t_e, then L - t_e (the last tile is flush with the far edge).
+// Weight of tile offset i: r(i) = min(i + 1, t_e - i, o_e + 1); a tile pixel weighs r_y * r_x (an exact integer).
+#pragma once
+#include <cstdint>
+#include "aux_kernels.cuh"
+
+namespace fdsr {
+
+struct TileAxis {
+  int32_t L;   // canvas extent
+  int32_t te;  // effective tile extent (multiple of 8, <= L)
+  int32_t oe;  // effective overlap
+  int32_t s;   // stride te - oe (>= 8)
+  int32_t n;   // tiles on this axis: starts i*s for i < n - 1, then L - te
+};
+
+__host__ __device__ __forceinline__ int tile_start(const TileAxis& a, int i) { return i + 1 < a.n ? i * a.s : a.L - a.te; }
+__host__ __device__ __forceinline__ int tile_ramp(const TileAxis& a, int i) {
+  return min(min(i + 1, a.te - i), a.oe + 1);
+}
+
+// Tiles of one axis covering position y, in ascending start order: the regular tiles lo..hi, then the flush last tile
+// n - 1 when it covers y (it starts after every regular tile, so the order is the global one).
+struct TileCover {
+  int lo, cnt_reg, last;  // last = n - 1 or -1
+  __device__ __forceinline__ int count() const { return cnt_reg + (last >= 0 ? 1 : 0); }
+  __device__ __forceinline__ int at(int k) const { return k < cnt_reg ? lo + k : last; }
+};
+__device__ __forceinline__ TileCover tile_cover(const TileAxis& a, int y) {
+  const int d = y - a.te + 1;
+  const int lo = d <= 0 ? 0 : (d + a.s - 1) / a.s;
+  const int hi = min(y / a.s, a.n - 2);
+  TileCover c;
+  c.lo = lo;
+  c.cnt_reg = hi >= lo ? hi - lo + 1 : 0;
+  c.last = y >= a.L - a.te ? a.n - 1 : -1;
+  return c;
+}
+
+// Packed 16-channel NHWC network input of one chunk of `bc` tiles ([x (3) 0 | cond (3) 0 | 0 x 8], pack_pixel), read
+// from the canvases at each tile's window.  Chunk slot j holds global tile min(tile0 + j, n_tiles - 1): the last chunk
+// is padded with repeats of the last tile.  One thread per tile pixel.
+template <typename T>
+__global__ void tile_pack_kernel(const float* __restrict__ cond, const float* __restrict__ x, T* __restrict__ out,
+                                 TileAxis ay, TileAxis ax, int64_t tile0, int64_t n_tiles, int bc) {
+  const int64_t i = blockIdx.x * int64_t(blockDim.x) + threadIdx.x;
+  const int64_t tpx = int64_t(ay.te) * ax.te;
+  if (i >= bc * tpx) return;
+  const int64_t j = i / tpx;
+  const int p = int(i - j * tpx);
+  const int64_t g = min(tile0 + j, n_tiles - 1);
+  const int64_t per_canvas = int64_t(ay.n) * ax.n;
+  const int64_t b = g / per_canvas;
+  const int r = int(g - b * per_canvas);
+  const int py = p / ax.te, px = p - py * ax.te;
+  const int y = tile_start(ay, r / ax.n) + py, xx = tile_start(ax, r % ax.n) + px;
+  const int64_t plane = int64_t(ay.L) * ax.L;
+  const int64_t o = b * 3 * plane + int64_t(y) * ax.L + xx;
+  pack_pixel<T>(out + i * 16, x + o, cond + o, plane);
+}
+
+// One step on every canvas: eps of each pixel = the normalised-weight blend of the eps of the tiles covering it (global
+// tile order, fp32, round-to-nearest, the sum starting from the first term so that a pixel covered once gets its tile's
+// eps exactly), then x_{t-1} = post1(x_t, eps, z) in place.  z: block z_block of args->noise, else the generator's
+// stream `stream` at (image0 + canvas, pixel index y*W + x); add_noise = 0 (t == 0): z = 0.  No atomics: each thread
+// owns its pixel.  grid (ceil(H W / 256), B); eps_store: [tile][3][te_y][te_x].
+__global__ void tile_blend_posterior_kernel(float* __restrict__ x, const float* __restrict__ eps_store, TileAxis ay,
+                                            TileAxis ax, PostCoef k, const SampleArgs* __restrict__ args,
+                                            int64_t z_block, uint32_t stream, int add_noise) {
+  const uint32_t HW = uint32_t(ay.L) * uint32_t(ax.L);
+  const uint32_t p = blockIdx.x * blockDim.x + threadIdx.x;
+  if (p >= HW) return;
+  const int b = blockIdx.y;
+  const int y = int(p / uint32_t(ax.L)), xx = int(p - uint32_t(y) * uint32_t(ax.L));
+  const TileCover cy = tile_cover(ay, y), cx = tile_cover(ax, xx);
+  const int ny = cy.count(), nx = cx.count();
+  float wsum = 0.f;
+  for (int a = 0; a < ny; ++a) {
+    const int ry = tile_ramp(ay, y - tile_start(ay, cy.at(a)));
+    for (int c = 0; c < nx; ++c) {
+      const float w = float(ry * tile_ramp(ax, xx - tile_start(ax, cx.at(c))));
+      wsum = (a | c) ? __fadd_rn(wsum, w) : w;
+    }
+  }
+  const int64_t tpx = int64_t(ay.te) * ax.te;
+  float e[3] = {0.f, 0.f, 0.f};
+  for (int a = 0; a < ny; ++a) {
+    const int ty = cy.at(a), oy = y - tile_start(ay, ty);
+    const int ry = tile_ramp(ay, oy);
+    for (int c = 0; c < nx; ++c) {
+      const int tx = cx.at(c), ox = xx - tile_start(ax, tx);
+      const float nk = __fdiv_rn(float(ry * tile_ramp(ax, ox)), wsum);
+      const int64_t g = (int64_t(b) * ay.n + ty) * ax.n + tx;
+      const float* ep = eps_store + g * 3 * tpx + int64_t(oy) * ax.te + ox;
+#pragma unroll
+      for (int ch = 0; ch < 3; ++ch) {
+        const float term = __fmul_rn(nk, ep[ch * tpx]);
+        e[ch] = (a | c) ? __fadd_rn(e[ch], term) : term;
+      }
+    }
+  }
+  const size_t o = size_t(b) * 3 * HW + p;
+  float zv[3] = {0.f, 0.f, 0.f};
+  if (add_noise) {
+    if (args->noise != nullptr) {
+      const float* nz = args->noise + size_t(z_block) * gridDim.y * 3 * HW;
+#pragma unroll
+      for (int ch = 0; ch < 3; ++ch) zv[ch] = nz[o + size_t(ch) * HW];
+    } else {
+      const float4 r = philox_normal4(args->seed, stream, args->image0 + b, p);
+      zv[0] = r.x;
+      zv[1] = r.y;
+      zv[2] = r.z;
+    }
+  }
+#pragma unroll
+  for (int ch = 0; ch < 3; ++ch) x[o + size_t(ch) * HW] = post1(x[o + size_t(ch) * HW], e[ch], zv[ch], k);
+}
+
+}  // namespace fdsr

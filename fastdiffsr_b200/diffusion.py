@@ -173,15 +173,21 @@ class GaussianDiffusion(nn.Module):
         return eng.posterior_step(x, eps, z, int(t))
 
     @torch.no_grad()
-    def p_sample_loop(self, x_in, continous=False, noise=None, seed=None, image_offset=0):
+    def p_sample_loop(self, x_in, continous=False, noise=None, seed=None, image_offset=0, *, tile=None, tile_overlap=32,
+                      tile_batch=16):
+        """`tile` (int or (th, tw), multiples of 8): sample canvases of any size (H, W >= 8) as overlapping tiles blended
+        at every step (Engine.sample_tiled; `tile_overlap` pixels, `tile_batch` tiles per UNet call).  None: one piece."""
         if not self.conditional:
             raise NotImplementedError("unconditional sampling is not on the SR path (unused by every config)")
+        if tile is not None and self.sr3:
+            raise NotImplementedError("tiled sampling is implemented for the FastDiffSR model only, not the SR3 baseline")
+        tiling = None if tile is None else (tile, tile_overlap, tile_batch)
         if seed is None:   # unseeded like the reference (SURVEY F7); ranks seeded alike must still draw different noise
             seed = int(torch.randint(0, 2 ** 62, (1,)).item())
             if torch.distributed.is_available() and torch.distributed.is_initialized():
                 seed = (seed + 0x9E3779B97F4A7C15 * torch.distributed.get_rank()) % (2 ** 63)
         try:
-            return self._sample_checked(x_in, continous, noise, seed, image_offset)
+            return self._sample_checked(x_in, continous, noise, seed, image_offset, tiling)
         except FdsrOverflowError:
             if not self.auto_dtype:
                 raise
@@ -190,22 +196,30 @@ class GaussianDiffusion(nn.Module):
             self.compute_dtype = "bf16"
             self._engine.close()
             self._engine = None
-            return self._sample_checked(x_in, continous, noise, seed, image_offset)
+            return self._sample_checked(x_in, continous, noise, seed, image_offset, tiling)
 
-    def _sample_checked(self, x_in, continous, noise, seed, image_offset):
+    def _sample_checked(self, x_in, continous, noise, seed, image_offset, tiling=None):
         eng = self.engine()
+        if tiling is None:
+            run = partial(eng.sample, x_in, noise=noise, seed=seed, image_offset=image_offset)
+        else:
+            run = partial(eng.sample_tiled, x_in, tiling[0], overlap=tiling[1], tile_batch=tiling[2], noise=noise,
+                          seed=seed, image_offset=image_offset)
         if not continous:
-            sr = eng.sample(x_in, noise=noise, seed=seed, image_offset=image_offset)
+            sr = run()
             eng.check_overflow()
             return sr[0] if (self.sr3 and sr.shape[0] == 1) else sr  # SR3: ret_img[-1] drops the batch axis
-        sr, tr = eng.sample(x_in, noise=noise, seed=seed, trace=True, image_offset=image_offset)
+        sr, tr = run(trace=True)
         eng.check_overflow()
         return tr.reshape(-1, *tr.shape[2:])  # B=1: (1+frames,3,H,W) exactly as the reference
 
     @torch.no_grad()
-    def super_resolution(self, x_in, continous=False, noise=None, seed=None, image_offset=0):
-        """`image_offset`: global index of x_in[0] in a job sharded over batches / ranks (see Engine.sample)."""
-        return self.p_sample_loop(x_in, continous, noise=noise, seed=seed, image_offset=image_offset)
+    def super_resolution(self, x_in, continous=False, noise=None, seed=None, image_offset=0, *, tile=None,
+                         tile_overlap=32, tile_batch=16):
+        """`image_offset`: global index of x_in[0] in a job sharded over batches / ranks (see Engine.sample).
+        `tile`, `tile_overlap`, `tile_batch`: tiled sampling of large canvases (see p_sample_loop)."""
+        return self.p_sample_loop(x_in, continous, noise=noise, seed=seed, image_offset=image_offset, tile=tile,
+                                  tile_overlap=tile_overlap, tile_batch=tile_batch)
 
     @torch.no_grad()
     def sample(self, batch_size=1, continous=False):

@@ -159,6 +159,27 @@ class Engine:
                                              self._stream()), "fdsr_sample")
         return (out, tr) if trace else out
 
+    def sample_tiled(self, cond, tile, overlap: int = 32, tile_batch: int = 16, noise=None, seed: int = 0,
+                     trace: bool = False, image_offset: int = 0):
+        """T-step sampling of (B,3,H,W) canvases of any size (H, W >= 8) as overlapping tiles blended at every step
+        (fdsr_sample_tiled).  `tile`: int or (th, tw), multiples of 8; `tile_batch`: tiles per UNet call (the activation
+        workspace scales with it, not with the canvas).  Noise, seed, image_offset and the trace are as in `sample`."""
+        th, tw = (tile, tile) if isinstance(tile, int) else (int(tile[0]), int(tile[1]))
+        self._check(self.lib.fdsr_set_image_offset(self._h, int(image_offset)), "fdsr_set_image_offset")
+        cond = self._img(cond, "cond")
+        B, _, H, W = cond.shape
+        if noise is not None:
+            if tuple(noise.shape) != (self.T, B, 3, H, W) or noise.dtype != torch.float32 or noise.device != self.device:
+                raise FdsrError(f"noise must be ({self.T},{B},3,{H},{W}) fp32 on {self.device}")
+            noise = noise.contiguous()
+        out = torch.empty_like(cond)
+        tr = torch.empty((B, self.trace_frames(), 3, H, W), device=self.device, dtype=torch.float32) if trace else None
+        with torch.cuda.device(self.device):
+            self._check(self.lib.fdsr_sample_tiled(self._h, _ptr(cond), _ptr(noise), seed, _ptr(out), _ptr(tr), B, H, W,
+                                                   th, tw, int(overlap), int(tile_batch), self._stream()),
+                        "fdsr_sample_tiled")
+        return (out, tr) if trace else out
+
     def bicubic_u8(self, lr_u8, H: int, W: int, want_u8=True, want_cond=True):
         """lr_u8: (B,h,w,3) uint8 on device -> (u8 (B,H,W,3) | None, cond (B,3,H,W) fp32 | None)."""
         if lr_u8.dtype != torch.uint8 or lr_u8.dim() != 4 or lr_u8.shape[3] != 3 or lr_u8.device != self.device:

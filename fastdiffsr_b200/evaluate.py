@@ -53,8 +53,14 @@ def _save_u8(img_chw, path):
 
 @torch.no_grad()
 def evaluate(netG, dataset, batch_size=16, scale=4, result_path=None, save_ext="tif", seed=0, current_step=0,
-             logger=None, max_images=None):
-    """Returns {'n', 'bic_mse', 'bic_psnr', 'bic_ssim', 'bic_ergas', 'sr_mse', ..., 'seconds', 'images_per_s'}."""
+             logger=None, max_images=None, tile=None, tile_overlap=32, tile_batch=16):
+    """Returns {'n', 'bic_mse', 'bic_psnr', 'bic_ssim', 'bic_ergas', 'sr_mse', ..., 'seconds', 'images_per_s'}.
+    `tile`: sample every image as one canvas of overlapping tiles (GaussianDiffusion.super_resolution(tile=...)), one
+    image per call (scenes may differ in size; the tiles of one canvas fill the GPU); the HR size is then `scale` x the
+    LR size, whatever that size is."""
+    if tile is not None:
+        batch_size = 1
+    tiling = {} if tile is None else dict(tile=tile, tile_overlap=tile_overlap, tile_batch=tile_batch)
     eng = netG.engine()
     dev = eng.device
     world = dist.get_world_size() if dist.is_initialized() else 1
@@ -70,13 +76,18 @@ def evaluate(netG, dataset, batch_size=16, scale=4, result_path=None, save_ext="
     for bi, batch in enumerate(loader):
         hr = u8_to_tensor(batch["HR"].to(dev, non_blocking=True))
         H, W = hr.shape[2], hr.shape[3]
+        if tile is not None and "LR" in batch:
+            H, W = scale * batch["LR"].shape[1], scale * batch["LR"].shape[2]
+            if (hr.shape[2], hr.shape[3]) != (H, W):
+                raise ValueError(f"image {batch['Index'][0]}: HR is {hr.shape[2]}x{hr.shape[3]}, not {scale} x the LR "
+                                 f"size ({H}x{W})")
         if "SR" in batch:                                          # the reference's precomputed bicubic image
             cond = u8_to_tensor(batch["SR"].to(dev, non_blocking=True)).contiguous()
         else:
             _, cond = eng.bicubic_u8(batch["LR"].to(dev, non_blocking=True), H, W, want_u8=False)
         # one seed for the whole job; the noise of an image depends on its global dataset index only, so the result
         # does not depend on the batch size or the number of ranks
-        sr = netG.super_resolution(cond, False, seed=seed, image_offset=start + bi * loader.bs)
+        sr = netG.super_resolution(cond, False, seed=seed, image_offset=start + bi * loader.bs, **tiling)
         if sr.dim() == 3:   # the SR3 baseline returns ret_img[-1] without the batch axis for a single image
             sr = sr[None]
         m_bic = eng.metrics_u8(cond, hr, scale)
@@ -142,6 +153,10 @@ def main(argv=None, default_config="config/sr_fastdiffsr_test_64_256.json", prog
     ap.add_argument('--no-save', action='store_true', help='do not write SR images')
     ap.add_argument('--max-images', type=int, default=None)
     ap.add_argument('--dtype', default=os.environ.get("FDSR_DTYPE", "auto"), choices=["auto", "fp16", "bf16", "fp32"])
+    ap.add_argument('--tile', type=int, default=None,
+                    help='sample each image as overlapping tiles of this size (multiple of 8): scenes of any size, one per call')
+    ap.add_argument('--tile-overlap', type=int, default=32, help='overlap of neighbouring tiles in pixels (with --tile)')
+    ap.add_argument('--tile-batch', type=int, default=16, help='tiles per UNet call (with --tile)')
     args = ap.parse_args(argv)
     if args.phase == 'train':
         raise NotImplementedError("training is outside the B200 sampling path: train with the reference and point "
@@ -177,7 +192,8 @@ def main(argv=None, default_config="config/sr_fastdiffsr_test_64_256.json", prog
     scale = int(val_opt['r_resolution']) // int(val_opt['l_resolution'])
     result_path = None if args.no_save else (paths.get('results') if isinstance(paths, dict) and paths.get('results') else 'results')
     res = evaluate(netG, val_set, batch_size=args.batch, scale=scale, result_path=result_path,
-                   save_ext="png" if prog == "infer.py" else "tif", logger=logger, max_images=args.max_images)
+                   save_ext="png" if prog == "infer.py" else "tif", logger=logger, max_images=args.max_images,
+                   tile=args.tile, tile_overlap=args.tile_overlap, tile_batch=args.tile_batch)
     if dist.is_initialized():
         dist.destroy_process_group()
     return res

@@ -126,6 +126,34 @@ int fdsr_sample(fdsr_ctx* ctx, const float* cond_dev, const float* noise_dev, ui
                 void* stream);
 int32_t fdsr_trace_frames(const fdsr_ctx* ctx); /* 1 + n_frames for the current schedule */
 
+/* Tiled sampling of B canvases of (3,H,W), any H, W >= 8 with H*W < 2^32 (FastDiffSR model only): overlapping tiles
+ * of one shared chain.  Every step, each tile's eps (the network on the tile's window [cond | x_t]; every tile is its
+ * own image for GroupNorm) is blended into one canvas-wide eps, and one posterior update moves the canvas-wide x_t.
+ *   Grid, per axis of length L with tile size t (tile_h / tile_w: multiples of 8, >= 8) and overlap o (>= 0):
+ *     t_e = min(t, 8*floor(L/8));  o_e = min(o, t_e - 8);  s = t_e - o_e;
+ *     starts = i*s for every i >= 0 with i*s < L - t_e, then L - t_e (the last tile is flush with the far edge).
+ *   Global tile order: canvas, then row start, then column start (all ascending).
+ *   Weights: tile pixel (i, j) weighs r_y(i) * r_x(j), r(i) = min(i+1, t_e-i, o_e+1) (an integer, exact in fp32 for
+ *     o_e < 4096).  Per canvas pixel, over the covering tiles in global order, in fp32 with round-to-nearest:
+ *     n_k = w_k / sum(w);  eps = n_1 eps_1 + n_2 eps_2 + ... (the sum starts from the first term, so a pixel covered
+ *     by one tile gets that tile's eps exactly);  x_{t-1} = the posterior update of fdsr_posterior_step.
+ *   Noise is drawn per canvas pixel: built-in = the generator of fdsr_sample at (seed, image offset + b, y*W + x,
+ *     step); injected = noise_dev (T,B,3,H,W) in fdsr_sample's draw order.  Canvas b is image fdsr_set_image_offset + b.
+ *   cond_dev, sr_out_dev and trace_out_dev are as in fdsr_sample, with the canvas shape.
+ *   Evaluation: the n_tiles = B * tiles_y * tiles_x tiles go through the UNet in n_chunks = ceil(n_tiles / tile_batch)
+ *     calls of Bc = ceil(n_tiles / n_chunks) tiles each (the last chunk is padded with repeats of its last tile), so the
+ *     activation workspace is fdsr_reserve(Bc, t_e_y, t_e_x), independent of the canvas; the canvas x_t and the
+ *     per-tile eps store (n_chunks * Bc * 3 * t_e_y * t_e_x floats) live in a separate grow-only context allocation.
+ *   A canvas that is exactly one tile gives fdsr_sample's bits; with o = 0 on a canvas the tiles partition, the result
+ *   equals fdsr_sample of the crops (with the noise cropped alike); tile_batch does not change the result.
+ *   Plain stream launches (no graph capture); the graphs cached by fdsr_sample are neither used nor evicted (a chunk
+ *   shape that grows the workspace drops them, like any larger fdsr_sample shape).  fp16 mode: check
+ *   fdsr_check_overflow as after fdsr_sample.  FDSR_E_INVALID: SR3 model, H or W < 8, H*W >= 2^32, bad tile sizes,
+ *   overlap < 0, tile_batch < 1, B outside 1..65535, null cond / sr_out. */
+int fdsr_sample_tiled(fdsr_ctx* ctx, const float* cond_dev, const float* noise_dev, uint64_t seed,
+                      float* sr_out_dev, float* trace_out_dev, int32_t B, int32_t H, int32_t W,
+                      int32_t tile_h, int32_t tile_w, int32_t overlap, int32_t tile_batch, void* stream);
+
 /* fp16 mode only (always FDSR_OK otherwise): synchronises `stream`, then returns FDSR_E_OVERFLOW if any activation
  * stored since the last check had left the fp16 range (it was stored saturated, so nothing downstream is inf / NaN,
  * but the image is not the network's output), and clears the flag.  fdsr_super_resolve_u8 performs this check itself;
