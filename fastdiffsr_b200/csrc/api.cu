@@ -122,11 +122,17 @@ struct fdsr_ctx {
   std::vector<F32Layer> f_layers;   // fp32 parity mode: the same plan for conv_f32_kernel
   std::vector<F32GnArgs> f_gn;
   std::vector<AttnParams> a_params;  // per HAttn of kind 1 (16-bit modes)
-  bool split_all = false;            // FDSR_SPLIT_ALL=1: every 256-wide layer runs as two 128-column halves (experiment)
-  bool s2d_tma = true;               // FDSR_S2D_TMA=0: stride-2 convs gather their parity planes with the producer warps
-  bool resid_mma = true;             // FDSR_RESID_MMA=0: identity residuals are always added by the epilogue
-  bool up_phases = true;             // FDSR_UP_PHASES=0: nearest-upsample convs gather a 2x patch and run all nine taps
-  bool attn_ref = false;             // FDSR_ATTN_REF=1: CUDA-core attention core in the 16-bit modes too
+  // Test hooks, read by fdsr_create: each forces a form that the automatic choice also picks for some layer or
+  // configuration, so that the tests can compare the two forms (INTEGRATION.md §2)
+  bool pair = true;        // FDSR_PAIR=0: never launch CTA pairs (cta_group::2); every layer runs the single-CTA kernel
+  bool half_tiles = true;  // FDSR_HALF_TILES=0: 32 x 8 tiles everywhere (the <= 64^2 wide layers then use split-N / single accumulators)
+  bool split_n = true;     // FDSR_SPLIT_N=0: never split a layer's output channels over two CTAs
+  bool epi2 = true;        // FDSR_EPI2=0: producer-free layers keep one epilogue team (warps 4..11)
+  bool tail_help = true;   // FDSR_TAIL_HELP=0: the last tile of a CTA is drained by warps 4..11 alone
+  bool resid_mma = true;   // FDSR_RESID_MMA=0: identity residuals are always added by the epilogue
+  bool up_phases = true;   // FDSR_UP_PHASES=0: nearest-upsample convs gather a 2x patch and run all nine taps
+  bool fused_tail = true;  // FDSR_FUSED_TAIL=0: the sampler runs pack_input / final conv -> eps / posterior as separate kernels
+  bool attn_ref = false;   // FDSR_ATTN_REF=1: CUDA-core attention core in the 16-bit modes too
   float* d_weights32 = nullptr;     // fp32 parity mode weights: per conv, per chunk [tap][ci][N]
   std::vector<size_t> w32_off;      // per conv (floats)
   size_t off_gntab = 0;             // [B][kMaxGnC] float2 scratch of the fp32 mode
@@ -159,22 +165,8 @@ struct fdsr_ctx {
   cudaStream_t copy_stream = nullptr;
   // graph cache
   bool use_graph = true;
-  bool precise = false;  // FDSR_PRECISE_SWISH=1: fp32 Swish in the producers
-  bool tma_store = true; // FDSR_TMA_STORE=0: per-lane 16-byte stores in the epilogue
-  bool two_rings = true; // FDSR_TWO_RINGS=0: one patch ring of three stages for every N = 64 layer
-  bool tma_in = true;    // FDSR_TMA_IN=0: producer warps gather every input patch (no TMA loads of the A operand)
-  bool pdl = true;       // FDSR_PDL=0: plain stream order between conv launches (no programmatic dependent launch)
-  bool split_n = true;   // FDSR_SPLIT_N=0: never split a layer's output channels over two CTAs
-  bool epi2 = true;        // FDSR_EPI2=0: producer-free layers keep one epilogue team (warps 4..11)
-  bool tail_help = true;   // FDSR_TAIL_HELP=0: the last tile of a CTA is drained by warps 4..11 alone
-  bool patch_first = true; // FDSR_PATCH_FIRST=0: weight stages are requested before griddepcontrol.wait, the first patch after
-  bool defer_csync = true; // FDSR_DEFER_CSYNC=0: CTA pairs run a full cluster barrier in the prologue
-  bool half_tiles = true;  // FDSR_HALF_TILES=0: 32 x 8 tiles everywhere (the <= 64^2 wide layers then use split-N / single accumulators)
-  bool stem_tma = true;  // FDSR_STEM_TMA=0: the 16-channel stem input is gathered by the producer warps
-  bool fused_tail = true;  // FDSR_FUSED_TAIL=0: the sampler runs pack_input / final conv -> eps / posterior as separate kernels
   PostStep* d_post = nullptr;      // [T] per-step posterior arguments of the fused final-conv epilogue
   ConvLayer final_fused{};         // the final conv's descriptor in kOutPosterior mode (h_layers holds the eps form)
-  bool pair = true;      // FDSR_PAIR=0: never launch CTA pairs (cta_group::2); every layer runs the single-CTA kernel
   // Captured sampling loops, keyed on what the captured launches depend on: the shape and whether noise is injected /
   // a trace is written.  Seed, image offset and the noise / trace POINTERS are read from device memory (SampleArgs),
   // so a fresh noise tensor, a new seed or a ragged last batch followed by a full one never forces a re-capture.
@@ -213,6 +205,12 @@ int fail(fdsr_ctx* c, int code, const char* fmt, ...) {
   if (c) c->err = buf;
   else g_global_error = buf;
   return code;
+}
+
+// Test hooks (fdsr_ctx): "0" / "1" in the environment turn one off / on; unset or any other value keeps the default
+bool env_hook(const char* name, bool dflt) {
+  const char* e = getenv(name);
+  return e && (e[0] == '0' || e[0] == '1') ? e[0] == '1' : dflt;
 }
 
 #define CUDA_TRY(c, expr)                                                                    \
@@ -487,7 +485,7 @@ int build_plan(fdsr_ctx* c) {
       // fall on the same source pixel are added up front (pack_weights), so each output parity is a 2x2 conv on
       // the low-resolution tensor -- 4 instead of 9 MACs per weight, TMA-fed like every other stride-1 layer.
       // An exact identity up to the rounding of the summed weights; the fp32 parity mode keeps the nine-tap form.
-      k.phases = (c->up_phases && c->tma_in && g.dtype != FDSR_DTYPE_FP32 && pre >= 128) ? 4 : 1;
+      k.phases = (c->up_phases && g.dtype != FDSR_DTYPE_FP32 && pre >= 128) ? 4 : 1;
       k.mode = k.phases == 4 ? kModeNormal : kModeUp2x;
       for (int c0 = 0; c0 < pre; c0 += 64) {
         if (k.phases == 4)
@@ -1091,6 +1089,7 @@ int launch_conv_f32(fdsr_ctx* c, int li, int t, cudaStream_t st) {
 int upload_layers(fdsr_ctx* c) {
   if (c->cfg.dtype == FDSR_DTYPE_FP32) return upload_layers_f32(c);
   const int B = c->B, H = c->H, W = c->W;
+  const bool bf = c->cfg.dtype == FDSR_DTYPE_BF16;
   if (!c->d_prof) {
     CUDA_TRY(c, cudaMalloc(&c->d_prof, size_t(c->num_sms) * kProfRoles * 64));
     CUDA_TRY(c, cudaMemset(c->d_prof, 0, size_t(c->num_sms) * kProfRoles * 64));
@@ -1112,18 +1111,16 @@ int upload_layers(fdsr_ctx* c) {
     // each CTA loads and normalises, and N = 256 gets a second TMEM accumulator stage.  The weight bytes per pixel double,
     // which is why layers with enough full tiles keep them (64^2 at B = 16: measured 1.3 % slower per step as half tiles).
     // Results are bit-identical for either shape (per-warp statistics are added as integers), so the choice may follow B.
-    const bool tma_normal = c->tma_in && k.mode == kModeNormal && k.ncg == 8;
     const int full_tiles = B * l.tiles_x * ((l.H + kTileH - 1) / kTileH);
-    const bool half = c->half_tiles && c->pair && tma_normal && k.phases == 1 && k.out_mode == kOutAct && k.N >= 128 &&
-                      l.tiles_x % 2 == 0 && l.H % 16 == 0 && full_tiles <= c->num_sms;
+    const bool half = c->half_tiles && c->pair && k.mode == kModeNormal && k.ncg == 8 && k.phases == 1 &&
+                      k.out_mode == kOutAct && k.N >= 128 && l.tiles_x % 2 == 0 && l.H % 16 == 0 && full_tiles <= c->num_sms;
     l.tile_h = half ? 16 : kTileH;
     l.tiles_y = (l.H + l.tile_h - 1) / l.tile_h;
     l.ntiles = B * k.phases * l.tiles_x * l.tiles_y;
     // Split-N: a low-resolution layer with fewer 256-pixel tiles than half the SMs is computed as two
     // 128-column halves by twice as many CTAs.  Only 256 -> 2 x 128: both widths use the same
     // per-tile statistics path, so results stay bitwise independent of the batch size.
-    l.nsplit = (!half && c->split_n && k.out_mode == kOutAct && k.N == 256 &&
-                (2 * l.ntiles <= c->num_sms || c->split_all)) ? 2 : 1;
+    l.nsplit = (!half && c->split_n && k.out_mode == kOutAct && k.N == 256 && 2 * l.ntiles <= c->num_sms) ? 2 : 1;
     l.n_full = k.N;
     l.N = k.N / l.nsplit;
     l.ncg = k.ncg;
@@ -1136,18 +1133,16 @@ int upload_layers(fdsr_ctx* c) {
       l.src[s].H = H >> t.level;
       l.src[s].W = W >> t.level;
     }
-    const bool s2d_tma = k.mode == kModeS2D && c->s2d_tma;
-    l.a_tma = (c->tma_in && (k.mode == kModeNormal || s2d_tma) && k.ncg == 8) ? 1 : 0;
-    if (c->tma_in && c->stem_tma && k.ncg == 2 && k.mode == kModeNormal && l.src[0].C == 16 &&
-        make_in_map(&l.in_map[0], l.src[0].ptr, B, l.src[0].H, l.src[0].W, 16, c->cfg.dtype == FDSR_DTYPE_BF16, 3))
-      l.a_tma = 2;  // the stem: two 8-channel TMA plane loads per tile, no producer work
+    // Input patches arrive by TMA, except in the nine-tap upsample convs, whose producer warps gather the 2x patch.
+    // The stem's 16-channel input arrives as two 8-channel plane loads (no producer work).
+    l.a_tma = k.mode == kModeUp2x ? 0 : (k.ncg == 2 ? 2 : 1);
+    bool maps_ok = l.a_tma != 2 || make_in_map(&l.in_map[0], l.src[0].ptr, B, l.src[0].H, l.src[0].W, l.src[0].C, bf, 3);
     for (int s = 0; s < k.nsrc && l.a_tma == 1; ++s)
-      if (!make_in_map(&l.in_map[s], l.src[s].ptr, B, l.src[s].H, l.src[s].W, l.src[s].C,
-                       c->cfg.dtype == FDSR_DTYPE_BF16, 0, l.tile_h) ||
-          !make_in_map(&l.in_map_c[s], l.src[s].ptr, B, l.src[s].H, l.src[s].W, l.src[s].C,
-                       c->cfg.dtype == FDSR_DTYPE_BF16, s2d_tma ? 2 : 1, l.tile_h))
-        l.a_tma = 0;
-    if (half && l.a_tma != 1) return fail(c, FDSR_E_CUDA, "layer %s: tensor maps of the half-tile form failed", k.name.c_str());
+      maps_ok = maps_ok &&
+                make_in_map(&l.in_map[s], l.src[s].ptr, B, l.src[s].H, l.src[s].W, l.src[s].C, bf, 0, l.tile_h) &&
+                make_in_map(&l.in_map_c[s], l.src[s].ptr, B, l.src[s].H, l.src[s].W, l.src[s].C, bf,
+                            k.mode == kModeS2D ? 2 : 1, l.tile_h);
+    if (!maps_ok) return fail(c, FDSR_E_CUDA, "layer %s: tensor maps of the input patches failed", k.name.c_str());
     l.nchunks = int(k.chunks.size());
     int any_center = 0;
     size_t woff = 0;
@@ -1158,27 +1153,24 @@ int upload_layers(fdsr_ctx* c) {
       d.c0 = ch.c0;
       d.gn = ch.gn;
       d.vc0 = ch.vc0;
-      d.pix_delta = ch.parity < 0 ? 0 : (ch.parity >> 1) * l.src[ch.slot].W + (ch.parity & 1);
       d.ntaps = int(ch.taps.size());
       d.w_off = int(woff);
       for (int tp = 0; tp < d.ntaps; ++tp) d.tap_pos[tp] = ch.taps[tp].pos;
       d.parity = ch.parity < 0 ? 0 : ch.parity;
-      d.center = (l.a_tma && k.mode == kModeNormal && ch.gn == 0 && d.ntaps == 1 && d.tap_pos[0] == kPatchW + 1) ? 1 : 0;
+      d.center = (k.mode == kModeNormal && ch.gn == 0 && d.ntaps == 1 && d.tap_pos[0] == kPatchW + 1) ? 1 : 0;
       any_center += d.center;
       woff += ch.taps.size() * size_t(k.ncg) * k.N * 16;
     }
     // patch rings (see ConvCfg): N = 64 layers with 1x1-residual chunks use 2 full + 2 centre-box stages
-    // (with three or more centre boxes per tile two 32 KB stages stall on the third: measured slower)
     // (with three centre boxes per tile two 32 KB stages stall on the third: measured slower in both rounds,
     //  ups.12.block2 189.6 -> 200.9 us as CTA pairs, profiles/r2/epilogue_costs.log)
-    l.nR = (c->two_rings && any_center >= 1 && any_center <= 2 && l.N == 64) ? 2 : 0;
+    l.nR = (any_center >= 1 && any_center <= 2 && l.N == 64) ? 2 : 0;
     l.nG = l.nR ? 2 : (l.N >= 256 ? 2 : 3);
     for (int j = 0; j < l.nchunks; ++j) l.chunk[j].ring = (l.nR && l.chunk[j].center) ? 1 : 0;
     l.gn_C = k.gn_C;
     l.gn_nsrc = k.gn_nsrc;
     l.gn_groups = c->cfg.norm_groups;
     l.gn_eps = 1e-5f;
-    l.precise = c->precise ? 1 : 0;
     if (k.gn_C) {
       l.gamma = c->d_params + k.gamma_off;
       l.beta = c->d_params + k.gamma_off + k.gn_C;
@@ -1194,15 +1186,13 @@ int upload_layers(fdsr_ctx* c) {
     if (k.out_mode == kOutAct) {
       const HTensor& t = c->tensors[k.out];
       l.out = c->d_ws + t.off;
-      const bool bf = c->cfg.dtype == FDSR_DTYPE_BF16;
-      if (k.phases == 4) {
-        bool ok = l.a_tma != 0;
+      bool ok = true;  // (the epilogue stores N >= 32 activations by TMA)
+      if (k.phases == 4)
         for (int ph = 0; ph < 4 && ok; ++ph)
           ok = make_out_map_phase(ph == 0 ? &l.out_map : &l.out_map_ph[ph - 1], l.out, B, l.H, l.W, k.N, ph, bf);
-        if (!ok) return fail(c, FDSR_E_CUDA, "layer %s: tensor maps of the phase-decomposed upsample conv failed", k.name.c_str());
-        l.use_tma_store = 1;
-      } else
-      l.use_tma_store = (c->tma_store && k.N >= 32 && make_out_map(&l.out_map, l.out, B, l.H, l.W, k.N, bf)) ? 1 : 0;
+      else if (k.N >= 32)
+        ok = make_out_map(&l.out_map, l.out, B, l.H, l.W, k.N, bf);
+      if (!ok) return fail(c, FDSR_E_CUDA, "layer %s: tensor maps of the output failed", k.name.c_str());
       l.out_stats = t.stats ? reinterpret_cast<unsigned long long*>(c->d_ws + t.stats_off) : nullptr;
       l.out_sq_scale = float(stat_sq_scale((long long)(H >> t.level) * (W >> t.level)));
       int su = 1;
@@ -1225,8 +1215,7 @@ int upload_layers(fdsr_ctx* c) {
     {  // second epilogue team (warps 12..19) for layers whose producer warps have nothing to do
       // (not the stride-2 convs: they stream four parity-plane chunks per tile and lose more from giving up the third
       //  patch stage than they gain — measured 49.6 -> 58.8 us for downs.3)
-      bool raw = l.a_tma != 0 && k.mode == kModeNormal && k.out_mode == kOutAct && l.use_tma_store && l.tile_h == kTileH &&
-                 l.nsplit == 1 && k.resid < 0;
+      bool raw = k.mode == kModeNormal && k.out_mode == kOutAct && l.tile_h == kTileH && l.nsplit == 1 && k.resid < 0;
       for (const HChunk& ch : k.chunks) raw = raw && ch.gn == 0;
       l.epi2 = (c->epi2 && raw) ? 1 : 0;
       if (l.epi2 && l.N <= 128) {  // their staging blocks live in the third patch stage
@@ -1236,14 +1225,8 @@ int upload_layers(fdsr_ctx* c) {
       }
     }
     l.tail2 = (c->tail_help && !l.epi2 && k.out_mode == kOutAct && l.N >= 64) ? 1 : 0;
-    l.patch_first = c->patch_first ? 1 : 0;
-    l.defer_csync = c->defer_csync ? 1 : 0;
     l.prof = c->d_prof;
     l.flags = reinterpret_cast<unsigned int*>(c->d_ws + kOffFlags);
-    {
-      const char* e = getenv("FDSR_DBG_SKIP");
-      l.dbg = e ? atoi(e) : 0;
-    }
   }
   static_assert(sizeof(ConvLayer) <= 4000, "ConvLayer must fit the kernel parameter space");
   // the sampler's form of the final conv: eps stays in registers, the epilogue performs the posterior update
@@ -1262,18 +1245,12 @@ int upload_layers(fdsr_ctx* c) {
 
 template <int N, typename T>
 cudaError_t set_conv_attr() {
-  cudaError_t e = cudaFuncSetAttribute(conv_gemm_kernel<N, T, false, false>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                       ConvCfg<N, false>::kSmemBytes);
-  if (e == cudaSuccess)
-    e = cudaFuncSetAttribute(conv_gemm_kernel<N, T, true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                             ConvCfg<N, false>::kSmemBytes);
+  cudaError_t e = cudaFuncSetAttribute(conv_gemm_kernel<N, T, false>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                       ConvCfg<N>::kSmemBytes);
   if constexpr (N >= 64) {
     if (e == cudaSuccess)
-      e = cudaFuncSetAttribute(conv_gemm_kernel<N, T, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                               ConvCfg<N, true>::kSmemBytes);
-    if (e == cudaSuccess)
-      e = cudaFuncSetAttribute(conv_gemm_kernel<N, T, true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                               ConvCfg<N, true>::kSmemBytes);
+      e = cudaFuncSetAttribute(conv_gemm_kernel<N, T, true>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                               ConvCfg<N>::kSmemBytes);
   }
   return e;
 }
@@ -1304,7 +1281,7 @@ int launch_conv_t(fdsr_ctx* c, int li, int ntiles, int t, cudaStream_t st, const
   cudaLaunchConfig_t cfg{};
   cfg.gridDim = dim3(grid);
   cfg.blockDim = dim3(kConvThreads);
-  cfg.dynamicSmemBytes = pair ? ConvCfg<N, true>::kSmemBytes : ConvCfg<N, false>::kSmemBytes;
+  cfg.dynamicSmemBytes = ConvCfg<N>::kSmemBytes;
   cfg.stream = st;
   cudaLaunchAttribute attr[2];
   attr[0].id = cudaLaunchAttributeClusterDimension;
@@ -1314,21 +1291,12 @@ int launch_conv_t(fdsr_ctx* c, int li, int ntiles, int t, cudaStream_t st, const
   attr[1].id = cudaLaunchAttributeProgrammaticStreamSerialization;
   attr[1].val.programmaticStreamSerializationAllowed = 1;
   cfg.attrs = attr;
-  cfg.numAttrs = c->pdl ? 2 : 1;
-  const bool fast = !c->precise;
+  cfg.numAttrs = 2;
+  void (*kernel)(ConvLayer, int) = conv_gemm_kernel<N, T, false>;
   if constexpr (N >= 64) {
-    if (pair) {
-      if (fast) CUDA_TRY(c, cudaLaunchKernelEx(&cfg, conv_gemm_kernel<N, T, true, true>, LY, t));
-      else CUDA_TRY(c, cudaLaunchKernelEx(&cfg, conv_gemm_kernel<N, T, false, true>, LY, t));
-      CUDA_TRY(c, cudaGetLastError());
-      ++c->launches;
-      return FDSR_OK;
-    }
+    if (pair) kernel = conv_gemm_kernel<N, T, true>;
   }
-  if (fast)
-    CUDA_TRY(c, cudaLaunchKernelEx(&cfg, conv_gemm_kernel<N, T, true, false>, LY, t));
-  else
-    CUDA_TRY(c, cudaLaunchKernelEx(&cfg, conv_gemm_kernel<N, T, false, false>, LY, t));
+  CUDA_TRY(c, cudaLaunchKernelEx(&cfg, kernel, LY, t));
   CUDA_TRY(c, cudaGetLastError());
   ++c->launches;
   return FDSR_OK;
@@ -1678,46 +1646,15 @@ int fdsr_create(const fdsr_config* cfg, fdsr_ctx** out) {
     return fail(nullptr, FDSR_E_CUDA, "libfdsr needs an sm_100 (B200) device");
   }
   c->num_sms = prop.multiProcessorCount;
-  {
-    const char* e = getenv("FDSR_PRECISE_SWISH");
-    c->precise = e && e[0] == '1';
-    const char* e2 = getenv("FDSR_TMA_STORE");
-    c->tma_store = !(e2 && e2[0] == '0');
-    const char* e3 = getenv("FDSR_PAIR");
-    c->pair = !(e3 && e3[0] == '0');
-    const char* e16 = getenv("FDSR_EPI2");
-    c->epi2 = !(e16 && e16[0] == '0');
-    const char* e17 = getenv("FDSR_TAIL_HELP");
-    c->tail_help = !(e17 && e17[0] == '0');
-    const char* e18 = getenv("FDSR_PATCH_FIRST");
-    c->patch_first = !(e18 && e18[0] == '0');
-    const char* e19 = getenv("FDSR_DEFER_CSYNC");
-    c->defer_csync = !(e19 && e19[0] == '0');
-    const char* e15 = getenv("FDSR_HALF_TILES");
-    c->half_tiles = !(e15 && e15[0] == '0');
-    const char* e13 = getenv("FDSR_STEM_TMA");
-    c->stem_tma = !(e13 && e13[0] == '0');
-    const char* e14 = getenv("FDSR_FUSED_TAIL");
-    c->fused_tail = !(e14 && e14[0] == '0');
-    const char* e4 = getenv("FDSR_SPLIT_N");
-    c->split_n = !(e4 && e4[0] == '0');
-    const char* e5 = getenv("FDSR_PDL");
-    c->pdl = !(e5 && e5[0] == '0');
-    const char* e6 = getenv("FDSR_TMA_IN");
-    c->tma_in = !(e6 && e6[0] == '0');
-    const char* e7 = getenv("FDSR_TWO_RINGS");
-    c->two_rings = !(e7 && e7[0] == '0');
-    const char* e12 = getenv("FDSR_SPLIT_ALL");
-    c->split_all = e12 && e12[0] == '1';
-    const char* e11 = getenv("FDSR_S2D_TMA");
-    c->s2d_tma = !(e11 && e11[0] == '0');
-    const char* e10 = getenv("FDSR_RESID_MMA");
-    c->resid_mma = !(e10 && e10[0] == '0');
-    const char* e9 = getenv("FDSR_UP_PHASES");
-    c->up_phases = !(e9 && e9[0] == '0');
-    const char* e8 = getenv("FDSR_ATTN_REF");
-    c->attn_ref = e8 && e8[0] == '1';
-  }
+  c->pair = env_hook("FDSR_PAIR", c->pair);
+  c->half_tiles = env_hook("FDSR_HALF_TILES", c->half_tiles);
+  c->split_n = env_hook("FDSR_SPLIT_N", c->split_n);
+  c->epi2 = env_hook("FDSR_EPI2", c->epi2);
+  c->tail_help = env_hook("FDSR_TAIL_HELP", c->tail_help);
+  c->resid_mma = env_hook("FDSR_RESID_MMA", c->resid_mma);
+  c->up_phases = env_hook("FDSR_UP_PHASES", c->up_phases);
+  c->fused_tail = env_hook("FDSR_FUSED_TAIL", c->fused_tail);
+  c->attn_ref = env_hook("FDSR_ATTN_REF", c->attn_ref);
   if (cfg->dtype != FDSR_DTYPE_FP16 && cfg->dtype != FDSR_DTYPE_BF16 && cfg->dtype != FDSR_DTYPE_FP32) {
     delete c;
     return fail(nullptr, FDSR_E_INVALID, "dtype must be FDSR_DTYPE_FP16, FDSR_DTYPE_BF16 or FDSR_DTYPE_FP32");

@@ -72,7 +72,6 @@ struct ConvChunk {
   int32_t c0;         // first channel inside the source tensor
   int32_t gn;         // 1: GroupNorm+Swish with scale/shift table entries [vc0, vc0+64); 2: GroupNorm only (no activation)
   int32_t vc0;        // channel offset on the virtual (concatenated) GroupNorm axis
-  int32_t pix_delta;  // extra source pixel offset (parity plane of the space-to-depth view)
   int32_t ntaps;
   int32_t ring;       // patch ring of this chunk: 0 = full stages, 1 = 32 KB centre-box stages (ConvLayer::nR > 0)
   int32_t center;     // 1: TMA-fed raw chunk whose only tap is the centre one: staged as a dense 32x8 box (no halo)
@@ -90,11 +89,11 @@ struct ConvSrc {
 
 struct ConvLayer {
   // TMA descriptor of the 16-bit NHWC output tensor, dims {C, W, H, B}, box {32 ch, 8, 4, 1},
-  // 64B swizzle: each epilogue warp stores its 32 px x 32 ch block with one bulk tensor copy
+  // 64B swizzle: each epilogue warp stores its 32 px x 32 ch block with one bulk tensor copy (kOutAct, N >= 32)
   alignas(64) CUtensorMap out_map;
   // TMA descriptors of the 16-bit NHWC source tensors, dims {C, W, H, B}, box {64 ch, 10, 34, 1},
   // 128B swizzle: one bulk tensor load stages a whole (32+2)x(8+2) x 64-channel input patch,
-  // out-of-image positions zero-filled (valid when a_tma = 1)
+  // out-of-image positions zero-filled (a_tma = 1; a_tma = 2: in_map[0] is the stem's 8-channel plane map)
   CUtensorMap in_map[kMaxSrc];
   CUtensorMap in_map_c[kMaxSrc];  // same tensors, box {64 ch, 8, 32, 1}: centre-only chunks (1x1 residual conv);
                                   // kModeS2D: box {64 ch, 20, 68, 1} traversed with element strides {1, 2, 2, 1}: one
@@ -109,8 +108,9 @@ struct ConvLayer {
   int32_t ncg;          // 16-byte channel groups per chunk (8, or 2 for the 16-channel stem input)
   int32_t mode;         // ConvMode
   int32_t nG, nR;       // patch stages in ring 0 (full) / ring 1 (centre boxes); nR = 0: single ring
-  int32_t a_tma;        // 1: input patches arrive by TMA (kModeNormal, 64-channel chunks); 0: gathered by the producer warps;
-                        // 2: the 16-channel stem input arrives as two 8-channel TMA plane loads (no-swizzle patch layout)
+  int32_t a_tma;        // 1: input patches arrive by TMA (kModeNormal and kModeS2D, 64-channel chunks); 2: the 16-channel
+                        // stem input arrives as two 8-channel TMA plane loads (no-swizzle patch layout); 0 (kModeUp2x in
+                        // the nine-tap form): gathered by the producer warps
   int32_t B, H, W;      // output size
   int32_t N;            // MMA N of one CTA (16 / 64 / 128 / 256)
   int32_t n_full;       // channel width of the output tensor and of the packed weight blobs (= N * nsplit)
@@ -122,7 +122,6 @@ struct ConvLayer {
   const float* gamma;   // [gn_C]
   const float* beta;    // [gn_C]
   float gn_eps;
-  int32_t precise;      // 1: fp32 EX2/RCP Swish (always for bf16); 0: packed-half tanh Swish (fp16)
   // epilogue
   const float* bias;    // [T or 1][N] fp32: conv bias (+ residual-conv bias) (+ FiLM vector of step t)
   int32_t bias_tstride; // floats between steps (0 when the bias does not depend on t)
@@ -131,7 +130,6 @@ struct ConvLayer {
   unsigned long long* out_stats;  // [B][N/2][2] fixed point, or null
   float out_sq_scale;   // fixed-point scale of the sums of squares of the OUTPUT tensor (power of two, see stat_sq_scale)
   double gn_inv_sum, gn_inv_sq;  // GroupNorm input: 1 / (scale * elements per group) for the sums / sums of squares
-  int32_t use_tma_store;  // 1: out_map is valid
   int32_t out_su;       // channel pairs per statistics entry (1, 2, 4, 8): coarsest unit every consumer can use
   int32_t out_mode;     // OutMode
   int32_t out_c;
@@ -144,8 +142,6 @@ struct ConvLayer {
                            //    stem) turn producer warps 12..19 into a second epilogue team (odd 32-column blocks)
   int32_t tail2;           // 1: producer warps 12..19 join the epilogue of the CTA's LAST tile as a second team (layers with
                            //    producer work; the last tile's epilogue is exposed — nothing is left to overlap it with)
-  int32_t patch_first;     // 1: the loader requests the CTA's first input patch before its first weight stages
-  int32_t defer_csync;     // 1 (pairs): the opening cluster barrier is split — arrive in the prologue, wait where needed
   int32_t tile_h;          // output rows per CTA tile: 32 (two 128-row MMA tiles) or 16 (one: "half tiles", see upload_layers)
   int32_t tiles_x, tiles_y, ntiles;
   int32_t group;           // tiles per assignment group (divides tiles_x * tiles_y)
@@ -155,7 +151,6 @@ struct ConvLayer {
   void* xin;               // 16-bit NHWC16 network input: channels 0-2 receive x_{t-1}
   const SampleArgs* args;
   unsigned int* flags;     // context status word: bit 0 = an fp16 activation store saturated (overflow)
-  int32_t dbg;             // experiments (tools/): bit0 skip epilogue work, bit1 skip producer work
   long long* prof;         // role cycle counters [grid][5 roles][8 slots] (FDSR_PROFILE builds only)
 };
 

@@ -11,9 +11,9 @@
 //   warps 4-11  epilogue (one warpgroup per 128-row MMA tile): tcgen05.ld -> bias/FiLM -> residual
 //               -> 16-bit TMA store -> GroupNorm pair statistics
 //   warps 2,3,12-19  producers: GroupNorm scale/shift + Swish applied in place to the TMA-delivered
-//               patch (pixel-major, 128 B per position); for the gathered layers (nearest-upsample,
-//               stride-2, 16-channel stem) coalesced 16B global loads, transform in registers, 16B
-//               stores into a no-swizzle [channel group][position][8 ch] patch.
+//               patch (pixel-major, 128 B per position); for the nine-tap nearest-upsample convs
+//               coalesced 16B global loads of the 2x-upsampled patch, 16B stores into a no-swizzle
+//               [channel group][position][8 ch] patch.
 // The patch is loaded and transformed ONCE per 64-channel chunk and then serves all nine 3x3
 // taps as shifted shared-memory descriptor views (start address + 128 B * (dy*10 + dx), SBO =
 // 1280 B; the MMA unit swizzles on absolute address bits, tools/probe_umma.cu), so the A operand is
@@ -58,7 +58,7 @@ __host__ __device__ inline double stat_sq_scale(long long hw) {
   return double(1LL << e);
 }
 
-template <int N, bool kPair = false>
+template <int N>
 struct ConvCfg {
   static constexpr int kAccStride = N < 32 ? 32 : N;        // TMEM columns per 128-row accumulator
   static constexpr int kAccCols = 2 * kAccStride;           // two MMA tiles per CTA tile
@@ -71,26 +71,17 @@ struct ConvCfg {
   static constexpr int kTmemCols =
       kTmemNeed <= 32 ? 32 : (kTmemNeed <= 64 ? 64 : (kTmemNeed <= 128 ? 128 : (kTmemNeed <= 256 ? 256 : 512)));
   // a B stage holds as many consecutive tap blobs of one chunk as fit (N=64: 4 taps, 128: 2, 256: 1)
-#ifndef FDSR_B128_BYTES
-#define FDSR_B128_BYTES 32768
-#define FDSR_B128_STAGES 2
-#endif
   // CTA pairs stage half-width blobs, so a stage of the same size holds twice the taps.  Cutting the same memory into
-  // twice as many stages of half the size (FDSR_PAIR_BSPLIT=2: more loads in flight) was measured 1.7 % SLOWER over the
-  // UNet (A/B on one box, profiles/r2/ab_bsplit.log): the MMA warp's weight waits are shared-memory bandwidth (the bulk
-  // copies' writes queue behind the tensor core's operand reads), not L2 latency, and more stages only add barrier work.
-#ifndef FDSR_PAIR_BSPLIT
-#define FDSR_PAIR_BSPLIT 1
-#endif
-  static constexpr int kBSplit = kPair ? FDSR_PAIR_BSPLIT : 1;
-  static constexpr int kBStageBytes =
-      (N < 32 ? 9 * N * 128 : (N == 64 ? 24576 : (N == 128 ? FDSR_B128_BYTES : 32768))) / kBSplit;
+  // twice as many stages of half the size (more loads in flight) was measured 1.7 % SLOWER over the UNet (A/B on one
+  // box, profiles/r2/ab_bsplit.log): the MMA warp's weight waits are shared-memory bandwidth (the bulk copies' writes
+  // queue behind the tensor core's operand reads), not L2 latency, and more stages only add barrier work.
+  static constexpr int kBStageBytes = N < 32 ? 9 * N * 128 : (N == 64 ? 24576 : 32768);
   // N <= 128 layers are bounded by the producer/epilogue roles, not by weight streaming: give the
   // input patch a third stage (deeper decoupling of producers and MMA) and the weights two.
   // (Measured: four patch stages with four one-tap weight stages for N = 64 removes the a_full waits
   // of the GroupNorm + 1x1-residual layers but starves the MMA warp of weights: 101 -> 132 us.)
   static constexpr int kAStages = N >= 256 ? 2 : 3;
-  static constexpr int kBStages = (N >= 256 ? 3 : (N == 128 ? FDSR_B128_STAGES : 2)) * kBSplit;
+  static constexpr int kBStages = N >= 256 ? 3 : 2;
   // N = 64 layers that mix a GroupNorm 3x3 chunk with 1x1-residual chunks split the patch memory into
   // two rings (ConvLayer::nG / nR): two full stages for the 3x3 chunks and two 32 KB stages for the dense
   // centre boxes.  In a single ring of three the 3x3 chunk of the next tile could only be requested two
@@ -153,8 +144,6 @@ struct Cvt<__nv_bfloat16> {
   __device__ static __forceinline__ uint32_t pack_store(float a, float b) { return pack(a, b); }  // fp32 exponent range
 };
 
-__device__ __forceinline__ float swish_f(float y) { return __fdividef(y, 1.0f + __expf(-y)); }
-
 // swish(x*2sc + 2sh) for a packed pair, with sc/sh pre-halved: h = x*sc + sh; h*tanh(h) + h
 __device__ __forceinline__ uint32_t swish_h2(uint32_t x, uint32_t sc, uint32_t sh) {
   uint32_t h, t, o;
@@ -174,14 +163,13 @@ template <typename T>
 using GnOperand = __half;
 
 // GroupNorm scale/shift + Swish on 8 packed 16-bit activations; the result is packed as GnOperand<T> (fp16).
-// kFast, fp16 storage: packed fp16 throughout (hsc/hsh hold scale/2, shift/2): swish(y) = h tanh(h) + h, h = y/2.
-// kFast, bf16 storage: the affine part in fp32 (sc/sh hold scale/2, shift/2; the input may be far outside the fp16
-//   range), then the same packed-half tanh form.
-// otherwise: fp32 EX2/RCP with sc/sh.
-template <typename T, bool kFast>
+// fp16 storage: packed fp16 throughout (hsc/hsh hold scale/2, shift/2): swish(y) = h tanh(h) + h, h = y/2.
+// bf16 storage: the affine part in fp32 (sc/sh hold scale/2, shift/2; the input may be far outside the fp16 range),
+//   then the same packed-half tanh form.
+template <typename T>
 __device__ __forceinline__ uint4 gn_swish_unit(uint4 o, const uint4& hsc, const uint4& hsh, const float (&sc)[8],
                                                const float (&sh)[8]) {
-  if constexpr (kFast && Cvt<T>::kFmt == 0) {
+  if constexpr (Cvt<T>::kFmt == 0) {
     o.x = swish_h2(o.x, hsc.x, hsh.x);
     o.y = swish_h2(o.y, hsc.y, hsh.y);
     o.z = swish_h2(o.z, hsc.z, hsh.z);
@@ -194,25 +182,21 @@ __device__ __forceinline__ uint4 gn_swish_unit(uint4 o, const uint4& hsc, const 
     for (int e = 0; e < 4; ++e) {
       const float2 f = Cvt<T>::unpack(w4[e]);
       const float ya = fmaf(f.x, sc[2 * e], sh[2 * e]), yb = fmaf(f.y, sc[2 * e + 1], sh[2 * e + 1]);
-      if constexpr (kFast) {
-        const uint32_t h = Cvt<__half>::pack(ya, yb);  // = y/2 (pre-halved table)
-        uint32_t t;
-        asm("tanh.approx.f16x2 %0, %1;" : "=r"(t) : "r"(h));
-        asm("fma.rn.f16x2 %0, %1, %2, %1;" : "=r"(r4[e]) : "r"(h), "r"(t));
-      } else {
-        r4[e] = Cvt<GnOperand<T>>::pack(swish_f(ya), swish_f(yb));
-      }
+      const uint32_t h = Cvt<__half>::pack(ya, yb);  // = y/2 (pre-halved table)
+      uint32_t t;
+      asm("tanh.approx.f16x2 %0, %1;" : "=r"(t) : "r"(h));
+      asm("fma.rn.f16x2 %0, %1, %2, %1;" : "=r"(r4[e]) : "r"(h), "r"(t));
     }
     return make_uint4(r4[0], r4[1], r4[2], r4[3]);
   }
 }
 
 // GroupNorm scale/shift only (the SelfAttention norm of the SR3 baseline has no activation,
-// ddpm_modules/unet.py:105,115): y = x*sc + sh; the packed-half table holds sc/2, sh/2, so y = h + h.
-template <typename T, bool kFast>
+// ddpm_modules/unet.py:105,115): y = x*sc + sh; the tables hold sc/2, sh/2, so y = h + h.
+template <typename T>
 __device__ __forceinline__ uint4 gn_affine_unit(uint4 o, const uint4& hsc, const uint4& hsh, const float (&sc)[8],
                                                 const float (&sh)[8]) {
-  if constexpr (kFast && Cvt<T>::kFmt == 0) {
+  if constexpr (Cvt<T>::kFmt == 0) {
     const uint32_t w4[4] = {o.x, o.y, o.z, o.w}, s4[4] = {hsc.x, hsc.y, hsc.z, hsc.w}, b4[4] = {hsh.x, hsh.y, hsh.z, hsh.w};
     uint32_t r4[4];
 #pragma unroll
@@ -225,11 +209,10 @@ __device__ __forceinline__ uint4 gn_affine_unit(uint4 o, const uint4& hsc, const
   }
   const uint32_t w4[4] = {o.x, o.y, o.z, o.w};
   uint32_t r4[4];
-  const float k = (kFast && Cvt<T>::kFmt != 0) ? 2.0f : 1.0f;  // (bf16 fast table: scale/2, shift/2)
 #pragma unroll
   for (int e = 0; e < 4; ++e) {
     const float2 f = Cvt<T>::unpack(w4[e]);
-    r4[e] = Cvt<GnOperand<T>>::pack(k * fmaf(f.x, sc[2 * e], sh[2 * e]), k * fmaf(f.y, sc[2 * e + 1], sh[2 * e + 1]));
+    r4[e] = Cvt<GnOperand<T>>::pack(2.0f * fmaf(f.x, sc[2 * e], sh[2 * e]), 2.0f * fmaf(f.y, sc[2 * e + 1], sh[2 * e + 1]));
   }
   return make_uint4(r4[0], r4[1], r4[2], r4[3]);
 }
@@ -338,7 +321,6 @@ constexpr int kProfRoles = 5;  // 8 slots each per CTA: MMA, epilogue, producers
 #define PROF_TS4(slot)
 #endif
 
-// kFast: GroupNorm-affine + Swish in packed fp16 (tanh form); otherwise fp32 EX2/RCP.
 // kPair: CTA-pair form.  The kernel runs as clusters of two CTAs (one per SM of a TPC) and every MMA is a
 //   tcgen05.mma.cta_group::2 of M = 256 rows: each CTA still owns a whole 32x8-pixel tile (its own input patch,
 //   producers, TMEM accumulators and epilogue) but stages only HALF of the weight columns — CTA r supplies columns
@@ -349,10 +331,10 @@ constexpr int kProfRoles = 5;  // 8 slots each per CTA: MMA, epilogue, producers
 //   phase and therefore the weights.  Only the leader's warp 0 issues MMAs; the peer's warp 0 walks the same sequence
 //   and forwards "my patch stage / weight half / accumulator is ready" to relay barriers in the leader's shared memory;
 //   completions are multicast to both CTAs by tcgen05.commit.cta_group::2.
-template <int N, typename T, bool kFast, bool kPair>
+template <int N, typename T, bool kPair>
 __global__ void __launch_bounds__(kConvThreads, 1)
 conv_gemm_kernel(const __grid_constant__ ConvLayer L, int t_step) {
-  using Cfg = ConvCfg<N, kPair>;
+  using Cfg = ConvCfg<N>;
   PROF_T0;
   constexpr int kRow = Cfg::kRow;
   constexpr int kAStages = Cfg::kAStages;  // gathered layers: one ring of kAStages full stages
@@ -392,7 +374,7 @@ conv_gemm_kernel(const __grid_constant__ ConvLayer L, int t_step) {
       prefetch_tensormap(&L.in_map[lane]);
       if (L.a_tma == 1) prefetch_tensormap(&L.in_map_c[lane]);
     }
-    if (lane == 8 && L.out_mode == kOutAct && L.use_tma_store != 0) prefetch_tensormap(&L.out_map);
+    if (lane == 8 && N >= 32 && L.out_mode == kOutAct) prefetch_tensormap(&L.out_map);
     if (lane >= 9 && lane < 12 && L.phases > 1) prefetch_tensormap(&L.out_map_ph[lane - 9]);
   }
   if (tid == 0) {
@@ -418,17 +400,13 @@ conv_gemm_kernel(const __grid_constant__ ConvLayer L, int t_step) {
   tc_fence_before();
   __syncthreads();
   // both CTAs' barriers and TMEM exist before any remote arrive / pair MMA.  Only the two MMA warps ever touch the other
-  // CTA (relay arrives, cta_group::2 MMAs and commits): with L.defer_csync every thread just ARRIVES here, the MMA warps
-  // wait before their loop and everyone else before the closing cluster barrier — the loader and the producers of a CTA
-  // start earlier (tools/timeline.py: entry -> prologue done 1.4 us as a pair, 0.6 us alone)
-  const bool defer_cs = kPair && L.defer_csync != 0;
-  if (kPair) {
-    if (defer_cs) cluster_arrive();
-    else cluster_sync_all();
-  }
+  // CTA (relay arrives, cta_group::2 MMAs and commits): every thread just ARRIVES here, the MMA warps wait before their
+  // loop and everyone else before the closing cluster barrier — the loader and the producers of a CTA start earlier
+  // (tools/timeline.py: entry -> prologue done 1.4 us as a pair, 0.6 us alone; profiles/r2/ab_defer_csync.log)
+  if (kPair) cluster_arrive();
   tc_fence_after();
   const uint32_t tmem = *tmem_slot;
-  if (kPair && warp == 0 && defer_cs) cluster_wait();
+  if (kPair && warp == 0) cluster_wait();
   if (kPair && tid == 0) {
     // the pair MMA writes the same TMEM address in both CTAs: the two allocations must agree (they do: one CTA per
     // SM, one allocation per CTA); a mismatch would corrupt results silently, so fail loudly instead
@@ -630,18 +608,13 @@ conv_gemm_kernel(const __grid_constant__ ConvLayer L, int t_step) {
     // GroupNorm chunks land on raw_full (the producer warps transform them in place and then arrive on
     // a_full); raw chunks complete a_full directly, so the MMA warp starts as soon as the bytes are there.
     const bool tma_in = L.a_tma != 0;
-    // Patches are the previous layer's output: no patch request before griddepcontrol.wait.  Weights are
-    // constants, so the first weight stages are requested before it and land while the previous launch drains.
-    bool dep_ok = !tma_in;
-    // ... unless the layer asks for its first patch FIRST (L.patch_first, the default): a CTA only becomes resident when
-    // the previous launch's CTA on this SM has exited, so the dependency resolves within a few microseconds anyway, and
-    // then 64 - 96 KB of weight stages queued ahead of the 43 KB patch on the SM's inbound link delay the longer chain
-    // (patch -> GroupNorm pass -> first MMA; the weights are only needed at the end of it).  Measured -0.6 % of a UNet
-    // step's op time, -1.6 % of the sampler at B = 16 (profiles/r2/ab_tail.log).
-    if (L.patch_first != 0 && !dep_ok) {
-      asm volatile("griddepcontrol.wait;" ::: "memory");
-      dep_ok = true;
-    }
+    // Patches are the previous layer's output: no patch request before griddepcontrol.wait.  The loader of a TMA-fed
+    // layer waits for it before its first weight stage too, so that the first patch is requested first: a CTA only
+    // becomes resident when the previous launch's CTA on this SM has exited, so the dependency resolves within a few
+    // microseconds anyway, and 64 - 96 KB of weight stages queued ahead of the 43 KB patch on the SM's inbound link
+    // would delay the longer chain (patch -> GroupNorm pass -> first MMA; the weights are only needed at the end of it).
+    // Measured -0.6 % of a UNet step's op time, -1.6 % of the sampler at B = 16 (profiles/r2/ab_tail.log).
+    if (tma_in) asm volatile("griddepcontrol.wait;" ::: "memory");
     const int total = (tile_end - tile_begin) * L.nchunks;
     // patch cursor
     int a_next = tma_in ? 0 : total, a_c = 0, a_gs = 0, a_gph = 0, a_rs = 0, a_rph = 0;
@@ -660,7 +633,6 @@ conv_gemm_kernel(const __grid_constant__ ConvLayer L, int t_step) {
     int b_q = 0, b_qq = 0, bs = 0, bph = 0;  // next tap overall / inside its tile
     // (pair mode: the weights are packed as two half-width copies of the single-CTA layout, half r for CTA r)
     const uint8_t* const w0 = L.weights + (kPair ? size_t(crank) * size_t(L.w_half) : size_t(n_off) * 16);
-    int b_issued = 0;
     // phase layers: the weights of phase p follow those of phase p-1 (taps_tile blobs each); w_bv / w_tin = virtual
     // image / tile-in-image of the tile that tap b_q belongs to
     const int phsh = L.phases > 1 ? 2 : 0;
@@ -668,11 +640,7 @@ conv_gemm_kernel(const __grid_constant__ ConvLayer L, int t_step) {
     int w_bv = tile_first / tiles_per_img, w_tin = tile_first - w_bv * tiles_per_img;
     while (a_next < total || b_q < total_taps) {
       bool progress = false;
-      if (!dep_ok && (b_issued >= Cfg::kBStages || b_q >= total_taps)) {
-        asm volatile("griddepcontrol.wait;" ::: "memory");
-        dep_ok = true;
-      }
-      if (dep_ok && a_next < total) {
+      if (a_next < total) {
         const bool a_r1 = L.chunk[a_c].ring != 0;
         const int a_as = a_r1 ? nG + a_rs : a_gs;
         const uint32_t ok = mbar_test(bar_a_empty(a_as), (a_r1 ? a_rph : a_gph) ^ 1) ? 1u : 0u;
@@ -766,7 +734,6 @@ conv_gemm_kernel(const __grid_constant__ ConvLayer L, int t_step) {
           b_q += g;
           for (b_qq += g; b_qq >= taps_tile; b_qq -= taps_tile)
             if ((w_tin += kTStep) >= tiles_per_img) { w_tin -= tiles_per_img; ++w_bv; }
-          ++b_issued;
           progress = true;
         }
       }
@@ -776,7 +743,7 @@ conv_gemm_kernel(const __grid_constant__ ConvLayer L, int t_step) {
     // =========================================================== input producers
     const int pw = warp < 4 ? warp - 2 : warp - 10;  // warps 2,3,12..19 -> 0..9
     const int pidx = pw * 32 + lane;                  // 0..319
-    const int H = L.H, W = L.W, mode = L.mode, tiles_x = L.tiles_x;
+    const int H = L.H, W = L.W, tiles_x = L.tiles_x;
     __half* table_h = reinterpret_cast<__half*>(table);
     int as = 0, aph = 0, cur_b = -1;
     int b = tile_first / tiles_per_img;
@@ -842,13 +809,12 @@ conv_gemm_kernel(const __grid_constant__ ConvLayer L, int t_step) {
           const float rstd = rsqrtf(float(var) + L.gn_eps);
           const float sc = ga[j] * rstd;
           const float sh = be[j] - float(mean) * sc;
-          if constexpr (kFast && Cvt<T>::kFmt == 0) {  // half-scaled so that swish(y) = h*tanh(h) + h with h = y/2
+          // half-scaled so that swish(y) = h*tanh(h) + h with h = y/2
+          if constexpr (Cvt<T>::kFmt == 0) {
             table_h[c] = __float2half_rn(0.5f * sc);
             table_h[kMaxGnC + c] = __float2half_rn(0.5f * sh);
-          } else if constexpr (kFast) {  // bf16 storage: fp32 affine, then the packed-half tanh form
+          } else {  // bf16 storage: fp32 affine, then the packed-half tanh form
             table[c] = make_float2(0.5f * sc, 0.5f * sh);
-          } else {
-            table[c] = make_float2(sc, sh);
           }
         }
       }
@@ -909,37 +875,35 @@ conv_gemm_kernel(const __grid_constant__ ConvLayer L, int t_step) {
           rph ^= 1u << as;
           if (pidx == 0 && tile == tile_begin && c == 0) PROF_TS(3);  // first patch landed
           PROF_MARK(1);
-          if (!(L.dbg & 2)) {
-            const int cgs = (pidx & 7) ^ ((pos0 + 5 * as) & 7);
-            float sc[8], sh[8];
-            uint4 hsc = make_uint4(0u, 0u, 0u, 0u), hsh = hsc;
-            if constexpr (kFast && Cvt<T>::kFmt == 0) {
-              hsc = *reinterpret_cast<const uint4*>(table_h + ck.vc0 + cgs * 8);
-              hsh = *reinterpret_cast<const uint4*>(table_h + kMaxGnC + ck.vc0 + cgs * 8);
-            } else {
+          const int cgs = (pidx & 7) ^ ((pos0 + 5 * as) & 7);
+          float sc[8], sh[8];
+          uint4 hsc = make_uint4(0u, 0u, 0u, 0u), hsh = hsc;
+          if constexpr (Cvt<T>::kFmt == 0) {
+            hsc = *reinterpret_cast<const uint4*>(table_h + ck.vc0 + cgs * 8);
+            hsh = *reinterpret_cast<const uint4*>(table_h + kMaxGnC + ck.vc0 + cgs * 8);
+          } else {
 #pragma unroll
-              for (int j = 0; j < 8; ++j) {
-                const float2 e = table[ck.vc0 + cgs * 8 + j];
-                sc[j] = e.x;
-                sh[j] = e.y;
-              }
+            for (int j = 0; j < 8; ++j) {
+              const float2 e = table[ck.vc0 + cgs * 8 + j];
+              sc[j] = e.x;
+              sh[j] = e.y;
             }
-            const uint32_t a0 = sA + as * kAStageBytes + uint32_t(pidx) * 16;  // (GroupNorm chunks: ring 0)
-            uint4 rv[kMaxUnits];
+          }
+          const uint32_t a0 = sA + as * kAStageBytes + uint32_t(pidx) * 16;  // (GroupNorm chunks: ring 0)
+          uint4 rv[kMaxUnits];
+#pragma unroll
+          for (int i = 0; i < kMaxUnits; ++i)
+            if ((vmask >> i) & 1u) rv[i] = lds128(a0 + i * (40 * 128));
+          if (ck.gn == 1) {
 #pragma unroll
             for (int i = 0; i < kMaxUnits; ++i)
-              if ((vmask >> i) & 1u) rv[i] = lds128(a0 + i * (40 * 128));
-            if (ck.gn == 1) {
+              if ((vmask >> i) & 1u) sts128(a0 + i * (40 * 128), gn_swish_unit<T>(rv[i], hsc, hsh, sc, sh));
+          } else {  // GroupNorm without activation
 #pragma unroll
-              for (int i = 0; i < kMaxUnits; ++i)
-                if ((vmask >> i) & 1u) sts128(a0 + i * (40 * 128), gn_swish_unit<T, kFast>(rv[i], hsc, hsh, sc, sh));
-            } else {  // GroupNorm without activation
-#pragma unroll
-              for (int i = 0; i < kMaxUnits; ++i)
-                if ((vmask >> i) & 1u) sts128(a0 + i * (40 * 128), gn_affine_unit<T, kFast>(rv[i], hsc, hsh, sc, sh));
-            }
-            fence_proxy_async_smem();
+            for (int i = 0; i < kMaxUnits; ++i)
+              if ((vmask >> i) & 1u) sts128(a0 + i * (40 * 128), gn_affine_unit<T>(rv[i], hsc, hsh, sc, sh));
           }
+          fence_proxy_async_smem();
           PROF_MARK(3);
           __syncwarp();
           if (lane == 0) mbar_arrive(bar_a_full(as));
@@ -951,101 +915,54 @@ conv_gemm_kernel(const __grid_constant__ ConvLayer L, int t_step) {
         }
       }
     } else {
-      // ----------------------------------------------------------------- gathered layers (nearest-upsample,
-      // space-to-depth, the 16-channel stem): predicated 16-byte global loads into registers,
-      // GroupNorm + Swish, 16-byte stores into the no-swizzle [channel group][position][8 ch] patch
-      const int lg = ncg == 8 ? 3 : (ncg == 4 ? 2 : (ncg == 2 ? 1 : 0));
-      const int cg = pidx & (ncg - 1);
-      const int nunits = kPatchPos * ncg;
+      // ----------------------------------------------------------------- nearest-upsample convs in the nine-tap form
+      // (64-channel raw chunks, no GroupNorm): predicated 16-byte global loads of the 2x-upsampled patch, 16-byte stores
+      // into the no-swizzle [channel group][position][8 ch] patch
+      const int cg = pidx & 7;
       // per-thread patch coordinates of the (up to) 9 16-byte units it fills: fixed for the launch
       uint32_t pcoord[kMaxUnits];  // py | px << 8
-      uint32_t emask = 0u, smask = 0u;  // bit i: unit i carries data / unit i has a smem slot to fill
-      uint32_t cenmask = 0u;            // bit i: unit i lies in the 32x8 centre of the patch (no halo)
+      uint32_t smask = 0u;         // bit i: unit i has a smem slot to fill
 #pragma unroll
       for (int i = 0; i < kMaxUnits; ++i) {
         const int u = pidx + i * kProdThreads;
-        const int pos = u >> lg;
+        const int pos = u >> 3;
         const int py = pos / kPatchW, px = pos - py * kPatchW;
-        bool ex = u < nunits;
-        smask |= ex ? (1u << i) : 0u;
-        if (mode == kModeS2D && (py > kTileH || px > kTileW)) ex = false;  // 33x9 block patch
-        emask |= ex ? (1u << i) : 0u;
-        cenmask |= (py >= 1 && py <= kTileH && px >= 1 && px <= kTileW) ? (1u << i) : 0u;
+        smask |= u < kPatchPos * 8 ? (1u << i) : 0u;
         pcoord[i] = uint32_t(py) | (uint32_t(px) << 8);
       }
-      const int shl = mode == kModeS2D ? 1 : 0, shr = mode == kModeUp2x ? 1 : 0;
-      const int src_w = mode == kModeS2D ? 2 * W : (mode == kModeUp2x ? (W >> 1) : W);
+      const int src_w = W >> 1;
       for (int tile = tile_begin; tile < tile_end; ++tile) {
         const int y0 = ty * kTileH - 1, x0 = tx * kTileW - 1;
-        if (L.gn_C > 0 && b != cur_b) {
-          cur_b = b;
-          build_table(b);
-        }
         // ---- source pixel offsets of this thread's patch positions; vmask bit i = inside the image
         int pixoff[kMaxUnits];
         uint32_t vmask = 0u;
 #pragma unroll
         for (int i = 0; i < kMaxUnits; ++i) {
           const int y = y0 + int(pcoord[i] & 0xffu), x = x0 + int((pcoord[i] >> 8) & 0xffu);
-          const bool ok = ((emask >> i) & 1u) != 0u && unsigned(y) < unsigned(H) && unsigned(x) < unsigned(W);
-          const int off = ((y << shl) >> shr) * src_w + ((x << shl) >> shr);
+          const bool ok = ((smask >> i) & 1u) != 0u && unsigned(y) < unsigned(H) && unsigned(x) < unsigned(W);
+          const int off = (y >> 1) * src_w + (x >> 1);
           pixoff[i] = ok ? off : 0;
           vmask |= ok ? (1u << i) : 0u;
         }
         PROF_MARK(0);
         for (int c = 0; c < L.nchunks; ++c) {
-          if (L.dbg & 2) {  // experiment: producers only hand over (stale) stages
-            mbar_wait(bar_a_empty(as), aph ^ 1);
-            fence_proxy_async_smem();
-            __syncwarp();
-            if (lane == 0) mbar_arrive(bar_a_full(as));
-            if (++as == kAStages) { as = 0; aph ^= 1; }
-            continue;
-          }
           const ConvChunk& ck = L.chunk[c];
           const ConvSrc& s = L.src[ck.src];
           const int sC = s.C;
-          const uint32_t tmask = ck.gn != 0 ? vmask : 0u;  // units that get GroupNorm + Swish
-          // a chunk whose only tap is the centre one (one space-to-depth plane) never reads the halo:
-          // neither load nor store it
-          const uint32_t cm = (ck.ntaps == 1 && ck.tap_pos[0] == kPatchW + 1) ? cenmask : 0xffffffffu;
-          const uint32_t lmask = vmask & cm, stmask = smask & cm;
-          const bool gn = ck.gn != 0;
           const uint8_t* base = reinterpret_cast<const uint8_t*>(
-              reinterpret_cast<const T*>(s.ptr) + (size_t(b) * s.H * s.W + ck.pix_delta) * sC + ck.c0 + cg * 8);
+              reinterpret_cast<const T*>(s.ptr) + size_t(b) * s.H * s.W * sC + ck.c0 + cg * 8);
           const uint32_t pix_bytes = uint32_t(sC) * 2u;
           uint4 rv[kMaxUnits];
 #pragma unroll
           for (int i = 0; i < kMaxUnits; ++i)
-            rv[i] = ldg16_pred(base + uint32_t(pixoff[i]) * pix_bytes, ((lmask >> i) & 1u) != 0u);
-          float sc[8], sh[8];
-          uint4 hsc = make_uint4(0u, 0u, 0u, 0u), hsh = hsc;
-          if (gn) {
-            if constexpr (kFast && Cvt<T>::kFmt == 0) {
-              hsc = *reinterpret_cast<const uint4*>(table_h + ck.vc0 + cg * 8);
-              hsh = *reinterpret_cast<const uint4*>(table_h + kMaxGnC + ck.vc0 + cg * 8);
-            } else {
-#pragma unroll
-              for (int j = 0; j < 8; ++j) {
-                const float2 e = table[ck.vc0 + cg * 8 + j];
-                sc[j] = e.x;
-                sh[j] = e.y;
-              }
-            }
-          }
+            rv[i] = ldg16_pred(base + uint32_t(pixoff[i]) * pix_bytes, ((vmask >> i) & 1u) != 0u);
           PROF_MARK(1);
           mbar_wait(bar_a_empty(as), aph ^ 1);
           PROF_MARK(2);
-          const uint32_t dst0 = sA + as * kAStageBytes + cg * kPlaneBytes + uint32_t(pidx >> lg) * 16;
+          const uint32_t dst0 = sA + as * kAStageBytes + cg * kPlaneBytes + uint32_t(pidx >> 3) * 16;
 #pragma unroll
-          for (int i = 0; i < kMaxUnits; ++i) {
-            if ((stmask >> i) & 1u) {
-              uint4 o = rv[i];
-              if ((tmask >> i) & 1u)
-                o = ck.gn == 1 ? gn_swish_unit<T, kFast>(o, hsc, hsh, sc, sh) : gn_affine_unit<T, kFast>(o, hsc, hsh, sc, sh);
-              sts128(dst0 + uint32_t((i * kProdThreads) >> lg) * 16, o);
-            }
-          }
+          for (int i = 0; i < kMaxUnits; ++i)
+            if ((smask >> i) & 1u) sts128(dst0 + uint32_t((i * kProdThreads) >> 3) * 16, rv[i]);
           fence_proxy_async_smem();
           __syncwarp();
           if (lane == 0) mbar_arrive(bar_a_full(as));
@@ -1094,7 +1011,7 @@ conv_gemm_kernel(const __grid_constant__ ConvLayer L, int t_step) {
     const bool act = L.out_mode == kOutAct;
     const bool do_stats = (L.out_stats != nullptr) && act;
     const bool has_res = (L.resid != nullptr) && act;
-    const bool use_tma = (N >= 32) && act && L.use_tma_store != 0;
+    const bool use_tma = N >= 32 && act;  // (N = 16 has no staging blocks)
     // staging blocks (2 KB, 512-byte aligned for the 64B swizzle).  Team 1: the third patch stage, which a producer-free
     // layer does not use (N <= 128); N = 256 has only two: the tail of the allocation + the unused GroupNorm table
     uint32_t stage_s = smem_u32(smem + Cfg::kOffStage) + uint32_t(ew) * 2048;
@@ -1184,7 +1101,7 @@ conv_gemm_kernel(const __grid_constant__ ConvLayer L, int t_step) {
       tc_fence_after();
       const uint32_t taddr = lane_base + acc * acc_cols + mt * Cfg::kAccStride;
 #pragma unroll 1
-      for (int cb = cb_first; cb < ((L.dbg & 1) ? 0 : Cfg::kNcb); cb += cb_step) {
+      for (int cb = cb_first; cb < Cfg::kNcb; cb += cb_step) {
         uint32_t raw[32];
         tmem_ld32(taddr + cb * 32, raw);
         tmem_ld_wait();
@@ -1227,7 +1144,7 @@ conv_gemm_kernel(const __grid_constant__ ConvLayer L, int t_step) {
             vmax = fmaxf(vmax, cbmax);
           }
           PROF_MARK(4);
-          if (use_tma && !(L.dbg & 4)) {
+          if (use_tma) {
             // stage the warp's 32 px x 32 ch block (64B-swizzled rows), then one bulk tensor store:
             // full 64-byte segments per pixel instead of 32 scattered 16-byte writes per instruction
             if (lane == 0) bulk_wait_read0();  // previous store has drained the staging block
@@ -1248,7 +1165,7 @@ conv_gemm_kernel(const __grid_constant__ ConvLayer L, int t_step) {
                            ty * TH + mt * 16 + q * 4, b_img);
               bulk_commit_group();
             }
-          } else if (valid && !(L.dbg & 4)) {
+          } else if (valid) {
             uint4* op = reinterpret_cast<uint4*>(orow + cb * 64);
 #pragma unroll
             for (int k = 0; k < 4; ++k) {
@@ -1261,7 +1178,7 @@ conv_gemm_kernel(const __grid_constant__ ConvLayer L, int t_step) {
             }
           }
           PROF_MARK(6);
-          if (do_stats && !(L.dbg & 8)) {
+          if (do_stats) {
             // in place: v[2p] <- pair sum, v[2p+1] <- pair sum of squares (zero for masked rows)
             if (all_valid) {
 #pragma unroll
@@ -1391,7 +1308,7 @@ conv_gemm_kernel(const __grid_constant__ ConvLayer L, int t_step) {
         tx -= tiles_x;
         if (++ty == L.tiles_y) { ty = 0; ++b; }
       }
-      if (do_stats && !(L.dbg & 1)) {
+      if (do_stats) {
         const bool flush = !Cfg::kStatsInTmem || (tile + 1) % tgroup == 0;
         if (flush) {
           if (Cfg::kStatsInTmem) {
@@ -1439,7 +1356,7 @@ conv_gemm_kernel(const __grid_constant__ ConvLayer L, int t_step) {
   }
 
   tc_fence_before();
-  if (kPair && defer_cs && warp != 0) cluster_wait();  // (the opening barrier's wait, see above)
+  if (kPair && warp != 0) cluster_wait();  // (the opening barrier's wait, see above)
   __syncthreads();
   if (kPair) cluster_sync_all();  // neither CTA frees its TMEM / exits while the pair's MMAs or commits may still touch it
   if (tid == 0) PROF_TS(7);

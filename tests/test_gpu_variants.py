@@ -1,15 +1,12 @@
-"""The kernel's alternative code paths against each other (B200, `pytest -m gpu`): every optimisation that replaces one
-way of computing a layer by another keeps an environment switch, and the two forms must agree —
-bitwise where the arithmetic is identical, within 16-bit rounding noise where the association changes (a one-ulp change of
-an early activation reshuffles every later rounding: the whole-network difference is the same ~1e-3 as between either
-form and the fp32 reference).
+"""The kernel's alternative code paths against each other (B200, `pytest -m gpu`): where the automatic per-layer choice
+picks between two forms of a computation, each for some supported layer or configuration, an environment switch read at
+context creation forces one form everywhere, and the two forms must agree — bitwise where the arithmetic is identical,
+within 16-bit rounding noise where the association changes (a one-ulp change of an early activation reshuffles every
+later rounding: the whole-network difference is the same ~1e-3 as between either form and the fp32 reference).
 
   FDSR_UP_PHASES=0   nearest-upsample convs: nine-tap form on the gathered 2x patch  vs  four 2x2 phase convs with
                      pre-summed weights on the low-resolution input (exact identity up to the rounding of the sums)
-  FDSR_S2D_TMA=0     stride-2 convs: parity planes gathered by the producer warps    vs  one strided tensor load each
   FDSR_RESID_MMA=0   identity residual of the N = 64 layers added by the epilogue    vs  an identity-matrix K chunk
-  FDSR_TMA_IN=0      every input patch gathered by the producer warps (which also selects the nine-tap upsample
-                     form)                                                           vs  TMA tensor loads
   FDSR_SPLIT_N=0     256-wide low-resolution layers on one CTA per tile              vs  two 128-column halves
   FDSR_PAIR=0        every layer on single CTAs (tcgen05.mma.cta_group::1)           vs  CTA pairs (cta_group::2, M = 256,
                      each CTA staging half of the weight columns) where the tile rows are even
@@ -18,10 +15,6 @@ form and the fp32 reference).
                      epilogue team (odd 32-column blocks) in the layers that have no producer work
   FDSR_TAIL_HELP=0   the last tile of every CTA drained by warps 4..11 alone        vs  producer warps 12..19 joining as a
                      second team for that one tile (its epilogue is exposed: nothing left to overlap it with)
-  FDSR_PATCH_FIRST=0 weight stages requested before the launch dependency resolves, the first patch after  vs  the first
-                     patch first (it heads the longer chain: patch -> GroupNorm pass -> first MMA)
-  FDSR_DEFER_CSYNC=0 CTA pairs: full cluster barrier in the prologue               vs  arrive there, wait where needed
-  FDSR_STEM_TMA=0    16-channel stem input gathered by the producer warps           vs  two 8-channel TMA plane loads
   FDSR_FUSED_TAIL=0  sampler: pack_input / final conv -> eps / posterior kernels    vs  the final conv's epilogue doing the
                      posterior update in registers and rewriting the next step's input (checked on the sampler)
 """
@@ -66,10 +59,9 @@ def base(oracle, schedule, inputs):
     return eng, eng.unet_forward(inputs[0], inputs[1], 9)
 
 
-@pytest.mark.parametrize("switch,tol", [("FDSR_S2D_TMA", 0.0), ("FDSR_SPLIT_N", 0.0), ("FDSR_STEM_TMA", 0.0),
-                                        ("FDSR_HALF_TILES", 0.0), ("FDSR_EPI2", 0.0), ("FDSR_TAIL_HELP", 0.0), ("FDSR_PATCH_FIRST", 0.0), ("FDSR_DEFER_CSYNC", 0.0),
-                                        ("FDSR_PAIR", 3e-3), ("FDSR_RESID_MMA", 3e-3),
-                                        ("FDSR_UP_PHASES", 3e-3), ("FDSR_TMA_IN", 3e-3)])
+@pytest.mark.parametrize("switch,tol", [("FDSR_SPLIT_N", 0.0), ("FDSR_HALF_TILES", 0.0), ("FDSR_EPI2", 0.0),
+                                        ("FDSR_TAIL_HELP", 0.0), ("FDSR_PAIR", 3e-3), ("FDSR_RESID_MMA", 3e-3),
+                                        ("FDSR_UP_PHASES", 3e-3)])
 def test_alternative_paths_agree(oracle, schedule, inputs, base, switch, tol):
     eng0, eps0 = base
     eng1 = make(oracle, schedule, {switch: "0"})

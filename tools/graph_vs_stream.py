@@ -1,5 +1,5 @@
-"""Sampler time per batch with / without CUDA-graph replay and with / without programmatic dependent launch.
-python tools/graph_vs_stream.py [B] [H]   (each combination in a fresh subprocess: the switches are read at context creation)"""
+"""Sampler time per batch with / without CUDA-graph replay.
+python tools/graph_vs_stream.py [B] [H]   (each run in a fresh subprocess)"""
 import os
 import subprocess
 import sys
@@ -29,8 +29,6 @@ B = sys.argv[1] if len(sys.argv) > 1 else "16"
 H = sys.argv[2] if len(sys.argv) > 2 else "256"
 for rnd in range(2):
     for graph in ("1", "0"):
-        for pdl in ("1", "0"):
-            env = dict(os.environ, FDSR_PDL=pdl)
-            out = subprocess.run([sys.executable, "-c", CHILD, B, H, graph], env=env, capture_output=True, text=True)
-            ms = out.stdout.strip().splitlines()[-1] if out.stdout.strip() else out.stderr[-300:]
-            print(f"round {rnd}: graph={graph} pdl={pdl}: {ms} ms / batch (B={B}, {H}x{H})", flush=True)
+        out = subprocess.run([sys.executable, "-c", CHILD, B, H, graph], capture_output=True, text=True)
+        ms = out.stdout.strip().splitlines()[-1] if out.stdout.strip() else out.stderr[-300:]
+        print(f"round {rnd}: graph={graph}: {ms} ms / batch (B={B}, {H}x{H})", flush=True)
