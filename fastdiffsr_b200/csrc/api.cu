@@ -44,8 +44,8 @@ struct HChunk {
   int wc0;      // first input channel inside the weight tensor
   int creal;    // real (non-padded) channels in this chunk
   int kk = 3;   // kernel size of the weight tensor (3, or 1 for res_conv / attention projections)
-  // stem only: the packed network input is [x0 x1 x2 0 | c0 c1 c2 0 | 0 ...] (pack_input_kernel) while the reference
-  // concatenates cat([cond, x]) (diffusion.py:173): perm[j] = reference input channel of packed channel j, or -1
+  // stem only: the packed network input holds x_t in channels [0, C) and cond in [P, P + C) (pack_pixel) while the
+  // reference concatenates cat([cond, x]) (diffusion.py:173): perm[j] = reference input channel of packed channel j, or -1
   std::vector<int> perm;
   int wchan(int ci) const { return perm.empty() ? (ci < creal ? wc0 + ci : -1) : (ci < int(perm.size()) ? perm[ci] : -1); }
   int nreal() const {
@@ -137,6 +137,7 @@ struct fdsr_ctx {
   std::vector<size_t> w32_off;      // per conv (floats)
   size_t off_gntab = 0;             // [B][kMaxGnC] float2 scratch of the fp32 mode
   int esize() const { return cfg.dtype == FDSR_DTYPE_FP32 ? 4 : 2; }
+  int bands() const { return cfg.out_channel; }  // C: channels of every image tensor (cond, x_t, eps, noise, SR, u8)
   long long* d_prof = nullptr;  // role cycle counters (FDSR_PROFILE builds)
   bool layers_dirty = true;
   // bicubic tables (cached per size pair)
@@ -188,7 +189,7 @@ struct fdsr_ctx {
   }
   int64_t launches = 0;
   double flops_per_px = 0.0;  // conv FLOPs per full-resolution output pixel per image
-  // fdsr_sample_tiled: [SampleArgs | canvas x_t (B,3,H,W) fp32 | per-tile eps store [slot][3][te_y][te_x] fp32],
+  // fdsr_sample_tiled: [SampleArgs | canvas x_t (B,C,H,W) fp32 | per-tile eps store [slot][C][te_y][te_x] fp32],
   // grow-only, apart from the workspace (which only ever holds one chunk of tiles)
   uint8_t* d_tiled = nullptr;
   size_t tiled_cap = 0;
@@ -379,8 +380,10 @@ int add_res_attn(fdsr_ctx* c, const std::string& name, const std::vector<int>& s
 int build_plan(fdsr_ctx* c) {
   const fdsr_config& g = c->cfg;
   const int inner = g.inner_channel;
-  if (g.in_channel != 6 || g.out_channel != 3)
-    return fail(c, FDSR_E_INVALID, "only in_channel=6 / out_channel=3 (conditional SR) is supported");
+  if (g.out_channel < 1 || g.out_channel > 8 || g.in_channel != 2 * g.out_channel)
+    return fail(c, FDSR_E_INVALID,
+                "in_channel must be 2 * out_channel with 1 <= out_channel <= 8 (conditional SR of C-band images; got "
+                "in_channel=%d, out_channel=%d)", g.in_channel, g.out_channel);
   if (inner % 64 != 0) return fail(c, FDSR_E_INVALID, "inner_channel must be a multiple of 64");
   if (g.norm_groups != 32) return fail(c, FDSR_E_INVALID, "norm_groups must be 32");
   if (g.n_levels < 1 || g.n_levels > FDSR_MAX_LEVELS) return fail(c, FDSR_E_INVALID, "bad n_levels");
@@ -401,8 +404,14 @@ int build_plan(fdsr_ctx* c) {
     k.ncg = 2;
     k.nsrc = 1;
     k.src[0] = c->t_xin;
-    HChunk stem{0, 0, 0, 0, -1, taps3x3(), "denoise_fn.downs.0.weight", 0, 7};
-    stem.perm = {3, 4, 5, -1, 0, 1, 2};  // packed [x | 0 | cond] -> reference cat([cond, x]) channels
+    // packed [x (C) | 0 | cond (C) | 0] with cond at P = 4 (C <= 4) or 8 -> reference cat([cond, x]) channels
+    const int C = g.out_channel, P = C <= 4 ? 4 : 8;
+    HChunk stem{0, 0, 0, 0, -1, taps3x3(), "denoise_fn.downs.0.weight", 0, P + C};
+    stem.perm.assign(16, -1);
+    for (int j = 0; j < C; ++j) {
+      stem.perm[j] = C + j;
+      stem.perm[P + j] = j;
+    }
     k.chunks.push_back(stem);
     k.bias_names = {"denoise_fn.downs.0.bias"};
     k.out = cur;
@@ -1393,7 +1402,7 @@ int pack_input(fdsr_ctx* c, cudaStream_t st) {
   const int64_t npix = int64_t(c->B) * HW;
   pack_input_kernel<T><<<unsigned((npix + 255) / 256), 256, 0, st>>>(
       reinterpret_cast<const float*>(c->d_ws + c->off_cond), reinterpret_cast<const float*>(c->d_ws + c->off_x),
-      reinterpret_cast<T*>(c->d_ws + c->tensors[c->t_xin].off), c->B, HW);
+      reinterpret_cast<T*>(c->d_ws + c->tensors[c->t_xin].off), c->B, HW, c->bands());
   CUDA_TRY(c, cudaGetLastError());
   ++c->launches;
   return FDSR_OK;
@@ -1445,10 +1454,11 @@ int check_ready(fdsr_ctx* c) {
 // injected noise / the generator's stream t
 int posterior_launch(fdsr_ctx* c, const float* x, const float* eps, const float* z, int t, float* out,
                      int64_t numel_img, int images, const SampleArgs* args, int64_t z_block, cudaStream_t st) {
-  if (numel_img % 3 || numel_img / 3 > 0x7fffffffLL || images < 1 || images > 65535)
-    return fail(c, FDSR_E_INVALID, "posterior: images are (3,H,W) blocks, 1..65535 of them");
-  const uint32_t hw = uint32_t(numel_img / 3);
-  posterior_kernel<<<dim3((hw + 255) / 256, images), 256, 0, st>>>(x, eps, z, out, hw, c->post[t], args, z_block,
+  const int C = c->bands();
+  if (numel_img % C || numel_img / C > 0x7fffffffLL || images < 1 || images > 65535)
+    return fail(c, FDSR_E_INVALID, "posterior: images are (%d,H,W) blocks, 1..65535 of them", C);
+  const uint32_t hw = uint32_t(numel_img / C);
+  posterior_kernel<<<dim3((hw + 255) / 256, images), 256, 0, st>>>(x, eps, z, out, hw, C, c->post[t], args, z_block,
                                                                     uint32_t(t), t > 0 ? 1 : 0);
   CUDA_TRY(c, cudaGetLastError());
   ++c->launches;
@@ -1460,14 +1470,15 @@ int posterior_launch(fdsr_ctx* c, const float* x, const float* eps, const float*
 int sample_enqueue(fdsr_ctx* c, bool has_trace, cudaStream_t st) {
   const SampleArgs* args = reinterpret_cast<const SampleArgs*>(c->d_ws + c->off_seed);
   const int T = c->T, B = c->B;
-  const int64_t per = int64_t(3) * c->H * c->W, numel = per * B;
+  const int64_t per = int64_t(c->bands()) * c->H * c->W, numel = per * B;
   float* x = reinterpret_cast<float*>(c->d_ws + c->off_x);
   float* cond = reinterpret_cast<float*>(c->d_ws + c->off_cond);
   float* eps = reinterpret_cast<float*>(c->d_ws + c->off_eps);
   float* sr = reinterpret_cast<float*>(c->d_ws + c->off_sr);
   const int nfr = fdsr_trace_frames(c);
   const unsigned gb = unsigned((numel + 255) / 256);
-  noise_init_kernel<<<dim3((uint32_t(c->H) * c->W + 255) / 256, B), 256, 0, st>>>(x, uint32_t(c->H) * c->W, args, uint32_t(T));
+  noise_init_kernel<<<dim3((uint32_t(c->H) * c->W + 255) / 256, B), 256, 0, st>>>(x, uint32_t(c->H) * c->W, c->bands(), args,
+                                                                              uint32_t(T));
   ++c->launches;
   // FastDiffSR predicts the residual: frames and result go through res2img (diffusion.py:213-216, 275-281).
   // The SR3 baseline predicts the image: frames are the raw x, the first frame is the conditioning image itself
@@ -1519,7 +1530,7 @@ TileAxis make_axis(int L, int t, int overlap) {
   return a;
 }
 
-// The T-step tiled loop.  d_tiled holds [SampleArgs | x (B,3,H,W) | eps store of n_chunks * bc tile slots]; the
+// The T-step tiled loop.  d_tiled holds [SampleArgs | x (B,C,H,W) | eps store of n_chunks * bc tile slots]; the
 // workspace is reserved for one chunk (bc tiles of te_y x te_x).  Plain stream launches: a chunk's UNet (~5 ms at
 // bc = 16, 256^2) keeps the device well behind the host's ~0.3 ms of launch calls.
 template <typename T>
@@ -1527,10 +1538,11 @@ int tiled_enqueue(fdsr_ctx* c, const float* cond, float* sr_out, bool has_trace,
                   const TileAxis& ax, int64_t n_tiles, int64_t n_chunks, int bc, cudaStream_t st) {
   const SampleArgs* args = reinterpret_cast<const SampleArgs*>(c->d_tiled);
   const uint32_t HW = uint32_t(ay.L) * uint32_t(ax.L);
-  const int64_t per = int64_t(3) * HW;
+  const int C = c->bands();
+  const int64_t per = int64_t(C) * HW;
   float* x = reinterpret_cast<float*>(c->d_tiled + 256);
   float* eps_store = reinterpret_cast<float*>(c->d_tiled + 256 + align_up(size_t(per) * B * 4, 256));
-  const int64_t tile_floats = int64_t(3) * ay.te * ax.te;
+  const int64_t tile_floats = int64_t(C) * ay.te * ax.te;
   const size_t chunk_bytes = size_t(bc) * tile_floats * 4;
   const dim3 pgrid(unsigned((uint64_t(HW) + 255) / 256), unsigned(B));
   const unsigned gb = unsigned((per * B + 255) / 256);
@@ -1538,7 +1550,7 @@ int tiled_enqueue(fdsr_ctx* c, const float* cond, float* sr_out, bool has_trace,
   T* xin = reinterpret_cast<T*>(c->d_ws + c->tensors[c->t_xin].off);
   const float* eps_chunk = reinterpret_cast<const float*>(c->d_ws + c->off_eps);
   const int T_ = c->T, nfr = fdsr_trace_frames(c), inter = 1 | (T_ / 10);
-  noise_init_kernel<<<pgrid, 256, 0, st>>>(x, HW, args, uint32_t(T_));
+  noise_init_kernel<<<pgrid, 256, 0, st>>>(x, HW, C, args, uint32_t(T_));
   ++c->launches;
   int frame = 0;
   if (has_trace) {
@@ -1548,14 +1560,14 @@ int tiled_enqueue(fdsr_ctx* c, const float* cond, float* sr_out, bool has_trace,
   }
   for (int k = 0, t = T_ - 1; t >= 0; --t, ++k) {
     for (int64_t ch = 0; ch < n_chunks; ++ch) {
-      tile_pack_kernel<T><<<pack_blocks, 256, 0, st>>>(cond, x, xin, ay, ax, ch * bc, n_tiles, bc);
+      tile_pack_kernel<T><<<pack_blocks, 256, 0, st>>>(cond, x, xin, ay, ax, ch * bc, n_tiles, bc, C);
       CUDA_TRY(c, cudaGetLastError());
       ++c->launches;
       int rc = unet_internal<T>(c, t, st, false, true);
       if (rc) return rc;
       CUDA_TRY(c, cudaMemcpyAsync(eps_store + ch * bc * tile_floats, eps_chunk, chunk_bytes, cudaMemcpyDeviceToDevice, st));
     }
-    tile_blend_posterior_kernel<<<pgrid, 256, 0, st>>>(x, eps_store, ay, ax, c->post[t], args, k + 1, uint32_t(t),
+    tile_blend_posterior_kernel<<<pgrid, 256, 0, st>>>(x, eps_store, ay, ax, C, c->post[t], args, k + 1, uint32_t(t),
                                                        t > 0 ? 1 : 0);
     ++c->launches;
     if (has_trace && t % inter == 0) {
@@ -1855,7 +1867,7 @@ int fdsr_reserve(fdsr_ctx* c, int32_t B, int32_t H, int32_t W) {
   off = align_up(off + size_t(B) * cmax * 4, 256);
   c->off_sp = off;
   off = align_up(off + (lmin < 99 ? size_t(B) * (H >> lmin) * (W >> lmin) * 8 : 0), 256);
-  const size_t img = align_up(size_t(B) * 3 * H * W * 4, 256);
+  const size_t img = align_up(size_t(B) * c->bands() * H * W * 4, 256);
   c->off_cond = off;
   off += img;
   c->off_x = off;
@@ -1897,7 +1909,7 @@ int fdsr_unet_forward(fdsr_ctx* c, const float* cond, const float* xt, int32_t t
   rc = fdsr_reserve(c, B, H, W);
   if (rc) return rc;
   cudaStream_t st = static_cast<cudaStream_t>(stream);
-  const size_t bytes = size_t(B) * 3 * H * W * 4;
+  const size_t bytes = size_t(B) * c->bands() * H * W * 4;
   CUDA_TRY(c, cudaMemcpyAsync(c->d_ws + c->off_cond, cond, bytes, cudaMemcpyDeviceToDevice, st));
   CUDA_TRY(c, cudaMemcpyAsync(c->d_ws + c->off_x, xt, bytes, cudaMemcpyDeviceToDevice, st));
   rc = unet_dispatch(c, t, st);
@@ -1912,10 +1924,12 @@ int fdsr_posterior_step(fdsr_ctx* c, const float* xt, const float* eps, const fl
   if (c->T == 0) return fail(c, FDSR_E_STATE, "fdsr_set_schedule has not been called");
   if (t < 0 || t >= c->T) return fail(c, FDSR_E_INVALID, "t out of range");
   if (t > 0 && !z) return fail(c, FDSR_E_INVALID, "z is required for t > 0");
-  if (numel < 3 || numel % 3) return fail(c, FDSR_E_INVALID, "numel must be a positive multiple of 3 ((B,3,H,W) tensors)");
-  // elementwise with an explicit z: treated as one (3, numel/3) image (split into equal blocks if it is huge)
+  const int C = c->bands();
+  if (numel < C || numel % C)
+    return fail(c, FDSR_E_INVALID, "numel must be a positive multiple of %d ((B,%d,H,W) tensors)", C, C);
+  // elementwise with an explicit z: treated as one (C, numel/C) image (split into equal blocks if it is huge)
   int64_t blocks = 1;
-  while (numel % (3 * blocks) != 0 || (numel / blocks) / 3 > 0x7fffffffLL) ++blocks;
+  while (numel % (C * blocks) != 0 || (numel / blocks) / C > 0x7fffffffLL) ++blocks;
   return posterior_launch(c, xt, eps, z, t, out, numel / blocks, int(blocks), nullptr, 0, static_cast<cudaStream_t>(stream));
 }
 
@@ -1936,7 +1950,7 @@ int fdsr_sample(fdsr_ctx* c, const float* cond, const float* noise, uint64_t see
   rc = fdsr_reserve(c, B, H, W);
   if (rc) return rc;
   cudaStream_t st = static_cast<cudaStream_t>(stream);
-  const size_t bytes = size_t(B) * 3 * H * W * 4;
+  const size_t bytes = size_t(B) * c->bands() * H * W * 4;
   CUDA_TRY(c, cudaMemcpyAsync(c->d_ws + c->off_cond, cond, bytes, cudaMemcpyDeviceToDevice, st));
   // seed, image offset and the noise / trace pointers are read from device memory: one captured graph per shape
   SampleArgs a{seed, c->image0, noise, trace};
@@ -2020,7 +2034,8 @@ int fdsr_sample_tiled(fdsr_ctx* c, const float* cond, const float* noise, uint64
   const int bc = int((n_tiles + n_chunks - 1) / n_chunks);
   rc = fdsr_reserve(c, bc, ay.te, ax.te);
   if (rc) return rc;
-  const size_t need = 256 + align_up(size_t(B) * 3 * H * W * 4, 256) + size_t(n_chunks) * bc * 3 * ay.te * ax.te * 4;
+  const size_t need = 256 + align_up(size_t(B) * c->bands() * H * W * 4, 256) +
+                      size_t(n_chunks) * bc * c->bands() * ay.te * ax.te * 4;
   if (need > c->tiled_cap) {
     cudaFree(c->d_tiled);
     c->d_tiled = nullptr;
@@ -2047,7 +2062,8 @@ int fdsr_bicubic_u8(fdsr_ctx* c, const uint8_t* lr, int32_t B, int32_t h, int32_
   rc = ensure_bic(c, h, H);
   if (rc) return rc;
   const fdsr_ctx::BicTab *th = find_bic(c, w, W), *tv = find_bic(c, h, H);
-  const size_t tmp = size_t(B) * h * W * 3;
+  const int C = c->bands();
+  const size_t tmp = size_t(B) * h * W * C;
   if (tmp > c->bic_tmp_bytes) {
     cudaFree(c->d_bic_tmp);
     c->d_bic_tmp = nullptr;
@@ -2056,9 +2072,9 @@ int fdsr_bicubic_u8(fdsr_ctx* c, const uint8_t* lr, int32_t B, int32_t h, int32_
   }
   const int64_t n1 = int64_t(B) * h * W, n2 = int64_t(B) * H * W;
   bicubic_h_kernel<<<unsigned((n1 + 255) / 256), 256, 0, st>>>(lr, c->d_bic_tmp, th->d_min, th->d_cnt, th->d_taps,
-                                                            th->ksize, B, h, w, W);
+                                                            th->ksize, B, h, w, W, C);
   bicubic_v_kernel<<<unsigned((n2 + 255) / 256), 256, 0, st>>>(c->d_bic_tmp, out_u8, cond, tv->d_min, tv->d_cnt,
-                                                            tv->d_taps, tv->ksize, B, h, H, W);
+                                                            tv->d_taps, tv->ksize, B, h, H, W, C);
   CUDA_TRY(c, cudaGetLastError());
   c->launches += 2;
   return FDSR_OK;
@@ -2077,7 +2093,8 @@ int fdsr_super_resolve_u8_submit(fdsr_ctx* c, int32_t slot, const uint8_t* lr_ho
     CUDA_TRY(c, cudaEventCreateWithFlags(&sl.computed, cudaEventDisableTiming));
     CUDA_TRY(c, cudaEventCreateWithFlags(&sl.copied, cudaEventDisableTiming));
   }
-  const size_t in_b = size_t(B) * h * w * 3, out_b = size_t(B) * 3 * H * W * 4, in_a = align_up(in_b, 256);
+  const size_t in_b = size_t(B) * h * w * c->bands(), out_b = size_t(B) * c->bands() * H * W * 4,
+               in_a = align_up(in_b, 256);
   const size_t need_pin = in_a + out_b + 256, need_dev = in_a + 2 * out_b + 256;
   if (need_pin > sl.h_pin_bytes) {
     if (sl.h_pin) cudaFreeHost(sl.h_pin);
@@ -2148,7 +2165,7 @@ int fdsr_sse_u8(fdsr_ctx* c, const float* a, const float* b, int32_t B, int32_t 
   if (!c || !a || !b || !sse) return fail(c, FDSR_E_INVALID, "null argument");
   cudaStream_t st = static_cast<cudaStream_t>(stream);
   CUDA_TRY(c, cudaMemsetAsync(sse, 0, size_t(B) * 8, st));
-  const int64_t per = int64_t(3) * H * W;
+  const int64_t per = int64_t(c->bands()) * H * W;
   int gx = int((per + 256 * 8 - 1) / (256 * 8));
   sse_u8_kernel<<<dim3(gx > 0 ? gx : 1, B), 256, 0, st>>>(a, b, sse, per);
   CUDA_TRY(c, cudaGetLastError());
@@ -2167,9 +2184,10 @@ int fdsr_metrics_u8(fdsr_ctx* c, const float* a, const float* b, int32_t B, int3
     c->metric_bytes = size_t(B) * 32;
   }
   CUDA_TRY(c, cudaMemsetAsync(c->d_metric, 0, size_t(B) * 32, st));
-  metrics_u8_kernel<<<dim3((W + kSsimTile - 1) / kSsimTile, (H + kSsimTile - 1) / kSsimTile, B * 3), 256, 0, st>>>(
-      a, b, c->d_metric, H, W);
-  metrics_finalize_kernel<<<(B + 127) / 128, 128, 0, st>>>(c->d_metric, out, B, H, W, ergas_scale);
+  const int C = c->bands();
+  metrics_u8_kernel<<<dim3((W + kSsimTile - 1) / kSsimTile, (H + kSsimTile - 1) / kSsimTile, B * C), 256, 0, st>>>(
+      a, b, c->d_metric, H, W, C);
+  metrics_finalize_kernel<<<(B + 127) / 128, 128, 0, st>>>(c->d_metric, out, B, H, W, C, ergas_scale);
   CUDA_TRY(c, cudaGetLastError());
   c->launches += 2;
   return FDSR_OK;
@@ -2364,7 +2382,7 @@ int fdsr_debug_noise(fdsr_ctx* c, float* out, int32_t B, int32_t H, int32_t W, u
   CUDA_TRY(c, cudaMallocAsync(reinterpret_cast<void**>(&slot), sizeof(SampleArgs), st));
   set_args_kernel<<<1, 1, 0, st>>>(slot, SampleArgs{seed, first_image, nullptr, nullptr});
   const uint32_t hw = uint32_t(H) * uint32_t(W);
-  noise_init_kernel<<<dim3((hw + 255) / 256, B), 256, 0, st>>>(out, hw, slot, uint32_t(stream_id));
+  noise_init_kernel<<<dim3((hw + 255) / 256, B), 256, 0, st>>>(out, hw, c->bands(), slot, uint32_t(stream_id));
   CUDA_TRY(c, cudaGetLastError());
   CUDA_TRY(c, cudaFreeAsync(slot, st));
   c->launches += 2;

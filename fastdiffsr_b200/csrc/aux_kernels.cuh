@@ -11,9 +11,9 @@ namespace fdsr {
 
 // ------------------------------------------------------------------------------------------
 // Counter-based Gaussian noise: Philox4x32-10 keyed by the seed.  The counter is (PIXEL index inside the image,
-// GLOBAL image index, stream) and one block of four normals serves the three channels of that pixel (the fourth is
-// unused), so the thread that owns a pixel — in particular the final conv's epilogue thread, which performs the
-// posterior update in registers — needs exactly one Philox evaluation.  The noise of an image depends on the seed, the
+// GLOBAL image index, stream) and one block of four normals serves up to four channels of that pixel (a second block
+// serves channels 4-7, philox_pixel_normals), so the thread that owns a pixel — in particular the final conv's epilogue
+// thread, which performs the posterior update in registers — needs one Philox evaluation for C <= 4.  The noise of an image depends on the seed, the
 // image's index in the whole job and the step only — not on the batch it happens to be sampled in, nor on which rank
 // samples it — so a batch sharded over N ranks reproduces the single-rank result bit for bit.
 // Streams: T for x_T, t for the z of step t.
@@ -22,28 +22,28 @@ namespace fdsr {
 // ------------------------------------------------------------------------------------------
 __global__ void set_args_kernel(SampleArgs* slot, SampleArgs a) { *slot = a; }
 
-// x_T: the first (B,3,H,W) block of the injected noise, or stream T of the generator.  grid (HW / 256, B), thread = pixel
-__global__ void noise_init_kernel(float* __restrict__ out, uint32_t HW, const SampleArgs* __restrict__ args,
+// x_T: the first (B,C,H,W) block of the injected noise, or stream T of the generator.  grid (HW / 256, B), thread = pixel
+__global__ void noise_init_kernel(float* __restrict__ out, uint32_t HW, int C, const SampleArgs* __restrict__ args,
                                   uint32_t stream) {
   const uint32_t p = blockIdx.x * blockDim.x + threadIdx.x;
   if (p >= HW) return;
-  const size_t o = size_t(blockIdx.y) * 3 * HW + p;
+  const size_t o = size_t(blockIdx.y) * C * HW + p;
   const float* nz = args->noise;
+  float z[8];
   if (nz != nullptr) {
-    out[o] = nz[o];
-    out[o + HW] = nz[o + HW];
-    out[o + 2 * size_t(HW)] = nz[o + 2 * size_t(HW)];
+#pragma unroll
+    for (int c = 0; c < 8; ++c) z[c] = c < C ? nz[o + size_t(c) * HW] : 0.f;
   } else {
-    const float4 z = philox_normal4(args->seed, stream, args->image0 + blockIdx.y, p);
-    out[o] = z.x;
-    out[o + HW] = z.y;
-    out[o + 2 * size_t(HW)] = z.z;
+    philox_pixel_normals(z, C, args->seed, stream, args->image0 + blockIdx.y, p);
   }
+#pragma unroll
+  for (int c = 0; c < 8; ++c)
+    if (c < C) out[o + size_t(c) * HW] = z[c];
 }
 
 // ------------------------------------------------------------------------------------------
 // Input assembly: cat([cond, x_t], 1) (diffusion.py:173) as a 16-channel NHWC 16-bit tensor
-// (channels 0-2 cond, 3-5 x_t, 6-15 zero) feeding the stem conv as a single 16-wide K chunk.
+// (layout below) feeding the stem conv as a single 16-wide K chunk.
 // ------------------------------------------------------------------------------------------
 // Two consecutive channels of an activation tensor (16-bit packed pair, or two floats in fp32 mode)
 template <typename T>
@@ -57,40 +57,52 @@ __device__ __forceinline__ void st_pair(T* p, float a, float b) {
   else *reinterpret_cast<uint32_t*>(p) = Cvt<T>::pack(a, b);
 }
 
-// Channel order of the packed input: [x0 x1 x2 0 | c0 c1 c2 0 | 0 ...] (x_t first, so that the fused posterior
-// epilogue of the final conv rewrites it with one aligned 8-byte store per pixel); the stem weights are packed with
-// the matching permutation of the reference's cat([cond, x]) order (kXinPerm in api.cu).
-// One pixel of the packed input from the three x / cond channels at xp[0], xp[plane], xp[2 plane] (likewise cp);
-// shared with the tiled sampler's tile_pack_kernel, whose one-tile result must equal fdsr_sample's bit for bit.
+// Channel order of the packed input for C bands, P = 4 if C <= 4 else 8: x_t in channels [0, C), cond in [P, P + C),
+// every other channel 0 — for C = 3 [x0 x1 x2 0 | c0 c1 c2 0 | 0 x 8].  x_t comes first so that the fused posterior
+// epilogue of the final conv rewrites it with one aligned store per pixel (8 bytes for P = 4, 16 for P = 8); the stem
+// weights are packed with the matching permutation of the reference's cat([cond, x]) order (stem.perm in api.cu).
+// One pixel of the packed input from the C x / cond channels at xp[c plane] (likewise cp); shared with the tiled
+// sampler's tile_pack_kernel, whose one-tile result must equal fdsr_sample's bit for bit.
 template <typename T>
 __device__ __forceinline__ void pack_pixel(T* __restrict__ out, const float* __restrict__ xp,
-                                           const float* __restrict__ cp, int64_t plane) {
+                                           const float* __restrict__ cp, int64_t plane, int C) {
+  float xv[8], cv[8];
+#pragma unroll
+  for (int c = 0; c < 8; ++c) {
+    xv[c] = c < C ? xp[c * plane] : 0.f;
+    cv[c] = c < C ? cp[c * plane] : 0.f;
+  }
   if constexpr (sizeof(T) == 4) {
     float4* o = reinterpret_cast<float4*>(out);
-    o[0] = make_float4(xp[0], xp[plane], xp[2 * plane], 0.f);
-    o[1] = make_float4(cp[0], cp[plane], cp[2 * plane], 0.f);
-    o[2] = make_float4(0.f, 0.f, 0.f, 0.f);
-    o[3] = make_float4(0.f, 0.f, 0.f, 0.f);
+    const float4 z4 = make_float4(0.f, 0.f, 0.f, 0.f);
+    o[0] = make_float4(xv[0], xv[1], xv[2], xv[3]);
+    o[1] = C <= 4 ? make_float4(cv[0], cv[1], cv[2], cv[3]) : make_float4(xv[4], xv[5], xv[6], xv[7]);
+    o[2] = C <= 4 ? z4 : make_float4(cv[0], cv[1], cv[2], cv[3]);
+    o[3] = C <= 4 ? z4 : make_float4(cv[4], cv[5], cv[6], cv[7]);
   } else {
-    uint4 lo, hi = make_uint4(0u, 0u, 0u, 0u);
-    lo.x = Cvt<T>::pack(xp[0], xp[plane]);
-    lo.y = Cvt<T>::pack(xp[2 * plane], 0.f);
-    lo.z = Cvt<T>::pack(cp[0], cp[plane]);
-    lo.w = Cvt<T>::pack(cp[2 * plane], 0.f);
+    const uint4 xs = make_uint4(Cvt<T>::pack(xv[0], xv[1]), Cvt<T>::pack(xv[2], xv[3]), Cvt<T>::pack(xv[4], xv[5]),
+                                Cvt<T>::pack(xv[6], xv[7]));
+    const uint4 cs = make_uint4(Cvt<T>::pack(cv[0], cv[1]), Cvt<T>::pack(cv[2], cv[3]), Cvt<T>::pack(cv[4], cv[5]),
+                                Cvt<T>::pack(cv[6], cv[7]));
     uint4* o = reinterpret_cast<uint4*>(out);
-    o[0] = lo;
-    o[1] = hi;
+    if (C <= 4) {
+      o[0] = make_uint4(xs.x, xs.y, cs.x, cs.y);
+      o[1] = make_uint4(0u, 0u, 0u, 0u);
+    } else {
+      o[0] = xs;
+      o[1] = cs;
+    }
   }
 }
 
 template <typename T>
 __global__ void pack_input_kernel(const float* __restrict__ cond, const float* __restrict__ x,
-                                  T* __restrict__ out, int B, int HW) {
+                                  T* __restrict__ out, int B, int HW, int C) {
   const int64_t i = blockIdx.x * int64_t(blockDim.x) + threadIdx.x;
   if (i >= int64_t(B) * HW) return;
   const int b = int(i / HW);
   const int p = int(i - int64_t(b) * HW);
-  pack_pixel<T>(out + i * 16, x + int64_t(b) * 3 * HW + p, cond + int64_t(b) * 3 * HW + p, HW);
+  pack_pixel<T>(out + i * 16, x + int64_t(b) * C * HW + p, cond + int64_t(b) * C * HW + p, HW, C);
 }
 
 // ------------------------------------------------------------------------------------------
@@ -99,31 +111,30 @@ __global__ void pack_input_kernel(const float* __restrict__ cond, const float* _
 //   x0 = clamp(a*x - b*eps, -1, 1);  mean = c1*x0 + c2*x;  x_prev = mean + z*sigma
 // z comes from `z` (injected) or from the Philox stream when z == nullptr and seed != nullptr.
 // ------------------------------------------------------------------------------------------
-// grid (HW / 256, B), thread = pixel (3 channels).  z: explicit tensor (fdsr_posterior_step), else block `z_block` of
+// grid (HW / 256, B), thread = pixel (C channels).  z: explicit tensor (fdsr_posterior_step), else block `z_block` of
 // args->noise, else the generator's stream `stream`; add_noise = 0 (t == 0): z = 0.
 __global__ void posterior_kernel(const float* __restrict__ x, const float* __restrict__ eps,
-                                 const float* __restrict__ z, float* __restrict__ out, uint32_t HW,
+                                 const float* __restrict__ z, float* __restrict__ out, uint32_t HW, int C,
                                  PostCoef k, const SampleArgs* __restrict__ args, int64_t z_block, uint32_t stream,
                                  int add_noise) {
   const uint32_t p = blockIdx.x * blockDim.x + threadIdx.x;
   if (p >= HW) return;
-  const size_t o = size_t(blockIdx.y) * 3 * HW + p;
-  float zv[3] = {0.f, 0.f, 0.f};
+  const size_t o = size_t(blockIdx.y) * C * HW + p;
+  float zv[8] = {0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f};
   if (add_noise) {
     const float* nz = z != nullptr ? z : (args != nullptr && args->noise != nullptr
-                                              ? args->noise + size_t(z_block) * gridDim.y * 3 * HW : nullptr);
+                                              ? args->noise + size_t(z_block) * gridDim.y * C * HW : nullptr);
     if (nz != nullptr) {
 #pragma unroll
-      for (int c = 0; c < 3; ++c) zv[c] = nz[o + size_t(c) * HW];
+      for (int c = 0; c < 8; ++c)
+        if (c < C) zv[c] = nz[o + size_t(c) * HW];
     } else if (args != nullptr) {
-      const float4 r = philox_normal4(args->seed, stream, args->image0 + blockIdx.y, p);
-      zv[0] = r.x;
-      zv[1] = r.y;
-      zv[2] = r.z;
+      philox_pixel_normals(zv, C, args->seed, stream, args->image0 + blockIdx.y, p);
     }
   }
 #pragma unroll
-  for (int c = 0; c < 3; ++c) out[o + size_t(c) * HW] = post1(x[o + size_t(c) * HW], eps[o + size_t(c) * HW], zv[c], k);
+  for (int c = 0; c < 8; ++c)
+    if (c < C) out[o + size_t(c) * HW] = post1(x[o + size_t(c) * HW], eps[o + size_t(c) * HW], zv[c], k);
 }
 
 // res2img (diffusion.py:275-281): clamp(x,-1,1)/2 + cond.  `out` rows may be strided per sample
@@ -288,63 +299,61 @@ __global__ void slam_apply_kernel(const T* __restrict__ x, const float* __restri
 // point taps, uint8 rounding + clipping after each pass.  bounds/taps are built on the host.
 // ------------------------------------------------------------------------------------------
 constexpr int kBicPrec = 22;
-// in: [B][inH][inW][3] u8 -> out: [B][inH][outW][3] u8
+// C <= 8 bands, each resized on its own exactly as Pillow resizes one 8-bit band.
+// in: [B][inH][inW][C] u8 -> out: [B][inH][outW][C] u8
 __global__ void bicubic_h_kernel(const uint8_t* __restrict__ in, uint8_t* __restrict__ out,
                                  const int* __restrict__ xmin, const int* __restrict__ xcnt,
-                                 const int* __restrict__ taps, int ksize, int B, int inH, int inW, int outW) {
+                                 const int* __restrict__ taps, int ksize, int B, int inH, int inW, int outW, int C) {
   const int64_t i = blockIdx.x * int64_t(blockDim.x) + threadIdx.x;
   const int64_t total = int64_t(B) * inH * outW;
   if (i >= total) return;
   const int xo = int(i % outW);
   const int64_t row = i / outW;
-  const uint8_t* src = in + (row * inW + xmin[xo]) * 3;
+  const uint8_t* src = in + (row * inW + xmin[xo]) * C;
   const int* k = taps + xo * ksize;
-  int a0 = 1 << (kBicPrec - 1), a1 = a0, a2 = a0;
-  for (int j = 0; j < xcnt[xo]; ++j) {
-    a0 += int(src[3 * j]) * k[j];
-    a1 += int(src[3 * j + 1]) * k[j];
-    a2 += int(src[3 * j + 2]) * k[j];
-  }
-  uint8_t* o = out + i * 3;
-  o[0] = uint8_t(min(max(a0 >> kBicPrec, 0), 255));
-  o[1] = uint8_t(min(max(a1 >> kBicPrec, 0), 255));
-  o[2] = uint8_t(min(max(a2 >> kBicPrec, 0), 255));
+  int a[8];
+#pragma unroll
+  for (int c = 0; c < 8; ++c) a[c] = 1 << (kBicPrec - 1);
+  for (int j = 0; j < xcnt[xo]; ++j)
+#pragma unroll
+    for (int c = 0; c < 8; ++c)
+      if (c < C) a[c] += int(src[C * j + c]) * k[j];
+  uint8_t* o = out + i * C;
+#pragma unroll
+  for (int c = 0; c < 8; ++c)
+    if (c < C) o[c] = uint8_t(min(max(a[c] >> kBicPrec, 0), 255));
 }
-// in: [B][inH][W][3] u8 -> out_u8: [B][outH][W][3] (optional), cond: [B][3][outH][W] fp32 (optional)
+// in: [B][inH][W][C] u8 -> out_u8: [B][outH][W][C] (optional), cond: [B][C][outH][W] fp32 (optional)
 __global__ void bicubic_v_kernel(const uint8_t* __restrict__ in, uint8_t* __restrict__ out_u8,
                                  float* __restrict__ cond, const int* __restrict__ ymin,
                                  const int* __restrict__ ycnt, const int* __restrict__ taps, int ksize,
-                                 int B, int inH, int outH, int W) {
+                                 int B, int inH, int outH, int W, int C) {
   const int64_t i = blockIdx.x * int64_t(blockDim.x) + threadIdx.x;
   const int64_t total = int64_t(B) * outH * W;
   if (i >= total) return;
   const int x = int(i % W);
   const int yo = int((i / W) % outH);
   const int b = int(i / (int64_t(W) * outH));
-  const uint8_t* src = in + ((int64_t(b) * inH + ymin[yo]) * W + x) * 3;
+  const uint8_t* src = in + ((int64_t(b) * inH + ymin[yo]) * W + x) * C;
   const int* k = taps + yo * ksize;
-  int a0 = 1 << (kBicPrec - 1), a1 = a0, a2 = a0;
+  int a[8];
+#pragma unroll
+  for (int c = 0; c < 8; ++c) a[c] = 1 << (kBicPrec - 1);
   for (int j = 0; j < ycnt[yo]; ++j) {
-    const uint8_t* s = src + int64_t(j) * W * 3;
-    a0 += int(s[0]) * k[j];
-    a1 += int(s[1]) * k[j];
-    a2 += int(s[2]) * k[j];
+    const uint8_t* s = src + int64_t(j) * W * C;
+#pragma unroll
+    for (int c = 0; c < 8; ++c)
+      if (c < C) a[c] += int(s[c]) * k[j];
   }
-  const int v0 = min(max(a0 >> kBicPrec, 0), 255), v1 = min(max(a1 >> kBicPrec, 0), 255),
-            v2 = min(max(a2 >> kBicPrec, 0), 255);
-  if (out_u8 != nullptr) {
-    uint8_t* o = out_u8 + i * 3;
-    o[0] = uint8_t(v0);
-    o[1] = uint8_t(v1);
-    o[2] = uint8_t(v2);
-  }
-  if (cond != nullptr) {
+  const int64_t plane = int64_t(outH) * W;
+  float* cp = cond != nullptr ? cond + int64_t(b) * C * plane + int64_t(yo) * W + x : nullptr;
+#pragma unroll
+  for (int c = 0; c < 8; ++c) {
+    if (c >= C) continue;
+    const int v = min(max(a[c] >> kBicPrec, 0), 255);
+    if (out_u8 != nullptr) out_u8[i * C + c] = uint8_t(v);
     // ToTensor (/255) then *2-1 (data/util.py:66-75), fp32, same operation order
-    const int64_t plane = int64_t(outH) * W;
-    float* c = cond + int64_t(b) * 3 * plane + int64_t(yo) * W + x;
-    c[0] = __fsub_rn(__fmul_rn(__fdiv_rn(float(v0), 255.0f), 2.0f), 1.0f);
-    c[plane] = __fsub_rn(__fmul_rn(__fdiv_rn(float(v1), 255.0f), 2.0f), 1.0f);
-    c[2 * plane] = __fsub_rn(__fmul_rn(__fdiv_rn(float(v2), 255.0f), 2.0f), 1.0f);
+    if (cp != nullptr) cp[c * plane] = __fsub_rn(__fmul_rn(__fdiv_rn(float(v), 255.0f), 2.0f), 1.0f);
   }
 }
 
@@ -375,7 +384,7 @@ __global__ void sse_u8_kernel(const float* __restrict__ a, const float* __restri
 // Evaluation metrics of sr_mfe.py:315-345 on tensor2img-quantised uint8 images, per image:
 //   acc[b][0] = sum (a-b)^2            (compare_mse / compare_psnr / calculate_ergas)
 //   acc[b][1] = sum a                  (calculate_ergas: mean of the first image)
-//   acc[b][2] = sum of the SSIM map over the cropped interior and the 3 channels, 2^-40 fixed point
+//   acc[b][2] = sum of the SSIM map over the cropped interior and the C channels, 2^-40 fixed point
 // SSIM follows skimage.measure.compare_ssim(X, Y, multichannel=True) as the reference calls it
 // (scikit-image 0.15, _structural_similarity.py): 7x7 uniform window, K1 = 0.01, K2 = 0.03,
 // data_range = 255, sample covariance (x 49/48), float64, mean over the map cropped by 3 pixels per
@@ -385,12 +394,12 @@ constexpr int kSsimWin = 7, kSsimPad = 3, kSsimTile = 16;
 constexpr double kSsimScale = 1099511627776.0;  // 2^40
 
 __global__ void __launch_bounds__(256) metrics_u8_kernel(const float* __restrict__ a, const float* __restrict__ b,
-                                                         unsigned long long* __restrict__ acc, int H, int W) {
+                                                         unsigned long long* __restrict__ acc, int H, int W, int C) {
   __shared__ uint8_t sa[kSsimTile + 6][kSsimTile + 6 + 2], sb[kSsimTile + 6][kSsimTile + 6 + 2];
   __shared__ long long red[8][3];
-  const int img = blockIdx.z / 3, ch = blockIdx.z % 3;
-  const float* ap = a + (int64_t(img) * 3 + ch) * H * W;
-  const float* bp = b + (int64_t(img) * 3 + ch) * H * W;
+  const int img = blockIdx.z / C, ch = blockIdx.z % C;  // grid z = B * C
+  const float* ap = a + (int64_t(img) * C + ch) * H * W;
+  const float* bp = b + (int64_t(img) * C + ch) * H * W;
   // the block owns the 16x16 pixels at (y0, x0); its SSIM windows need a 3-pixel apron
   const int y0 = blockIdx.y * kSsimTile, x0 = blockIdx.x * kSsimTile;
   for (int e = threadIdx.x; e < (kSsimTile + 6) * (kSsimTile + 6); e += 256) {
@@ -448,21 +457,22 @@ __global__ void __launch_bounds__(256) metrics_u8_kernel(const float* __restrict
   }
 }
 
-// out[b] = (mse, psnr, ssim, ergas) in float64, exactly as sr_mfe.py derives them from the sums
+// out[b] = (mse, psnr, ssim, ergas) in float64, exactly as sr_mfe.py derives them from the sums (C bands: n = C H W,
+// SSIM averaged over the C channels, ERGAS divided by C)
 __global__ void metrics_finalize_kernel(const unsigned long long* __restrict__ acc, double* __restrict__ out, int B,
-                                        int H, int W, double scale) {
+                                        int H, int W, int C, double scale) {
   const int b = blockIdx.x * blockDim.x + threadIdx.x;
   if (b >= B) return;
-  const double n = 3.0 * H * W;
+  const double n = double(C) * H * W;
   const double sse = double(static_cast<long long>(acc[b * 4 + 0]));
   const double mean = double(static_cast<long long>(acc[b * 4 + 1])) / n;
   const double mse = sse / n;
-  const double nss = 3.0 * double(H - 2 * kSsimPad) * double(W - 2 * kSsimPad);
+  const double nss = double(C) * double(H - 2 * kSsimPad) * double(W - 2 * kSsimPad);
   out[b * 4 + 0] = mse;
   out[b * 4 + 1] = mse > 0.0 ? 10.0 * log10(255.0 * 255.0 / mse) : INFINITY;
   out[b * 4 + 2] = (H > 2 * kSsimPad && W > 2 * kSsimPad)
                        ? double(static_cast<long long>(acc[b * 4 + 2])) / kSsimScale / nss : NAN;
-  out[b * 4 + 3] = 100.0 * sqrt(mse / (mean * mean) / 3.0) / scale;
+  out[b * 4 + 3] = 100.0 * sqrt(mse / (mean * mean) / double(C)) / scale;
 }
 
 // NHWC 16-bit -> NCHW fp32 (debug hook only)

@@ -53,8 +53,8 @@ enum OutMode : int32_t {
 struct SampleArgs {
   uint64_t seed;         // Philox key
   uint64_t image0;       // global index of the first image of this batch
-  const float* noise;    // (T,B,3,H,W) injected noise, or null: built-in generator
-  float* trace;          // (B, frames, 3, H, W), or null
+  const float* noise;    // (T,B,C,H,W) injected noise, or null: built-in generator
+  float* trace;          // (B, frames, C, H, W), or null
 };
 // posterior coefficients of one step (diffusion.py:140-155 tables as fp32, like the reference's registered buffers)
 struct PostCoef {
@@ -147,8 +147,8 @@ struct ConvLayer {
   int32_t group;           // tiles per assignment group (divides tiles_x * tiles_y)
   // kOutPosterior
   const PostStep* post;    // [T]
-  float* x_state;          // fp32 NCHW (B,3,H,W): x_t in, x_{t-1} out (in place)
-  void* xin;               // 16-bit NHWC16 network input: channels 0-2 receive x_{t-1}
+  float* x_state;          // fp32 NCHW (B,out_c,H,W): x_t in, x_{t-1} out (in place)
+  void* xin;               // 16-bit NHWC16 network input: channels [0, out_c) receive x_{t-1} (pack_pixel's layout)
   const SampleArgs* args;
   unsigned int* flags;     // context status word: bit 0 = an fp16 activation store saturated (overflow)
   long long* prof;         // role cycle counters [grid][5 roles][8 slots] (FDSR_PROFILE builds only)

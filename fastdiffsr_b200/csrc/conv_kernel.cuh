@@ -1254,44 +1254,46 @@ conv_gemm_kernel(const __grid_constant__ ConvLayer L, int t_step) {
           }
           PROF_MARK(7);
         } else if (L.out_mode == kOutPosterior) {
-          // final conv inside the sampler: this thread holds eps of one pixel (3 channels).  p_sample in registers:
-          // x0 = clamp(a x - b eps), mean, + sigma z (z injected or one Philox block keyed by the pixel), fp32 state
+          // final conv inside the sampler: this thread holds eps of one pixel (C = out_c <= 8 channels).  p_sample in
+          // registers: x0 = clamp(a x - b eps), mean, + sigma z (z injected or the pixel's Philox blocks), fp32 state
           // updated in place, and the next step's network input rewritten — diffusion.py:157-190, 173
           if (valid && cb == 0) {
             const PostStep ps = L.post[t_step];
-            const size_t HWs = size_t(H) * W, o0 = (size_t(b) * 3 * H + y) * W + x;
-            float zv[3] = {0.f, 0.f, 0.f};
+            const int C = L.out_c;
+            const size_t HWs = size_t(H) * W, o0 = (size_t(b) * C * H + y) * W + x;
+            float zv[8] = {0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f};
             if (ps.add_noise) {
               const float* nz = L.args->noise;
               if (nz != nullptr) {
-                nz += size_t(ps.z_block) * L.B * 3 * HWs;
+                nz += size_t(ps.z_block) * L.B * C * HWs;
 #pragma unroll
-                for (int c = 0; c < 3; ++c) zv[c] = nz[o0 + c * HWs];
+                for (int c = 0; c < 8; ++c)
+                  if (c < C) zv[c] = nz[o0 + c * HWs];
               } else {
-                const float4 r4 = philox_normal4(L.args->seed, uint32_t(t_step), L.args->image0 + b, uint32_t(y * W + x));
-                zv[0] = r4.x;
-                zv[1] = r4.y;
-                zv[2] = r4.z;
+                philox_pixel_normals(zv, C, L.args->seed, uint32_t(t_step), L.args->image0 + b, uint32_t(y * W + x));
               }
             }
-            float xp[3];
+            float xp[8];
 #pragma unroll
-            for (int c = 0; c < 3; ++c) {
-              xp[c] = post1(L.x_state[o0 + c * HWs], v[c], zv[c], ps.k);
-              L.x_state[o0 + c * HWs] = xp[c];
+            for (int c = 0; c < 8; ++c) {
+              xp[c] = 0.f;
+              if (c < C) {
+                xp[c] = post1(L.x_state[o0 + c * HWs], v[c], zv[c], ps.k);
+                L.x_state[o0 + c * HWs] = xp[c];
+              }
             }
-            if constexpr (sizeof(T) == 2) {   // channels [x0 x1 x2 0] of the packed input (pack_input_kernel's layout)
-              uint2 w;
-              w.x = Cvt<T>::pack(xp[0], xp[1]);
-              w.y = Cvt<T>::pack(xp[2], 0.f);
-              *reinterpret_cast<uint2*>(reinterpret_cast<T*>(L.xin) + (size_t(b) * HWs + size_t(y) * W + x) * 16) = w;
+            if constexpr (sizeof(T) == 2) {   // channels [0, P) of the packed input (pack_pixel's layout): x_t, then 0
+              T* dst = reinterpret_cast<T*>(L.xin) + (size_t(b) * HWs + size_t(y) * W + x) * 16;
+              const uint32_t w0 = Cvt<T>::pack(xp[0], xp[1]), w1 = Cvt<T>::pack(xp[2], xp[3]);
+              if (C <= 4) *reinterpret_cast<uint2*>(dst) = make_uint2(w0, w1);
+              else *reinterpret_cast<uint4*>(dst) = make_uint4(w0, w1, Cvt<T>::pack(xp[4], xp[5]), Cvt<T>::pack(xp[6], xp[7]));
             }
           }
         } else {  // fp32 NCHW, first out_c channels (final conv -> eps)
           if (valid && cb == 0) {
             float* o = reinterpret_cast<float*>(L.out);
 #pragma unroll
-            for (int c = 0; c < 4; ++c)
+            for (int c = 0; c < 8; ++c)
               if (c < L.out_c) o[((size_t(b) * L.out_c + c) * H + y) * W + x] = v[c];
           }
         }

@@ -42,12 +42,12 @@ __device__ __forceinline__ TileCover tile_cover(const TileAxis& a, int y) {
   return c;
 }
 
-// Packed 16-channel NHWC network input of one chunk of `bc` tiles ([x (3) 0 | cond (3) 0 | 0 x 8], pack_pixel), read
+// Packed 16-channel NHWC network input of one chunk of `bc` tiles (x_t and cond of C bands, pack_pixel), read
 // from the canvases at each tile's window.  Chunk slot j holds global tile min(tile0 + j, n_tiles - 1): the last chunk
 // is padded with repeats of the last tile.  One thread per tile pixel.
 template <typename T>
 __global__ void tile_pack_kernel(const float* __restrict__ cond, const float* __restrict__ x, T* __restrict__ out,
-                                 TileAxis ay, TileAxis ax, int64_t tile0, int64_t n_tiles, int bc) {
+                                 TileAxis ay, TileAxis ax, int64_t tile0, int64_t n_tiles, int bc, int C) {
   const int64_t i = blockIdx.x * int64_t(blockDim.x) + threadIdx.x;
   const int64_t tpx = int64_t(ay.te) * ax.te;
   if (i >= bc * tpx) return;
@@ -60,17 +60,17 @@ __global__ void tile_pack_kernel(const float* __restrict__ cond, const float* __
   const int py = p / ax.te, px = p - py * ax.te;
   const int y = tile_start(ay, r / ax.n) + py, xx = tile_start(ax, r % ax.n) + px;
   const int64_t plane = int64_t(ay.L) * ax.L;
-  const int64_t o = b * 3 * plane + int64_t(y) * ax.L + xx;
-  pack_pixel<T>(out + i * 16, x + o, cond + o, plane);
+  const int64_t o = b * C * plane + int64_t(y) * ax.L + xx;
+  pack_pixel<T>(out + i * 16, x + o, cond + o, plane, C);
 }
 
 // One step on every canvas: eps of each pixel = the normalised-weight blend of the eps of the tiles covering it (global
 // tile order, fp32, round-to-nearest, the sum starting from the first term so that a pixel covered once gets its tile's
 // eps exactly), then x_{t-1} = post1(x_t, eps, z) in place.  z: block z_block of args->noise, else the generator's
 // stream `stream` at (image0 + canvas, pixel index y*W + x); add_noise = 0 (t == 0): z = 0.  No atomics: each thread
-// owns its pixel.  grid (ceil(H W / 256), B); eps_store: [tile][3][te_y][te_x].
+// owns its pixel.  grid (ceil(H W / 256), B); x: (B,C,H,W); eps_store: [tile][C][te_y][te_x].
 __global__ void tile_blend_posterior_kernel(float* __restrict__ x, const float* __restrict__ eps_store, TileAxis ay,
-                                            TileAxis ax, PostCoef k, const SampleArgs* __restrict__ args,
+                                            TileAxis ax, int C, PostCoef k, const SampleArgs* __restrict__ args,
                                             int64_t z_block, uint32_t stream, int add_noise) {
   const uint32_t HW = uint32_t(ay.L) * uint32_t(ax.L);
   const uint32_t p = blockIdx.x * blockDim.x + threadIdx.x;
@@ -88,7 +88,7 @@ __global__ void tile_blend_posterior_kernel(float* __restrict__ x, const float* 
     }
   }
   const int64_t tpx = int64_t(ay.te) * ax.te;
-  float e[3] = {0.f, 0.f, 0.f};
+  float e[8] = {0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f};
   for (int a = 0; a < ny; ++a) {
     const int ty = cy.at(a), oy = y - tile_start(ay, ty);
     const int ry = tile_ramp(ay, oy);
@@ -96,30 +96,30 @@ __global__ void tile_blend_posterior_kernel(float* __restrict__ x, const float* 
       const int tx = cx.at(c), ox = xx - tile_start(ax, tx);
       const float nk = __fdiv_rn(float(ry * tile_ramp(ax, ox)), wsum);
       const int64_t g = (int64_t(b) * ay.n + ty) * ax.n + tx;
-      const float* ep = eps_store + g * 3 * tpx + int64_t(oy) * ax.te + ox;
+      const float* ep = eps_store + g * C * tpx + int64_t(oy) * ax.te + ox;
 #pragma unroll
-      for (int ch = 0; ch < 3; ++ch) {
+      for (int ch = 0; ch < 8; ++ch) {
+        if (ch >= C) continue;
         const float term = __fmul_rn(nk, ep[ch * tpx]);
         e[ch] = (a | c) ? __fadd_rn(e[ch], term) : term;
       }
     }
   }
-  const size_t o = size_t(b) * 3 * HW + p;
-  float zv[3] = {0.f, 0.f, 0.f};
+  const size_t o = size_t(b) * C * HW + p;
+  float zv[8] = {0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f};
   if (add_noise) {
     if (args->noise != nullptr) {
-      const float* nz = args->noise + size_t(z_block) * gridDim.y * 3 * HW;
+      const float* nz = args->noise + size_t(z_block) * gridDim.y * C * HW;
 #pragma unroll
-      for (int ch = 0; ch < 3; ++ch) zv[ch] = nz[o + size_t(ch) * HW];
+      for (int ch = 0; ch < 8; ++ch)
+        if (ch < C) zv[ch] = nz[o + size_t(ch) * HW];
     } else {
-      const float4 r = philox_normal4(args->seed, stream, args->image0 + b, p);
-      zv[0] = r.x;
-      zv[1] = r.y;
-      zv[2] = r.z;
+      philox_pixel_normals(zv, C, args->seed, stream, args->image0 + b, p);
     }
   }
 #pragma unroll
-  for (int ch = 0; ch < 3; ++ch) x[o + size_t(ch) * HW] = post1(x[o + size_t(ch) * HW], e[ch], zv[ch], k);
+  for (int ch = 0; ch < 8; ++ch)
+    if (ch < C) x[o + size_t(ch) * HW] = post1(x[o + size_t(ch) * HW], e[ch], zv[ch], k);
 }
 
 }  // namespace fdsr

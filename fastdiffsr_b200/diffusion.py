@@ -5,15 +5,15 @@ touches: set_loss, set_new_noise_schedule (12 registered fp32 buffers + numpy
 sqrt_alphas_cumprod_prev), super_resolution / p_sample_loop / p_sample, res2img / img2res,
 state_dict compatibility.  Differences, all deliberate (SURVEY.md section 0):
   * super_resolution is batch-safe (the reference crashes for B>1, F2); for B=1 the
-    continous=True layout is identical: (1+frames, 3, H, W);
+    continous=True layout is identical: (1+frames, C, H, W), C = the UNet's out_channel (image bands, 1..8);
   * Gaussian noise may be injected (`noise=`) for parity, else it comes from the library's
     counter-based generator seeded from torch's global RNG (the reference is unseeded, F7);
   * training (`forward` -> p_losses) is out of scope for this path and raises.
 
 The same class serves the SR3 baseline (which_model_G == "ddpm", model/ddpm_modules/diffusion.py:79-298) when
 its denoise_fn is an SR3UNet: the UNet is conditioned on the integer step t (not on a noise level), the image
-itself is predicted (no res2img), and `super_resolution` returns `ret_img[-1]` — for B = 1 the (3,H,W) image
-without the batch axis, exactly as the reference does (ddpm diffusion.py:228-231); B > 1 returns (B,3,H,W).
+itself is predicted (no res2img), and `super_resolution` returns `ret_img[-1]` — for B = 1 the (C,H,W) image
+without the batch axis, exactly as the reference does (ddpm diffusion.py:228-231); B > 1 returns (B,C,H,W).
 """
 from __future__ import annotations
 
@@ -159,7 +159,8 @@ class GaussianDiffusion(nn.Module):
     @torch.no_grad()
     def denoise(self, x_cat, t: int):
         """eps = UNet(cat[cond, x_t], noise_level_t): the reference's denoise_fn call in p_mean_variance."""
-        return self.engine().unet_forward(x_cat[:, :3].contiguous(), x_cat[:, 3:].contiguous(), int(t))
+        c = self.denoise_fn.cfg["out_channel"]
+        return self.engine().unet_forward(x_cat[:, :c].contiguous(), x_cat[:, c:].contiguous(), int(t))
 
     @torch.no_grad()
     def p_sample(self, x, t, clip_denoised=True, condition_x=None, noise=None):
@@ -211,7 +212,7 @@ class GaussianDiffusion(nn.Module):
             return sr[0] if (self.sr3 and sr.shape[0] == 1) else sr  # SR3: ret_img[-1] drops the batch axis
         sr, tr = run(trace=True)
         eng.check_overflow()
-        return tr.reshape(-1, *tr.shape[2:])  # B=1: (1+frames,3,H,W) exactly as the reference
+        return tr.reshape(-1, *tr.shape[2:])  # B=1: (1+frames,C,H,W) exactly as the reference
 
     @torch.no_grad()
     def super_resolution(self, x_in, continous=False, noise=None, seed=None, image_offset=0, *, tile=None,

@@ -49,6 +49,7 @@ class Engine:
                     cfg.attn_levels |= 1 << i
                 res //= 2
         self.dtype = dtype
+        self.C = int(cfg.out_channel)  # image bands: every image tensor is (B,C,H,W), u8 images (B,h,w,C)
         self._h = C.c_void_p()
         with torch.cuda.device(self.device):
             rc = self.lib.fdsr_create(C.byref(cfg), C.byref(self._h))
@@ -117,8 +118,8 @@ class Engine:
 
     # ---- compute
     def _img(self, t, name):
-        if t.device != self.device or t.dtype != torch.float32 or t.dim() != 4 or t.shape[1] != 3:
-            raise FdsrError(f"{name} must be a (B,3,H,W) fp32 tensor on {self.device}")
+        if t.device != self.device or t.dtype != torch.float32 or t.dim() != 4 or t.shape[1] != self.C:
+            raise FdsrError(f"{name} must be a (B,{self.C},H,W) fp32 tensor on {self.device}")
         return t.contiguous()
 
     def unet_forward(self, cond, x_t, t: int):
@@ -149,11 +150,11 @@ class Engine:
         cond = self._img(cond, "cond")
         B, _, H, W = cond.shape
         if noise is not None:
-            if tuple(noise.shape) != (self.T, B, 3, H, W) or noise.dtype != torch.float32 or noise.device != self.device:
-                raise FdsrError(f"noise must be ({self.T},{B},3,{H},{W}) fp32 on {self.device}")
+            if tuple(noise.shape) != (self.T, B, self.C, H, W) or noise.dtype != torch.float32 or noise.device != self.device:
+                raise FdsrError(f"noise must be ({self.T},{B},{self.C},{H},{W}) fp32 on {self.device}")
             noise = noise.contiguous()
         out = torch.empty_like(cond)
-        tr = torch.empty((B, self.trace_frames(), 3, H, W), device=self.device, dtype=torch.float32) if trace else None
+        tr = torch.empty((B, self.trace_frames(), self.C, H, W), device=self.device, dtype=torch.float32) if trace else None
         with torch.cuda.device(self.device):
             self._check(self.lib.fdsr_sample(self._h, _ptr(cond), _ptr(noise), seed, _ptr(out), _ptr(tr), B, H, W,
                                              self._stream()), "fdsr_sample")
@@ -161,7 +162,7 @@ class Engine:
 
     def sample_tiled(self, cond, tile, overlap: int = 32, tile_batch: int = 16, noise=None, seed: int = 0,
                      trace: bool = False, image_offset: int = 0):
-        """T-step sampling of (B,3,H,W) canvases of any size (H, W >= 8) as overlapping tiles blended at every step
+        """T-step sampling of (B,C,H,W) canvases of any size (H, W >= 8) as overlapping tiles blended at every step
         (fdsr_sample_tiled).  `tile`: int or (th, tw), multiples of 8; `tile_batch`: tiles per UNet call (the activation
         workspace scales with it, not with the canvas).  Noise, seed, image_offset and the trace are as in `sample`."""
         th, tw = (tile, tile) if isinstance(tile, int) else (int(tile[0]), int(tile[1]))
@@ -169,11 +170,11 @@ class Engine:
         cond = self._img(cond, "cond")
         B, _, H, W = cond.shape
         if noise is not None:
-            if tuple(noise.shape) != (self.T, B, 3, H, W) or noise.dtype != torch.float32 or noise.device != self.device:
-                raise FdsrError(f"noise must be ({self.T},{B},3,{H},{W}) fp32 on {self.device}")
+            if tuple(noise.shape) != (self.T, B, self.C, H, W) or noise.dtype != torch.float32 or noise.device != self.device:
+                raise FdsrError(f"noise must be ({self.T},{B},{self.C},{H},{W}) fp32 on {self.device}")
             noise = noise.contiguous()
         out = torch.empty_like(cond)
-        tr = torch.empty((B, self.trace_frames(), 3, H, W), device=self.device, dtype=torch.float32) if trace else None
+        tr = torch.empty((B, self.trace_frames(), self.C, H, W), device=self.device, dtype=torch.float32) if trace else None
         with torch.cuda.device(self.device):
             self._check(self.lib.fdsr_sample_tiled(self._h, _ptr(cond), _ptr(noise), seed, _ptr(out), _ptr(tr), B, H, W,
                                                    th, tw, int(overlap), int(tile_batch), self._stream()),
@@ -181,21 +182,21 @@ class Engine:
         return (out, tr) if trace else out
 
     def bicubic_u8(self, lr_u8, H: int, W: int, want_u8=True, want_cond=True):
-        """lr_u8: (B,h,w,3) uint8 on device -> (u8 (B,H,W,3) | None, cond (B,3,H,W) fp32 | None)."""
-        if lr_u8.dtype != torch.uint8 or lr_u8.dim() != 4 or lr_u8.shape[3] != 3 or lr_u8.device != self.device:
-            raise FdsrError("lr must be (B,h,w,3) uint8 on the engine's device")
+        """lr_u8: (B,h,w,C) uint8 on device -> (u8 (B,H,W,C) | None, cond (B,C,H,W) fp32 | None)."""
+        if lr_u8.dtype != torch.uint8 or lr_u8.dim() != 4 or lr_u8.shape[3] != self.C or lr_u8.device != self.device:
+            raise FdsrError(f"lr must be (B,h,w,{self.C}) uint8 on the engine's device")
         lr_u8 = lr_u8.contiguous()
         B, h, w, _ = lr_u8.shape
-        o8 = torch.empty((B, H, W, 3), dtype=torch.uint8, device=self.device) if want_u8 else None
-        oc = torch.empty((B, 3, H, W), dtype=torch.float32, device=self.device) if want_cond else None
+        o8 = torch.empty((B, H, W, self.C), dtype=torch.uint8, device=self.device) if want_u8 else None
+        oc = torch.empty((B, self.C, H, W), dtype=torch.float32, device=self.device) if want_cond else None
         with torch.cuda.device(self.device):
             self._check(self.lib.fdsr_bicubic_u8(self._h, _ptr(lr_u8), B, h, w, H, W, _ptr(o8), _ptr(oc),
                                                  self._stream()), "fdsr_bicubic_u8")
         return o8, oc
 
     def debug_noise(self, B: int, H: int, W: int, seed: int, stream_id: int, image_offset: int = 0):
-        """(B,3,H,W) N(0,1) values of the built-in generator for step stream `stream_id` (T: x_T, t: z of step t)."""
-        out = torch.empty((B, 3, H, W), dtype=torch.float32, device=self.device)
+        """(B,C,H,W) N(0,1) values of the built-in generator for step stream `stream_id` (T: x_T, t: z of step t)."""
+        out = torch.empty((B, self.C, H, W), dtype=torch.float32, device=self.device)
         with torch.cuda.device(self.device):
             self._check(self.lib.fdsr_debug_noise(self._h, _ptr(out), B, H, W, int(seed), int(image_offset),
                                                   int(stream_id), self._stream()), "fdsr_debug_noise")
@@ -204,16 +205,22 @@ class Engine:
     def graph_captures(self):
         return int(self.lib.fdsr_graph_captures(self._h))
 
+    def _host_u8(self, lr_host):
+        lr_host = np.ascontiguousarray(lr_host, dtype=np.uint8)
+        if lr_host.ndim != 4 or lr_host.shape[3] != self.C:
+            raise FdsrError(f"lr must be a (B,h,w,{self.C}) uint8 array")
+        return lr_host
+
     def super_resolve_u8_host(self, lr_host: np.ndarray, H: int, W: int, noise=None, seed: int = 0, out=None,
                               image_offset: int = 0):
-        """Host uint8 (B,h,w,3) -> host fp32 (B,3,H,W): H2D, bicubic, T-step sampling, D2H.
-        `out`: optional caller-owned C-contiguous float32 (B,3,H,W) array to fill (avoids a fresh allocation per call)."""
-        lr_host = np.ascontiguousarray(lr_host, dtype=np.uint8)
+        """Host uint8 (B,h,w,C) -> host fp32 (B,C,H,W): H2D, bicubic, T-step sampling, D2H.
+        `out`: optional caller-owned C-contiguous float32 (B,C,H,W) array to fill (avoids a fresh allocation per call)."""
+        lr_host = self._host_u8(lr_host)
         B, h, w, _ = lr_host.shape
         if out is None:
-            out = np.empty((B, 3, H, W), dtype=np.float32)
-        elif out.shape != (B, 3, H, W) or out.dtype != np.float32 or not out.flags["C_CONTIGUOUS"]:
-            raise FdsrError(f"out must be a C-contiguous float32 array of shape {(B, 3, H, W)}")
+            out = np.empty((B, self.C, H, W), dtype=np.float32)
+        elif out.shape != (B, self.C, H, W) or out.dtype != np.float32 or not out.flags["C_CONTIGUOUS"]:
+            raise FdsrError(f"out must be a C-contiguous float32 array of shape {(B, self.C, H, W)}")
         self._check(self.lib.fdsr_set_image_offset(self._h, int(image_offset)), "fdsr_set_image_offset")
         with torch.cuda.device(self.device):
             self._check(self.lib.fdsr_super_resolve_u8(self._h, lr_host.ctypes.data_as(C.c_void_p), B, h, w, H, W,
@@ -224,14 +231,14 @@ class Engine:
     def super_resolve_u8_submit(self, slot: int, lr_host: np.ndarray, H: int, W: int, noise=None, seed: int = 0,
                                 image_offset: int = 0):
         """Pipelined host path: enqueue one batch into `slot` (0 / 1) and return; see super_resolve_u8_wait."""
-        lr_host = np.ascontiguousarray(lr_host, dtype=np.uint8)
+        lr_host = self._host_u8(lr_host)
         B, h, w, _ = lr_host.shape
         self._check(self.lib.fdsr_set_image_offset(self._h, int(image_offset)), "fdsr_set_image_offset")
         with torch.cuda.device(self.device):
             self._check(self.lib.fdsr_super_resolve_u8_submit(self._h, slot, lr_host.ctypes.data_as(C.c_void_p), B, h, w, H, W,
                                                               _ptr(noise), seed, self._stream()),
                         "fdsr_super_resolve_u8_submit")
-        return (B, 3, H, W)
+        return (B, self.C, H, W)
 
     def super_resolve_u8_wait(self, slot: int, out: np.ndarray):
         """Block until the batch in `slot` is on the host; fills the C-contiguous float32 array `out`."""
@@ -252,7 +259,7 @@ class Engine:
         return out
 
     def metrics_u8(self, a, b, scale: float = 4.0):
-        """Per-image (mse, psnr, ssim, ergas) of `a` (SR or bicubic image) against `b` (HR), both (B,3,H,W) fp32
+        """Per-image (mse, psnr, ssim, ergas) of `a` (SR or bicubic image) against `b` (HR), both (B,C,H,W) fp32
         in [-1,1]: the reference's evaluation block (sr_mfe.py:315-345) on the device.  Returns (B,4) float64."""
         a, b = self._img(a, "a"), self._img(b, "b")
         B, _, H, W = a.shape

@@ -45,10 +45,20 @@ def load_network(netG, opt, logger=None):
 
 
 def _save_u8(img_chw, path):
+    """RGB for 3 bands, a single-band 'L' image for 1, an (H,W,C) uint8 `.npy` array (extension replaced) otherwise.
+    Returns the path written."""
     from PIL import Image
     a = img_chw.detach().float().clamp(-1, 1)
     a = ((a + 1) / 2).permute(1, 2, 0).cpu().numpy()
-    Image.fromarray((a * 255.0).round().astype(np.uint8)).save(path)
+    u8 = (a * 255.0).round().astype(np.uint8)
+    if u8.shape[2] == 3:
+        Image.fromarray(u8).save(path)
+    elif u8.shape[2] == 1:
+        Image.fromarray(u8[:, :, 0]).save(path)  # 2-D uint8: mode L
+    else:
+        path = os.path.splitext(path)[0] + ".npy"
+        np.save(path, u8)
+    return path
 
 
 @torch.no_grad()
@@ -187,7 +197,7 @@ def main(argv=None, default_config="config/sr_fastdiffsr_test_64_256.json", prog
     netG.eval()
     val_opt = opt['datasets']['val']
     from .data import create_dataset
-    val_set = create_dataset(val_opt, 'val')
+    val_set = create_dataset(val_opt, 'val', channels=int(opt['model']['unet']['out_channel']))
     logger.info('Dataset [{:s} - {:s}] is created: {} images.'.format("LRHRDataset", str(val_opt['name']), len(val_set)))
     scale = int(val_opt['r_resolution']) // int(val_opt['l_resolution'])
     result_path = None if args.no_save else (paths.get('results') if isinstance(paths, dict) and paths.get('results') else 'results')

@@ -59,8 +59,8 @@ def psnr_from_sse(sse: torch.Tensor, numel_per_image: int):
 
 @torch.no_grad()
 def sharded_super_resolution(netG, cond_global: torch.Tensor, noise_global=None, seed: int = 0, group=None):
-    """Run netG.super_resolution on this rank's shard of `cond_global` (B,3,H,W) and return the
-    gathered (B,3,H,W) result on every rank.  `noise_global`, if given, is (T,B,3,H,W)."""
+    """Run netG.super_resolution on this rank's shard of `cond_global` (B,C,H,W) and return the
+    gathered (B,C,H,W) result on every rank.  `noise_global`, if given, is (T,B,C,H,W)."""
     rank = dist.get_rank(group) if dist.is_initialized() else 0
     world = dist.get_world_size(group) if dist.is_initialized() else 1
     local, _ = shard_batch(cond_global, rank, world)

@@ -9,7 +9,8 @@
  *     fdsr_last_error() returns a human-readable message for the last failure on that context
  *   - "dev" pointers are CUDA device pointers owned by the caller, valid until the stream work
  *     enqueued by the call has completed; "host" pointers are ordinary host memory
- *   - all image tensors are fp32 NCHW (B,3,H,W), the reference's layout; H and W must be
+ *   - C = out_channel is the number of image bands (1..8; 3 for RGB).  All image tensors are fp32 NCHW
+ *     (B,C,H,W), the reference's layout, and uint8 images are HWC (B,h,w,C); H and W must be
  *     multiples of 2^(n_levels-1): 8 for the FastDiffSR UNet (three stride-2 levels,
  *     model/fastdiffsr_modules/unet.py:77-83), 32 for the SR3 baseline (five)
  *   - calls are asynchronous with respect to the host (enqueue on `stream` and return) unless
@@ -52,8 +53,8 @@ typedef struct fdsr_ctx fdsr_ctx;
 /* UNet hyper-parameters: opt['model']['unet'] consumed by define_G (model/networks.py:82-119)
  * and UNet.__init__ (model/fastdiffsr_modules/unet.py:224-297). */
 typedef struct fdsr_config {
-  int32_t in_channel;     /* 6: cat[cond, x_t] */
-  int32_t out_channel;    /* 3 */
+  int32_t in_channel;     /* 2 * out_channel: cat[cond, x_t] */
+  int32_t out_channel;    /* C, the image bands: 1..8 (3 = RGB) */
   int32_t inner_channel;  /* 64 */
   int32_t norm_groups;    /* 32 */
   int32_t n_levels;       /* len(channel_multiplier) */
@@ -65,7 +66,11 @@ typedef struct fdsr_config {
                              i.e. (image_size >> l) is in attn_res (ddpm_modules/unet.py:184, 211); mid[0] always does */
 } fdsr_config;
 
-/* Replaces UNet.__init__ + GaussianDiffusion.__init__ (diffusion.py:80-99): builds the layer plan. */
+/* Replaces UNet.__init__ + GaussianDiffusion.__init__ (diffusion.py:80-99): builds the layer plan.  Channel rule:
+ * in_channel == 2 * out_channel and 1 <= out_channel <= 8 (both models); anything else is FDSR_E_INVALID.
+ * The network input is packed as one 16-channel NHWC tensor: with P = 4 for C <= 4 and P = 8 otherwise, x_t occupies
+ * channels [0, C), cond [P, P + C), every other channel is 0 (C = 3: [x0 x1 x2 0 | c0 c1 c2 0 | 0 x 8]); the stem
+ * weights are permuted to match the reference's cat([cond, x_t]) order. */
 int fdsr_create(const fdsr_config* cfg, fdsr_ctx** out);
 int fdsr_destroy(fdsr_ctx* ctx);
 const char* fdsr_last_error(const fdsr_ctx* ctx);
@@ -105,28 +110,28 @@ int fdsr_reserve(fdsr_ctx* ctx, int32_t B, int32_t H, int32_t W);
 size_t fdsr_workspace_bytes(const fdsr_ctx* ctx);
 
 /* Replaces UNet.forward as called from p_mean_variance (diffusion.py:169-173): eps for step t,
- * noise_level = sqrt_alphas_cumprod_prev[t+1].  cond, x_t: (B,3,H,W) dev; eps_out: (B,3,H,W) dev. */
+ * noise_level = sqrt_alphas_cumprod_prev[t+1].  cond, x_t: (B,C,H,W) dev; eps_out: (B,C,H,W) dev. */
 int fdsr_unet_forward(fdsr_ctx* ctx, const float* cond_dev, const float* xt_dev, int32_t t,
                       float* eps_out_dev, int32_t B, int32_t H, int32_t W, void* stream);
 
 /* Replaces p_sample (diffusion.py:157-190) given eps: x0 = clamp(a_t x - b_t eps), mean, + sigma_t z.
- * z_dev may be NULL for t == 0.  In-place allowed (x_prev_dev == xt_dev). */
+ * z_dev may be NULL for t == 0.  In-place allowed (x_prev_dev == xt_dev).  numel: a positive multiple of C. */
 int fdsr_posterior_step(fdsr_ctx* ctx, const float* xt_dev, const float* eps_dev, const float* z_dev,
                         int32_t t, float* x_prev_dev, int64_t numel, void* stream);
 
 /* Replaces GaussianDiffusion.super_resolution / p_sample_loop (diffusion.py:192-231), batch-safe.
- *   cond_dev  (B,3,H,W) bicubic conditioning in [-1,1]
- *   noise_dev (T,B,3,H,W) injected Gaussian noise in the reference's draw order (x_T, then z for
+ *   cond_dev  (B,C,H,W) bicubic conditioning in [-1,1]
+ *   noise_dev (T,B,C,H,W) injected Gaussian noise in the reference's draw order (x_T, then z for
  *             t=T-1..1), or NULL to draw from the built-in counter-based generator with `seed`
- *   sr_out_dev (B,3,H,W) = clamp(x_0,-1,1)/2 + cond   (res2img, diffusion.py:275-281)
- *   trace_out_dev NULL, or (B, 1+n_frames, 3, H, W): per sample, res2img(cond) followed by
+ *   sr_out_dev (B,C,H,W) = clamp(x_0,-1,1)/2 + cond   (res2img, diffusion.py:275-281)
+ *   trace_out_dev NULL, or (B, 1+n_frames, C, H, W): per sample, res2img(cond) followed by
  *             res2img of x after every step with t % (1 | T/10) == 0 — the continous=True output. */
 int fdsr_sample(fdsr_ctx* ctx, const float* cond_dev, const float* noise_dev, uint64_t seed,
                 float* sr_out_dev, float* trace_out_dev, int32_t B, int32_t H, int32_t W,
                 void* stream);
 int32_t fdsr_trace_frames(const fdsr_ctx* ctx); /* 1 + n_frames for the current schedule */
 
-/* Tiled sampling of B canvases of (3,H,W), any H, W >= 8 with H*W < 2^32 (FastDiffSR model only): overlapping tiles
+/* Tiled sampling of B canvases of (C,H,W), any H, W >= 8 with H*W < 2^32 (FastDiffSR model only): overlapping tiles
  * of one shared chain.  Every step, each tile's eps (the network on the tile's window [cond | x_t]; every tile is its
  * own image for GroupNorm) is blended into one canvas-wide eps, and one posterior update moves the canvas-wide x_t.
  *   Grid, per axis of length L with tile size t (tile_h / tile_w: multiples of 8, >= 8) and overlap o (>= 0):
@@ -138,12 +143,12 @@ int32_t fdsr_trace_frames(const fdsr_ctx* ctx); /* 1 + n_frames for the current 
  *     n_k = w_k / sum(w);  eps = n_1 eps_1 + n_2 eps_2 + ... (the sum starts from the first term, so a pixel covered
  *     by one tile gets that tile's eps exactly);  x_{t-1} = the posterior update of fdsr_posterior_step.
  *   Noise is drawn per canvas pixel: built-in = the generator of fdsr_sample at (seed, image offset + b, y*W + x,
- *     step); injected = noise_dev (T,B,3,H,W) in fdsr_sample's draw order.  Canvas b is image fdsr_set_image_offset + b.
+ *     step); injected = noise_dev (T,B,C,H,W) in fdsr_sample's draw order.  Canvas b is image fdsr_set_image_offset + b.
  *   cond_dev, sr_out_dev and trace_out_dev are as in fdsr_sample, with the canvas shape.
  *   Evaluation: the n_tiles = B * tiles_y * tiles_x tiles go through the UNet in n_chunks = ceil(n_tiles / tile_batch)
  *     calls of Bc = ceil(n_tiles / n_chunks) tiles each (the last chunk is padded with repeats of its last tile), so the
  *     activation workspace is fdsr_reserve(Bc, t_e_y, t_e_x), independent of the canvas; the canvas x_t and the
- *     per-tile eps store (n_chunks * Bc * 3 * t_e_y * t_e_x floats) live in a separate grow-only context allocation.
+ *     per-tile eps store (n_chunks * Bc * C * t_e_y * t_e_x floats) live in a separate grow-only context allocation.
  *   A canvas that is exactly one tile gives fdsr_sample's bits; with o = 0 on a canvas the tiles partition, the result
  *   equals fdsr_sample of the crops (with the noise cropped alike); tile_batch does not change the result.
  *   Plain stream launches (no graph capture); the graphs cached by fdsr_sample are neither used nor evicted (a chunk
@@ -164,11 +169,15 @@ int fdsr_check_overflow(fdsr_ctx* ctx, void* stream);
  * fdsr_super_resolve_u8 batches.  The built-in generator's counter is (position in the image, GLOBAL image index,
  * step), so image k of a job receives the same noise whether it is sampled alone, inside a batch, or by another rank:
  * a batch sharded over N ranks (rank r passes the index of its first image) equals the single-rank result bit for bit.
- * Sticky; default 0.  Read from device memory by the captured graph (no re-capture). */
+ * Sticky; default 0.  Read from device memory by the captured graph (no re-capture).
+ * The generator: Philox4x32-10 keyed by the 64-bit seed, counter (pixel index y*W + x, low 32 bits of the global image
+ * index, step stream, (0x5eed + high 32 bits of the image index) ^ f), four normals per evaluation by Box-Muller.  Band c
+ * of a pixel takes normal c mod 4 of block c div 4, where block 0 has f = 0 and block 1 has f = 0x80000000; so bands
+ * 0-2 receive the same values for every C. */
 int fdsr_set_image_offset(fdsr_ctx* ctx, uint64_t first_image);
 
 /* Host-buffer convenience for callers without device memory management (the end-to-end path that
- * bench.py times): uint8 LR (B,h,w,3) host -> PIL-exact bicubic -> sampling -> fp32 SR (B,3,H,W)
+ * bench.py times): uint8 LR (B,h,w,C) host -> PIL-exact bicubic -> sampling -> fp32 SR (B,C,H,W)
  * host.  Copies go through context-owned pinned staging buffers.  Synchronous. */
 int fdsr_super_resolve_u8(fdsr_ctx* ctx, const uint8_t* lr_host, int32_t B, int32_t h, int32_t w,
                           int32_t H, int32_t W, const float* noise_dev, uint64_t seed,
@@ -184,22 +193,24 @@ int fdsr_super_resolve_u8_wait(fdsr_ctx* ctx, int32_t slot, float* sr_out_host);
 
 /* New at the boundary (the reference precomputes it offline with PIL, data/prepare_data_mfe_dm.py
  * :30-40): bit-exact Pillow BICUBIC resize of uint8 HWC images (horizontal pass, uint8 rounding,
- * vertical pass; 22-bit fixed-point taps), then optional /255*2-1 to fp32 NCHW (data/util.py:66-75).
- *   lr_dev (B,h,w,3) u8;  out_u8_dev (B,H,W,3) u8 or NULL;  cond_out_dev (B,3,H,W) fp32 or NULL */
+ * vertical pass; 22-bit fixed-point taps; each band resized as Pillow resizes an 'L' image), then optional /255*2-1
+ * to fp32 NCHW (data/util.py:66-75).
+ *   lr_dev (B,h,w,C) u8;  out_u8_dev (B,H,W,C) u8 or NULL;  cond_out_dev (B,C,H,W) fp32 or NULL */
 int fdsr_bicubic_u8(fdsr_ctx* ctx, const uint8_t* lr_dev, int32_t B, int32_t h, int32_t w,
                     int32_t H, int32_t W, uint8_t* out_u8_dev, float* cond_out_dev, void* stream);
 
 /* PSNR accumulators for the sharded evaluation loop (sr_mfe.py:315-356, core/metrics.py:16-42,
  * 94-101): per image, quantise both tensors like tensor2img (clamp [-1,1] -> uint8) and add the
- * squared error sum to sse_out_dev[b] (double, B entries).  PSNR = 10 log10(255^2 * 3HW / sse). */
+ * squared error sum to sse_out_dev[b] (double, B entries) of (B,C,H,W) tensors.  PSNR = 10 log10(255^2 * CHW / sse). */
 int fdsr_sse_u8(fdsr_ctx* ctx, const float* a_dev, const float* b_dev, int32_t B, int32_t H,
                 int32_t W, double* sse_out_dev, void* stream);
 
 /* Device-side evaluation metrics replacing the host block of sr_mfe.py:315-356 (skimage compare_mse /
  * compare_psnr / compare_ssim(multichannel=True) and core/metrics.py:88-93 calculate_ergas on
  * Metrics.tensor2img uint8 images, core/metrics.py:16-42).  a = the evaluated image (SR or bicubic),
- * b = HR, both (B,3,H,W) fp32 in [-1,1] on the device.  out_dev: B x 4 doubles (mse, psnr, ssim, ergas).
- * SSIM: 7x7 uniform window, sample covariance, K1 = .01, K2 = .03, data_range 255, 3-pixel crop. */
+ * b = HR, both (B,C,H,W) fp32 in [-1,1] on the device.  out_dev: B x 4 doubles (mse, psnr, ssim, ergas).
+ * MSE / PSNR over the C*H*W values; SSIM: 7x7 uniform window, sample covariance, K1 = .01, K2 = .03, data_range 255,
+ * 3-pixel crop, mean over the C channels; ERGAS: 100 sqrt(mse / mean(a)^2 / C) / ergas_scale. */
 int fdsr_metrics_u8(fdsr_ctx* ctx, const float* a_dev, const float* b_dev, int32_t B, int32_t H, int32_t W,
                     double ergas_scale, double* out_dev, void* stream);
 
@@ -236,7 +247,7 @@ int fdsr_debug_role_cycles(fdsr_ctx* ctx, int32_t op, int32_t t, int64_t* out_ho
  * last one (cap >= num_ops * num_sms * 40 entries).  Consecutive launches on one SM share its clock, so
  * first-MMA(op k+1) - last-MMA(op k) is the tensor pipe's idle time between two layers.  Returns the number of ops. */
 int fdsr_debug_timeline(fdsr_ctx* ctx, int32_t t, int32_t reps, int64_t* out_host, int64_t cap, void* stream);
-/* Fills out_dev (B,3,H,W) with the N(0,1) values the built-in generator hands the sampler for step stream
+/* Fills out_dev (B,C,H,W) with the N(0,1) values the built-in generator hands the sampler for step stream
  * `stream_id` (T for x_T, t for the z of step t) of images first_image .. first_image+B-1 under `seed`: lets tests
  * check the distribution (moments, Kolmogorov-Smirnov) and reproduce a built-in-noise sample through the
  * injected-noise path bit for bit. */
