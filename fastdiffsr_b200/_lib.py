@@ -94,6 +94,7 @@ _SIGS = {
     "fdsr_debug_op_name": (C.c_char_p, [C.c_void_p, C.c_int32]),
     "fdsr_debug_op_flops": (C.c_double, [C.c_void_p, C.c_int32]),
     "fdsr_debug_op_flops_executed": (C.c_double, [C.c_void_p, C.c_int32]),
+    "fdsr_debug_op_schedule": (C.c_int, [C.c_void_p, C.c_int32, C.POINTER(C.c_int32), C.c_int32]),
     "fdsr_debug_profile_unet": (C.c_int, [C.c_void_p, C.c_int32, C.c_int32, C.POINTER(C.c_float), C.c_int32,
                                           C.c_void_p]),
     "fdsr_debug_role_cycles": (C.c_int, [C.c_void_p, C.c_int32, C.c_int32, C.POINTER(C.c_int64), C.c_int32,

@@ -224,6 +224,8 @@ bool env_hook(const char* name, bool dflt) {
 
 int pad_n(int cout) { return cout <= 16 ? 16 : (cout <= 64 ? 64 : (cout <= 128 ? 128 : 256)); }
 
+constexpr int kOpScheduleFields = 17;  // fdsr_debug_op_schedule
+
 int add_tensor(fdsr_ctx* c, const std::string& name, int C, int level, bool stats) {
   HTensor t;
   t.name = name;
@@ -389,10 +391,15 @@ int build_plan(fdsr_ctx* c) {
   if (g.n_levels < 1 || g.n_levels > FDSR_MAX_LEVELS) return fail(c, FDSR_E_INVALID, "bad n_levels");
   if (g.model != FDSR_MODEL_FASTDIFFSR && g.model != FDSR_MODEL_SR3) return fail(c, FDSR_E_INVALID, "unknown model %d", g.model);
   const bool sr3 = g.model == FDSR_MODEL_SR3;
-  for (int i = 0; i < g.n_levels; ++i)
-    if (g.channel_mults[i] < 1 || inner * g.channel_mults[i] > 256)
-      return fail(c, FDSR_E_INVALID, "channel width %d unsupported (max 256 output channels)",
-                  inner * g.channel_mults[i]);
+  // a level's tensors are allocated with its width and its convs are planned at pad_n(width) channels: the two agree
+  // only for 64, 128 and 256 (a 192-wide level would be written at a 256-channel pitch)
+  for (int i = 0; i < g.n_levels; ++i) {
+    const int w = inner * g.channel_mults[i];
+    if (g.channel_mults[i] < 1 || (w != 64 && w != 128 && w != 256))
+      return fail(c, FDSR_E_INVALID,
+                  "level %d: channel width inner_channel * channel_mults[%d] = %d unsupported (every level width must be "
+                  "64, 128 or 256)", i, i, w);
+  }
   c->t_xin = add_tensor(c, "xin", 16, 0, false);
   int level = 0, pre = inner, idx = 1;
   int cur = add_tensor(c, "downs.0", inner, 0, true);
@@ -1275,18 +1282,24 @@ cudaError_t set_conv_attrs() {
 template <typename T>
 int launch_conv16(fdsr_ctx* c, int li, int t, cudaStream_t st, const ConvLayer* override_layer = nullptr);
 
+// CTAs of one conv launch (the kernel divides the layer's tile groups evenly over them, see conv_gemm_kernel)
+int conv_grid(const fdsr_ctx* c, const ConvLayer& l) {
+  const int cs = l.pair ? 2 : 1;  // CTA pairs are clusters of two; the unit of work is then a pair of tiles
+  const int ngroups = l.ntiles / cs / l.group;
+  int grid = (ngroups < c->num_sms / cs ? ngroups : c->num_sms / cs) * cs;
+  if (l.nsplit > 1) {  // nsplit CTAs per tile group; persistent over the groups when there are more than fit one wave
+    grid = ngroups * l.nsplit;
+    if (grid > c->num_sms) grid = c->num_sms - c->num_sms % l.nsplit;
+  }
+  return grid;
+}
+
 template <int N, typename T>
-int launch_conv_t(fdsr_ctx* c, int li, int ntiles, int t, cudaStream_t st, const ConvLayer* override_layer) {
+int launch_conv_t(fdsr_ctx* c, int li, int t, cudaStream_t st, const ConvLayer* override_layer) {
   const ConvLayer& LY = override_layer ? *override_layer : c->h_layers[li];
   const bool pair = c->h_layers[li].pair != 0;
-  const int cs = pair ? 2 : 1;  // CTA pairs are clusters of two; the unit of work is then a pair of tiles
-  const int ngroups = ntiles / cs / c->h_layers[li].group;
-  const int nsplit = c->h_layers[li].nsplit;
-  int grid = (ngroups < c->num_sms / cs ? ngroups : c->num_sms / cs) * cs;
-  if (nsplit > 1) {  // nsplit CTAs per tile group; persistent over the groups when there are more than fit one wave
-    grid = ngroups * nsplit;
-    if (grid > c->num_sms) grid = c->num_sms - c->num_sms % nsplit;
-  }
+  const int cs = pair ? 2 : 1;
+  const int grid = conv_grid(c, c->h_layers[li]);
   cudaLaunchConfig_t cfg{};
   cfg.gridDim = dim3(grid);
   cfg.blockDim = dim3(kConvThreads);
@@ -1320,12 +1333,11 @@ int launch_conv(fdsr_ctx* c, int li, int t, cudaStream_t st, const ConvLayer* ov
 template <typename T>
 int launch_conv16(fdsr_ctx* c, int li, int t, cudaStream_t st, const ConvLayer* override_layer) {
   const HConv& k = c->convs[li];
-  const int ntiles = c->h_layers[li].ntiles;
   switch (c->h_layers[li].N) {
-    case 16: return launch_conv_t<16, T>(c, li, ntiles, t, st, override_layer);
-    case 64: return launch_conv_t<64, T>(c, li, ntiles, t, st, override_layer);
-    case 128: return launch_conv_t<128, T>(c, li, ntiles, t, st, override_layer);
-    case 256: return launch_conv_t<256, T>(c, li, ntiles, t, st, override_layer);
+    case 16: return launch_conv_t<16, T>(c, li, t, st, override_layer);
+    case 64: return launch_conv_t<64, T>(c, li, t, st, override_layer);
+    case 128: return launch_conv_t<128, T>(c, li, t, st, override_layer);
+    case 256: return launch_conv_t<256, T>(c, li, t, st, override_layer);
   }
   return fail(c, FDSR_E_INVALID, "unsupported N=%d", k.N);
 }
@@ -2246,6 +2258,35 @@ static double op_flops(const fdsr_ctx* c, int32_t i, bool executed) {
 }
 double fdsr_debug_op_flops(const fdsr_ctx* c, int32_t i) { return op_flops(c, i, false); }
 double fdsr_debug_op_flops_executed(const fdsr_ctx* c, int32_t i) { return op_flops(c, i, true); }
+
+int fdsr_debug_op_schedule(fdsr_ctx* c, int32_t i, int32_t* out_host, int32_t cap) {
+  if (!c || !out_host) return fail(c, FDSR_E_INVALID, "null argument");
+  if (i < 0 || i >= int(c->ops.size()) || c->ops[i].kind != 0) return fail(c, FDSR_E_INVALID, "op %d is not a conv", i);
+  if (c->cfg.dtype == FDSR_DTYPE_FP32) return fail(c, FDSR_E_INVALID, "the fp32 parity mode has no tile schedule");
+  if (c->layers_dirty || c->h_layers.empty()) return fail(c, FDSR_E_STATE, "run fdsr_unet_forward at the shape first");
+  if (cap < kOpScheduleFields) return fail(c, FDSR_E_INVALID, "capacity too small (%d needed)", kOpScheduleFields);
+  const ConvLayer& l = c->h_layers[c->ops[i].idx];
+  const int grid = conv_grid(c, l);
+  // the CTA ranges of conv_gemm_kernel: nclusters contiguous, balanced ranges of tile groups (pair mode: groups of
+  // tile pairs, CTA r of a pair computing tile 2k + r); split-N CTAs of one range share its tiles
+  const int cs = l.pair ? 2 : 1, ngroups = l.ntiles / cs / l.group, nclusters = grid / cs / l.nsplit;
+  const int tq = ngroups / nclusters, tr = ngroups - tq * nclusters, tpi = l.tiles_x * l.tiles_y;
+  int max_tiles = 0, spans_image = 0, spans_phase = 0;
+  for (int cid = 0; cid < nclusters; ++cid) {
+    const int units = tq + (cid < tr ? 1 : 0);
+    if (units == 0) continue;
+    const int tb = (cid * tq + (cid < tr ? cid : tr)) * l.group, te = tb + units * l.group;
+    max_tiles = std::max(max_tiles, te - tb);
+    const int b0 = tb * cs / tpi, b1 = ((te - 1) * cs + cs - 1) / tpi;  // first and last virtual image of the range
+    spans_image |= b0 / l.phases != b1 / l.phases;
+    for (int b = b0; b < b1 && l.phases > 1; ++b) spans_phase |= b / l.phases == (b + 1) / l.phases;
+  }
+  const int32_t v[kOpScheduleFields] = {l.N,     l.pair,  l.tile_h, l.nsplit, l.group,  grid,        l.ntiles,    max_tiles,
+                                        l.epi2,  l.tail2, l.nR,     l.nG,     l.phases, l.a_tma,     spans_image, spans_phase,
+                                        l.nchunks};
+  std::copy(v, v + kOpScheduleFields, out_host);
+  return kOpScheduleFields;
+}
 
 int fdsr_debug_profile_unet(fdsr_ctx* c, int32_t t, int32_t reps, float* ms_out_host, int32_t cap, void* stream) {
   if (!c || !ms_out_host) return fail(c, FDSR_E_INVALID, "null argument");

@@ -288,6 +288,18 @@ class Engine:
         n = self.lib.fdsr_debug_num_ops(self._h)
         return [float(self.lib.fdsr_debug_op_flops_executed(self._h, i)) for i in range(n)]
 
+    OP_SCHEDULE_FIELDS = ("N", "pair", "tile_h", "nsplit", "group", "grid", "ntiles", "max_tiles", "epi2", "tail2", "nR",
+                          "nG", "phases", "a_tma", "spans_image", "spans_phase", "nchunks")
+
+    def op_names(self):
+        return [self.lib.fdsr_debug_op_name(self._h, i).decode() for i in range(self.lib.fdsr_debug_num_ops(self._h))]
+
+    def op_schedule(self, op: int):
+        """The launch schedule of conv op `op` at the shape of the last forward (fdsr_debug_op_schedule), as a dict."""
+        buf = (C.c_int32 * len(self.OP_SCHEDULE_FIELDS))()
+        n = self._check(self.lib.fdsr_debug_op_schedule(self._h, op, buf, len(buf)), "fdsr_debug_op_schedule")
+        return dict(zip(self.OP_SCHEDULE_FIELDS, buf[:n]))
+
     def profile_unet(self, t: int, reps: int = 3):
         """[(op name, mean ms, algorithmic conv FLOPs)] for one UNet evaluation at the current shape."""
         n = self.lib.fdsr_debug_num_ops(self._h)

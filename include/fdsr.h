@@ -58,7 +58,9 @@ typedef struct fdsr_config {
   int32_t inner_channel;  /* 64 */
   int32_t norm_groups;    /* 32 */
   int32_t n_levels;       /* len(channel_multiplier) */
-  int32_t channel_mults[FDSR_MAX_LEVELS];
+  int32_t channel_mults[FDSR_MAX_LEVELS];  /* level widths inner_channel * channel_mults[l] must each be 64, 128 or
+                                              256 (e.g. 64 * [1, 2, 4, 4]); any other width, 192 included, is
+                                              FDSR_E_INVALID */
   int32_t res_blocks;     /* 2 */
   int32_t dtype;          /* FDSR_DTYPE_* */
   int32_t model;          /* FDSR_MODEL_* (networks.py:84-91) */
@@ -233,6 +235,13 @@ double fdsr_debug_op_flops(const fdsr_ctx* ctx, int32_t i);
 /* The multiply-adds the op really executes: equal to the algorithmic figure except for the three nearest-upsample convs,
  * which run as four 2x2 phase convs on the low-resolution input (4/9 of the nine-tap MACs). */
 double fdsr_debug_op_flops_executed(const fdsr_ctx* ctx, int32_t i);
+/* The schedule conv op `i` is launched with at the current shape (16-bit modes, after a forward at that shape; host
+ * only), as the launch computes it: out_host[0..16] = N (per CTA), pair (CTA pairs), tile_h (32, or 16 = half tiles),
+ * nsplit (split-N parts), group (tiles per statistics group), grid (CTAs), ntiles, the largest tile count of one CTA,
+ * epi2, tail2, nR, nG (patch ring stages), phases (4 = phase-decomposed upsample), a_tma, whether some CTA's range
+ * holds tiles of two images, whether some CTA's range holds tiles of two phases of one image, and the K chunk count.
+ * Returns the number of fields written (17); cap must be at least that. */
+int fdsr_debug_op_schedule(fdsr_ctx* ctx, int32_t i, int32_t* out_host, int32_t cap);
 int fdsr_debug_profile_unet(fdsr_ctx* ctx, int32_t t, int32_t reps, float* ms_out_host, int32_t cap,
                             void* stream);
 /* Role-level cycle counters of one conv op (only populated by -DFDSR_PROFILE builds of the library,
