@@ -9,6 +9,7 @@
 #include <cstring>
 #include <map>
 #include <string>
+#include <utility>
 #include <vector>
 
 #include <cuda_runtime.h>
@@ -48,6 +49,7 @@ struct HChunk {
   // reference concatenates cat([cond, x]) (diffusion.py:173): perm[j] = reference input channel of packed channel j, or -1
   std::vector<int> perm;
   int wchan(int ci) const { return perm.empty() ? (ci < creal ? wc0 + ci : -1) : (ci < int(perm.size()) ? perm[ci] : -1); }
+  int wchan_end() const { return perm.empty() ? wc0 + creal : *std::max_element(perm.begin(), perm.end()) + 1; }
   int nreal() const {
     if (perm.empty()) return creal;
     int n = 0;
@@ -87,6 +89,31 @@ struct HOp {
   int idx;
 };
 
+// Device memory owned by a context, freed with it.  grow(bytes) keeps the allocation when it is already large enough:
+// cached graphs and tensor maps hold pointers into it.
+template <typename T>
+struct DevBuf {
+  T* ptr = nullptr;
+  size_t cap = 0;  // bytes
+  DevBuf() = default;
+  DevBuf(DevBuf&& o) noexcept : ptr(o.ptr), cap(o.cap) {
+    o.ptr = nullptr;
+    o.cap = 0;
+  }
+  DevBuf(const DevBuf&) = delete;
+  ~DevBuf() { cudaFree(ptr); }
+  operator T*() const { return ptr; }
+  cudaError_t grow(size_t bytes) {
+    if (bytes <= cap) return cudaSuccess;
+    cudaFree(ptr);
+    ptr = nullptr;
+    cap = 0;
+    const cudaError_t e = cudaMalloc(&ptr, bytes);
+    if (e == cudaSuccess) cap = bytes;
+    return e;
+  }
+};
+
 }  // namespace
 
 struct fdsr_ctx {
@@ -101,19 +128,16 @@ struct fdsr_ctx {
   // weights
   std::map<std::string, std::vector<float>> host_w;
   bool weights_loaded = false;
-  uint8_t* d_weights = nullptr;
-  size_t weights_bytes = 0;
-  float* d_params = nullptr;  // gamma/beta, clam/slam weights
-  size_t params_floats = 0;
-  float* d_bias = nullptr;  // per conv [T][N]
-  size_t bias_floats = 0;
+  DevBuf<uint8_t> d_weights;
+  DevBuf<float> d_params;  // gamma/beta, clam/slam weights
+  DevBuf<float> d_bias;    // per conv [T][N]
   // schedule
   int T = 0;
   std::map<std::string, std::vector<double>> tables;
   std::vector<PostCoef> post;
   // workspace
   int B = 0, H = 0, W = 0;
-  uint8_t* d_ws = nullptr;
+  DevBuf<uint8_t> d_ws;  // grow-only: the captured graphs of other shapes hold pointers into it
   size_t ws_bytes = 0;
   size_t stats_off = 0, stats_bytes = 0;
   size_t off_cond = 0, off_x = 0, off_eps = 0, off_sr = 0, off_psum = 0, off_pmax = 0, off_gate = 0,
@@ -133,30 +157,27 @@ struct fdsr_ctx {
   bool up_phases = true;   // FDSR_UP_PHASES=0: nearest-upsample convs gather a 2x patch and run all nine taps
   bool fused_tail = true;  // FDSR_FUSED_TAIL=0: the sampler runs pack_input / final conv -> eps / posterior as separate kernels
   bool attn_ref = false;   // FDSR_ATTN_REF=1: CUDA-core attention core in the 16-bit modes too
-  float* d_weights32 = nullptr;     // fp32 parity mode weights: per conv, per chunk [tap][ci][N]
+  DevBuf<float> d_weights32;        // fp32 parity mode weights: per conv, per chunk [tap][ci][N]
   std::vector<size_t> w32_off;      // per conv (floats)
   size_t off_gntab = 0;             // [B][kMaxGnC] float2 scratch of the fp32 mode
   int esize() const { return cfg.dtype == FDSR_DTYPE_FP32 ? 4 : 2; }
   int bands() const { return cfg.out_channel; }  // C: channels of every image tensor (cond, x_t, eps, noise, SR, u8)
-  long long* d_prof = nullptr;  // role cycle counters (FDSR_PROFILE builds)
+  DevBuf<long long> d_prof;  // role cycle counters (FDSR_PROFILE builds)
   bool layers_dirty = true;
   // bicubic tables (cached per size pair)
   struct BicTab {
     int in, out, ksize;
-    int *d_min, *d_cnt, *d_taps;
+    DevBuf<int> d_min, d_cnt, d_taps;
   };
   std::vector<BicTab> bic;
-  uint8_t* d_bic_tmp = nullptr;
-  size_t bic_tmp_bytes = 0;
-  unsigned long long* d_metric = nullptr;  // [B][4] integer accumulators of fdsr_metrics_u8
-  size_t metric_bytes = 0;
+  DevBuf<uint8_t> d_bic_tmp;
+  DevBuf<unsigned long long> d_metric;  // [B][4] integer accumulators of fdsr_metrics_u8
   // pinned staging for the host-buffer path
   // host-buffer path: two slots so that the copies of one batch overlap the sampling of the next
   struct HostSlot {
     uint8_t* h_pin = nullptr;      // pinned: [LR u8 | SR fp32 | status word]
     size_t h_pin_bytes = 0;
-    uint8_t* d_stage = nullptr;    // device: [LR u8 | cond fp32 | SR fp32 | status word]
-    size_t d_stage_bytes = 0;
+    DevBuf<uint8_t> d_stage;       // device: [LR u8 | cond fp32 | SR fp32 | status word]
     size_t in_b = 0, out_b = 0;
     cudaEvent_t computed = nullptr, copied = nullptr;
     bool busy = false;
@@ -166,7 +187,7 @@ struct fdsr_ctx {
   cudaStream_t copy_stream = nullptr;
   // graph cache
   bool use_graph = true;
-  PostStep* d_post = nullptr;      // [T] per-step posterior arguments of the fused final-conv epilogue
+  DevBuf<PostStep> d_post;         // [T] per-step posterior arguments of the fused final-conv epilogue
   ConvLayer final_fused{};         // the final conv's descriptor in kOutPosterior mode (h_layers holds the eps form)
   // Captured sampling loops, keyed on what the captured launches depend on: the shape and whether noise is injected /
   // a trace is written.  Seed, image offset and the noise / trace POINTERS are read from device memory (SampleArgs),
@@ -182,7 +203,6 @@ struct fdsr_ctx {
   uint64_t graph_clock = 0;
   int64_t graph_captures = 0;
   uint64_t image0 = 0;              // fdsr_set_image_offset
-  size_t ws_cap = 0;                // allocated bytes of d_ws (grow-only: cached graphs hold pointers into it)
   void drop_graphs() {
     for (auto& g : graphs) cudaGraphExecDestroy(g.exec);
     graphs.clear();
@@ -191,8 +211,7 @@ struct fdsr_ctx {
   double flops_per_px = 0.0;  // conv FLOPs per full-resolution output pixel per image
   // fdsr_sample_tiled: [SampleArgs | canvas x_t (B,C,H,W) fp32 | per-tile eps store [slot][C][te_y][te_x] fp32],
   // grow-only, apart from the workspace (which only ever holds one chunk of tiles)
-  uint8_t* d_tiled = nullptr;
-  size_t tiled_cap = 0;
+  DevBuf<uint8_t> d_tiled;
 };
 
 namespace {
@@ -222,9 +241,58 @@ bool env_hook(const char* name, bool dflt) {
                   __LINE__);                                                                 \
   } while (0)
 
+// The tail of every kernel launch: check it where it happens, and count it (fdsr_launch_count)
+int launched(fdsr_ctx* c, cudaError_t e, const void* kernel) {
+  if (e == cudaSuccess) e = cudaGetLastError();
+  if (e != cudaSuccess) {
+    const char* name = nullptr;
+    if (cudaFuncGetName(&name, kernel) != cudaSuccess || !name) name = "kernel";
+    return fail(c, FDSR_E_CUDA, "launch of %s failed: %s", name, cudaGetErrorString(e));
+  }
+  ++c->launches;
+  return FDSR_OK;
+}
+
+template <typename... P, typename... A>
+int launch(fdsr_ctx* c, void (*kernel)(P...), dim3 grid, dim3 block, size_t smem, cudaStream_t st, A&&... args) {
+  kernel<<<grid, block, smem, st>>>(std::forward<A>(args)...);
+  return launched(c, cudaSuccess, reinterpret_cast<const void*>(kernel));
+}
+
+// Replaces the buffer with a device copy of `host`, allocated `pad` bytes longer
+template <typename T, typename H>
+int upload(fdsr_ctx* c, DevBuf<T>& b, const std::vector<H>& host, size_t pad = 0) {
+  cudaFree(b.ptr);
+  b.ptr = nullptr;
+  b.cap = 0;
+  CUDA_TRY(c, b.grow(host.size() * sizeof(H) + pad));
+  CUDA_TRY(c, cudaMemcpy(b.ptr, host.data(), host.size() * sizeof(H), cudaMemcpyHostToDevice));
+  return FDSR_OK;
+}
+
+// f(Elem<T>{}) with the context's element type T: __half, __nv_bfloat16, or float (the fp32 parity mode).
+// with_dtype16 serves the paths that exist for the 16-bit types only; their callers have ruled out fp32.
+template <typename T>
+struct Elem {
+  using type = T;
+};
+template <typename F>
+auto with_dtype16(const fdsr_ctx* c, F&& f) {
+  return c->cfg.dtype == FDSR_DTYPE_BF16 ? f(Elem<__nv_bfloat16>{}) : f(Elem<__half>{});
+}
+template <typename F>
+auto with_dtype(const fdsr_ctx* c, F&& f) {
+  return c->cfg.dtype == FDSR_DTYPE_FP32 ? f(Elem<float>{}) : with_dtype16(c, f);
+}
+
 int pad_n(int cout) { return cout <= 16 ? 16 : (cout <= 64 ? 64 : (cout <= 128 ? 128 : 256)); }
 
 constexpr int kOpScheduleFields = 17;  // fdsr_debug_op_schedule
+
+void add_conv(fdsr_ctx* c, const HConv& k) {
+  c->convs.push_back(k);
+  c->ops.push_back({0, int(c->convs.size()) - 1});
+}
 
 int add_tensor(fdsr_ctx* c, const std::string& name, int C, int level, bool stats) {
   HTensor t;
@@ -270,8 +338,7 @@ int add_res(fdsr_ctx* c, const std::string& name, const std::vector<int>& srcs, 
     k.film_swish = c->cfg.model == FDSR_MODEL_SR3;
     k.film_name = k.film_swish ? p + ".mlp.1" : p + ".noise_func.noise_func.0";
     k.out = th;
-    c->convs.push_back(k);
-    c->ops.push_back({0, int(c->convs.size()) - 1});
+    add_conv(c, k);
   }
   {
     HConv k;
@@ -307,8 +374,7 @@ int add_res(fdsr_ctx* c, const std::string& name, const std::vector<int>& srcs, 
       k.resid = srcs[0];
     }
     k.out = to;
-    c->convs.push_back(k);
-    c->ops.push_back({0, int(c->convs.size()) - 1});
+    add_conv(c, k);
   }
   return to;
 }
@@ -339,8 +405,7 @@ int add_self_attn(fdsr_ctx* c, const std::string& name, int in, int level, const
     k.w_n0 = i * C;
     k.w_rows = 3 * C;
     k.out = tq[i];
-    c->convs.push_back(k);
-    c->ops.push_back({0, int(c->convs.size()) - 1});
+    add_conv(c, k);
   }
   HAttn a;
   a.name = name;
@@ -366,8 +431,7 @@ int add_self_attn(fdsr_ctx* c, const std::string& name, int in, int level, const
     k.bias_names = {p + ".out.bias"};
     k.resid = in;
     k.out = to;
-    c->convs.push_back(k);
-    c->ops.push_back({0, int(c->convs.size()) - 1});
+    add_conv(c, k);
   }
   return to;
 }
@@ -377,6 +441,15 @@ int add_res_attn(fdsr_ctx* c, const std::string& name, const std::vector<int>& s
   if (!attn) return add_res(c, name, srcs, cout, level, name);
   const int tr = add_res(c, name, srcs, cout, level, name + ".res");
   return add_self_attn(c, name, tr, level, name);
+}
+
+// MACs per output pixel of a conv (real channels only; identity-residual chunks are bookkeeping, not convolution work).
+// Algorithmic: a phase layer counts as the nine-tap conv it replaces; executed: as the four-tap convs it runs.
+double conv_macs(const HConv& k, bool executed) {
+  double macs = 0.0;
+  for (const HChunk& ch : k.chunks)
+    macs += ch.wname == "@identity" ? 0.0 : double((k.phases == 4 && !executed) ? 9 : ch.taps.size()) * ch.nreal();
+  return macs;
 }
 
 int build_plan(fdsr_ctx* c) {
@@ -422,8 +495,7 @@ int build_plan(fdsr_ctx* c) {
     k.chunks.push_back(stem);
     k.bias_names = {"denoise_fn.downs.0.bias"};
     k.out = cur;
-    c->convs.push_back(k);
-    c->ops.push_back({0, 0});
+    add_conv(c, k);
   }
   std::vector<int> feats{cur};
   for (int li = 0; li < g.n_levels; ++li) {
@@ -455,8 +527,7 @@ int build_plan(fdsr_ctx* c) {
           }
       k.bias_names = {"denoise_fn." + nm + ".conv.bias"};
       k.out = to;
-      c->convs.push_back(k);
-      c->ops.push_back({0, int(c->convs.size()) - 1});
+      add_conv(c, k);
       cur = to;
       ++level;
       feats.push_back(cur);
@@ -513,8 +584,7 @@ int build_plan(fdsr_ctx* c) {
       }
       k.bias_names = {"denoise_fn." + nm + ".conv.bias"};
       k.out = to;
-      c->convs.push_back(k);
-      c->ops.push_back({0, int(c->convs.size()) - 1});
+      add_conv(c, k);
       cur = to;
       --level;
     }
@@ -534,8 +604,7 @@ int build_plan(fdsr_ctx* c) {
     k.bias_names = {"denoise_fn.final_conv.block.3.bias"};
     k.out_mode = kOutEpsNCHW;
     k.out_c = g.out_channel;
-    c->convs.push_back(k);
-    c->ops.push_back({0, int(c->convs.size()) - 1});
+    add_conv(c, k);
   }
   c->t_last = cur;
   // Statistics granularity per tensor: a consumer GroupNorm with cpg channels per group over the
@@ -558,15 +627,22 @@ int build_plan(fdsr_ctx* c) {
     if (int(k.chunks.size()) > kMaxChunks) return fail(c, FDSR_E_INVALID, "layer %s: too many chunks", k.name.c_str());
     if (k.gn_C > kMaxGnC) return fail(c, FDSR_E_INVALID, "layer %s: GroupNorm width %d > %d", k.name.c_str(), k.gn_C, kMaxGnC);
     const int lvl = k.out >= 0 ? c->tensors[k.out].level : 0;
-    double macs = 0.0;  // algorithmic: a phase layer is accounted as the nine-tap conv it replaces
-    for (const HChunk& ch : k.chunks) macs += ch.wname == "@identity" ? 0.0 : double(k.phases == 4 ? 9 : ch.taps.size()) * ch.nreal();
-    fl += 2.0 * macs * k.cout / double(1 << (2 * lvl));
+    fl += 2.0 * conv_macs(k, false) * k.cout / double(1 << (2 * lvl));
   }
   c->flops_per_px = fl;
   return FDSR_OK;
 }
 
 const std::vector<float>* find_w(fdsr_ctx* c, const std::string& name);
+
+// The weight tensor [rows][cin][kk][kk] a chunk reads.  cin follows from the tensor's size, which validate_weights has
+// checked against the channels the plan reads (the 256 x 256 identity has no state_dict entry).
+struct WeightGeom {
+  size_t rows, kk, cin;
+  WeightGeom(const HConv& k, const HChunk& ch, size_t numel = 0)
+      : rows(k.w_rows ? k.w_rows : k.cout), kk(ch.kk), cin(ch.wname == "@identity" ? 256 : numel / (rows * kk * kk)) {}
+  size_t at(int n, int ci, int ky, int kx) const { return ((size_t(n) * cin + ci) * kk + ky) * kk + kx; }
+};
 
 // Exact element counts of every tensor the plan reads, before anything indexes into them: the C ABI is a public
 // boundary that does not go through torch's strict shape check, and a state_dict of a different inner_channel /
@@ -583,18 +659,16 @@ int validate_weights(fdsr_ctx* c) {
   const size_t inner = size_t(c->cfg.inner_channel);
   int rc;
   // conv weights: rows x (sum of the source channels this weight tensor spans) x k x k
-  std::map<std::string, size_t> cin_of, rows_of, kk_of;
+  std::map<std::string, size_t> numel_of;
   for (const HConv& k : c->convs)
     for (const HChunk& ch : k.chunks) {
       if (ch.wname == "@identity") continue;
-      size_t& ci = cin_of[ch.wname];
-      if (ch.perm.empty()) ci = std::max(ci, size_t(ch.wc0 + ch.creal));
-      else for (int v : ch.perm) ci = std::max(ci, size_t(v + 1));
-      rows_of[ch.wname] = size_t(k.w_rows ? k.w_rows : k.cout);
-      kk_of[ch.wname] = size_t(ch.kk);
+      const WeightGeom g(k, ch);
+      size_t& n = numel_of[ch.wname];
+      n = std::max(n, g.rows * ch.wchan_end() * g.kk * g.kk);
     }
-  for (const auto& it : cin_of)
-    if ((rc = need(it.first, rows_of[it.first] * it.second * kk_of[it.first] * kk_of[it.first], "conv weight"))) return rc;
+  for (const auto& it : numel_of)
+    if ((rc = need(it.first, it.second, "conv weight"))) return rc;
   for (const HConv& k : c->convs) {
     for (const std::string& bn : k.bias_names)
       if ((rc = need(bn, size_t(k.cout), "conv bias"))) return rc;
@@ -677,9 +751,7 @@ int pack_weights(fdsr_ctx* c) {
     for (const HChunk& ch : k.chunks) {
       const std::vector<float>* w = find_w(c, ch.wname);
       if (!w) return fail(c, FDSR_E_NOTFOUND, "missing weight %s", ch.wname.c_str());
-      const bool is1x1 = ch.kk == 1;
-      const int kk = ch.kk;
-      const size_t cin_w = ch.wname == "@identity" ? 256 : w->size() / (size_t(k.w_rows ? k.w_rows : k.cout) * kk * kk);
+      const WeightGeom g(k, ch, w->size());
       for (const HTap& tp : ch.taps) {
         T* blob = host.data() + off / sizeof(T);
         for (int cg = 0; cg < k.ncg; ++cg)
@@ -687,7 +759,6 @@ int pack_weights(fdsr_ctx* c) {
             for (int j = 0; j < 8; ++j) {
               const int wci = ch.wchan(cg * 8 + j);
               if (wci < 0) continue;
-              const size_t wbase = (size_t(k.w_n0 + n) * cin_w + wci) * kk * kk;
               if (k.phases == 4) {
                 // tap (ry, rx) of phase (py, px): the 3x3 taps whose upsampled source row / column is that one
                 const int py = ph >> 1, px = ph & 1;
@@ -695,12 +766,11 @@ int pack_weights(fdsr_ctx* c) {
                 for (int dy = 0; dy < 3; ++dy)
                   for (int dx = 0; dx < 3; ++dx)
                     if (((py + dy + 1) >> 1) - py == tp.ky && ((px + dx + 1) >> 1) - px == tp.kx)
-                      acc += (*w)[wbase + dy * 3 + dx];
+                      acc += (*w)[g.at(k.w_n0 + n, wci, dy, dx)];
                 blob[(size_t(cg) * k.N + n) * 8 + j] = to_w<T>(acc, ch.gn != 0);
                 continue;
               }
-              const size_t wi = wbase + (is1x1 ? 0 : tp.ky) * kk + (is1x1 ? 0 : tp.kx);
-              blob[(size_t(cg) * k.N + n) * 8 + j] = to_w<T>((*w)[wi], ch.gn != 0);
+              blob[(size_t(cg) * k.N + n) * 8 + j] = to_w<T>((*w)[g.at(k.w_n0 + n, wci, tp.ky, tp.kx)], ch.gn != 0);
             }
         off += size_t(k.ncg) * k.N * 16;
       }
@@ -717,12 +787,7 @@ int pack_weights(fdsr_ctx* c) {
                    src + bi * blob_e + (size_t(cg) * k.N + n) * 8, 8 * sizeof(T));
     }
   }
-  if (c->d_weights) cudaFree(c->d_weights);
-  c->d_weights = nullptr;
-  CUDA_TRY(c, cudaMalloc(&c->d_weights, total));
-  CUDA_TRY(c, cudaMemcpy(c->d_weights, host.data(), total, cudaMemcpyHostToDevice));
-  c->weights_bytes = total;
-  return FDSR_OK;
+  return upload(c, c->d_weights, host);
 }
 
 // fp32 parity mode: per conv, per chunk: [tap][ci < creal][N] floats
@@ -740,27 +805,19 @@ int pack_weights_f32(fdsr_ctx* c) {
     for (const HChunk& ch : k.chunks) {
       const std::vector<float>* w = find_w(c, ch.wname);
       if (!w) return fail(c, FDSR_E_NOTFOUND, "missing weight %s", ch.wname.c_str());
-      const bool is1x1 = ch.kk == 1;
-      const int kk = ch.kk;
-      const size_t cin_w = ch.wname == "@identity" ? 256 : w->size() / (size_t(k.w_rows ? k.w_rows : k.cout) * kk * kk);
+      const WeightGeom g(k, ch, w->size());
       for (const HTap& tp : ch.taps) {
         for (int ci = 0; ci < ch.creal; ++ci) {
           const int wci = ch.wchan(ci);
           if (wci < 0) continue;
           for (int n = 0; n < k.cout; ++n)
-            host[off + size_t(ci) * k.N + n] =
-                (*w)[((size_t(k.w_n0 + n) * cin_w + wci) * kk + (is1x1 ? 0 : tp.ky)) * kk + (is1x1 ? 0 : tp.kx)];
+            host[off + size_t(ci) * k.N + n] = (*w)[g.at(k.w_n0 + n, wci, tp.ky, tp.kx)];
         }
         off += size_t(ch.creal) * k.N;
       }
     }
   }
-  if (c->d_weights32) cudaFree(c->d_weights32);
-  c->d_weights32 = nullptr;
-  CUDA_TRY(c, cudaMalloc(&c->d_weights32, total * 4 + 16));
-  CUDA_TRY(c, cudaMemcpy(c->d_weights32, host.data(), total * 4, cudaMemcpyHostToDevice));
-  c->weights_bytes = total * 4;
-  return FDSR_OK;
+  return upload(c, c->d_weights32, host, 16);
 }
 
 int upload_params(fdsr_ctx* c) {
@@ -787,12 +844,7 @@ int upload_params(fdsr_ctx* c) {
     a.w7_off = p.size();
     p.insert(p.end(), w7->begin(), w7->end());
   }
-  if (c->d_params) cudaFree(c->d_params);
-  c->d_params = nullptr;
-  CUDA_TRY(c, cudaMalloc(&c->d_params, p.size() * 4 + 16));
-  CUDA_TRY(c, cudaMemcpy(c->d_params, p.data(), p.size() * 4, cudaMemcpyHostToDevice));
-  c->params_floats = p.size();
-  return FDSR_OK;
+  return upload(c, c->d_params, p, 16);
 }
 
 // y[o] = b[o] + sum_i w[o][i] x[i]   (fp32, like nn.Linear)
@@ -878,13 +930,8 @@ int build_bias_tables(fdsr_ctx* c) {
       }
     }
   }
-  if (c->d_bias) cudaFree(c->d_bias);
-  c->d_bias = nullptr;
-  CUDA_TRY(c, cudaMalloc(&c->d_bias, total * 4 + 16));
-  CUDA_TRY(c, cudaMemcpy(c->d_bias, tab.data(), total * 4, cudaMemcpyHostToDevice));
-  c->bias_floats = total;
   c->layers_dirty = true;
-  return FDSR_OK;
+  return upload(c, c->d_bias, tab, 16);
 }
 
 size_t align_up(size_t v, size_t a) { return (v + a - 1) / a * a; }
@@ -906,33 +953,33 @@ EncodeTiledFn get_encode_tiled() {
   return fn;
 }
 
+// A tiled TMA map of a 16-bit tensor: L2 promotion of 128 bytes, zero fill outside the tensor
+constexpr cuuint32_t kUnitStrides[4] = {1, 1, 1, 1};
+bool encode_map(CUtensorMap* m, const void* ptr, int rank, const cuuint64_t* dims, const cuuint64_t* strides,
+                const cuuint32_t* box, const cuuint32_t* elem_strides, CUtensorMapSwizzle swizzle, bool bf16) {
+  EncodeTiledFn enc = get_encode_tiled();
+  return enc && enc(m, bf16 ? CU_TENSOR_MAP_DATA_TYPE_BFLOAT16 : CU_TENSOR_MAP_DATA_TYPE_FLOAT16, rank,
+                    const_cast<void*>(ptr), dims, strides, box, elem_strides, CU_TENSOR_MAP_INTERLEAVE_NONE, swizzle,
+                    CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) == CUDA_SUCCESS;
+}
+
 // NHWC 16-bit activation [B][H][W][C] as a rank-4 TMA tensor {C, W, H, B}, box {32, 8, 4, 1}, 64B swizzle
 bool make_out_map(CUtensorMap* m, void* ptr, int B, int H, int W, int C, bool bf16) {
-  EncodeTiledFn enc = get_encode_tiled();
-  if (!enc) return false;
   const cuuint64_t dims[4] = {cuuint64_t(C), cuuint64_t(W), cuuint64_t(H), cuuint64_t(B)};
   const cuuint64_t strides[3] = {cuuint64_t(C) * 2, cuuint64_t(W) * C * 2, cuuint64_t(H) * W * C * 2};
   const cuuint32_t box[4] = {32, cuuint32_t(kTileW), 4, 1};
-  const cuuint32_t estr[4] = {1, 1, 1, 1};
-  return enc(m, bf16 ? CU_TENSOR_MAP_DATA_TYPE_BFLOAT16 : CU_TENSOR_MAP_DATA_TYPE_FLOAT16, 4, ptr, dims, strides, box,
-             estr, CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_64B, CU_TENSOR_MAP_L2_PROMOTION_L2_128B,
-             CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) == CUDA_SUCCESS;
+  return encode_map(m, ptr, 4, dims, strides, box, kUnitStrides, CU_TENSOR_MAP_SWIZZLE_64B, bf16);
 }
 
 // Output of a phase-decomposed upsample conv: parity (py, px) = (ph >> 1, ph & 1) of the NHWC 16-bit tensor
 // [B][2h][2w][C] viewed as a rank-4 tensor {C, w, h, B} over the low-resolution grid
 bool make_out_map_phase(CUtensorMap* m, void* ptr, int B, int h, int w, int C, int ph, bool bf16) {
-  EncodeTiledFn enc = get_encode_tiled();
-  if (!enc) return false;
   const int Wo = 2 * w, Ho = 2 * h;
   uint8_t* base = static_cast<uint8_t*>(ptr) + (size_t(ph >> 1) * Wo + (ph & 1)) * C * 2;
   const cuuint64_t dims[4] = {cuuint64_t(C), cuuint64_t(w), cuuint64_t(h), cuuint64_t(B)};
   const cuuint64_t strides[3] = {cuuint64_t(C) * 4, cuuint64_t(Wo) * C * 4, cuuint64_t(Ho) * Wo * C * 2};
   const cuuint32_t box[4] = {32, cuuint32_t(kTileW), 4, 1};
-  const cuuint32_t estr[4] = {1, 1, 1, 1};
-  return enc(m, bf16 ? CU_TENSOR_MAP_DATA_TYPE_BFLOAT16 : CU_TENSOR_MAP_DATA_TYPE_FLOAT16, 4, base, dims, strides, box,
-             estr, CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_64B, CU_TENSOR_MAP_L2_PROMOTION_L2_128B,
-             CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) == CUDA_SUCCESS;
+  return encode_map(m, base, 4, dims, strides, box, kUnitStrides, CU_TENSOR_MAP_SWIZZLE_64B, bf16);
 }
 
 // NHWC 16-bit source [B][H][W][C] as a rank-4 TMA tensor {C, W, H, B}, box {64 ch, 10, 34, 1}, 128B swizzle:
@@ -940,44 +987,26 @@ bool make_out_map_phase(CUtensorMap* m, void* ptr, int B, int h, int w, int C, i
 // kind 0: full patch; 1: centre box {64, 8, 32}; 2: space-to-depth plane = box {64, 20, 68} traversed with element
 // strides {1, 2, 2, 1} (every second pixel in x and y: 10 x 34 positions land in shared memory)
 bool make_in_map(CUtensorMap* m, const void* ptr, int B, int H, int W, int C, bool bf16, int kind, int tile_h = kTileH) {
-  EncodeTiledFn enc = get_encode_tiled();
-  if (kind == 3) {  // 16-channel stem input: one 8-channel plane of the patch per load (box {8, 10, 34}), no swizzle
-    if (!enc || C != 16) return false;
-    const cuuint64_t dims[4] = {cuuint64_t(C), cuuint64_t(W), cuuint64_t(H), cuuint64_t(B)};
-    const cuuint64_t strides[3] = {cuuint64_t(C) * 2, cuuint64_t(W) * C * 2, cuuint64_t(H) * W * C * 2};
-    const cuuint32_t box[4] = {8, cuuint32_t(kPatchW), cuuint32_t(kPatchH), 1};
-    const cuuint32_t estr[4] = {1, 1, 1, 1};
-    return enc(m, bf16 ? CU_TENSOR_MAP_DATA_TYPE_BFLOAT16 : CU_TENSOR_MAP_DATA_TYPE_FLOAT16, 4, const_cast<void*>(ptr),
-               dims, strides, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_NONE,
-               CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) == CUDA_SUCCESS;
-  }
-  if (!enc || C < 64) return false;
   const cuuint64_t dims[4] = {cuuint64_t(C), cuuint64_t(W), cuuint64_t(H), cuuint64_t(B)};
   const cuuint64_t strides[3] = {cuuint64_t(C) * 2, cuuint64_t(W) * C * 2, cuuint64_t(H) * W * C * 2};
+  if (kind == 3) {  // 16-channel stem input: one 8-channel plane of the patch per load (box {8, 10, 34}), no swizzle
+    const cuuint32_t box[4] = {8, cuuint32_t(kPatchW), cuuint32_t(kPatchH), 1};
+    return C == 16 && encode_map(m, ptr, 4, dims, strides, box, kUnitStrides, CU_TENSOR_MAP_SWIZZLE_NONE, bf16);
+  }
   const cuuint32_t sc = kind == 2 ? 2 : 1;
   const cuuint32_t box[4] = {64, cuuint32_t(kind == 1 ? kTileW : kPatchW) * sc, cuuint32_t(kind == 1 ? tile_h : tile_h + 2) * sc, 1};
   const cuuint32_t estr[4] = {1, sc, sc, 1};
-  return enc(m, bf16 ? CU_TENSOR_MAP_DATA_TYPE_BFLOAT16 : CU_TENSOR_MAP_DATA_TYPE_FLOAT16, 4, const_cast<void*>(ptr),
-             dims, strides, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B,
-             CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) == CUDA_SUCCESS;
+  return C >= 64 && encode_map(m, ptr, 4, dims, strides, box, estr, CU_TENSOR_MAP_SWIZZLE_128B, bf16);
 }
 
 // [B][HW][C] 16-bit token matrix (an NHWC activation seen as rows of C channels) as a rank-3 TMA tensor
 // {C, HW, B}, box {64 ch, rows, 1}, 128B swizzle: K-major (q, k) / MN-major (v) MMA operand tiles
 bool make_token_map(CUtensorMap* m, const void* ptr, int B, int HW, int C, int rows, bool bf16) {
-  EncodeTiledFn enc = get_encode_tiled();
-  if (!enc) return false;
   const cuuint64_t dims[3] = {cuuint64_t(C), cuuint64_t(HW), cuuint64_t(B)};
   const cuuint64_t strides[2] = {cuuint64_t(C) * 2, cuuint64_t(HW) * C * 2};
   const cuuint32_t box[3] = {64, cuuint32_t(rows), 1};
-  const cuuint32_t estr[3] = {1, 1, 1};
-  return enc(m, bf16 ? CU_TENSOR_MAP_DATA_TYPE_BFLOAT16 : CU_TENSOR_MAP_DATA_TYPE_FLOAT16, 3, const_cast<void*>(ptr),
-             dims, strides, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B,
-             CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) == CUDA_SUCCESS;
+  return encode_map(m, ptr, 3, dims, strides, box, kUnitStrides, CU_TENSOR_MAP_SWIZZLE_128B, bf16);
 }
-
-template <typename T, int C>
-cudaError_t launch_attn_core_tc(const AttnParams& p, int B, int HW, cudaStream_t st);
 
 // SelfAttention cores of the SR3 baseline (16-bit modes): tensor maps of q / k / v at the reserved shape
 int upload_attn(fdsr_ctx* c) {
@@ -996,12 +1025,6 @@ int upload_attn(fdsr_ctx* c) {
     p.out = c->d_ws + c->tensors[a.out].off;
     p.HW = HW;
     p.scale_log2 = 1.4426950408889634f / sqrtf(float(a.C));
-    cudaError_t e = cudaErrorInvalidValue;  // B = 0: only sets the kernel's shared-memory attribute (not capturable)
-    if (a.C == 64) e = bf ? launch_attn_core_tc<__nv_bfloat16, 64>(p, 0, 0, 0) : launch_attn_core_tc<__half, 64>(p, 0, 0, 0);
-    else if (a.C == 128) e = bf ? launch_attn_core_tc<__nv_bfloat16, 128>(p, 0, 0, 0) : launch_attn_core_tc<__half, 128>(p, 0, 0, 0);
-    else if (a.C == 256) e = bf ? launch_attn_core_tc<__nv_bfloat16, 256>(p, 0, 0, 0) : launch_attn_core_tc<__half, 256>(p, 0, 0, 0);
-    if (e != cudaSuccess)
-      return fail(c, FDSR_E_CUDA, "SelfAttention with %d channels: %s", a.C, cudaGetErrorString(e));
   }
   return FDSR_OK;
 }
@@ -1092,14 +1115,11 @@ int launch_conv_f32(fdsr_ctx* c, int li, int t, cudaStream_t st) {
   const HConv& k = c->convs[li];
   const F32Layer& l = c->f_layers[li];
   if (k.gn_C) {
-    f32_gn_table_kernel<<<c->B, 256, 0, st>>>(c->f_gn[li]);
-    ++c->launches;
+    const int rc = launch(c, f32_gn_table_kernel, c->B, 256, 0, st, c->f_gn[li]);
+    if (rc) return rc;
   }
   const int tiles = c->B * ((l.W + kF32Tile - 1) / kF32Tile) * ((l.H + kF32Tile - 1) / kF32Tile);
-  conv_f32_kernel<<<dim3(tiles, (l.N + kF32NBlk - 1) / kF32NBlk), 256, 0, st>>>(l, t);
-  CUDA_TRY(c, cudaGetLastError());
-  ++c->launches;
-  return FDSR_OK;
+  return launch(c, conv_f32_kernel, dim3(tiles, (l.N + kF32NBlk - 1) / kF32NBlk), 256, 0, st, l, t);
 }
 
 int upload_layers(fdsr_ctx* c) {
@@ -1107,7 +1127,7 @@ int upload_layers(fdsr_ctx* c) {
   const int B = c->B, H = c->H, W = c->W;
   const bool bf = c->cfg.dtype == FDSR_DTYPE_BF16;
   if (!c->d_prof) {
-    CUDA_TRY(c, cudaMalloc(&c->d_prof, size_t(c->num_sms) * kProfRoles * 64));
+    CUDA_TRY(c, c->d_prof.grow(size_t(c->num_sms) * kProfRoles * 64));
     CUDA_TRY(c, cudaMemset(c->d_prof, 0, size_t(c->num_sms) * kProfRoles * 64));
   }
   std::vector<ConvLayer> L(c->convs.size());
@@ -1259,6 +1279,10 @@ int upload_layers(fdsr_ctx* c) {
   return FDSR_OK;
 }
 
+// The launch descriptors point into the workspace and the weight, parameter, bias and posterior buffers: rebuilt after
+// any of them moved or changed shape
+int ensure_layers(fdsr_ctx* c) { return c->layers_dirty ? upload_layers(c) : FDSR_OK; }
+
 template <int N, typename T>
 cudaError_t set_conv_attr() {
   cudaError_t e = cudaFuncSetAttribute(conv_gemm_kernel<N, T, false>, cudaFuncAttributeMaxDynamicSharedMemorySize,
@@ -1318,10 +1342,7 @@ int launch_conv_t(fdsr_ctx* c, int li, int t, cudaStream_t st, const ConvLayer* 
   if constexpr (N >= 64) {
     if (pair) kernel = conv_gemm_kernel<N, T, true>;
   }
-  CUDA_TRY(c, cudaLaunchKernelEx(&cfg, kernel, LY, t));
-  CUDA_TRY(c, cudaGetLastError());
-  ++c->launches;
-  return FDSR_OK;
+  return launched(c, cudaLaunchKernelEx(&cfg, kernel, LY, t), reinterpret_cast<const void*>(kernel));
 }
 
 template <typename T>
@@ -1342,18 +1363,13 @@ int launch_conv16(fdsr_ctx* c, int li, int t, cudaStream_t st, const ConvLayer* 
   return fail(c, FDSR_E_INVALID, "unsupported N=%d", k.N);
 }
 
-template <typename T, int C>
-cudaError_t launch_attn_core_tc(const AttnParams& p, int B, int HW, cudaStream_t st) {
-  static bool attr_set = false;  // (set outside stream capture: upload_layers calls this with B = 0 first)
-  if (!attr_set) {
-    cudaError_t e = cudaFuncSetAttribute(attn_core_kernel<T, C>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                         AttnCfg<C>::kSmemBytes);
-    if (e != cudaSuccess) return e;
-    attr_set = true;
-  }
-  if (B == 0) return cudaSuccess;
-  attn_core_kernel<T, C><<<dim3((HW + kAttnQ - 1) / kAttnQ, B), kAttnQ, AttnCfg<C>::kSmemBytes, st>>>(p);
-  return cudaGetLastError();
+// The tensor-core SelfAttention core for C channels (64, 128 or 256) and its dynamic shared memory
+template <typename T>
+std::pair<void (*)(AttnParams), int> attn_core(int C) {
+  if (C == 64) return {attn_core_kernel<T, 64>, AttnCfg<64>::kSmemBytes};
+  if (C == 128) return {attn_core_kernel<T, 128>, AttnCfg<128>::kSmemBytes};
+  if (C == 256) return {attn_core_kernel<T, 256>, AttnCfg<256>::kSmemBytes};
+  return {nullptr, 0};
 }
 
 template <typename T>
@@ -1363,22 +1379,15 @@ int launch_self_attn(fdsr_ctx* c, int ai, cudaStream_t st) {
   const int HW = (c->H >> tq.level) * (c->W >> tq.level), C = a.C;
   if constexpr (sizeof(T) == 2) {
     if (!c->attn_ref) {
-      cudaError_t e = cudaErrorInvalidValue;
-      if (C == 64) e = launch_attn_core_tc<T, 64>(c->a_params[ai], c->B, HW, st);
-      else if (C == 128) e = launch_attn_core_tc<T, 128>(c->a_params[ai], c->B, HW, st);
-      else if (C == 256) e = launch_attn_core_tc<T, 256>(c->a_params[ai], c->B, HW, st);
-      if (e != cudaSuccess) return fail(c, FDSR_E_CUDA, "attention core launch failed: %s", cudaGetErrorString(e));
-      ++c->launches;
-      return FDSR_OK;
+      const auto core = attn_core<T>(C);
+      if (!core.first) return fail(c, FDSR_E_INVALID, "SelfAttention with %d channels", C);
+      return launch(c, core.first, dim3((HW + kAttnQ - 1) / kAttnQ, c->B), kAttnQ, core.second, st, c->a_params[ai]);
     }
   }
-  attn_core_ref_kernel<T><<<dim3((HW + 7) / 8, c->B), 256, 0, st>>>(
-      reinterpret_cast<const T*>(c->d_ws + tq.off), reinterpret_cast<const T*>(c->d_ws + c->tensors[a.tk].off),
-      reinterpret_cast<const T*>(c->d_ws + c->tensors[a.tv].off), reinterpret_cast<T*>(c->d_ws + c->tensors[a.out].off),
-      HW, C, 1.0f / sqrtf(float(C)));
-  CUDA_TRY(c, cudaGetLastError());
-  ++c->launches;
-  return FDSR_OK;
+  return launch(c, attn_core_ref_kernel<T>, dim3((HW + 7) / 8, c->B), 256, 0, st,
+                reinterpret_cast<const T*>(c->d_ws + tq.off), reinterpret_cast<const T*>(c->d_ws + c->tensors[a.tk].off),
+                reinterpret_cast<const T*>(c->d_ws + c->tensors[a.tv].off),
+                reinterpret_cast<T*>(c->d_ws + c->tensors[a.out].off), HW, C, 1.0f / sqrtf(float(C)));
 }
 
 template <typename T>
@@ -1395,29 +1404,26 @@ int launch_attn(fdsr_ctx* c, int ai, cudaStream_t st) {
   float* gate = reinterpret_cast<float*>(c->d_ws + c->off_gate);
   float2* sp = reinterpret_cast<float2*>(c->d_ws + c->off_sp);
   const int ppb = 32;
-  clam_pool_kernel<T><<<dim3((HW + ppb - 1) / ppb, c->B), 128, 0, st>>>(x, psum, pmax, HW, C, ppb);
-  clam_gate_kernel<<<c->B, 256, (2 * C + 2 * R) * 4, st>>>(psum, pmax, c->d_params + a.w1_off,
-                                                         c->d_params + a.w2_off, gate, HW, C, R);
   const int64_t nwarp = int64_t(c->B) * HW;
-  slam_pool_kernel<T><<<unsigned((nwarp * 32 + 255) / 256), 256, 0, st>>>(x, gate, sp, c->B, HW, C);
-  slam_apply_kernel<T><<<dim3((HW + 7) / 8, c->B), 256, 8 * C * 4, st>>>(
-      x, gate, sp, c->d_params + a.w7_off, y, reinterpret_cast<unsigned long long*>(c->d_ws + to.stats_off), h, w, C,
-      stat_sq_scale((long long)h * w));
-  CUDA_TRY(c, cudaGetLastError());
-  c->launches += 4;
-  return FDSR_OK;
+  int rc = launch(c, clam_pool_kernel<T>, dim3((HW + ppb - 1) / ppb, c->B), 128, 0, st, x, psum, pmax, HW, C, ppb);
+  if (!rc)
+    rc = launch(c, clam_gate_kernel, c->B, 256, (2 * C + 2 * R) * 4, st, psum, pmax, c->d_params + a.w1_off,
+                c->d_params + a.w2_off, gate, HW, C, R);
+  if (!rc) rc = launch(c, slam_pool_kernel<T>, unsigned((nwarp * 32 + 255) / 256), 256, 0, st, x, gate, sp, c->B, HW, C);
+  if (!rc)
+    rc = launch(c, slam_apply_kernel<T>, dim3((HW + 7) / 8, c->B), 256, 8 * C * 4, st, x, gate, sp,
+                c->d_params + a.w7_off, y, reinterpret_cast<unsigned long long*>(c->d_ws + to.stats_off), h, w, C,
+                stat_sq_scale((long long)h * w));
+  return rc;
 }
 
 template <typename T>
 int pack_input(fdsr_ctx* c, cudaStream_t st) {
   const int HW = c->H * c->W;
   const int64_t npix = int64_t(c->B) * HW;
-  pack_input_kernel<T><<<unsigned((npix + 255) / 256), 256, 0, st>>>(
-      reinterpret_cast<const float*>(c->d_ws + c->off_cond), reinterpret_cast<const float*>(c->d_ws + c->off_x),
-      reinterpret_cast<T*>(c->d_ws + c->tensors[c->t_xin].off), c->B, HW, c->bands());
-  CUDA_TRY(c, cudaGetLastError());
-  ++c->launches;
-  return FDSR_OK;
+  return launch(c, pack_input_kernel<T>, unsigned((npix + 255) / 256), 256, 0, st,
+                reinterpret_cast<const float*>(c->d_ws + c->off_cond), reinterpret_cast<const float*>(c->d_ws + c->off_x),
+                reinterpret_cast<T*>(c->d_ws + c->tensors[c->t_xin].off), c->B, HW, c->bands());
 }
 
 // One UNet evaluation on the context's internal cond / x buffers.
@@ -1427,19 +1433,17 @@ int pack_input(fdsr_ctx* c, cudaStream_t st) {
 //   packed = true (tiled sampler): the network input was assembled by tile_pack_kernel; eps lands in the eps buffer.
 template <typename T>
 int unet_internal(fdsr_ctx* c, int t, cudaStream_t st, bool fused, bool packed = false) {
-  if (c->layers_dirty) {
-    int rc = upload_layers(c);
-    if (rc) return rc;
-  }
+  int rc = ensure_layers(c);
+  if (rc) return rc;
   CUDA_TRY(c, cudaMemsetAsync(c->d_ws + c->stats_off, 0, c->stats_bytes, st));
   if (!fused && !packed) {
-    int rc = pack_input<T>(c, st);
+    rc = pack_input<T>(c, st);
     if (rc) return rc;
   }
   for (size_t i = 0; i < c->ops.size(); ++i) {
     const HOp& op = c->ops[i];
     const bool last = fused && i + 1 == c->ops.size();
-    int rc = op.kind == 0 ? launch_conv<T>(c, op.idx, t, st, last ? &c->final_fused : nullptr) : launch_attn<T>(c, op.idx, st);
+    rc = op.kind == 0 ? launch_conv<T>(c, op.idx, t, st, last ? &c->final_fused : nullptr) : launch_attn<T>(c, op.idx, st);
     if (rc) return rc;
   }
   return FDSR_OK;
@@ -1447,13 +1451,11 @@ int unet_internal(fdsr_ctx* c, int t, cudaStream_t st, bool fused, bool packed =
 
 // the fused tail exists for the 16-bit tensor-core path of the FastDiffSR model
 bool can_fuse_tail(const fdsr_ctx* c) {
-  return c->fused_tail && c->cfg.dtype != FDSR_DTYPE_FP32 && c->cfg.model == FDSR_MODEL_FASTDIFFSR && c->d_post != nullptr;
+  return c->fused_tail && c->cfg.dtype != FDSR_DTYPE_FP32 && c->cfg.model == FDSR_MODEL_FASTDIFFSR && c->d_post.ptr != nullptr;
 }
 
 int unet_dispatch(fdsr_ctx* c, int t, cudaStream_t st, bool fused = false) {
-  if (c->cfg.dtype == FDSR_DTYPE_FP32) return unet_internal<float>(c, t, st, false);
-  return c->cfg.dtype == FDSR_DTYPE_BF16 ? unet_internal<__nv_bfloat16>(c, t, st, fused)
-                                         : unet_internal<__half>(c, t, st, fused);
+  return with_dtype(c, [&](auto e) { return unet_internal<typename decltype(e)::type>(c, t, st, fused); });
 }
 
 int check_ready(fdsr_ctx* c) {
@@ -1470,65 +1472,67 @@ int posterior_launch(fdsr_ctx* c, const float* x, const float* eps, const float*
   if (numel_img % C || numel_img / C > 0x7fffffffLL || images < 1 || images > 65535)
     return fail(c, FDSR_E_INVALID, "posterior: images are (%d,H,W) blocks, 1..65535 of them", C);
   const uint32_t hw = uint32_t(numel_img / C);
-  posterior_kernel<<<dim3((hw + 255) / 256, images), 256, 0, st>>>(x, eps, z, out, hw, C, c->post[t], args, z_block,
-                                                                    uint32_t(t), t > 0 ? 1 : 0);
-  CUDA_TRY(c, cudaGetLastError());
-  ++c->launches;
-  return FDSR_OK;
+  return launch(c, posterior_kernel, dim3((hw + 255) / 256, images), 256, 0, st, x, eps, z, out, hw, C, c->post[t], args,
+                z_block, uint32_t(t), t > 0 ? 1 : 0);
 }
 
-// The T-step loop on the context's buffers.  Everything that differs between two calls of the same shape (seed,
-// image offset, noise / trace pointers) is read from the SampleArgs slot in device memory.
-int sample_enqueue(fdsr_ctx* c, bool has_trace, cudaStream_t st) {
-  const SampleArgs* args = reinterpret_cast<const SampleArgs*>(c->d_ws + c->off_seed);
-  const int T = c->T, B = c->B;
-  const int64_t per = int64_t(c->bands()) * c->H * c->W, numel = per * B;
-  float* x = reinterpret_cast<float*>(c->d_ws + c->off_x);
-  float* cond = reinterpret_cast<float*>(c->d_ws + c->off_cond);
-  float* eps = reinterpret_cast<float*>(c->d_ws + c->off_eps);
-  float* sr = reinterpret_cast<float*>(c->d_ws + c->off_sr);
-  const int nfr = fdsr_trace_frames(c);
-  const unsigned gb = unsigned((numel + 255) / 256);
-  noise_init_kernel<<<dim3((uint32_t(c->H) * c->W + 255) / 256, B), 256, 0, st>>>(x, uint32_t(c->H) * c->W, c->bands(), args,
-                                                                              uint32_t(T));
-  ++c->launches;
+// Trace frames are written after the steps t with t % trace_every(T) == 0 (and one frame before the first step)
+int trace_every(int T) { return 1 | (T / 10); }
+
+// The T-step chain of both samplers on B images of C x HW values: x_T from the generator, a trace frame before the
+// first step, step(t, k) for the k-th step t = T-1 .. 0, a trace frame after every trace_every(T)-th step, and the
+// result sr.  Everything that differs between two calls of the same shape (seed, image offset, noise / trace pointers)
+// is read from the SampleArgs slot in device memory.
+template <typename Step>
+int sample_chain(fdsr_ctx* c, const SampleArgs* args, float* x, const float* cond, float* sr, int B, uint32_t HW,
+                 bool has_trace, cudaStream_t st, Step&& step) {
+  const int T = c->T, nfr = fdsr_trace_frames(c), inter = trace_every(T);
+  const int64_t per = int64_t(c->bands()) * HW;
+  const unsigned gb = unsigned((per * B + 255) / 256);
   // FastDiffSR predicts the residual: frames and result go through res2img (diffusion.py:213-216, 275-281).
   // The SR3 baseline predicts the image: frames are the raw x, the first frame is the conditioning image itself
   // (ddpm_modules/diffusion.py:218-227).
   const int sr3 = c->cfg.model == FDSR_MODEL_SR3 ? 1 : 0;
+  const dim3 grid(unsigned((uint64_t(HW) + 255) / 256), unsigned(B));
+  int rc = launch(c, noise_init_kernel, grid, 256, 0, st, x, HW, c->bands(), args, uint32_t(T));
+  if (rc) return rc;
   int frame = 0;
   if (has_trace) {
-    res2img_kernel<<<gb, 256, 0, st>>>(cond, cond, nullptr, per, per * nfr, B, args, 0, sr3);
-    ++c->launches;
+    rc = launch(c, res2img_kernel, gb, 256, 0, st, cond, cond, nullptr, per, per * nfr, B, args, 0, sr3);
+    if (rc) return rc;
     frame = 1;
   }
-  const int inter = 1 | (T / 10);
-  const bool fused = can_fuse_tail(c);
-  if (fused) {  // cat[cond, x_T] once; afterwards every step's epilogue rewrites the x channels of the packed input
-    if (c->layers_dirty) {
-      int rc = upload_layers(c);
-      if (rc) return rc;
-    }
-    int rc = c->cfg.dtype == FDSR_DTYPE_BF16 ? pack_input<__nv_bfloat16>(c, st) : pack_input<__half>(c, st);
-    if (rc) return rc;
-  }
   for (int k = 0, t = T - 1; t >= 0; --t, ++k) {
-    int rc = unet_dispatch(c, t, st, fused);
+    rc = step(t, k);
     if (rc) return rc;
-    if (!fused) {
-      rc = posterior_launch(c, x, eps, nullptr, t, x, per, B, args, k + 1, st);
-      if (rc) return rc;
-    }
     if (has_trace && t % inter == 0) {
-      res2img_kernel<<<gb, 256, 0, st>>>(x, cond, nullptr, per, per * nfr, B, args, per * frame, sr3);
-      ++c->launches;
+      rc = launch(c, res2img_kernel, gb, 256, 0, st, x, cond, nullptr, per, per * nfr, B, args, per * frame, sr3);
+      if (rc) return rc;
       ++frame;
     }
   }
-  res2img_kernel<<<gb, 256, 0, st>>>(x, cond, sr, per, per, B, args, 0, sr3);
-  ++c->launches;
-  CUDA_TRY(c, cudaGetLastError());
-  return FDSR_OK;
+  return launch(c, res2img_kernel, gb, 256, 0, st, x, cond, sr, per, per, B, args, 0, sr3);
+}
+
+// The T-step loop on the context's buffers
+int sample_enqueue(fdsr_ctx* c, bool has_trace, cudaStream_t st) {
+  const SampleArgs* args = reinterpret_cast<const SampleArgs*>(c->d_ws + c->off_seed);
+  const int64_t per = int64_t(c->bands()) * c->H * c->W;
+  float* x = reinterpret_cast<float*>(c->d_ws + c->off_x);
+  const float* cond = reinterpret_cast<const float*>(c->d_ws + c->off_cond);
+  const float* eps = reinterpret_cast<const float*>(c->d_ws + c->off_eps);
+  float* sr = reinterpret_cast<float*>(c->d_ws + c->off_sr);
+  const bool fused = can_fuse_tail(c);
+  return sample_chain(c, args, x, cond, sr, c->B, uint32_t(c->H) * c->W, has_trace, st, [&](int t, int k) {
+    int rc = FDSR_OK;
+    if (fused && k == 0) {  // cat[cond, x_T] once; afterwards every step's epilogue rewrites the x channels of the packed input
+      rc = ensure_layers(c);
+      if (!rc) rc = with_dtype16(c, [&](auto e) { return pack_input<typename decltype(e)::type>(c, st); });
+    }
+    if (!rc) rc = unet_dispatch(c, t, st, fused);
+    if (!rc && !fused) rc = posterior_launch(c, x, eps, nullptr, t, x, per, c->B, args, k + 1, st);
+    return rc;
+  });
 }
 
 // One axis of the tile grid (the rule stated in tile_kernels.cuh / include/fdsr.h)
@@ -1548,50 +1552,27 @@ TileAxis make_axis(int L, int t, int overlap) {
 template <typename T>
 int tiled_enqueue(fdsr_ctx* c, const float* cond, float* sr_out, bool has_trace, int B, const TileAxis& ay,
                   const TileAxis& ax, int64_t n_tiles, int64_t n_chunks, int bc, cudaStream_t st) {
-  const SampleArgs* args = reinterpret_cast<const SampleArgs*>(c->d_tiled);
+  const SampleArgs* args = reinterpret_cast<const SampleArgs*>(c->d_tiled.ptr);
   const uint32_t HW = uint32_t(ay.L) * uint32_t(ax.L);
   const int C = c->bands();
-  const int64_t per = int64_t(C) * HW;
   float* x = reinterpret_cast<float*>(c->d_tiled + 256);
-  float* eps_store = reinterpret_cast<float*>(c->d_tiled + 256 + align_up(size_t(per) * B * 4, 256));
+  float* eps_store = reinterpret_cast<float*>(c->d_tiled + 256 + align_up(size_t(C) * HW * B * 4, 256));
   const int64_t tile_floats = int64_t(C) * ay.te * ax.te;
   const size_t chunk_bytes = size_t(bc) * tile_floats * 4;
   const dim3 pgrid(unsigned((uint64_t(HW) + 255) / 256), unsigned(B));
-  const unsigned gb = unsigned((per * B + 255) / 256);
   const unsigned pack_blocks = unsigned((int64_t(bc) * ay.te * ax.te + 255) / 256);
   T* xin = reinterpret_cast<T*>(c->d_ws + c->tensors[c->t_xin].off);
   const float* eps_chunk = reinterpret_cast<const float*>(c->d_ws + c->off_eps);
-  const int T_ = c->T, nfr = fdsr_trace_frames(c), inter = 1 | (T_ / 10);
-  noise_init_kernel<<<pgrid, 256, 0, st>>>(x, HW, C, args, uint32_t(T_));
-  ++c->launches;
-  int frame = 0;
-  if (has_trace) {
-    res2img_kernel<<<gb, 256, 0, st>>>(cond, cond, nullptr, per, per * nfr, B, args, 0, 0);
-    ++c->launches;
-    frame = 1;
-  }
-  for (int k = 0, t = T_ - 1; t >= 0; --t, ++k) {
+  return sample_chain(c, args, x, cond, sr_out, B, HW, has_trace, st, [&](int t, int k) {
     for (int64_t ch = 0; ch < n_chunks; ++ch) {
-      tile_pack_kernel<T><<<pack_blocks, 256, 0, st>>>(cond, x, xin, ay, ax, ch * bc, n_tiles, bc, C);
-      CUDA_TRY(c, cudaGetLastError());
-      ++c->launches;
-      int rc = unet_internal<T>(c, t, st, false, true);
+      int rc = launch(c, tile_pack_kernel<T>, pack_blocks, 256, 0, st, cond, x, xin, ay, ax, ch * bc, n_tiles, bc, C);
+      if (!rc) rc = unet_internal<T>(c, t, st, false, true);
       if (rc) return rc;
       CUDA_TRY(c, cudaMemcpyAsync(eps_store + ch * bc * tile_floats, eps_chunk, chunk_bytes, cudaMemcpyDeviceToDevice, st));
     }
-    tile_blend_posterior_kernel<<<pgrid, 256, 0, st>>>(x, eps_store, ay, ax, C, c->post[t], args, k + 1, uint32_t(t),
-                                                       t > 0 ? 1 : 0);
-    ++c->launches;
-    if (has_trace && t % inter == 0) {
-      res2img_kernel<<<gb, 256, 0, st>>>(x, cond, nullptr, per, per * nfr, B, args, per * frame, 0);
-      ++c->launches;
-      ++frame;
-    }
-  }
-  res2img_kernel<<<gb, 256, 0, st>>>(x, cond, sr_out, per, per, B, args, 0, 0);
-  ++c->launches;
-  CUDA_TRY(c, cudaGetLastError());
-  return FDSR_OK;
+    return launch(c, tile_blend_posterior_kernel, pgrid, 256, 0, st, x, eps_store, ay, ax, C, c->post[t], args, k + 1,
+                  uint32_t(t), t > 0 ? 1 : 0);
+  });
 }
 
 // Pillow precompute_coeffs + normalize_coeffs_8bpc for the bicubic filter, full-image box
@@ -1632,15 +1613,12 @@ int ensure_bic(fdsr_ctx* c, int in, int out) {
     vmin[xx] = xmin;
     vcnt[xx] = xmax;
   }
-  fdsr_ctx::BicTab b{in, out, ksize, nullptr, nullptr, nullptr};
-  CUDA_TRY(c, cudaMalloc(&b.d_min, out * 4));
-  CUDA_TRY(c, cudaMalloc(&b.d_cnt, out * 4));
-  CUDA_TRY(c, cudaMalloc(&b.d_taps, taps.size() * 4));
-  CUDA_TRY(c, cudaMemcpy(b.d_min, vmin.data(), out * 4, cudaMemcpyHostToDevice));
-  CUDA_TRY(c, cudaMemcpy(b.d_cnt, vcnt.data(), out * 4, cudaMemcpyHostToDevice));
-  CUDA_TRY(c, cudaMemcpy(b.d_taps, taps.data(), taps.size() * 4, cudaMemcpyHostToDevice));
-  c->bic.push_back(b);
-  return FDSR_OK;
+  fdsr_ctx::BicTab b{in, out, ksize};
+  int rc = upload(c, b.d_min, vmin);
+  if (!rc) rc = upload(c, b.d_cnt, vcnt);
+  if (!rc) rc = upload(c, b.d_taps, taps);
+  if (!rc) c->bic.push_back(std::move(b));
+  return rc;
 }
 const fdsr_ctx::BicTab* find_bic(const fdsr_ctx* c, int in, int out) {
   for (const auto& b : c->bic)
@@ -1679,7 +1657,7 @@ int fdsr_create(const fdsr_config* cfg, fdsr_ctx** out) {
   c->up_phases = env_hook("FDSR_UP_PHASES", c->up_phases);
   c->fused_tail = env_hook("FDSR_FUSED_TAIL", c->fused_tail);
   c->attn_ref = env_hook("FDSR_ATTN_REF", c->attn_ref);
-  if (cfg->dtype != FDSR_DTYPE_FP16 && cfg->dtype != FDSR_DTYPE_BF16 && cfg->dtype != FDSR_DTYPE_FP32) {
+  if (cfg->dtype < FDSR_DTYPE_FP16 || cfg->dtype > FDSR_DTYPE_FP32) {
     delete c;
     return fail(nullptr, FDSR_E_INVALID, "dtype must be FDSR_DTYPE_FP16, FDSR_DTYPE_BF16 or FDSR_DTYPE_FP32");
   }
@@ -1689,9 +1667,16 @@ int fdsr_create(const fdsr_config* cfg, fdsr_ctx** out) {
     delete c;
     return rc;
   }
-  const cudaError_t ae = cfg->dtype == FDSR_DTYPE_FP32 ? cudaSuccess
-                         : cfg->dtype == FDSR_DTYPE_BF16 ? set_conv_attrs<__nv_bfloat16>()
-                                                         : set_conv_attrs<__half>();
+  // the 16-bit kernels' dynamic shared memory limits (the fp32 parity mode uses static shared memory only)
+  const cudaError_t ae = cfg->dtype == FDSR_DTYPE_FP32 ? cudaSuccess : with_dtype16(c, [&](auto e) {
+    using T = typename decltype(e)::type;
+    cudaError_t r = set_conv_attrs<T>();
+    for (const HAttn& a : c->attns)  // SelfAttention cores of the SR3 baseline
+      if (r == cudaSuccess && a.kind == 1)
+        r = cudaFuncSetAttribute(attn_core<T>(a.C).first, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                 attn_core<T>(a.C).second);
+    return r;
+  });
   if (ae != cudaSuccess) {
     delete c;
     return fail(nullptr, FDSR_E_CUDA, "cudaFuncSetAttribute(max dynamic smem) failed: %s", cudaGetErrorString(ae));
@@ -1703,29 +1688,13 @@ int fdsr_create(const fdsr_config* cfg, fdsr_ctx** out) {
 int fdsr_destroy(fdsr_ctx* c) {
   if (!c) return FDSR_OK;
   c->drop_graphs();
-  cudaFree(c->d_weights);
-  cudaFree(c->d_weights32);
-  cudaFree(c->d_params);
-  cudaFree(c->d_bias);
-  cudaFree(c->d_post);
-  cudaFree(c->d_ws);
-  cudaFree(c->d_prof);
-  cudaFree(c->d_bic_tmp);
-  cudaFree(c->d_metric);
-  cudaFree(c->d_tiled);
   for (auto& sl : c->slot) {
-    cudaFree(sl.d_stage);
     if (sl.h_pin) cudaFreeHost(sl.h_pin);
     if (sl.computed) cudaEventDestroy(sl.computed);
     if (sl.copied) cudaEventDestroy(sl.copied);
   }
   if (c->copy_stream) cudaStreamDestroy(c->copy_stream);
-  for (auto& b : c->bic) {
-    cudaFree(b.d_min);
-    cudaFree(b.d_cnt);
-    cudaFree(b.d_taps);
-  }
-  delete c;
+  delete c;  // and with it every device buffer
   return FDSR_OK;
 }
 
@@ -1766,8 +1735,11 @@ static int finish_load_weights(fdsr_ctx* c) {
     c->weights_loaded = false;
     return rc;
   }
-  rc = c->cfg.dtype == FDSR_DTYPE_FP32 ? pack_weights_f32(c)
-       : c->cfg.dtype == FDSR_DTYPE_BF16 ? pack_weights<__nv_bfloat16>(c) : pack_weights<__half>(c);
+  rc = with_dtype(c, [&](auto e) {
+    using T = typename decltype(e)::type;
+    if constexpr (sizeof(T) == 4) return pack_weights_f32(c);
+    else return pack_weights<T>(c);
+  });
   if (rc) return rc;
   rc = upload_params(c);
   if (rc) return rc;
@@ -1825,11 +1797,9 @@ int fdsr_set_schedule(fdsr_ctx* c, const double* betas, int32_t T) {
   {  // per-step arguments of the fused final-conv epilogue: step t is the (T-1-t)-th of the loop, its z block T-t
     std::vector<PostStep> ps(T);
     for (int t = 0; t < T; ++t) ps[t] = PostStep{c->post[t], T - t, t > 0 ? 1 : 0, {0}};
-    cudaFree(c->d_post);
-    c->d_post = nullptr;
-    CUDA_TRY(c, cudaMalloc(&c->d_post, sizeof(PostStep) * size_t(T)));
-    CUDA_TRY(c, cudaMemcpy(c->d_post, ps.data(), sizeof(PostStep) * size_t(T), cudaMemcpyHostToDevice));
     c->layers_dirty = true;
+    const int rc = upload(c, c->d_post, ps);
+    if (rc) return rc;
   }
   c->drop_graphs();
   return build_bias_tables(c);
@@ -1893,14 +1863,10 @@ int fdsr_reserve(fdsr_ctx* c, int32_t B, int32_t H, int32_t W) {
   off += c->cfg.dtype == FDSR_DTYPE_FP32 ? size_t(B) * kMaxGnC * 8 : 0;
   // grow-only: the captured graphs of other shapes hold pointers into the workspace and stay valid as long as it is
   // not reallocated (alternating shapes / a ragged last batch re-use their graphs)
-  if (off > c->ws_cap) {
+  if (off > c->d_ws.cap) {
     c->drop_graphs();
-    if (c->d_ws) cudaFree(c->d_ws);
-    c->d_ws = nullptr;
-    c->ws_cap = 0;
-    CUDA_TRY(c, cudaMalloc(&c->d_ws, off));
+    CUDA_TRY(c, c->d_ws.grow(off));
     CUDA_TRY(c, cudaMemset(c->d_ws, 0, 256));
-    c->ws_cap = off;
   }
   c->ws_bytes = off;
   c->B = B;
@@ -1947,10 +1913,9 @@ int fdsr_posterior_step(fdsr_ctx* c, const float* xt, const float* eps, const fl
 
 int32_t fdsr_trace_frames(const fdsr_ctx* c) {
   if (!c || c->T == 0) return 0;
-  const int inter = 1 | (c->T / 10);
   int n = 1;
   for (int t = c->T - 1; t >= 0; --t)
-    if (t % inter == 0) ++n;
+    if (t % trace_every(c->T) == 0) ++n;
   return n;
 }
 
@@ -1965,17 +1930,15 @@ int fdsr_sample(fdsr_ctx* c, const float* cond, const float* noise, uint64_t see
   const size_t bytes = size_t(B) * c->bands() * H * W * 4;
   CUDA_TRY(c, cudaMemcpyAsync(c->d_ws + c->off_cond, cond, bytes, cudaMemcpyDeviceToDevice, st));
   // seed, image offset and the noise / trace pointers are read from device memory: one captured graph per shape
-  SampleArgs a{seed, c->image0, noise, trace};
-  set_args_kernel<<<1, 1, 0, st>>>(reinterpret_cast<SampleArgs*>(c->d_ws + c->off_seed), a);
-  ++c->launches;
+  rc = launch(c, set_args_kernel, 1, 1, 0, st, reinterpret_cast<SampleArgs*>(c->d_ws + c->off_seed),
+              SampleArgs{seed, c->image0, noise, trace});
+  if (rc) return rc;
   // a T = 1000 schedule would be a graph of ~10^5 nodes: long schedules are enqueued directly (the host runs
   // far ahead of the device: ~0.3 ms of launch calls per ~5 ms UNet step)
   const bool want_graph = c->use_graph && c->T <= 100;
   if (want_graph) {
-    if (c->layers_dirty) {
-      rc = upload_layers(c);
-      if (rc) return rc;
-    }
+    rc = ensure_layers(c);
+    if (rc) return rc;
     fdsr_ctx::GraphEntry* hit = nullptr;
     for (auto& g : c->graphs)
       if (g.B == B && g.H == H && g.W == W && g.noise == (noise != nullptr) && g.trace == (trace != nullptr)) hit = &g;
@@ -2048,21 +2011,15 @@ int fdsr_sample_tiled(fdsr_ctx* c, const float* cond, const float* noise, uint64
   if (rc) return rc;
   const size_t need = 256 + align_up(size_t(B) * c->bands() * H * W * 4, 256) +
                       size_t(n_chunks) * bc * c->bands() * ay.te * ax.te * 4;
-  if (need > c->tiled_cap) {
-    cudaFree(c->d_tiled);
-    c->d_tiled = nullptr;
-    c->tiled_cap = 0;
-    CUDA_TRY(c, cudaMalloc(&c->d_tiled, need));
-    c->tiled_cap = need;
-  }
+  CUDA_TRY(c, c->d_tiled.grow(need));
   cudaStream_t st = static_cast<cudaStream_t>(stream);
-  set_args_kernel<<<1, 1, 0, st>>>(reinterpret_cast<SampleArgs*>(c->d_tiled), SampleArgs{seed, c->image0, noise, trace});
-  ++c->launches;
-  if (c->cfg.dtype == FDSR_DTYPE_FP32)
-    return tiled_enqueue<float>(c, cond, sr_out, trace != nullptr, B, ay, ax, n_tiles, n_chunks, bc, st);
-  if (c->cfg.dtype == FDSR_DTYPE_BF16)
-    return tiled_enqueue<__nv_bfloat16>(c, cond, sr_out, trace != nullptr, B, ay, ax, n_tiles, n_chunks, bc, st);
-  return tiled_enqueue<__half>(c, cond, sr_out, trace != nullptr, B, ay, ax, n_tiles, n_chunks, bc, st);
+  rc = launch(c, set_args_kernel, 1, 1, 0, st, reinterpret_cast<SampleArgs*>(c->d_tiled.ptr),
+              SampleArgs{seed, c->image0, noise, trace});
+  if (rc) return rc;
+  return with_dtype(c, [&](auto e) {
+    return tiled_enqueue<typename decltype(e)::type>(c, cond, sr_out, trace != nullptr, B, ay, ax, n_tiles, n_chunks, bc,
+                                                     st);
+  });
 }
 
 int fdsr_bicubic_u8(fdsr_ctx* c, const uint8_t* lr, int32_t B, int32_t h, int32_t w, int32_t H, int32_t W,
@@ -2076,20 +2033,13 @@ int fdsr_bicubic_u8(fdsr_ctx* c, const uint8_t* lr, int32_t B, int32_t h, int32_
   const fdsr_ctx::BicTab *th = find_bic(c, w, W), *tv = find_bic(c, h, H);
   const int C = c->bands();
   const size_t tmp = size_t(B) * h * W * C;
-  if (tmp > c->bic_tmp_bytes) {
-    cudaFree(c->d_bic_tmp);
-    c->d_bic_tmp = nullptr;
-    CUDA_TRY(c, cudaMalloc(&c->d_bic_tmp, tmp));
-    c->bic_tmp_bytes = tmp;
-  }
+  CUDA_TRY(c, c->d_bic_tmp.grow(tmp));
   const int64_t n1 = int64_t(B) * h * W, n2 = int64_t(B) * H * W;
-  bicubic_h_kernel<<<unsigned((n1 + 255) / 256), 256, 0, st>>>(lr, c->d_bic_tmp, th->d_min, th->d_cnt, th->d_taps,
-                                                            th->ksize, B, h, w, W, C);
-  bicubic_v_kernel<<<unsigned((n2 + 255) / 256), 256, 0, st>>>(c->d_bic_tmp, out_u8, cond, tv->d_min, tv->d_cnt,
-                                                            tv->d_taps, tv->ksize, B, h, H, W, C);
-  CUDA_TRY(c, cudaGetLastError());
-  c->launches += 2;
-  return FDSR_OK;
+  rc = launch(c, bicubic_h_kernel, unsigned((n1 + 255) / 256), 256, 0, st, lr, c->d_bic_tmp.ptr, th->d_min.ptr,
+              th->d_cnt.ptr, th->d_taps.ptr, th->ksize, B, h, w, W, C);
+  if (rc) return rc;
+  return launch(c, bicubic_v_kernel, unsigned((n2 + 255) / 256), 256, 0, st, c->d_bic_tmp.ptr, out_u8, cond,
+                tv->d_min.ptr, tv->d_cnt.ptr, tv->d_taps.ptr, tv->ksize, B, h, H, W, C);
 }
 
 int fdsr_super_resolve_u8_submit(fdsr_ctx* c, int32_t slot, const uint8_t* lr_host, int32_t B, int32_t h, int32_t w,
@@ -2115,13 +2065,7 @@ int fdsr_super_resolve_u8_submit(fdsr_ctx* c, int32_t slot, const uint8_t* lr_ho
     CUDA_TRY(c, cudaMallocHost(&sl.h_pin, need_pin));
     sl.h_pin_bytes = need_pin;
   }
-  if (need_dev > sl.d_stage_bytes) {
-    cudaFree(sl.d_stage);
-    sl.d_stage = nullptr;
-    sl.d_stage_bytes = 0;
-    CUDA_TRY(c, cudaMalloc(&sl.d_stage, need_dev));
-    sl.d_stage_bytes = need_dev;
-  }
+  CUDA_TRY(c, sl.d_stage.grow(need_dev));
   sl.in_b = in_b;
   sl.out_b = out_b;
   uint8_t* d_lr = sl.d_stage;
@@ -2179,30 +2123,20 @@ int fdsr_sse_u8(fdsr_ctx* c, const float* a, const float* b, int32_t B, int32_t 
   CUDA_TRY(c, cudaMemsetAsync(sse, 0, size_t(B) * 8, st));
   const int64_t per = int64_t(c->bands()) * H * W;
   int gx = int((per + 256 * 8 - 1) / (256 * 8));
-  sse_u8_kernel<<<dim3(gx > 0 ? gx : 1, B), 256, 0, st>>>(a, b, sse, per);
-  CUDA_TRY(c, cudaGetLastError());
-  ++c->launches;
-  return FDSR_OK;
+  return launch(c, sse_u8_kernel, dim3(gx > 0 ? gx : 1, B), 256, 0, st, a, b, sse, per);
 }
 
 int fdsr_metrics_u8(fdsr_ctx* c, const float* a, const float* b, int32_t B, int32_t H, int32_t W, double ergas_scale,
                     double* out, void* stream) {
   if (!c || !a || !b || !out || B < 1 || H < 1 || W < 1) return fail(c, FDSR_E_INVALID, "bad argument");
   cudaStream_t st = static_cast<cudaStream_t>(stream);
-  if (size_t(B) * 32 > c->metric_bytes) {
-    cudaFree(c->d_metric);
-    c->d_metric = nullptr;
-    CUDA_TRY(c, cudaMalloc(&c->d_metric, size_t(B) * 32));
-    c->metric_bytes = size_t(B) * 32;
-  }
+  CUDA_TRY(c, c->d_metric.grow(size_t(B) * 32));
   CUDA_TRY(c, cudaMemsetAsync(c->d_metric, 0, size_t(B) * 32, st));
   const int C = c->bands();
-  metrics_u8_kernel<<<dim3((W + kSsimTile - 1) / kSsimTile, (H + kSsimTile - 1) / kSsimTile, B * C), 256, 0, st>>>(
-      a, b, c->d_metric, H, W, C);
-  metrics_finalize_kernel<<<(B + 127) / 128, 128, 0, st>>>(c->d_metric, out, B, H, W, C, ergas_scale);
-  CUDA_TRY(c, cudaGetLastError());
-  c->launches += 2;
-  return FDSR_OK;
+  const dim3 grid((W + kSsimTile - 1) / kSsimTile, (H + kSsimTile - 1) / kSsimTile, B * C);
+  const int rc = launch(c, metrics_u8_kernel, grid, 256, 0, st, a, b, c->d_metric.ptr, H, W, C);
+  if (rc) return rc;
+  return launch(c, metrics_finalize_kernel, (B + 127) / 128, 128, 0, st, c->d_metric.ptr, out, B, H, W, C, ergas_scale);
 }
 
 int32_t fdsr_debug_num_tensors(const fdsr_ctx* c) { return c ? int32_t(c->tensors.size()) : 0; }
@@ -2219,17 +2153,12 @@ int fdsr_debug_read_tensor(fdsr_ctx* c, const char* name, float* out, int64_t ca
       const int h = c->H >> t.level, w = c->W >> t.level;
       const int64_t n = int64_t(c->B) * h * w * t.C;
       if (cap < n) return fail(c, FDSR_E_INVALID, "capacity too small (%lld needed)", (long long)n);
-      cudaStream_t st = static_cast<cudaStream_t>(stream);
-      if (c->cfg.dtype == FDSR_DTYPE_FP32)
-        nhwc_to_nchw_kernel<float><<<unsigned((n + 255) / 256), 256, 0, st>>>(
-            reinterpret_cast<const float*>(c->d_ws + t.off), out, c->B, h * w, t.C);
-      else if (c->cfg.dtype == FDSR_DTYPE_BF16)
-        nhwc_to_nchw_kernel<__nv_bfloat16><<<unsigned((n + 255) / 256), 256, 0, st>>>(
-            reinterpret_cast<const __nv_bfloat16*>(c->d_ws + t.off), out, c->B, h * w, t.C);
-      else
-        nhwc_to_nchw_kernel<__half><<<unsigned((n + 255) / 256), 256, 0, st>>>(
-            reinterpret_cast<const __half*>(c->d_ws + t.off), out, c->B, h * w, t.C);
-      CUDA_TRY(c, cudaGetLastError());
+      const int rc = with_dtype(c, [&](auto e) {
+        using T = typename decltype(e)::type;
+        return launch(c, nhwc_to_nchw_kernel<T>, unsigned((n + 255) / 256), 256, 0, static_cast<cudaStream_t>(stream),
+                      reinterpret_cast<const T*>(c->d_ws + t.off), out, c->B, h * w, t.C);
+      });
+      if (rc) return rc;
       if (C) *C = t.C;
       if (H) *H = h;
       if (W) *W = w;
@@ -2251,10 +2180,7 @@ static double op_flops(const fdsr_ctx* c, int32_t i, bool executed) {
   if (!c || i < 0 || i >= int(c->ops.size()) || c->ops[i].kind != 0) return 0.0;
   const HConv& k = c->convs[c->ops[i].idx];
   const int lvl = k.out >= 0 ? c->tensors[k.out].level : 0;
-  double macs = 0.0;  // real channels only; identity-residual chunks are bookkeeping, not convolution work
-  for (const HChunk& ch : k.chunks)
-    macs += ch.wname == "@identity" ? 0.0 : double((k.phases == 4 && !executed) ? 9 : ch.taps.size()) * ch.nreal();
-  return 2.0 * macs * k.cout * double(c->B) * (c->H >> lvl) * (c->W >> lvl);
+  return 2.0 * conv_macs(k, executed) * k.cout * double(c->B) * (c->H >> lvl) * (c->W >> lvl);
 }
 double fdsr_debug_op_flops(const fdsr_ctx* c, int32_t i) { return op_flops(c, i, false); }
 double fdsr_debug_op_flops_executed(const fdsr_ctx* c, int32_t i) { return op_flops(c, i, true); }
@@ -2296,21 +2222,19 @@ int fdsr_debug_profile_unet(fdsr_ctx* c, int32_t t, int32_t reps, float* ms_out_
   const int nops = int(c->ops.size());
   if (cap < nops) return fail(c, FDSR_E_INVALID, "capacity too small");
   cudaStream_t st = static_cast<cudaStream_t>(stream);
-  if (c->layers_dirty) {
-    rc = upload_layers(c);
-    if (rc) return rc;
-  }
+  rc = ensure_layers(c);
+  if (rc) return rc;
   std::vector<cudaEvent_t> ev(size_t(nops) * 2 * reps);
   for (auto& e : ev) CUDA_TRY(c, cudaEventCreate(&e));
-  const bool bf = c->cfg.dtype == FDSR_DTYPE_BF16, f32 = c->cfg.dtype == FDSR_DTYPE_FP32;
   for (int r = 0; r < reps; ++r) {
     CUDA_TRY(c, cudaMemsetAsync(c->d_ws + c->stats_off, 0, c->stats_bytes, st));
     for (int i = 0; i < nops; ++i) {
       const HOp& op = c->ops[i];
       CUDA_TRY(c, cudaEventRecord(ev[(size_t(r) * nops + i) * 2], st));
-      if (f32) rc = op.kind == 0 ? launch_conv<float>(c, op.idx, t, st) : launch_attn<float>(c, op.idx, st);
-      else if (op.kind == 0) rc = bf ? launch_conv<__nv_bfloat16>(c, op.idx, t, st) : launch_conv<__half>(c, op.idx, t, st);
-      else rc = bf ? launch_attn<__nv_bfloat16>(c, op.idx, st) : launch_attn<__half>(c, op.idx, st);
+      rc = with_dtype(c, [&](auto e) {
+        using T = typename decltype(e)::type;
+        return op.kind == 0 ? launch_conv<T>(c, op.idx, t, st) : launch_attn<T>(c, op.idx, st);
+      });
       if (rc) return rc;
       CUDA_TRY(c, cudaEventRecord(ev[(size_t(r) * nops + i) * 2 + 1], st));
     }
@@ -2341,14 +2265,11 @@ int fdsr_debug_role_cycles(fdsr_ctx* c, int32_t op, int32_t t, int64_t* out_host
   if (c->cfg.dtype == FDSR_DTYPE_FP32) return fail(c, FDSR_E_INVALID, "role cycles exist for the tensor-core kernel only");
   const int n = c->num_sms * kProfRoles * 8;
   if (cap < n) return fail(c, FDSR_E_INVALID, "capacity too small");
-  if (c->layers_dirty) {
-    rc = upload_layers(c);
-    if (rc) return rc;
-  }
+  rc = ensure_layers(c);
+  if (rc) return rc;
   cudaStream_t st = static_cast<cudaStream_t>(stream);
   CUDA_TRY(c, cudaMemsetAsync(c->d_prof, 0, size_t(n) * 8, st));
-  rc = c->cfg.dtype == FDSR_DTYPE_BF16 ? launch_conv<__nv_bfloat16>(c, c->ops[op].idx, t, st)
-                                        : launch_conv<__half>(c, c->ops[op].idx, t, st);
+  rc = with_dtype16(c, [&](auto e) { return launch_conv<typename decltype(e)::type>(c, c->ops[op].idx, t, st); });
   if (rc) return rc;
   CUDA_TRY(c, cudaMemcpyAsync(out_host, c->d_prof, size_t(n) * 8, cudaMemcpyDeviceToHost, st));
   CUDA_TRY(c, cudaStreamSynchronize(st));
@@ -2366,10 +2287,8 @@ int fdsr_debug_timeline(fdsr_ctx* c, int32_t t, int32_t reps, int64_t* out_host,
   if (c->cfg.dtype == FDSR_DTYPE_FP32) return fail(c, FDSR_E_INVALID, "timelines exist for the tensor-core kernel only");
   const size_t per_op = size_t(c->num_sms) * kProfRoles * 8, n = per_op * c->ops.size();
   if (size_t(cap) < n) return fail(c, FDSR_E_INVALID, "capacity too small");
-  if (c->layers_dirty) {
-    rc = upload_layers(c);
-    if (rc) return rc;
-  }
+  rc = ensure_layers(c);
+  if (rc) return rc;
   cudaStream_t st = static_cast<cudaStream_t>(stream);
   long long* buf = nullptr;
   CUDA_TRY(c, cudaMalloc(&buf, n * 8));
@@ -2421,13 +2340,12 @@ int fdsr_debug_noise(fdsr_ctx* c, float* out, int32_t B, int32_t H, int32_t W, u
   cudaStream_t st = static_cast<cudaStream_t>(stream);
   SampleArgs* slot = nullptr;  // a private argument slot: the workspace may not exist yet
   CUDA_TRY(c, cudaMallocAsync(reinterpret_cast<void**>(&slot), sizeof(SampleArgs), st));
-  set_args_kernel<<<1, 1, 0, st>>>(slot, SampleArgs{seed, first_image, nullptr, nullptr});
   const uint32_t hw = uint32_t(H) * uint32_t(W);
-  noise_init_kernel<<<dim3((hw + 255) / 256, B), 256, 0, st>>>(out, hw, c->bands(), slot, uint32_t(stream_id));
-  CUDA_TRY(c, cudaGetLastError());
+  int rc = launch(c, set_args_kernel, 1, 1, 0, st, slot, SampleArgs{seed, first_image, nullptr, nullptr});
+  if (!rc)
+    rc = launch(c, noise_init_kernel, dim3((hw + 255) / 256, B), 256, 0, st, out, hw, c->bands(), slot, uint32_t(stream_id));
   CUDA_TRY(c, cudaFreeAsync(slot, st));
-  c->launches += 2;
-  return FDSR_OK;
+  return rc;
 }
 
 int64_t fdsr_graph_captures(const fdsr_ctx* c) { return c ? c->graph_captures : 0; }

@@ -74,13 +74,17 @@ class Engine:
             raise cls(f"{what}: {self.lib.fdsr_last_error(self._h).decode()} (code {rc})")
         return rc
 
+    def _call(self, fn_name, *args):
+        """self.lib.<fn_name>(handle, *args) on this engine's device; a negative return code raises."""
+        with torch.cuda.device(self.device):
+            return self._check(getattr(self.lib, fn_name)(self._h, *args), fn_name)
+
     def check_overflow(self):
         """fp16 mode: synchronise the current stream and raise FdsrOverflowError if an activation left the fp16 range
         since the last check (the value was stored saturated; the result is not the network's output)."""
         if self.dtype not in ("fp16", "float16"):
             return
-        with torch.cuda.device(self.device):
-            self._check(self.lib.fdsr_check_overflow(self._h, self._stream()), "fdsr_check_overflow")
+        self._call("fdsr_check_overflow", self._stream())
 
     def _stream(self):
         return C.c_void_p(torch.cuda.current_stream(self.device).cuda_stream)
@@ -97,23 +101,19 @@ class Engine:
         names = (C.c_char_p * n)(*[k.encode() for k, _ in items])
         ptrs = (C.c_void_p * n)(*[v.data_ptr() for _, v in items])
         numels = (C.c_int64 * n)(*[v.numel() for _, v in items])
-        with torch.cuda.device(self.device):
-            if on_dev:
-                self._check(self.lib.fdsr_load_weights_dev(self._h, names, ptrs, numels, n, self._stream()),
-                            "fdsr_load_weights_dev")
-            else:
-                self._check(self.lib.fdsr_load_weights(self._h, names, ptrs, numels, n), "fdsr_load_weights")
+        if on_dev:
+            self._call("fdsr_load_weights_dev", names, ptrs, numels, n, self._stream())
+        else:
+            self._call("fdsr_load_weights", names, ptrs, numels, n)
 
     def set_schedule(self, betas):
         b = np.ascontiguousarray(np.asarray(betas, dtype=np.float64))
-        with torch.cuda.device(self.device):
-            self._check(self.lib.fdsr_set_schedule(self._h, b.ctypes.data_as(C.POINTER(C.c_double)), len(b)),
-                        "fdsr_set_schedule")
+        self._call("fdsr_set_schedule", b.ctypes.data_as(C.POINTER(C.c_double)), len(b))
         self.T = len(b)
 
     def table(self, name: str):
         buf = (C.c_double * (self.T + 1))()
-        n = self._check(self.lib.fdsr_get_table(self._h, name.encode(), buf, self.T + 1), "fdsr_get_table")
+        n = self._call("fdsr_get_table", name.encode(), buf, self.T + 1)
         return np.array(buf[:n], dtype=np.float64)
 
     # ---- compute
@@ -126,27 +126,22 @@ class Engine:
         cond, x_t = self._img(cond, "cond"), self._img(x_t, "x_t")
         B, _, H, W = cond.shape
         out = torch.empty_like(cond)
-        with torch.cuda.device(self.device):
-            self._check(self.lib.fdsr_unet_forward(self._h, _ptr(cond), _ptr(x_t), t, _ptr(out), B, H, W,
-                                                   self._stream()), "fdsr_unet_forward")
+        self._call("fdsr_unet_forward", _ptr(cond), _ptr(x_t), t, _ptr(out), B, H, W, self._stream())
         return out
 
     def posterior_step(self, x_t, eps, z, t: int):
         x_t, eps = x_t.contiguous(), eps.contiguous()
         z = z.contiguous() if z is not None else None
         out = torch.empty_like(x_t)
-        with torch.cuda.device(self.device):
-            self._check(self.lib.fdsr_posterior_step(self._h, _ptr(x_t), _ptr(eps), _ptr(z), t, _ptr(out),
-                                                     x_t.numel(), self._stream()), "fdsr_posterior_step")
+        self._call("fdsr_posterior_step", _ptr(x_t), _ptr(eps), _ptr(z), t, _ptr(out), x_t.numel(), self._stream())
         return out
 
     def trace_frames(self):
         return self.lib.fdsr_trace_frames(self._h)
 
-    def sample(self, cond, noise=None, seed: int = 0, trace: bool = False, image_offset: int = 0):
-        """T-step sampling of a batch.  `image_offset` = global index of cond[0] in the whole job: the built-in noise of
-        an image depends on (seed, global index, step) only, so shards of a job reproduce the unsharded result."""
-        self._check(self.lib.fdsr_set_image_offset(self._h, int(image_offset)), "fdsr_set_image_offset")
+    def _sample_io(self, cond, noise, trace, image_offset):
+        """The preamble of sample / sample_tiled: image offset, checked inputs, output and trace tensors."""
+        self._call("fdsr_set_image_offset", int(image_offset))
         cond = self._img(cond, "cond")
         B, _, H, W = cond.shape
         if noise is not None:
@@ -155,9 +150,14 @@ class Engine:
             noise = noise.contiguous()
         out = torch.empty_like(cond)
         tr = torch.empty((B, self.trace_frames(), self.C, H, W), device=self.device, dtype=torch.float32) if trace else None
-        with torch.cuda.device(self.device):
-            self._check(self.lib.fdsr_sample(self._h, _ptr(cond), _ptr(noise), seed, _ptr(out), _ptr(tr), B, H, W,
-                                             self._stream()), "fdsr_sample")
+        return cond, noise, out, tr
+
+    def sample(self, cond, noise=None, seed: int = 0, trace: bool = False, image_offset: int = 0):
+        """T-step sampling of a batch.  `image_offset` = global index of cond[0] in the whole job: the built-in noise of
+        an image depends on (seed, global index, step) only, so shards of a job reproduce the unsharded result."""
+        cond, noise, out, tr = self._sample_io(cond, noise, trace, image_offset)
+        B, _, H, W = cond.shape
+        self._call("fdsr_sample", _ptr(cond), _ptr(noise), seed, _ptr(out), _ptr(tr), B, H, W, self._stream())
         return (out, tr) if trace else out
 
     def sample_tiled(self, cond, tile, overlap: int = 32, tile_batch: int = 16, noise=None, seed: int = 0,
@@ -166,19 +166,10 @@ class Engine:
         (fdsr_sample_tiled).  `tile`: int or (th, tw), multiples of 8; `tile_batch`: tiles per UNet call (the activation
         workspace scales with it, not with the canvas).  Noise, seed, image_offset and the trace are as in `sample`."""
         th, tw = (tile, tile) if isinstance(tile, int) else (int(tile[0]), int(tile[1]))
-        self._check(self.lib.fdsr_set_image_offset(self._h, int(image_offset)), "fdsr_set_image_offset")
-        cond = self._img(cond, "cond")
+        cond, noise, out, tr = self._sample_io(cond, noise, trace, image_offset)
         B, _, H, W = cond.shape
-        if noise is not None:
-            if tuple(noise.shape) != (self.T, B, self.C, H, W) or noise.dtype != torch.float32 or noise.device != self.device:
-                raise FdsrError(f"noise must be ({self.T},{B},{self.C},{H},{W}) fp32 on {self.device}")
-            noise = noise.contiguous()
-        out = torch.empty_like(cond)
-        tr = torch.empty((B, self.trace_frames(), self.C, H, W), device=self.device, dtype=torch.float32) if trace else None
-        with torch.cuda.device(self.device):
-            self._check(self.lib.fdsr_sample_tiled(self._h, _ptr(cond), _ptr(noise), seed, _ptr(out), _ptr(tr), B, H, W,
-                                                   th, tw, int(overlap), int(tile_batch), self._stream()),
-                        "fdsr_sample_tiled")
+        self._call("fdsr_sample_tiled", _ptr(cond), _ptr(noise), seed, _ptr(out), _ptr(tr), B, H, W, th, tw,
+                   int(overlap), int(tile_batch), self._stream())
         return (out, tr) if trace else out
 
     def bicubic_u8(self, lr_u8, H: int, W: int, want_u8=True, want_cond=True):
@@ -189,17 +180,13 @@ class Engine:
         B, h, w, _ = lr_u8.shape
         o8 = torch.empty((B, H, W, self.C), dtype=torch.uint8, device=self.device) if want_u8 else None
         oc = torch.empty((B, self.C, H, W), dtype=torch.float32, device=self.device) if want_cond else None
-        with torch.cuda.device(self.device):
-            self._check(self.lib.fdsr_bicubic_u8(self._h, _ptr(lr_u8), B, h, w, H, W, _ptr(o8), _ptr(oc),
-                                                 self._stream()), "fdsr_bicubic_u8")
+        self._call("fdsr_bicubic_u8", _ptr(lr_u8), B, h, w, H, W, _ptr(o8), _ptr(oc), self._stream())
         return o8, oc
 
     def debug_noise(self, B: int, H: int, W: int, seed: int, stream_id: int, image_offset: int = 0):
         """(B,C,H,W) N(0,1) values of the built-in generator for step stream `stream_id` (T: x_T, t: z of step t)."""
         out = torch.empty((B, self.C, H, W), dtype=torch.float32, device=self.device)
-        with torch.cuda.device(self.device):
-            self._check(self.lib.fdsr_debug_noise(self._h, _ptr(out), B, H, W, int(seed), int(image_offset),
-                                                  int(stream_id), self._stream()), "fdsr_debug_noise")
+        self._call("fdsr_debug_noise", _ptr(out), B, H, W, int(seed), int(image_offset), int(stream_id), self._stream())
         return out
 
     def graph_captures(self):
@@ -221,11 +208,9 @@ class Engine:
             out = np.empty((B, self.C, H, W), dtype=np.float32)
         elif out.shape != (B, self.C, H, W) or out.dtype != np.float32 or not out.flags["C_CONTIGUOUS"]:
             raise FdsrError(f"out must be a C-contiguous float32 array of shape {(B, self.C, H, W)}")
-        self._check(self.lib.fdsr_set_image_offset(self._h, int(image_offset)), "fdsr_set_image_offset")
-        with torch.cuda.device(self.device):
-            self._check(self.lib.fdsr_super_resolve_u8(self._h, lr_host.ctypes.data_as(C.c_void_p), B, h, w, H, W,
-                                                       _ptr(noise), seed, out.ctypes.data_as(C.c_void_p),
-                                                       self._stream()), "fdsr_super_resolve_u8")
+        self._call("fdsr_set_image_offset", int(image_offset))
+        self._call("fdsr_super_resolve_u8", lr_host.ctypes.data_as(C.c_void_p), B, h, w, H, W, _ptr(noise), seed,
+                   out.ctypes.data_as(C.c_void_p), self._stream())
         return out
 
     def super_resolve_u8_submit(self, slot: int, lr_host: np.ndarray, H: int, W: int, noise=None, seed: int = 0,
@@ -233,29 +218,23 @@ class Engine:
         """Pipelined host path: enqueue one batch into `slot` (0 / 1) and return; see super_resolve_u8_wait."""
         lr_host = self._host_u8(lr_host)
         B, h, w, _ = lr_host.shape
-        self._check(self.lib.fdsr_set_image_offset(self._h, int(image_offset)), "fdsr_set_image_offset")
-        with torch.cuda.device(self.device):
-            self._check(self.lib.fdsr_super_resolve_u8_submit(self._h, slot, lr_host.ctypes.data_as(C.c_void_p), B, h, w, H, W,
-                                                              _ptr(noise), seed, self._stream()),
-                        "fdsr_super_resolve_u8_submit")
+        self._call("fdsr_set_image_offset", int(image_offset))
+        self._call("fdsr_super_resolve_u8_submit", slot, lr_host.ctypes.data_as(C.c_void_p), B, h, w, H, W, _ptr(noise),
+                   seed, self._stream())
         return (B, self.C, H, W)
 
     def super_resolve_u8_wait(self, slot: int, out: np.ndarray):
         """Block until the batch in `slot` is on the host; fills the C-contiguous float32 array `out`."""
         if out.dtype != np.float32 or not out.flags["C_CONTIGUOUS"]:
             raise FdsrError("out must be a C-contiguous float32 array")
-        with torch.cuda.device(self.device):
-            self._check(self.lib.fdsr_super_resolve_u8_wait(self._h, slot, out.ctypes.data_as(C.c_void_p)),
-                        "fdsr_super_resolve_u8_wait")
+        self._call("fdsr_super_resolve_u8_wait", slot, out.ctypes.data_as(C.c_void_p))
         return out
 
     def sse_u8(self, a, b):
         a, b = self._img(a, "a"), self._img(b, "b")
         B, _, H, W = a.shape
         out = torch.empty(B, dtype=torch.float64, device=self.device)
-        with torch.cuda.device(self.device):
-            self._check(self.lib.fdsr_sse_u8(self._h, _ptr(a), _ptr(b), B, H, W, _ptr(out), self._stream()),
-                        "fdsr_sse_u8")
+        self._call("fdsr_sse_u8", _ptr(a), _ptr(b), B, H, W, _ptr(out), self._stream())
         return out
 
     def metrics_u8(self, a, b, scale: float = 4.0):
@@ -264,9 +243,7 @@ class Engine:
         a, b = self._img(a, "a"), self._img(b, "b")
         B, _, H, W = a.shape
         out = torch.empty((B, 4), dtype=torch.float64, device=self.device)
-        with torch.cuda.device(self.device):
-            self._check(self.lib.fdsr_metrics_u8(self._h, _ptr(a), _ptr(b), B, H, W, float(scale), _ptr(out),
-                                                 self._stream()), "fdsr_metrics_u8")
+        self._call("fdsr_metrics_u8", _ptr(a), _ptr(b), B, H, W, float(scale), _ptr(out), self._stream())
         return out
 
     # ---- hooks
@@ -277,9 +254,8 @@ class Engine:
     def read_tensor(self, name: str, B: int, max_elems: int):
         buf = torch.empty(max_elems, dtype=torch.float32, device=self.device)
         c, h, w = C.c_int32(), C.c_int32(), C.c_int32()
-        with torch.cuda.device(self.device):
-            self._check(self.lib.fdsr_debug_read_tensor(self._h, name.encode(), _ptr(buf), max_elems, C.byref(c),
-                                                        C.byref(h), C.byref(w), self._stream()), "fdsr_debug_read_tensor")
+        self._call("fdsr_debug_read_tensor", name.encode(), _ptr(buf), max_elems, C.byref(c), C.byref(h), C.byref(w),
+                   self._stream())
         n = B * c.value * h.value * w.value
         return buf[:n].view(B, c.value, h.value, w.value)
 
@@ -297,16 +273,14 @@ class Engine:
     def op_schedule(self, op: int):
         """The launch schedule of conv op `op` at the shape of the last forward (fdsr_debug_op_schedule), as a dict."""
         buf = (C.c_int32 * len(self.OP_SCHEDULE_FIELDS))()
-        n = self._check(self.lib.fdsr_debug_op_schedule(self._h, op, buf, len(buf)), "fdsr_debug_op_schedule")
+        n = self._call("fdsr_debug_op_schedule", op, buf, len(buf))
         return dict(zip(self.OP_SCHEDULE_FIELDS, buf[:n]))
 
     def profile_unet(self, t: int, reps: int = 3):
         """[(op name, mean ms, algorithmic conv FLOPs)] for one UNet evaluation at the current shape."""
         n = self.lib.fdsr_debug_num_ops(self._h)
         ms = (C.c_float * n)()
-        with torch.cuda.device(self.device):
-            self._check(self.lib.fdsr_debug_profile_unet(self._h, t, reps, ms, n, self._stream()),
-                        "fdsr_debug_profile_unet")
+        self._call("fdsr_debug_profile_unet", t, reps, ms, n, self._stream())
         return [(self.lib.fdsr_debug_op_name(self._h, i).decode(), float(ms[i]),
                  float(self.lib.fdsr_debug_op_flops(self._h, i))) for i in range(n)]
 
@@ -314,9 +288,7 @@ class Engine:
         """(n_cta, 5 roles, 8 slots) cycle counters of conv op `op` (FDSR_PROFILE builds only)."""
         n = 148 * 40 * 2
         buf = (C.c_int64 * n)()
-        with torch.cuda.device(self.device):
-            m = self._check(self.lib.fdsr_debug_role_cycles(self._h, op, t, buf, n, self._stream()),
-                            "fdsr_debug_role_cycles")
+        m = self._call("fdsr_debug_role_cycles", op, t, buf, n, self._stream())
         return np.array(buf[:m], dtype=np.int64).reshape(-1, 5, 8)
 
     def timeline(self, t: int = 0, reps: int = 3):
@@ -325,9 +297,7 @@ class Engine:
         nops = int(self.lib.fdsr_debug_num_ops(self._h))
         nsm = torch.cuda.get_device_properties(self.device).multi_processor_count
         out = np.zeros((nops, nsm, 5, 8), dtype=np.int64)
-        with torch.cuda.device(self.device):
-            self._check(self.lib.fdsr_debug_timeline(self._h, t, reps, out.ctypes.data_as(C.POINTER(C.c_int64)), out.size,
-                                                     self._stream()), "fdsr_debug_timeline")
+        self._call("fdsr_debug_timeline", t, reps, out.ctypes.data_as(C.POINTER(C.c_int64)), out.size, self._stream())
         return out
 
     def launch_count(self):
@@ -337,8 +307,7 @@ class Engine:
         return float(self.lib.fdsr_unet_flops(self._h))
 
     def reserve(self, B, H, W):
-        with torch.cuda.device(self.device):
-            self._check(self.lib.fdsr_reserve(self._h, B, H, W), "fdsr_reserve")
+        self._call("fdsr_reserve", B, H, W)
 
     def workspace_bytes(self):
         return int(self.lib.fdsr_workspace_bytes(self._h))
