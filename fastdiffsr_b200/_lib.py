@@ -36,6 +36,9 @@ class FdsrOverflowError(FdsrError, FloatingPointError):
 
 E_OVERFLOW = -5
 
+# fdsr_tile_exchange_fn: int (*)(void* user, int32_t step, void* stream)
+TILE_EXCHANGE_FN = C.CFUNCTYPE(C.c_int, C.c_void_p, C.c_int32, C.c_void_p)
+
 
 def build_library(force: bool = False, verbose: bool = False) -> str:
     """Compile libfdsr.so in-tree with nvcc for sm_100a (cross-compiles without a GPU)."""
@@ -74,6 +77,11 @@ _SIGS = {
     "fdsr_sample_tiled": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint64, C.c_void_p, C.c_void_p,
                                     C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.c_int32,
                                     C.c_void_p]),
+    "fdsr_tiled_plan": (C.c_int64, [C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.c_int32,
+                                    C.c_int32, C.POINTER(C.c_int64), C.c_int64]),
+    "fdsr_sample_tiled_part": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint64, C.c_void_p, C.c_void_p,
+                                         C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.c_int32,
+                                         C.c_int32, C.c_int32, C.c_void_p, TILE_EXCHANGE_FN, C.c_void_p, C.c_void_p]),
     "fdsr_trace_frames": (C.c_int32, [C.c_void_p]),
     "fdsr_super_resolve_u8": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int32, C.c_int32, C.c_int32, C.c_int32,
                                         C.c_int32, C.c_void_p, C.c_uint64, C.c_void_p, C.c_void_p]),

@@ -1479,13 +1479,20 @@ int posterior_launch(fdsr_ctx* c, const float* x, const float* eps, const float*
 // Trace frames are written after the steps t with t % trace_every(T) == 0 (and one frame before the first step)
 int trace_every(int T) { return 1 | (T / 10); }
 
+// The part of a tiled canvas one rank writes (fdsr_sample_tiled_part): the pixels whose first covering tile lies in the
+// own range [g0, g1); res2img_owned_kernel writes +0.0 everywhere else
+struct TileOwner {
+  TileAxis ay, ax;
+  int64_t g0, g1;
+};
+
 // The T-step chain of both samplers on B images of C x HW values: x_T from the generator, a trace frame before the
 // first step, step(t, k) for the k-th step t = T-1 .. 0, a trace frame after every trace_every(T)-th step, and the
 // result sr.  Everything that differs between two calls of the same shape (seed, image offset, noise / trace pointers)
-// is read from the SampleArgs slot in device memory.
+// is read from the SampleArgs slot in device memory.  owner != nullptr: frames and result at the owner's pixels only.
 template <typename Step>
 int sample_chain(fdsr_ctx* c, const SampleArgs* args, float* x, const float* cond, float* sr, int B, uint32_t HW,
-                 bool has_trace, cudaStream_t st, Step&& step) {
+                 bool has_trace, cudaStream_t st, Step&& step, const TileOwner* owner = nullptr) {
   const int T = c->T, nfr = fdsr_trace_frames(c), inter = trace_every(T);
   const int64_t per = int64_t(c->bands()) * HW;
   const unsigned gb = unsigned((per * B + 255) / 256);
@@ -1494,11 +1501,17 @@ int sample_chain(fdsr_ctx* c, const SampleArgs* args, float* x, const float* con
   // (ddpm_modules/diffusion.py:218-227).
   const int sr3 = c->cfg.model == FDSR_MODEL_SR3 ? 1 : 0;
   const dim3 grid(unsigned((uint64_t(HW) + 255) / 256), unsigned(B));
+  auto res2img = [&](const float* src, float* out, int64_t bstride, int64_t frame_off) {
+    if (owner)
+      return launch(c, res2img_owned_kernel, grid, 256, 0, st, src, cond, out, bstride, c->bands(), owner->ay, owner->ax,
+                    owner->g0, owner->g1, args, frame_off);
+    return launch(c, res2img_kernel, gb, 256, 0, st, src, cond, out, per, bstride, B, args, frame_off, sr3);
+  };
   int rc = launch(c, noise_init_kernel, grid, 256, 0, st, x, HW, c->bands(), args, uint32_t(T));
   if (rc) return rc;
   int frame = 0;
   if (has_trace) {
-    rc = launch(c, res2img_kernel, gb, 256, 0, st, cond, cond, nullptr, per, per * nfr, B, args, 0, sr3);
+    rc = res2img(cond, nullptr, per * nfr, 0);
     if (rc) return rc;
     frame = 1;
   }
@@ -1506,12 +1519,12 @@ int sample_chain(fdsr_ctx* c, const SampleArgs* args, float* x, const float* con
     rc = step(t, k);
     if (rc) return rc;
     if (has_trace && t % inter == 0) {
-      rc = launch(c, res2img_kernel, gb, 256, 0, st, x, cond, nullptr, per, per * nfr, B, args, per * frame, sr3);
+      rc = res2img(x, nullptr, per * nfr, per * frame);
       if (rc) return rc;
       ++frame;
     }
   }
-  return launch(c, res2img_kernel, gb, 256, 0, st, x, cond, sr, per, per, B, args, 0, sr3);
+  return res2img(x, sr, per, 0);
 }
 
 // The T-step loop on the context's buffers
@@ -1546,33 +1559,121 @@ TileAxis make_axis(int L, int t, int overlap) {
   return a;
 }
 
-// The T-step tiled loop.  d_tiled holds [SampleArgs | x (B,C,H,W) | eps store of n_chunks * bc tile slots]; the
-// workspace is reserved for one chunk (bc tiles of te_y x te_x).  Plain stream launches: a chunk's UNet (~5 ms at
-// bc = 16, 256^2) keeps the device well behind the host's ~0.3 ms of launch calls.
+// Chunking of a range of `tiles` tiles: n = ceil(tiles / tile_batch) UNet calls of bc = ceil(tiles / n) tiles each (the
+// last one padded with repeats of the range's last tile), so every call has the same shape
+struct TileChunks {
+  int64_t n;
+  int bc;
+};
+TileChunks tile_chunks(int64_t tiles, int tile_batch) {
+  const int64_t n = (tiles + tile_batch - 1) / tile_batch;
+  return {n, n ? int((tiles + n - 1) / n) : 0};
+}
+
+// The T-step tiled loop over the own tiles [g0, g1) of B canvases.  d_tiled holds [SampleArgs | x (B,C,H,W) | ...]; the
+// workspace is reserved for one chunk (bc tiles of te_y x te_x); eps_store is indexed by global tile.  Per step: the
+// own tiles' eps into the store, chunk by chunk, then exchange(user, t, st) when given, then the blend of the pixels the
+// own tiles cover.  fdsr_sample_tiled: [0, n_tiles), no exchange, no owner.  Plain stream launches: a chunk's UNet (~5 ms
+// at bc = 16, 256^2) keeps the device well behind the host's ~0.3 ms of launch calls.
 template <typename T>
 int tiled_enqueue(fdsr_ctx* c, const float* cond, float* sr_out, bool has_trace, int B, const TileAxis& ay,
-                  const TileAxis& ax, int64_t n_tiles, int64_t n_chunks, int bc, cudaStream_t st) {
+                  const TileAxis& ax, int64_t g0, int64_t g1, const TileChunks& ch, float* eps_store,
+                  fdsr_tile_exchange_fn exchange, void* user, const TileOwner* owner, cudaStream_t st) {
   const SampleArgs* args = reinterpret_cast<const SampleArgs*>(c->d_tiled.ptr);
   const uint32_t HW = uint32_t(ay.L) * uint32_t(ax.L);
   const int C = c->bands();
   float* x = reinterpret_cast<float*>(c->d_tiled + 256);
-  float* eps_store = reinterpret_cast<float*>(c->d_tiled + 256 + align_up(size_t(C) * HW * B * 4, 256));
   const int64_t tile_floats = int64_t(C) * ay.te * ax.te;
-  const size_t chunk_bytes = size_t(bc) * tile_floats * 4;
-  const dim3 pgrid(unsigned((uint64_t(HW) + 255) / 256), unsigned(B));
-  const unsigned pack_blocks = unsigned((int64_t(bc) * ay.te * ax.te + 255) / 256);
-  T* xin = reinterpret_cast<T*>(c->d_ws + c->tensors[c->t_xin].off);
-  const float* eps_chunk = reinterpret_cast<const float*>(c->d_ws + c->off_eps);
-  return sample_chain(c, args, x, cond, sr_out, B, HW, has_trace, st, [&](int t, int k) {
-    for (int64_t ch = 0; ch < n_chunks; ++ch) {
-      int rc = launch(c, tile_pack_kernel<T>, pack_blocks, 256, 0, st, cond, x, xin, ay, ax, ch * bc, n_tiles, bc, C);
-      if (!rc) rc = unet_internal<T>(c, t, st, false, true);
-      if (rc) return rc;
-      CUDA_TRY(c, cudaMemcpyAsync(eps_store + ch * bc * tile_floats, eps_chunk, chunk_bytes, cudaMemcpyDeviceToDevice, st));
+  const unsigned pack_blocks = unsigned((int64_t(ch.bc) * ay.te * ax.te + 255) / 256);
+  T* xin = ch.bc ? reinterpret_cast<T*>(c->d_ws + c->tensors[c->t_xin].off) : nullptr;
+  const float* eps_chunk = ch.bc ? reinterpret_cast<const float*>(c->d_ws + c->off_eps) : nullptr;
+  // the band of canvases / pixel indices that holds every pixel the own tiles cover: the rows of the range's windows
+  // when it lies in one canvas, else its canvases whole (an empty range: one block that updates nothing)
+  const int64_t per_canvas = int64_t(ay.n) * ax.n;
+  int b0 = 0, nb = B;
+  uint32_t p0 = 0, p1 = HW;
+  if (g0 == g1) {
+    nb = 1, p1 = 0;
+  } else if (g0 / per_canvas == (g1 - 1) / per_canvas) {
+    b0 = int(g0 / per_canvas), nb = 1;
+    p0 = uint32_t(tile_start(ay, int(g0 % per_canvas / ax.n))) * uint32_t(ax.L);
+    p1 = uint32_t(tile_start(ay, int((g1 - 1) % per_canvas / ax.n)) + ay.te) * uint32_t(ax.L);
+  } else if (g0 != 0 || g1 != int64_t(B) * per_canvas) {
+    b0 = int(g0 / per_canvas), nb = int((g1 - 1) / per_canvas) - b0 + 1;
+  }
+  const dim3 pgrid(std::max(1u, unsigned((uint64_t(p1 - p0) + 255) / 256)), unsigned(nb));
+  return sample_chain(
+      c, args, x, cond, sr_out, B, HW, has_trace, st,
+      [&](int t, int k) {
+        for (int64_t i = 0; i < ch.n; ++i) {
+          const int64_t tile0 = g0 + i * ch.bc, valid = std::min<int64_t>(ch.bc, g1 - tile0);
+          int rc = launch(c, tile_pack_kernel<T>, pack_blocks, 256, 0, st, cond, x, xin, ay, ax, tile0, g1 - 1, ch.bc, C);
+          if (!rc) rc = unet_internal<T>(c, t, st, false, true);
+          if (rc) return rc;
+          // padding slots repeat the last own tile and stay in the workspace: the store holds other ranks' slots
+          CUDA_TRY(c, cudaMemcpyAsync(eps_store + tile0 * tile_floats, eps_chunk, size_t(valid) * tile_floats * 4,
+                                      cudaMemcpyDeviceToDevice, st));
+        }
+        if (exchange) {
+          const int e = exchange(user, t, st);
+          if (e) return fail(c, FDSR_E_INVALID, "the tile exchange callback returned %d at step t = %d", e, t);
+        }
+        return launch(c, tile_blend_posterior_kernel, pgrid, 256, 0, st, x, eps_store, ay, ax, C, c->post[t], args,
+                      int64_t(k + 1), uint32_t(t), t > 0 ? 1 : 0, B, b0, p0, p1, g0, g1);
+      },
+      owner);
+}
+
+// The partition and need rule of fdsr_tiled_plan (include/fdsr.h).  Rank r owns [own_lo(r), own_lo(r + 1)).
+int64_t own_lo(int64_t n, int world, int r) {
+  return int64_t((unsigned __int128)n * unsigned(r) / unsigned(world));
+}
+
+// [lo, hi]: the tiles of one axis whose windows intersect the positions [s, e) (their starts ascend, so they are
+// contiguous); lo > hi when there are none
+void axis_hits(const TileAxis& a, int s, int e, int& lo, int& hi) {
+  lo = a.n, hi = -1;
+  for (int j = 0; j < a.n; ++j)
+    if (tile_start(a, j) < e && tile_start(a, j) + a.te > s) lo = std::min(lo, j), hi = j;
+}
+
+// The tiles of [s0, s1) whose windows intersect U = the union of the windows of [r0, r1), as the range [lo, hi) from
+// the first to the last of them (lo == hi == 0: none).  The own tiles of one tile row of U have one contiguous column
+// span; the windows meeting it form a rectangle of the tile grid, one g-interval per tile row.
+void tiles_needed(const TileAxis& ay, const TileAxis& ax, int64_t r0, int64_t r1, int64_t s0, int64_t s1, int64_t* lo,
+                  int64_t* hi) {
+  int64_t first = INT64_MAX, last = -1;
+  for (int64_t g = r0; g < r1 && s0 < s1;) {
+    const int64_t row = g / ax.n, row_end = std::min(r1, (row + 1) * ax.n);  // g .. row_end - 1: one tile row
+    const int ty = int(row % ay.n);
+    int ya, yb, xa, xb;
+    axis_hits(ay, tile_start(ay, ty), tile_start(ay, ty) + ay.te, ya, yb);
+    axis_hits(ax, tile_start(ax, int(g - row * ax.n)), tile_start(ax, int(row_end - 1 - row * ax.n)) + ax.te, xa, xb);
+    for (int y = ya; y <= yb; ++y) {
+      const int64_t base = (row - ty + y) * ax.n;
+      const int64_t a = std::max(base + xa, s0), z = std::min(base + xb + 1, s1);
+      if (a < z) first = std::min(first, a), last = std::max(last, z);
     }
-    return launch(c, tile_blend_posterior_kernel, pgrid, 256, 0, st, x, eps_store, ay, ax, C, c->post[t], args, k + 1,
-                  uint32_t(t), t > 0 ? 1 : 0);
-  });
+    g = row_end;
+  }
+  *lo = last < 0 ? 0 : first;
+  *hi = last < 0 ? 0 : last;
+}
+
+// The entries of peer q in rank's plan: o = {send lo, send hi, recv lo, recv hi}, all 0 for q == rank
+void peer_plan(const TileAxis& ay, const TileAxis& ax, int64_t n, int world, int rank, int q, int64_t* o) {
+  o[0] = o[1] = o[2] = o[3] = 0;
+  if (q == rank) return;
+  const int64_t lo = own_lo(n, world, rank), hi = own_lo(n, world, rank + 1);
+  const int64_t qlo = own_lo(n, world, q), qhi = own_lo(n, world, q + 1);
+  tiles_needed(ay, ax, qlo, qhi, lo, hi, o, o + 1);      // q needs of ours
+  tiles_needed(ay, ax, lo, hi, qlo, qhi, o + 2, o + 3);  // we need of q's
+}
+
+// out[0..5 + 4 world): n_tiles, te_y, te_x, own lo, own hi, then per peer q: send lo, send hi, recv lo, recv hi
+void tiled_plan(const TileAxis& ay, const TileAxis& ax, int64_t n, int world, int rank, int64_t* out) {
+  out[0] = n, out[1] = ay.te, out[2] = ax.te, out[3] = own_lo(n, world, rank), out[4] = own_lo(n, world, rank + 1);
+  for (int q = 0; q < world; ++q) peer_plan(ay, ax, n, world, rank, q, out + 5 + 4 * int64_t(q));
 }
 
 // Pillow precompute_coeffs + normalize_coeffs_8bpc for the bicubic filter, full-image box
@@ -1626,6 +1727,40 @@ const fdsr_ctx::BicTab* find_bic(const fdsr_ctx* c, int in, int out) {
   return nullptr;
 }
 
+// The checks fdsr_sample_tiled, fdsr_sample_tiled_part and fdsr_tiled_plan share (c == nullptr: the global error)
+int tiled_check(fdsr_ctx* c, int32_t B, int32_t H, int32_t W, int32_t tile_h, int32_t tile_w, int32_t overlap) {
+  if (B < 1 || B > 65535) return fail(c, FDSR_E_INVALID, "B must be 1..65535 (got %d)", B);
+  if (H < 8 || W < 8) return fail(c, FDSR_E_INVALID, "canvas H and W must be >= 8 (got %dx%d)", H, W);
+  if (uint64_t(H) * uint64_t(W) >= (uint64_t(1) << 32))
+    return fail(c, FDSR_E_INVALID, "canvas H*W must be below 2^32 (got %dx%d)", H, W);
+  if (tile_h < 8 || tile_w < 8 || tile_h % 8 || tile_w % 8)
+    return fail(c, FDSR_E_INVALID, "tile sizes must be multiples of 8 and >= 8 (got %dx%d)", tile_h, tile_w);
+  if (overlap < 0) return fail(c, FDSR_E_INVALID, "overlap must be >= 0 (got %d)", overlap);
+  return FDSR_OK;
+}
+
+int tiled_entry_check(fdsr_ctx* c, const float* cond, const float* sr_out, int32_t B, int32_t H, int32_t W,
+                      int32_t tile_h, int32_t tile_w, int32_t overlap, int32_t tile_batch) {
+  if (!cond || !sr_out) return fail(c, FDSR_E_INVALID, "null argument");
+  if (c->cfg.model != FDSR_MODEL_FASTDIFFSR)
+    return fail(c, FDSR_E_INVALID, "tiled sampling is implemented for the FastDiffSR model only, not the SR3 baseline");
+  int rc = tiled_check(c, B, H, W, tile_h, tile_w, overlap);
+  if (rc) return rc;
+  if (tile_batch < 1) return fail(c, FDSR_E_INVALID, "tile_batch must be >= 1 (got %d)", tile_batch);
+  return check_ready(c);
+}
+
+// Reserves the workspace for one chunk, grows d_tiled to [SampleArgs | canvas x | store_bytes] and writes SampleArgs
+int tiled_prepare(fdsr_ctx* c, const TileChunks& ch, const TileAxis& ay, const TileAxis& ax, int B, size_t store_bytes,
+                  const float* noise, uint64_t seed, float* trace, cudaStream_t st) {
+  if (ch.bc) {
+    int rc = fdsr_reserve(c, ch.bc, ay.te, ax.te);
+    if (rc) return rc;
+  }
+  CUDA_TRY(c, c->d_tiled.grow(256 + align_up(size_t(B) * c->bands() * ay.L * ax.L * 4, 256) + store_bytes));
+  return launch(c, set_args_kernel, 1, 1, 0, st, reinterpret_cast<SampleArgs*>(c->d_tiled.ptr),
+                SampleArgs{seed, c->image0, noise, trace});
+}
 }  // namespace
 
 // =============================================================================== C ABI
@@ -1989,36 +2124,65 @@ int fdsr_sample_tiled(fdsr_ctx* c, const float* cond, const float* noise, uint64
                       int32_t B, int32_t H, int32_t W, int32_t tile_h, int32_t tile_w, int32_t overlap,
                       int32_t tile_batch, void* stream) {
   if (!c) return FDSR_E_INVALID;
-  if (!cond || !sr_out) return fail(c, FDSR_E_INVALID, "null argument");
-  if (c->cfg.model != FDSR_MODEL_FASTDIFFSR)
-    return fail(c, FDSR_E_INVALID, "tiled sampling is implemented for the FastDiffSR model only, not the SR3 baseline");
-  if (B < 1 || B > 65535) return fail(c, FDSR_E_INVALID, "B must be 1..65535 (got %d)", B);
-  if (H < 8 || W < 8) return fail(c, FDSR_E_INVALID, "canvas H and W must be >= 8 (got %dx%d)", H, W);
-  if (uint64_t(H) * uint64_t(W) >= (uint64_t(1) << 32))
-    return fail(c, FDSR_E_INVALID, "canvas H*W must be below 2^32 (got %dx%d)", H, W);
-  if (tile_h < 8 || tile_w < 8 || tile_h % 8 || tile_w % 8)
-    return fail(c, FDSR_E_INVALID, "tile sizes must be multiples of 8 and >= 8 (got %dx%d)", tile_h, tile_w);
-  if (overlap < 0) return fail(c, FDSR_E_INVALID, "overlap must be >= 0 (got %d)", overlap);
-  if (tile_batch < 1) return fail(c, FDSR_E_INVALID, "tile_batch must be >= 1 (got %d)", tile_batch);
-  int rc = check_ready(c);
+  int rc = tiled_entry_check(c, cond, sr_out, B, H, W, tile_h, tile_w, overlap, tile_batch);
   if (rc) return rc;
   const TileAxis ay = make_axis(H, tile_h, overlap), ax = make_axis(W, tile_w, overlap);
-  // equal chunks: every UNet call has the shape (bc, te_y, te_x); the last chunk repeats its last tile
   const int64_t n_tiles = int64_t(B) * ay.n * ax.n;
-  const int64_t n_chunks = (n_tiles + tile_batch - 1) / tile_batch;
-  const int bc = int((n_tiles + n_chunks - 1) / n_chunks);
-  rc = fdsr_reserve(c, bc, ay.te, ax.te);
-  if (rc) return rc;
-  const size_t need = 256 + align_up(size_t(B) * c->bands() * H * W * 4, 256) +
-                      size_t(n_chunks) * bc * c->bands() * ay.te * ax.te * 4;
-  CUDA_TRY(c, c->d_tiled.grow(need));
+  const TileChunks ch = tile_chunks(n_tiles, tile_batch);
   cudaStream_t st = static_cast<cudaStream_t>(stream);
-  rc = launch(c, set_args_kernel, 1, 1, 0, st, reinterpret_cast<SampleArgs*>(c->d_tiled.ptr),
-              SampleArgs{seed, c->image0, noise, trace});
+  // the context's store has a slot for every chunk slot, padding included
+  const size_t store_bytes = size_t(ch.n) * ch.bc * c->bands() * ay.te * ax.te * 4;
+  rc = tiled_prepare(c, ch, ay, ax, B, store_bytes, noise, seed, trace, st);
+  if (rc) return rc;
+  float* eps_store = reinterpret_cast<float*>(c->d_tiled + 256 + align_up(size_t(B) * c->bands() * H * W * 4, 256));
+  return with_dtype(c, [&](auto e) {
+    return tiled_enqueue<typename decltype(e)::type>(c, cond, sr_out, trace != nullptr, B, ay, ax, 0, n_tiles, ch,
+                                                     eps_store, nullptr, nullptr, nullptr, st);
+  });
+}
+
+int64_t fdsr_tiled_plan(int32_t B, int32_t H, int32_t W, int32_t tile_h, int32_t tile_w, int32_t overlap, int32_t world,
+                        int32_t rank, int64_t* out_host, int64_t cap) {
+  int rc = tiled_check(nullptr, B, H, W, tile_h, tile_w, overlap);
+  if (rc) return rc;
+  if (world < 1) return fail(nullptr, FDSR_E_INVALID, "world must be >= 1 (got %d)", world);
+  if (rank < 0 || rank >= world) return fail(nullptr, FDSR_E_INVALID, "rank must be 0..world-1 (got %d of %d)", rank, world);
+  const int64_t need = 5 + 4 * int64_t(world);
+  if (!out_host || cap < need)
+    return fail(nullptr, FDSR_E_INVALID, "the plan needs %lld entries (5 + 4 * world), cap is %lld", (long long)need,
+                (long long)cap);
+  const TileAxis ay = make_axis(H, tile_h, overlap), ax = make_axis(W, tile_w, overlap);
+  tiled_plan(ay, ax, int64_t(B) * ay.n * ax.n, world, rank, out_host);
+  return need;
+}
+
+int fdsr_sample_tiled_part(fdsr_ctx* c, const float* cond, const float* noise, uint64_t seed, float* sr_out,
+                           float* trace, int32_t B, int32_t H, int32_t W, int32_t tile_h, int32_t tile_w,
+                           int32_t overlap, int32_t tile_batch, int32_t rank, int32_t world, float* eps_store,
+                           fdsr_tile_exchange_fn exchange, void* user, void* stream) {
+  if (!c) return FDSR_E_INVALID;
+  int rc = tiled_entry_check(c, cond, sr_out, B, H, W, tile_h, tile_w, overlap, tile_batch);
+  if (rc) return rc;
+  if (!eps_store) return fail(c, FDSR_E_INVALID, "null argument (eps_store)");
+  if (world < 1) return fail(c, FDSR_E_INVALID, "world must be >= 1 (got %d)", world);
+  if (rank < 0 || rank >= world) return fail(c, FDSR_E_INVALID, "rank must be 0..world-1 (got %d of %d)", rank, world);
+  const TileAxis ay = make_axis(H, tile_h, overlap), ax = make_axis(W, tile_w, overlap);
+  const int64_t n_tiles = int64_t(B) * ay.n * ax.n;
+  const TileOwner owner{ay, ax, own_lo(n_tiles, world, rank), own_lo(n_tiles, world, rank + 1)};
+  for (int q = 0; q < world && !exchange; ++q) {
+    int64_t o[4];
+    peer_plan(ay, ax, n_tiles, world, rank, q, o);
+    if (o[1] > o[0] || o[3] > o[2])
+      return fail(c, FDSR_E_INVALID, "rank %d of %d exchanges tiles with rank %d: the exchange callback is required",
+                  rank, world, q);
+  }
+  const TileChunks ch = tile_chunks(owner.g1 - owner.g0, tile_batch);
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  rc = tiled_prepare(c, ch, ay, ax, B, 0, noise, seed, trace, st);
   if (rc) return rc;
   return with_dtype(c, [&](auto e) {
-    return tiled_enqueue<typename decltype(e)::type>(c, cond, sr_out, trace != nullptr, B, ay, ax, n_tiles, n_chunks, bc,
-                                                     st);
+    return tiled_enqueue<typename decltype(e)::type>(c, cond, sr_out, trace != nullptr, B, ay, ax, owner.g0, owner.g1,
+                                                     ch, eps_store, exchange, user, &owner, st);
   });
 }
 

@@ -175,18 +175,28 @@ class GaussianDiffusion(nn.Module):
 
     @torch.no_grad()
     def p_sample_loop(self, x_in, continous=False, noise=None, seed=None, image_offset=0, *, tile=None, tile_overlap=32,
-                      tile_batch=16):
+                      tile_batch=16, tile_split=False):
         """`tile` (int or (th, tw), multiples of 8): sample canvases of any size (H, W >= 8) as overlapping tiles blended
-        at every step (Engine.sample_tiled; `tile_overlap` pixels, `tile_batch` tiles per UNet call).  None: one piece."""
+        at every step (Engine.sample_tiled; `tile_overlap` pixels, `tile_batch` tiles per UNet call).  None: one piece.
+        `tile_split` (with `tile`): every rank of the default process group samples the same canvases together, each
+        its share of the tiles (parallel.split_sample_tiled), and returns the whole, single-GPU result."""
         if not self.conditional:
             raise NotImplementedError("unconditional sampling is not on the SR path (unused by every config)")
         if tile is not None and self.sr3:
             raise NotImplementedError("tiled sampling is implemented for the FastDiffSR model only, not the SR3 baseline")
-        tiling = None if tile is None else (tile, tile_overlap, tile_batch)
+        if tile_split and tile is None:
+            raise ValueError("tile_split splits the tiles of a canvas: it needs tile=")
+        dist = torch.distributed
+        split = tile_split and dist.is_available() and dist.is_initialized() and dist.get_world_size() > 1
+        tiling = None if tile is None else (tile, tile_overlap, tile_batch, split)
         if seed is None:   # unseeded like the reference (SURVEY F7); ranks seeded alike must still draw different noise
             seed = int(torch.randint(0, 2 ** 62, (1,)).item())
-            if torch.distributed.is_available() and torch.distributed.is_initialized():
-                seed = (seed + 0x9E3779B97F4A7C15 * torch.distributed.get_rank()) % (2 ** 63)
+            if split:      # ... unless they sample the same canvases together: then every rank takes rank 0's seed
+                s = torch.tensor([seed], dtype=torch.int64, device=self._param_device())
+                dist.broadcast(s, src=0)
+                seed = int(s.item())
+            elif dist.is_available() and dist.is_initialized():
+                seed = (seed + 0x9E3779B97F4A7C15 * dist.get_rank()) % (2 ** 63)
         try:
             return self._sample_checked(x_in, continous, noise, seed, image_offset, tiling)
         except FdsrOverflowError:
@@ -203,6 +213,10 @@ class GaussianDiffusion(nn.Module):
         eng = self.engine()
         if tiling is None:
             run = partial(eng.sample, x_in, noise=noise, seed=seed, image_offset=image_offset)
+        elif tiling[3]:    # split_sample_tiled checks the overflow flag of every rank itself
+            from .parallel import split_sample_tiled
+            run = partial(split_sample_tiled, eng, x_in, tiling[0], overlap=tiling[1], tile_batch=tiling[2], noise=noise,
+                          seed=seed, image_offset=image_offset)
         else:
             run = partial(eng.sample_tiled, x_in, tiling[0], overlap=tiling[1], tile_batch=tiling[2], noise=noise,
                           seed=seed, image_offset=image_offset)
@@ -216,11 +230,12 @@ class GaussianDiffusion(nn.Module):
 
     @torch.no_grad()
     def super_resolution(self, x_in, continous=False, noise=None, seed=None, image_offset=0, *, tile=None,
-                         tile_overlap=32, tile_batch=16):
+                         tile_overlap=32, tile_batch=16, tile_split=False):
         """`image_offset`: global index of x_in[0] in a job sharded over batches / ranks (see Engine.sample).
-        `tile`, `tile_overlap`, `tile_batch`: tiled sampling of large canvases (see p_sample_loop)."""
+        `tile`, `tile_overlap`, `tile_batch`: tiled sampling of large canvases (see p_sample_loop); `tile_split`: split
+        each canvas's tiles over the ranks of the default process group."""
         return self.p_sample_loop(x_in, continous, noise=noise, seed=seed, image_offset=image_offset, tile=tile,
-                                  tile_overlap=tile_overlap, tile_batch=tile_batch)
+                                  tile_overlap=tile_overlap, tile_batch=tile_batch, tile_split=tile_split)
 
     @torch.no_grad()
     def sample(self, batch_size=1, continous=False):

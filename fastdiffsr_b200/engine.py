@@ -172,6 +172,53 @@ class Engine:
                    int(overlap), int(tile_batch), self._stream())
         return (out, tr) if trace else out
 
+    @staticmethod
+    def tiled_plan(B: int, H: int, W: int, tile, overlap: int, world: int, rank: int):
+        """The exchange plan of `rank` for a tiled job split over `world` ranks (fdsr_tiled_plan; host only, no
+        context or GPU needed): {"n_tiles", "te": (te_y, te_x), "own": (lo, hi), "send": [(lo, hi)] * world,
+        "recv": [(lo, hi)] * world}, ranges of global tile slots, (0, 0) = nothing."""
+        th, tw = (tile, tile) if isinstance(tile, int) else (int(tile[0]), int(tile[1]))
+        lib = _lib.load()
+        buf = (C.c_int64 * (5 + 4 * max(int(world), 1)))()
+        rc = lib.fdsr_tiled_plan(B, H, W, th, tw, int(overlap), int(world), int(rank), buf, len(buf))
+        if rc < 0:
+            raise FdsrError(f"fdsr_tiled_plan: {lib.fdsr_global_error().decode()} (code {rc})")
+        peers = [tuple(buf[5 + 4 * q:9 + 4 * q]) for q in range(world)]
+        return {"n_tiles": buf[0], "te": (buf[1], buf[2]), "own": (buf[3], buf[4]),
+                "send": [p[:2] for p in peers], "recv": [p[2:] for p in peers]}
+
+    def sample_tiled_part(self, cond, tile, overlap: int = 32, tile_batch: int = 16, noise=None, seed: int = 0,
+                          trace: bool = False, image_offset: int = 0, rank: int = 0, world: int = 1, exchange=None):
+        """Rank `rank`'s part of sample_tiled split over `world` ranks (fdsr_sample_tiled_part): every rank passes the
+        same arguments except tile_batch.  Allocates the (n_tiles, C, te_y, te_x) fp32 eps store and calls
+        exchange(step, eps_store) once per step, on the host, between the own tiles' eps and the blend: it must move the
+        plan's slot ranges (tiled_plan) on the current stream.  Returns the rank's pixels of the result (and trace),
+        +0.0 elsewhere: the int32 bit patterns of all ranks sum to sample_tiled's bits.  An exception raised by
+        `exchange` aborts the call and is re-raised here."""
+        th, tw = (tile, tile) if isinstance(tile, int) else (int(tile[0]), int(tile[1]))
+        cond, noise, out, tr = self._sample_io(cond, noise, trace, image_offset)
+        B, _, H, W = cond.shape
+        plan = self.tiled_plan(B, H, W, (th, tw), overlap, world, rank)
+        store = torch.empty((plan["n_tiles"], self.C) + tuple(plan["te"]), dtype=torch.float32, device=self.device)
+        errors = []
+
+        def call_exchange(user, step, stream):
+            try:
+                exchange(int(step), store)
+                return 0
+            except BaseException as e:     # never unwind through the C frames
+                errors.append(e)
+                return 1
+        fn = _lib.TILE_EXCHANGE_FN(call_exchange) if exchange is not None else _lib.TILE_EXCHANGE_FN()
+        with torch.cuda.device(self.device):
+            rc = self.lib.fdsr_sample_tiled_part(self._h, _ptr(cond), _ptr(noise), seed, _ptr(out), _ptr(tr), B, H, W,
+                                                 th, tw, int(overlap), int(tile_batch), int(rank), int(world),
+                                                 _ptr(store), fn, None, self._stream())
+        if errors:
+            raise errors[0]
+        self._check(rc, "fdsr_sample_tiled_part")
+        return (out, tr) if trace else out
+
     def bicubic_u8(self, lr_u8, H: int, W: int, want_u8=True, want_cond=True):
         """lr_u8: (B,h,w,C) uint8 on device -> (u8 (B,H,W,C) | None, cond (B,C,H,W) fp32 | None)."""
         if lr_u8.dtype != torch.uint8 or lr_u8.dim() != 4 or lr_u8.shape[3] != self.C or lr_u8.device != self.device:

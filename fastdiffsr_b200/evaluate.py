@@ -5,7 +5,8 @@ ERGAS against HR (for both the bicubic baseline 'INF' and the SR result), averag
 Differences, all deliberate: images are processed in batches (the reference feeds one image per step and
 crashes for B>1, SURVEY F2); metrics are computed on the device (`fdsr_metrics_u8`) instead of skimage +
 matplotlib on the host; LPIPS (an AlexNet download) and the per-image matplotlib plot are not produced;
-under torchrun the dataset is sharded by image and the sums are all-reduced.
+under torchrun the dataset is sharded by image and the sums are all-reduced, or, with `tile_split`, every rank samples
+every image together with the others (each its share of the tiles) and the metrics are counted once.
 """
 from __future__ import annotations
 
@@ -63,23 +64,29 @@ def _save_u8(img_chw, path):
 
 @torch.no_grad()
 def evaluate(netG, dataset, batch_size=16, scale=4, result_path=None, save_ext="tif", seed=0, current_step=0,
-             logger=None, max_images=None, tile=None, tile_overlap=32, tile_batch=16):
+             logger=None, max_images=None, tile=None, tile_overlap=32, tile_batch=16, tile_split=False):
     """Returns {'n', 'bic_mse', 'bic_psnr', 'bic_ssim', 'bic_ergas', 'sr_mse', ..., 'seconds', 'images_per_s'}.
     `tile`: sample every image as one canvas of overlapping tiles (GaussianDiffusion.super_resolution(tile=...)), one
     image per call (scenes may differ in size; the tiles of one canvas fill the GPU); the HR size is then `scale` x the
-    LR size, whatever that size is."""
+    LR size, whatever that size is.  `tile_split` (with `tile`, under torchrun): the ranks split each image's tiles
+    instead of sharding the images (GaussianDiffusion.super_resolution(tile_split=True)); rank 0 writes the images."""
+    if tile_split and tile is None:
+        raise ValueError("tile_split needs tile")
     if tile is not None:
         batch_size = 1
-    tiling = {} if tile is None else dict(tile=tile, tile_overlap=tile_overlap, tile_batch=tile_batch)
+    tiling = {} if tile is None else dict(tile=tile, tile_overlap=tile_overlap, tile_batch=tile_batch,
+                                          tile_split=tile_split)
     eng = netG.engine()
     dev = eng.device
     world = dist.get_world_size() if dist.is_initialized() else 1
     rank = dist.get_rank() if dist.is_initialized() else 0
     n_total = len(dataset) if max_images is None else min(len(dataset), max_images)
-    start, stop, _ = shard_bounds(n_total, rank, world)
+    # tile_split: every rank holds every image's result, so the images are not sharded and the sums not reduced
+    start, stop, _ = (0, n_total, n_total) if tile_split else shard_bounds(n_total, rank, world)
+    write = result_path and (rank == 0 or not tile_split)
     loader = BatchLoader(dataset, batch_size, indices=range(start, stop))
     acc = torch.zeros(9, dtype=torch.float64, device=dev)       # bic[4], sr[4], n
-    if result_path:                  # every rank writes its own shard's images there
+    if write:                        # every rank writes its own shard's images there (tile_split: rank 0 all of them)
         os.makedirs(result_path, exist_ok=True)
     torch.cuda.synchronize(dev)
     t0 = time.perf_counter()
@@ -105,12 +112,13 @@ def evaluate(netG, dataset, batch_size=16, scale=4, result_path=None, save_ext="
         acc[0:4] += m_bic.sum(0)
         acc[4:8] += m_sr.sum(0)
         acc[8] += hr.shape[0]
-        if result_path:
+        if write:
             for j, idx in enumerate(batch["Index"]):
                 _save_u8(sr[j], '{}/{}_{}_sr.{}'.format(result_path, current_step, idx + 1, save_ext))
     torch.cuda.synchronize(dev)
     dt = time.perf_counter() - t0
-    reduce_sums(acc)
+    if not tile_split:
+        reduce_sums(acc)
     n = max(acc[8].item(), 1.0)
     out = {"n": int(acc[8].item()), "seconds": dt, "images_per_s": acc[8].item() / dt if dt > 0 else float("nan")}
     for i, k in enumerate(METRIC_NAMES):
@@ -167,7 +175,12 @@ def main(argv=None, default_config="config/sr_fastdiffsr_test_64_256.json", prog
                     help='sample each image as overlapping tiles of this size (multiple of 8): scenes of any size, one per call')
     ap.add_argument('--tile-overlap', type=int, default=32, help='overlap of neighbouring tiles in pixels (with --tile)')
     ap.add_argument('--tile-batch', type=int, default=16, help='tiles per UNet call (with --tile)')
+    ap.add_argument('--tile-split', action='store_true',
+                    help='under torchrun, split the tiles of each image over the ranks instead of sharding the images '
+                         '(with --tile): one large scene on every GPU, the single-GPU result')
     args = ap.parse_args(argv)
+    if args.tile_split and args.tile is None:
+        ap.error('--tile-split needs --tile')
     if args.phase == 'train':
         raise NotImplementedError("training is outside the B200 sampling path: train with the reference and point "
                                   "path.resume_state at the checkpoint")
@@ -195,6 +208,11 @@ def main(argv=None, default_config="config/sr_fastdiffsr_test_64_256.json", prog
         logger.warning("no path.resume_state in the config: sampling with RANDOM-INIT weights")
     netG.set_new_noise_schedule(opt['model']['beta_schedule']['val'], dev)
     netG.eval()
+    if args.tile_split and dist.is_initialized():
+        # the ranks evaluate different tiles of one image: they must run the same network (a random init differs per rank)
+        for t in netG.state_dict().values():
+            dist.broadcast(t, src=0)
+        netG.refresh_weights()
     val_opt = opt['datasets']['val']
     from .data import create_dataset
     val_set = create_dataset(val_opt, 'val', channels=int(opt['model']['unet']['out_channel']))
@@ -203,7 +221,7 @@ def main(argv=None, default_config="config/sr_fastdiffsr_test_64_256.json", prog
     result_path = None if args.no_save else (paths.get('results') if isinstance(paths, dict) and paths.get('results') else 'results')
     res = evaluate(netG, val_set, batch_size=args.batch, scale=scale, result_path=result_path,
                    save_ext="png" if prog == "infer.py" else "tif", logger=logger, max_images=args.max_images,
-                   tile=args.tile, tile_overlap=args.tile_overlap, tile_batch=args.tile_batch)
+                   tile=args.tile, tile_overlap=args.tile_overlap, tile_batch=args.tile_batch, tile_split=args.tile_split)
     if dist.is_initialized():
         dist.destroy_process_group()
     return res

@@ -1,15 +1,21 @@
-"""Batch sharding of LR images over ranks (one process per GPU, torch.distributed).
+"""Batch sharding of LR images over ranks (one process per GPU, torch.distributed), and the split of one tiled canvas
+over ranks.
 
 The sampling path has no exchange step: every image's T-step chain is independent (GroupNorm is
 per-sample, SURVEY 8(e)).  Ranks therefore run the full loop on their shard with no data-path
 collective; NCCL (gloo in CPU tests) is used only after the loop to all-gather SR shards and to
 all-reduce metric accumulators — the two collectives the reference's single-GPU evaluation loop
 (sr_mfe.py:258-386) would need when spread over GPUs.
+
+A tiled canvas (split_sample_tiled) is the exception: its tiles share one chain, so the ranks that split its tiles
+exchange the eps of the tiles at their borders once per step (DESIGN §4.4).
 """
 from __future__ import annotations
 
 import torch
 import torch.distributed as dist
+
+from ._lib import FdsrOverflowError
 
 
 def shard_bounds(n_items: int, rank: int, world: int):
@@ -80,3 +86,78 @@ def sharded_super_resolution(netG, cond_global: torch.Tensor, noise_global=None,
     if sr_local.dim() == 3:   # SR3 baseline, one image per rank: ret_img[-1] has no batch axis
         sr_local = sr_local[None]
     return gather_batch(sr_local, cond_global.shape[0], group)
+
+
+def tile_exchange(plan, group=None):
+    """exchange(step, eps_store) of Engine.sample_tiled_part for the ranks of `group`: the plan's slot ranges as
+    point-to-point sends / receives.  NCCL moves the device slots directly, ordered on and waited for by the current
+    stream; a backend that sends host tensors only (gloo) gets them staged through host memory, after the stream's
+    prior work and copied back on the stream."""
+    peer = (lambda q: q) if group is None else (lambda q: dist.get_global_rank(group, q))
+    sends = [(peer(q), lo, hi) for q, (lo, hi) in enumerate(plan["send"]) if hi > lo]
+    recvs = [(peer(q), lo, hi) for q, (lo, hi) in enumerate(plan["recv"]) if hi > lo]
+    on_device = "nccl" in str(dist.get_backend(group))
+
+    def exchange(step, store):
+        if not (sends or recvs):
+            return
+        if on_device:
+            ops = [dist.P2POp(dist.isend, store[lo:hi], q, group) for q, lo, hi in sends]
+            ops += [dist.P2POp(dist.irecv, store[lo:hi], q, group) for q, lo, hi in recvs]
+            for req in dist.batch_isend_irecv(ops):
+                req.wait()
+            return
+        out = [store[lo:hi].cpu() for _, lo, hi in sends]     # synchronises with the stream's prior work
+        inc = [torch.empty(store[lo:hi].shape) for _, lo, hi in recvs]
+        reqs = [dist.isend(t, q, group) for t, (q, _, _) in zip(out, sends)]
+        reqs += [dist.irecv(t, q, group) for t, (q, _, _) in zip(inc, recvs)]
+        for req in reqs:
+            req.wait()
+        for t, (_, lo, hi) in zip(inc, recvs):
+            store[lo:hi].copy_(t)
+    return exchange
+
+
+def gather_owned(t: torch.Tensor, group=None):
+    """The whole fp32 tensor from the ranks' parts of it (each rank's part, +0.0 elsewhere): an integer sum of the bit
+    patterns, so the exact bits, -0.0 included, with no floating-point addition."""
+    if dist.is_initialized() and dist.get_world_size(group) > 1:
+        dist.all_reduce(t.view(torch.int32), op=dist.ReduceOp.SUM, group=group)
+    return t
+
+
+@torch.no_grad()
+def split_sample_tiled(engine, cond, tile, overlap: int = 32, tile_batch: int = 16, noise=None, seed: int = 0,
+                       trace: bool = False, image_offset: int = 0, group=None):
+    """engine.sample_tiled(cond, ...) split over the ranks of `group` (default: the default process group): every rank
+    passes the same arguments (tile_batch may differ), samples its share of the tiles (Engine.sample_tiled_part) with
+    an eps exchange every step (tile_exchange: NCCL, or gloo through host memory), and gets the whole result (and
+    trace), bit for bit sample_tiled's.  The ranks' networks must hold the same weights.  fp16 mode: the
+    overflow flags are combined over the ranks, so all of them raise FdsrOverflowError together."""
+    rank, world = dist.get_rank(group), dist.get_world_size(group)
+    B, _, H, W = cond.shape
+    # the ranks must agree on the job, or the exchange would pair mismatched ranges and hang
+    th, tw = (tile, tile) if isinstance(tile, int) else (int(tile[0]), int(tile[1]))
+    key = torch.tensor([B, H, W, th, tw, int(overlap), int(image_offset), int(seed) % (2 ** 62), noise is not None,
+                        bool(trace)], dtype=torch.int64, device=engine.device)
+    both = torch.cat([key, -key])
+    dist.all_reduce(both, op=dist.ReduceOp.MAX, group=group)
+    if not torch.equal(both[:key.numel()], -both[key.numel():]):
+        raise ValueError("split_sample_tiled: the ranks were called with different canvas, tile, seed or noise arguments")
+    plan = engine.tiled_plan(B, H, W, (th, tw), overlap, world, rank)
+    res = engine.sample_tiled_part(cond, (th, tw), overlap=overlap, tile_batch=tile_batch, noise=noise, seed=seed,
+                                   trace=trace, image_offset=image_offset, rank=rank, world=world,
+                                   exchange=tile_exchange(plan, group))
+    overflow = torch.zeros(1, dtype=torch.int32, device=engine.device)
+    try:
+        engine.check_overflow()
+    except FdsrOverflowError:
+        overflow.fill_(1)
+    dist.all_reduce(overflow, op=dist.ReduceOp.MAX, group=group)
+    if overflow.item():
+        raise FdsrOverflowError("split_sample_tiled: an activation left the fp16 range on at least one rank")
+    if not trace:
+        return gather_owned(res, group)
+    sr, tr = res
+    both = gather_owned(torch.cat([sr.reshape(-1), tr.reshape(-1)]), group)   # one collective for both
+    return both[:sr.numel()].view(sr.shape), both[sr.numel():].view(tr.shape)

@@ -161,6 +161,59 @@ int fdsr_sample_tiled(fdsr_ctx* ctx, const float* cond_dev, const float* noise_d
                       float* sr_out_dev, float* trace_out_dev, int32_t B, int32_t H, int32_t W,
                       int32_t tile_h, int32_t tile_w, int32_t overlap, int32_t tile_batch, void* stream);
 
+/* One tiled sampling job split over the `world` ranks of a group (one process and context per GPU): every rank samples
+ * its share of the tiles of the same B canvases, and the gathered result equals fdsr_sample_tiled of the same inputs
+ * bit for bit, for any world size.
+ *   The rule.  All ranks pass identical arguments (cond, noise or seed, image offset, canvas and tile sizes, overlap);
+ *     tile_batch may differ per rank.
+ *   - Tile ownership: the n = B * tiles_y * tiles_x tiles in their global order (canvas, row start, column start) are
+ *     split into contiguous ranges; rank r owns [floor(r n / world), floor((r+1) n / world)).  The range is empty iff
+ *     the two bounds are equal, which happens only when world > n.
+ *   - Update region U_r: the union of the windows of rank r's tiles.  Every step rank r computes the eps of its own tiles,
+ *     receives the eps of every other rank's tile whose window intersects U_r, and blends and updates exactly the
+ *     pixels of U_r (fdsr_sample_tiled's arithmetic).  Pixels a neighbour also updates get identical bits on both ranks
+ *     (same x_t, the same eps in the same order, the same noise), so x_t is never exchanged: only eps, once per step.
+ *   - Exchange plan (fdsr_tiled_plan): for each ordered pair q -> r, q sends one contiguous range of its own tile slots,
+ *     from the first to the last of its tiles r needs (a superset: every slot in it holds q's valid eps), into the same
+ *     slots of r's store.  With heavy overlaps (o_e >= t_e / 2) a pixel lies under 3 or more tile rows and r may need
+ *     tiles of ranks that are not adjacent to it; the plan covers them.
+ *   - Output: a pixel belongs to the rank that owns its first covering tile in global order (these owners partition the
+ *     canvas).  Each rank writes sr_out and the trace frames at its pixels and +0.0 everywhere else, so an integer sum
+ *     of the int32 bit patterns over the ranks (all_reduce SUM of the int32 view) rebuilds the exact bits, -0.0 included.
+ *   - Why the bits match: by induction over the steps, x_t on U_r equals the single-GPU x_t.  A tile's eps depends only
+ *     on x_t in its window (and not on the chunk it is evaluated in: tile_batch does not change the result), every own
+ *     window lies in U_r, every foreign window lies in its owner's update region, and the blend reads each covering
+ *     tile in global order.
+ *
+ * Host only, needs no context or GPU: the exchange plan of `rank`.  out_host[0 .. 5 + 4 world):
+ *   n_tiles, t_e_y, t_e_x, own_lo, own_hi, then for each peer q = 0 .. world-1: send_lo, send_hi (the slots rank sends
+ *   to q), recv_lo, recv_hi (the slots rank receives from q); empty ranges and q == rank are 0, 0.  recv of r from q
+ *   equals send of q to r.  Returns the entry count, or FDSR_E_INVALID (message in fdsr_global_error) for the arguments
+ *   fdsr_sample_tiled rejects, world < 1, rank outside 0..world-1, a null out_host or cap < 5 + 4 world. */
+int64_t fdsr_tiled_plan(int32_t B, int32_t H, int32_t W, int32_t tile_h, int32_t tile_w, int32_t overlap,
+                        int32_t world, int32_t rank, int64_t* out_host, int64_t cap);
+
+/* Moves the eps slots of one step between the ranks' stores (see fdsr_sample_tiled_part).  `step` is t (T-1 .. 0).
+ * Returns 0, or nonzero to abort the sampling call. */
+typedef int (*fdsr_tile_exchange_fn)(void* user, int32_t step, void* stream);
+
+/* Rank `rank`'s part of the split job above (arguments as in fdsr_sample_tiled).
+ *   eps_store_dev: caller-owned n_tiles x C x t_e_y x t_e_x fp32, indexed by global tile, so that the exchange can send
+ *     from it and receive into it directly.  The call writes its own slots.
+ *   exchange: called once per step on the host, after the own tiles' eps have been enqueued into the store on `stream`
+ *     and before the blend is enqueued.  It must order its transfers after prior work on `stream` and make `stream`
+ *     wait for their completion (for example NCCL send / recv of the plan's ranges).  A nonzero return aborts the call
+ *     with FDSR_E_INVALID.  NULL is accepted only when the plan of this rank has no transfers (for example world 1).
+ *   A rank with an empty range runs no UNet but still calls exchange every step, so that collectives match.
+ *   sr_out_dev / trace_out_dev: the rank's pixels, +0.0 elsewhere.  Launches per call: 2 + T (chunks (1 + UNet ops) + 1)
+ *     + trace frames + 1, with chunks = ceil(own tiles / tile_batch).
+ *   FDSR_E_INVALID: everything fdsr_sample_tiled rejects, a null eps_store_dev, world < 1, rank outside 0..world-1, a
+ *   NULL exchange when the plan has transfers. */
+int fdsr_sample_tiled_part(fdsr_ctx* ctx, const float* cond_dev, const float* noise_dev, uint64_t seed,
+                           float* sr_out_dev, float* trace_out_dev, int32_t B, int32_t H, int32_t W, int32_t tile_h,
+                           int32_t tile_w, int32_t overlap, int32_t tile_batch, int32_t rank, int32_t world,
+                           float* eps_store_dev, fdsr_tile_exchange_fn exchange, void* user, void* stream);
+
 /* fp16 mode only (always FDSR_OK otherwise): synchronises `stream`, then returns FDSR_E_OVERFLOW if any activation
  * stored since the last check had left the fp16 range (it was stored saturated, so nothing downstream is inf / NaN,
  * but the image is not the network's output), and clears the flag.  fdsr_super_resolve_u8 performs this check itself;
