@@ -94,6 +94,10 @@ _SIGS = {
                               C.c_void_p]),
     "fdsr_metrics_u8": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int32, C.c_int32, C.c_int32, C.c_double,
                                   C.c_void_p, C.c_void_p]),
+    "fdsr_bicubic_u16": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.c_int32,
+                                   C.c_int32, C.c_void_p, C.c_void_p, C.c_void_p]),
+    "fdsr_metrics_u16": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int32, C.c_int32, C.c_int32, C.c_int32,
+                                   C.c_double, C.c_void_p, C.c_void_p]),
     "fdsr_debug_num_tensors": (C.c_int32, [C.c_void_p]),
     "fdsr_debug_tensor_name": (C.c_char_p, [C.c_void_p, C.c_int32]),
     "fdsr_debug_read_tensor": (C.c_int, [C.c_void_p, C.c_char_p, C.c_void_p, C.c_int64, C.POINTER(C.c_int32),

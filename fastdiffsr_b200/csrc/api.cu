@@ -168,10 +168,11 @@ struct fdsr_ctx {
   struct BicTab {
     int in, out, ksize;
     DevBuf<int> d_min, d_cnt, d_taps;
+    DevBuf<double> d_wts;  // normalised weights before the fixed-point step (the 16-bit resize)
   };
   std::vector<BicTab> bic;
   DevBuf<uint8_t> d_bic_tmp;
-  DevBuf<unsigned long long> d_metric;  // [B][4] integer accumulators of fdsr_metrics_u8
+  DevBuf<unsigned long long> d_metric;  // [B][4] integer accumulators of fdsr_metrics_u8 / _u16
   // pinned staging for the host-buffer path
   // host-buffer path: two slots so that the copies of one batch overlap the sampling of the next
   struct HostSlot {
@@ -1676,16 +1677,17 @@ void tiled_plan(const TileAxis& ay, const TileAxis& ax, int64_t n, int world, in
   for (int q = 0; q < world; ++q) peer_plan(ay, ax, n, world, rank, q, out + 5 + 4 * int64_t(q));
 }
 
-// Pillow precompute_coeffs + normalize_coeffs_8bpc for the bicubic filter, full-image box
-int ensure_bic(fdsr_ctx* c, int in, int out) {
-  for (const auto& b : c->bic)
-    if (b.in == in && b.out == out) return FDSR_OK;
+// Pillow precompute_coeffs for the bicubic filter, full-image box: per output index the window's first input index
+// vmin, its length vcnt and the normalised double weights w[out][ksize] (zero past vcnt).  Both the 8-bit taps
+// (normalize_coeffs_8bpc of these weights) and the 16-bit resize (the weights as they are) start from here.
+int bic_coeffs(int in, int out, std::vector<int>& vmin, std::vector<int>& vcnt, std::vector<double>& w) {
   const double scale = double(in) / out;
   const double fscale = scale < 1.0 ? 1.0 : scale;
   const double support = 2.0 * fscale;
   const int ksize = int(ceil(support)) * 2 + 1;
-  std::vector<int> vmin(out), vcnt(out), taps(size_t(out) * ksize, 0);
-  std::vector<double> k(ksize);
+  vmin.assign(out, 0);
+  vcnt.assign(out, 0);
+  w.assign(size_t(out) * ksize, 0.0);
   auto filt = [](double x) {
     const double a = -0.5;
     if (x < 0.0) x = -x;
@@ -1701,23 +1703,35 @@ int ensure_bic(fdsr_ctx* c, int in, int out) {
     int xmax = int(center + support + 0.5);
     if (xmax > in) xmax = in;
     xmax -= xmin;
+    double* k = w.data() + size_t(xx) * ksize;
     double ww = 0.0;
     for (int x = 0; x < xmax; ++x) {
       k[x] = filt((x + xmin - center + 0.5) * ss);
       ww += k[x];
     }
-    for (int x = 0; x < xmax; ++x) {
+    for (int x = 0; x < xmax; ++x)
       if (ww != 0.0) k[x] /= ww;
-      taps[size_t(xx) * ksize + x] =
-          k[x] < 0 ? int(-0.5 + k[x] * (1 << kBicPrec)) : int(0.5 + k[x] * (1 << kBicPrec));
-    }
     vmin[xx] = xmin;
     vcnt[xx] = xmax;
   }
+  return ksize;
+}
+
+// The resize tables of one (in, out) pair, built once per context: bounds, 22-bit taps and the double weights
+int ensure_bic(fdsr_ctx* c, int in, int out) {
+  for (const auto& b : c->bic)
+    if (b.in == in && b.out == out) return FDSR_OK;
+  std::vector<int> vmin, vcnt;
+  std::vector<double> w;
+  const int ksize = bic_coeffs(in, out, vmin, vcnt, w);
+  std::vector<int> taps(w.size());
+  for (size_t i = 0; i < w.size(); ++i)
+    taps[i] = w[i] < 0 ? int(-0.5 + w[i] * (1 << kBicPrec)) : int(0.5 + w[i] * (1 << kBicPrec));
   fdsr_ctx::BicTab b{in, out, ksize};
   int rc = upload(c, b.d_min, vmin);
   if (!rc) rc = upload(c, b.d_cnt, vcnt);
   if (!rc) rc = upload(c, b.d_taps, taps);
+  if (!rc) rc = upload(c, b.d_wts, w);
   if (!rc) c->bic.push_back(std::move(b));
   return rc;
 }
@@ -1725,6 +1739,19 @@ const fdsr_ctx::BicTab* find_bic(const fdsr_ctx* c, int in, int out) {
   for (const auto& b : c->bic)
     if (b.in == in && b.out == out) return &b;
   return nullptr;
+}
+
+// fdsr_metrics_u8 / fdsr_metrics_u16: one kernel pair at white level M
+int metrics(fdsr_ctx* c, const float* a, const float* b, int32_t B, int32_t H, int32_t W, int M, double ergas_scale,
+            double* out, cudaStream_t st) {
+  CUDA_TRY(c, c->d_metric.grow(size_t(B) * 32));
+  CUDA_TRY(c, cudaMemsetAsync(c->d_metric, 0, size_t(B) * 32, st));
+  const int C = c->bands();
+  const dim3 grid((W + kSsimTile - 1) / kSsimTile, (H + kSsimTile - 1) / kSsimTile, B * C);
+  const int rc = launch(c, metrics_kernel, grid, 256, 0, st, a, b, c->d_metric.ptr, H, W, C, M);
+  if (rc) return rc;
+  return launch(c, metrics_finalize_kernel, (B + 127) / 128, 128, 0, st, c->d_metric.ptr, out, B, H, W, C, ergas_scale,
+                M);
 }
 
 // The checks fdsr_sample_tiled, fdsr_sample_tiled_part and fdsr_tiled_plan share (c == nullptr: the global error)
@@ -2206,6 +2233,32 @@ int fdsr_bicubic_u8(fdsr_ctx* c, const uint8_t* lr, int32_t B, int32_t h, int32_
                 tv->d_min.ptr, tv->d_cnt.ptr, tv->d_taps.ptr, tv->ksize, B, h, H, W, C);
 }
 
+int fdsr_bicubic_u16(fdsr_ctx* c, const uint16_t* lr, int32_t B, int32_t h, int32_t w, int32_t H, int32_t W,
+                     int32_t max_value, uint16_t* out_u16, float* cond, void* stream) {
+  if (!c) return FDSR_E_INVALID;
+  if (B < 1 || h < 1 || w < 1 || H < 1 || W < 1)
+    return fail(c, FDSR_E_INVALID, "B, h, w, H and W must be >= 1 (got %d, %dx%d -> %dx%d)", B, h, w, H, W);
+  if (max_value < 1 || max_value > 65535)
+    return fail(c, FDSR_E_INVALID, "max_value must be 1..65535 (got %d)", max_value);
+  if (!lr) return fail(c, FDSR_E_INVALID, "null argument (lr)");
+  if (!out_u16 && !cond) return fail(c, FDSR_E_INVALID, "both outputs are null: pass out_u16 and/or cond_out");
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  int rc = ensure_bic(c, w, W);
+  if (rc) return rc;
+  rc = ensure_bic(c, h, H);
+  if (rc) return rc;
+  const fdsr_ctx::BicTab *th = find_bic(c, w, W), *tv = find_bic(c, h, H);
+  const int C = c->bands();
+  CUDA_TRY(c, c->d_bic_tmp.grow(size_t(B) * h * W * C * sizeof(uint16_t)));
+  uint16_t* tmp = reinterpret_cast<uint16_t*>(c->d_bic_tmp.ptr);
+  const int64_t n1 = int64_t(B) * h * W, n2 = int64_t(B) * H * W;
+  rc = launch(c, bicubic16_h_kernel, unsigned((n1 + 255) / 256), 256, 0, st, lr, tmp, th->d_min.ptr, th->d_cnt.ptr,
+              th->d_wts.ptr, th->ksize, B, h, w, W, C);
+  if (rc) return rc;
+  return launch(c, bicubic16_v_kernel, unsigned((n2 + 255) / 256), 256, 0, st, tmp, out_u16, cond, tv->d_min.ptr,
+                tv->d_cnt.ptr, tv->d_wts.ptr, tv->ksize, B, h, H, W, C, int(max_value));
+}
+
 int fdsr_super_resolve_u8_submit(fdsr_ctx* c, int32_t slot, const uint8_t* lr_host, int32_t B, int32_t h, int32_t w,
                                  int32_t H, int32_t W, const float* noise_dev, uint64_t seed, void* stream) {
   if (!c || !lr_host || slot < 0 || slot >= fdsr_ctx::kHostSlots) return fail(c, FDSR_E_INVALID, "bad argument");
@@ -2293,14 +2346,17 @@ int fdsr_sse_u8(fdsr_ctx* c, const float* a, const float* b, int32_t B, int32_t 
 int fdsr_metrics_u8(fdsr_ctx* c, const float* a, const float* b, int32_t B, int32_t H, int32_t W, double ergas_scale,
                     double* out, void* stream) {
   if (!c || !a || !b || !out || B < 1 || H < 1 || W < 1) return fail(c, FDSR_E_INVALID, "bad argument");
-  cudaStream_t st = static_cast<cudaStream_t>(stream);
-  CUDA_TRY(c, c->d_metric.grow(size_t(B) * 32));
-  CUDA_TRY(c, cudaMemsetAsync(c->d_metric, 0, size_t(B) * 32, st));
-  const int C = c->bands();
-  const dim3 grid((W + kSsimTile - 1) / kSsimTile, (H + kSsimTile - 1) / kSsimTile, B * C);
-  const int rc = launch(c, metrics_u8_kernel, grid, 256, 0, st, a, b, c->d_metric.ptr, H, W, C);
-  if (rc) return rc;
-  return launch(c, metrics_finalize_kernel, (B + 127) / 128, 128, 0, st, c->d_metric.ptr, out, B, H, W, C, ergas_scale);
+  return metrics(c, a, b, B, H, W, 255, ergas_scale, out, static_cast<cudaStream_t>(stream));
+}
+
+int fdsr_metrics_u16(fdsr_ctx* c, const float* a, const float* b, int32_t B, int32_t H, int32_t W, int32_t max_value,
+                     double ergas_scale, double* out, void* stream) {
+  if (!c) return FDSR_E_INVALID;
+  if (B < 1 || H < 1 || W < 1) return fail(c, FDSR_E_INVALID, "B, H and W must be >= 1 (got %d, %dx%d)", B, H, W);
+  if (max_value < 1 || max_value > 65535)
+    return fail(c, FDSR_E_INVALID, "max_value must be 1..65535 (got %d)", max_value);
+  if (!a || !b || !out) return fail(c, FDSR_E_INVALID, "null argument");
+  return metrics(c, a, b, B, H, W, int(max_value), ergas_scale, out, static_cast<cudaStream_t>(stream));
 }
 
 int32_t fdsr_debug_num_tensors(const fdsr_ctx* c) { return c ? int32_t(c->tensors.size()) : 0; }

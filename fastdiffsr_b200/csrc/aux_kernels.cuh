@@ -1,5 +1,6 @@
 // HBM-bound helper kernels of the sampling path: input assembly, posterior update, res2img,
-// CLAM/SLAM gates, PIL-exact bicubic, uint8 SSE, layout conversion for the debug hook.
+// CLAM/SLAM gates, PIL-exact bicubic of 8- and 16-bit bands, uint8 SSE, metrics at a white level, layout conversion for
+// the debug hook.
 // All are coalesced/vectorised elementwise or small-reduction kernels; none needs tensor cores.
 #pragma once
 #include <cstdint>
@@ -358,13 +359,90 @@ __global__ void bicubic_v_kernel(const uint8_t* __restrict__ in, uint8_t* __rest
 }
 
 // ------------------------------------------------------------------------------------------
+// PIL-exact bicubic of 16-bit bands (Pillow ImagingResample of an 'I;16' image): the same bounds as the 8-bit pair and
+// the normalised double weights before their fixed-point step; per output sample ss = 0.0, ss = ss + double(p) * k[j]
+// with every multiply and add rounded on its own (no FMA contraction), rounded half away from zero, then stored the
+// way Pillow stores an I;16 sample byte by byte: lo = CLIP8(v % 256), hi = CLIP8(v >> 8).  So v < 0 -> 0 and
+// v > 65535 -> 65280 + v % 256 (not 65535).  The horizontal pass's result is stored the same way (uint16 intermediate).
+// ------------------------------------------------------------------------------------------
+__device__ __forceinline__ uint16_t pil_store_u16(double ss) {
+  const int v = int(ss >= 0.0 ? floor(__dadd_rn(ss, 0.5)) : -floor(__dadd_rn(-ss, 0.5)));
+  if (v < 0) return 0;
+  if (v > 65535) return uint16_t(0xff00 | (v & 0xff));
+  return uint16_t(v);
+}
+// in: [B][inH][inW][C] u16 -> out: [B][inH][outW][C] u16
+__global__ void bicubic16_h_kernel(const uint16_t* __restrict__ in, uint16_t* __restrict__ out,
+                                   const int* __restrict__ xmin, const int* __restrict__ xcnt,
+                                   const double* __restrict__ wts, int ksize, int B, int inH, int inW, int outW,
+                                   int C) {
+  const int64_t i = blockIdx.x * int64_t(blockDim.x) + threadIdx.x;
+  const int64_t total = int64_t(B) * inH * outW;
+  if (i >= total) return;
+  const int xo = int(i % outW);
+  const int64_t row = i / outW;
+  const uint16_t* src = in + (row * inW + xmin[xo]) * C;
+  const double* k = wts + xo * ksize;
+  double a[8];
+#pragma unroll
+  for (int c = 0; c < 8; ++c) a[c] = 0.0;
+  for (int j = 0; j < xcnt[xo]; ++j) {
+    const double kj = k[j];
+#pragma unroll
+    for (int c = 0; c < 8; ++c)
+      if (c < C) a[c] = __dadd_rn(a[c], __dmul_rn(double(src[C * j + c]), kj));
+  }
+  uint16_t* o = out + i * C;
+#pragma unroll
+  for (int c = 0; c < 8; ++c)
+    if (c < C) o[c] = pil_store_u16(a[c]);
+}
+// in: [B][inH][W][C] u16 -> out_u16: [B][outH][W][C] (optional, the stored levels), cond: [B][C][outH][W] fp32
+// (optional) = (min(v, M) / M) * 2 - 1 in fp32, the operation order of the 8-bit pass with 255 -> M
+__global__ void bicubic16_v_kernel(const uint16_t* __restrict__ in, uint16_t* __restrict__ out_u16,
+                                   float* __restrict__ cond, const int* __restrict__ ymin,
+                                   const int* __restrict__ ycnt, const double* __restrict__ wts, int ksize,
+                                   int B, int inH, int outH, int W, int C, int M) {
+  const int64_t i = blockIdx.x * int64_t(blockDim.x) + threadIdx.x;
+  const int64_t total = int64_t(B) * outH * W;
+  if (i >= total) return;
+  const int x = int(i % W);
+  const int yo = int((i / W) % outH);
+  const int b = int(i / (int64_t(W) * outH));
+  const uint16_t* src = in + ((int64_t(b) * inH + ymin[yo]) * W + x) * C;
+  const double* k = wts + yo * ksize;
+  double a[8];
+#pragma unroll
+  for (int c = 0; c < 8; ++c) a[c] = 0.0;
+  for (int j = 0; j < ycnt[yo]; ++j) {
+    const uint16_t* s = src + int64_t(j) * W * C;
+    const double kj = k[j];
+#pragma unroll
+    for (int c = 0; c < 8; ++c)
+      if (c < C) a[c] = __dadd_rn(a[c], __dmul_rn(double(s[c]), kj));
+  }
+  const int64_t plane = int64_t(outH) * W;
+  float* cp = cond != nullptr ? cond + int64_t(b) * C * plane + int64_t(yo) * W + x : nullptr;
+  const float fM = float(M);
+#pragma unroll
+  for (int c = 0; c < 8; ++c) {
+    if (c >= C) continue;
+    const int v = pil_store_u16(a[c]);
+    if (out_u16 != nullptr) out_u16[i * C + c] = uint16_t(v);
+    if (cp != nullptr) cp[c * plane] = __fsub_rn(__fmul_rn(__fdiv_rn(float(min(v, M)), fM), 2.0f), 1.0f);
+  }
+}
+
+// ------------------------------------------------------------------------------------------
 // Sum of squared uint8 differences per image after tensor2img quantisation (core/metrics.py:16-42)
 // ------------------------------------------------------------------------------------------
-__device__ __forceinline__ int quant_u8(float v) {
+// tensor2img at white level M: the level 0..M of an fp32 value in [-1, 1]
+__device__ __forceinline__ int quant_level(float v, float M) {
   v = fminf(fmaxf(v, -1.0f), 1.0f);
   v = __fdiv_rn(__fadd_rn(v, 1.0f), 2.0f);
-  return __float2int_rn(__fmul_rn(v, 255.0f));  // numpy .round(): half to even
+  return __float2int_rn(__fmul_rn(v, M));  // numpy .round(): half to even
 }
+__device__ __forceinline__ int quant_u8(float v) { return quant_level(v, 255.0f); }
 __global__ void sse_u8_kernel(const float* __restrict__ a, const float* __restrict__ b,
                               double* __restrict__ sse, int64_t per_image) {
   const int img = blockIdx.y;
@@ -381,33 +459,36 @@ __global__ void sse_u8_kernel(const float* __restrict__ a, const float* __restri
 }
 
 // ------------------------------------------------------------------------------------------
-// Evaluation metrics of sr_mfe.py:315-345 on tensor2img-quantised uint8 images, per image:
+// Evaluation metrics of sr_mfe.py:315-345 on tensor2img-quantised images at white level M (255: uint8), per image:
 //   acc[b][0] = sum (a-b)^2            (compare_mse / compare_psnr / calculate_ergas)
 //   acc[b][1] = sum a                  (calculate_ergas: mean of the first image)
 //   acc[b][2] = sum of the SSIM map over the cropped interior and the C channels, 2^-40 fixed point
 // SSIM follows skimage.measure.compare_ssim(X, Y, multichannel=True) as the reference calls it
 // (scikit-image 0.15, _structural_similarity.py): 7x7 uniform window, K1 = 0.01, K2 = 0.03,
-// data_range = 255, sample covariance (x 49/48), float64, mean over the map cropped by 3 pixels per
-// side, then mean over channels.  Window sums are exact integers; the map is evaluated in fp64.
+// data_range = M, sample covariance (x 49/48), float64, mean over the map cropped by 3 pixels per
+// side, then mean over channels.  Window sums are exact integers (int64: 49 * 65535^2 > 2^31); the map is evaluated
+// in fp64.  M = 255 computes exactly what the uint8 form of this kernel computed.
 // ------------------------------------------------------------------------------------------
 constexpr int kSsimWin = 7, kSsimPad = 3, kSsimTile = 16;
 constexpr double kSsimScale = 1099511627776.0;  // 2^40
 
-__global__ void __launch_bounds__(256) metrics_u8_kernel(const float* __restrict__ a, const float* __restrict__ b,
-                                                         unsigned long long* __restrict__ acc, int H, int W, int C) {
-  __shared__ uint8_t sa[kSsimTile + 6][kSsimTile + 6 + 2], sb[kSsimTile + 6][kSsimTile + 6 + 2];
+__global__ void __launch_bounds__(256) metrics_kernel(const float* __restrict__ a, const float* __restrict__ b,
+                                                      unsigned long long* __restrict__ acc, int H, int W, int C,
+                                                      int M) {
+  __shared__ uint16_t sa[kSsimTile + 6][kSsimTile + 6 + 2], sb[kSsimTile + 6][kSsimTile + 6 + 2];
   __shared__ long long red[8][3];
   const int img = blockIdx.z / C, ch = blockIdx.z % C;  // grid z = B * C
   const float* ap = a + (int64_t(img) * C + ch) * H * W;
   const float* bp = b + (int64_t(img) * C + ch) * H * W;
+  const float fM = float(M);
   // the block owns the 16x16 pixels at (y0, x0); its SSIM windows need a 3-pixel apron
   const int y0 = blockIdx.y * kSsimTile, x0 = blockIdx.x * kSsimTile;
   for (int e = threadIdx.x; e < (kSsimTile + 6) * (kSsimTile + 6); e += 256) {
     const int ly = e / (kSsimTile + 6), lx = e - ly * (kSsimTile + 6);
     const int y = y0 + ly - kSsimPad, x = x0 + lx - kSsimPad;
     const bool in = y >= 0 && y < H && x >= 0 && x < W;
-    sa[ly][lx] = in ? uint8_t(quant_u8(ap[int64_t(y) * W + x])) : 0;
-    sb[ly][lx] = in ? uint8_t(quant_u8(bp[int64_t(y) * W + x])) : 0;
+    sa[ly][lx] = in ? uint16_t(quant_level(ap[int64_t(y) * W + x], fM)) : 0;
+    sb[ly][lx] = in ? uint16_t(quant_level(bp[int64_t(y) * W + x], fM)) : 0;
   }
   __syncthreads();
   const int ly = threadIdx.x / kSsimTile, lx = threadIdx.x % kSsimTile;
@@ -415,15 +496,16 @@ __global__ void __launch_bounds__(256) metrics_u8_kernel(const float* __restrict
   long long sse = 0, suma = 0, ss = 0;
   if (y < H && x < W) {
     const int va = sa[ly + kSsimPad][lx + kSsimPad], vb = sb[ly + kSsimPad][lx + kSsimPad];
-    sse = (long long)((va - vb) * (va - vb));
+    sse = (long long)(va - vb) * (va - vb);
     suma = va;
     if (y >= kSsimPad && y < H - kSsimPad && x >= kSsimPad && x < W - kSsimPad) {
-      int s1 = 0, s2 = 0, s11 = 0, s22 = 0, s12 = 0;
+      int s1 = 0, s2 = 0;
+      long long s11 = 0, s22 = 0, s12 = 0;
 #pragma unroll
       for (int dy = 0; dy < kSsimWin; ++dy)
 #pragma unroll
         for (int dx = 0; dx < kSsimWin; ++dx) {
-          const int p = sa[ly + dy][lx + dx], q = sb[ly + dy][lx + dx];
+          const unsigned p = sa[ly + dy][lx + dx], q = sb[ly + dy][lx + dx];
           s1 += p;
           s2 += q;
           s11 += p * p;
@@ -433,7 +515,9 @@ __global__ void __launch_bounds__(256) metrics_u8_kernel(const float* __restrict
       const double np = double(kSsimWin * kSsimWin), cov = np / (np - 1.0);
       const double ux = s1 / np, uy = s2 / np;
       const double vx = cov * (s11 / np - ux * ux), vy = cov * (s22 / np - uy * uy), vxy = cov * (s12 / np - ux * uy);
-      const double C1 = (0.01 * 255.0) * (0.01 * 255.0), C2 = (0.03 * 255.0) * (0.03 * 255.0);
+      // C1, C2 rounded on their own, as the compile-time constants of M = 255 were (an FMA would fuse their last
+      // multiply into the sums below and change the bits)
+      const double R = double(M), C1 = __dmul_rn(0.01 * R, 0.01 * R), C2 = __dmul_rn(0.03 * R, 0.03 * R);
       const double S = ((2.0 * ux * uy + C1) * (2.0 * vxy + C2)) / ((ux * ux + uy * uy + C1) * (vx + vy + C2));
       ss = __double2ll_rn(S * kSsimScale);
     }
@@ -458,9 +542,9 @@ __global__ void __launch_bounds__(256) metrics_u8_kernel(const float* __restrict
 }
 
 // out[b] = (mse, psnr, ssim, ergas) in float64, exactly as sr_mfe.py derives them from the sums (C bands: n = C H W,
-// SSIM averaged over the C channels, ERGAS divided by C)
+// SSIM averaged over the C channels, ERGAS divided by C); PSNR = 10 log10(M^2 / mse)
 __global__ void metrics_finalize_kernel(const unsigned long long* __restrict__ acc, double* __restrict__ out, int B,
-                                        int H, int W, int C, double scale) {
+                                        int H, int W, int C, double scale, int M) {
   const int b = blockIdx.x * blockDim.x + threadIdx.x;
   if (b >= B) return;
   const double n = double(C) * H * W;
@@ -469,7 +553,7 @@ __global__ void metrics_finalize_kernel(const unsigned long long* __restrict__ a
   const double mse = sse / n;
   const double nss = double(C) * double(H - 2 * kSsimPad) * double(W - 2 * kSsimPad);
   out[b * 4 + 0] = mse;
-  out[b * 4 + 1] = mse > 0.0 ? 10.0 * log10(255.0 * 255.0 / mse) : INFINITY;
+  out[b * 4 + 1] = mse > 0.0 ? 10.0 * log10(double(M) * double(M) / mse) : INFINITY;
   out[b * 4 + 2] = (H > 2 * kSsimPad && W > 2 * kSsimPad)
                        ? double(static_cast<long long>(acc[b * 4 + 2])) / kSsimScale / nss : NAN;
   out[b * 4 + 3] = 100.0 * sqrt(mse / (mean * mean) / double(C)) / scale;

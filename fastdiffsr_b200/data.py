@@ -9,7 +9,10 @@ loader is the bottleneck (SURVEY 8f N2), so here
     `lr_{l}/` (SURVEY F3), and when the folder exists it is used as is, like the reference does;
   * batches are assembled in pinned memory by a background thread one batch ahead of the GPU;
   * images of C = 1..8 bands (`channels`, the UNet's out_channel): C = 3 reads RGB images exactly as the reference,
-    C = 1 reads images as single-band 'L' or `.npy` arrays, any other C reads `.npy` (H,W,C) uint8 arrays.
+    C = 1 reads images as single-band 'L' or `.npy` arrays, any other C reads `.npy` (H,W,C) uint8 arrays;
+  * 16-bit imagery (`max_value` = M, the white level that maps to +1, DESIGN.md §4.6): `.npy` (H,W,C) uint16 arrays
+    for any C, and for C = 1 also 16-bit single-band images (Pillow modes I;16 / I;16L / I;16B, or I with values in
+    0..65535); items stay uint16 up to the device, where `u16_to_tensor` normalises them with M.
 """
 from __future__ import annotations
 
@@ -27,20 +30,24 @@ def is_image_file(filename):
     return any(filename.endswith(ext) for ext in IMG_EXTENSIONS)
 
 
-def _is_band_file(filename, channels):
-    """Files an image folder of `channels` bands is made of: images for C = 3, images or .npy for C = 1, .npy else."""
+def _is_band_file(filename, channels, wide=False):
+    """Files an image folder of `channels` bands is made of: images for C = 3, images or .npy for C = 1, .npy else.
+    A 16-bit folder (`wide`) is made of .npy and image files for every C; the loader rejects what it cannot read."""
+    if wide:
+        return filename.endswith(".npy") or is_image_file(filename)
     if channels == 3:
         return is_image_file(filename)
     return filename.endswith(".npy") or (channels == 1 and is_image_file(filename))
 
 
-def get_paths_from_images(path, channels=3):
-    """data/util.py:13-24 (channels=3); other band counts keep the files _is_band_file accepts."""
+def get_paths_from_images(path, channels=3, wide=False):
+    """data/util.py:13-24 (channels=3); other band counts and 16-bit folders (`wide`) keep the files _is_band_file
+    accepts."""
     assert os.path.isdir(path), '{:s} is not a valid directory'.format(path)
     images, rejected = [], 0
     for dirpath, _, fnames in sorted(os.walk(path)):
         for fname in sorted(fnames):
-            if _is_band_file(fname, channels):
+            if _is_band_file(fname, channels, wide):
                 images.append(os.path.join(dirpath, fname))
             elif is_image_file(fname):
                 rejected += 1
@@ -69,6 +76,47 @@ def _load_u8(path, channels=3):
     from PIL import Image
     with Image.open(path) as im:
         return _pil_u8(im, channels)
+
+
+_I16_MODES = ("I;16", "I;16L", "I;16B")
+
+
+def _load_u16(path, channels):
+    """A file of a 16-bit dataset as (H,W,C) uint16: a .npy uint16 array ((H,W) too for C = 1), or for C = 1 a 16-bit
+    single-band image (I;16 / I;16L / I;16B, or I with values in 0..65535), read losslessly.  Anything else is a
+    ValueError naming the file."""
+    if path.endswith(".npy"):
+        a = np.load(path, allow_pickle=False)
+        if a.ndim == 2 and channels == 1:
+            a = a[:, :, None]
+        if a.dtype != np.uint16 or a.ndim != 3 or a.shape[2] != channels:
+            raise ValueError(f"{path}: a 16-bit dataset of {channels} band(s) needs (H,W,{channels}) uint16 arrays, got "
+                             f"{a.dtype} {a.shape}")
+        return np.ascontiguousarray(a)
+    from PIL import Image
+    with Image.open(path) as im:
+        mode = im.mode
+        if channels != 1:
+            raise ValueError(f"{path}: a 16-bit dataset of {channels} bands is read from .npy (H,W,{channels}) uint16 "
+                             f"arrays, not from {mode} images")
+        if mode in _I16_MODES:
+            a = np.asarray(im).astype(np.uint16)
+        elif mode == "I":
+            a = np.asarray(im)
+            if a.size and (a.min() < 0 or a.max() > 65535):
+                raise ValueError(f"{path}: mode I image with values outside 0..65535")
+            a = a.astype(np.uint16)
+        else:
+            raise ValueError(f"{path}: a 16-bit single-band dataset needs I;16 (or I) images, got mode {mode}")
+    return np.ascontiguousarray(a)[:, :, None]
+
+
+def u16_to_tensor(img_u16: torch.Tensor, max_value: int):
+    """(B,H,W,C) uint16 -> (B,C,H,W) fp32 in [-1,1] at white level M = max_value: (min(v, M) / M) * 2 - 1 in fp32,
+    each step rounded to nearest (fdsr_bicubic_u16's conditioning bit for bit).  The divisor is a tensor on the
+    data's device, so that no device divides by a reciprocal of M."""
+    v = img_u16.permute(0, 3, 1, 2).float().clamp(max=float(max_value))
+    return (v / torch.tensor(float(max_value), dtype=torch.float32, device=v.device)) * 2.0 - 1.0
 
 
 def u8_to_tensor(img_u8: torch.Tensor):
@@ -108,12 +156,21 @@ class LRHRDataset:
     `{dataroot}/hr_{r}`, `{dataroot}/lr_{l}`, optional `{dataroot}/sr_{l}_{r}`; datatype 'lmdb' = the key-value layout
     of data/LRHR_dataset.py:17-27, 60-93 (`kv`: any object with get(key: bytes) -> bytes | None; default: the LMDB
     environment at `dataroot`).  `channels`: bands per image (1..8, see the module docstring); 'lmdb' holds
-    encoded images and so serves 1 or 3 bands."""
+    encoded images and so serves 1 or 3 bands.  `max_value`: None = 8-bit data; an integer M in 1..65535 = 16-bit
+    data with white level M (datatype 'img' only), read by `_load_u16` and normalised by `u16_to_tensor`."""
 
     def __init__(self, dataroot, datatype="img", l_resolution=64, r_resolution=256, split="val", data_len=-1,
-                 need_LR=True, img_mask="no", kv=None, channels=3):
+                 need_LR=True, img_mask="no", kv=None, channels=3, max_value=None):
         if datatype not in ("img", "lmdb"):
             raise NotImplementedError('data_type [{:s}] is not recognized.'.format(str(datatype)))
+        if max_value is not None:
+            if isinstance(max_value, bool) or int(max_value) != max_value or not 1 <= int(max_value) <= 65535:
+                raise ValueError(f"max_value must be an integer 1..65535 (got {max_value!r})")
+            max_value = int(max_value)
+            if datatype != "img":
+                raise ValueError(f"max_value: 16-bit data is read from image folders (datatype 'img'); datatype "
+                                 f"'{datatype}' stores encoded 8-bit images")
+        self.max_value = max_value
         if not 1 <= int(channels) <= 8:
             raise ValueError(f"channels must be 1..8 (got {channels})")
         if datatype == "lmdb" and channels not in (1, 3):
@@ -133,11 +190,12 @@ class LRHRDataset:
             self.dataset_len = int(length)
             self.data_len = self.dataset_len if (data_len is None or data_len <= 0) else min(data_len, self.dataset_len)
             return
-        self.hr_path = get_paths_from_images('{}/hr_{}'.format(dataroot, r_resolution), self.channels)
+        wide = max_value is not None
+        self.hr_path = get_paths_from_images('{}/hr_{}'.format(dataroot, r_resolution), self.channels, wide)
         sr_dir = '{}/sr_{}_{}'.format(dataroot, l_resolution, r_resolution)
         lr_dir = '{}/lr_{}'.format(dataroot, l_resolution)
-        self.sr_path = get_paths_from_images(sr_dir, self.channels) if os.path.isdir(sr_dir) else None
-        self.lr_path = get_paths_from_images(lr_dir, self.channels) if os.path.isdir(lr_dir) else None
+        self.sr_path = get_paths_from_images(sr_dir, self.channels, wide) if os.path.isdir(sr_dir) else None
+        self.lr_path = get_paths_from_images(lr_dir, self.channels, wide) if os.path.isdir(lr_dir) else None
         if self.sr_path is None and self.lr_path is None:
             raise FileNotFoundError(f"{dataroot}: neither {os.path.basename(sr_dir)}/ nor {os.path.basename(lr_dir)}/ exists")
         for p in (self.sr_path, self.lr_path):
@@ -163,38 +221,53 @@ class LRHRDataset:
         item["path"] = keys["HR"]
         return item
 
-    def get_u8(self, index):
-        """uint8 HWC arrays: always 'HR'; 'LR' and/or 'SR' as present on disk."""
+    def get_raw(self, index):
+        """HWC arrays as stored, uint8 (8-bit data) or uint16 (max_value set): always 'HR'; 'LR' and/or 'SR' as present
+        on disk."""
         if self.datatype == "lmdb":
             return self._lmdb_u8(index)
-        item = {"HR": _load_u8(self.hr_path[index], self.channels), "Index": index, "path": self.hr_path[index]}
+        load = _load_u8 if self.max_value is None else _load_u16
+        item = {"HR": load(self.hr_path[index], self.channels), "Index": index, "path": self.hr_path[index]}
         if self.lr_path is not None:
-            item["LR"] = _load_u8(self.lr_path[index], self.channels)
+            item["LR"] = load(self.lr_path[index], self.channels)
         if self.sr_path is not None:
-            item["SR"] = _load_u8(self.sr_path[index], self.channels)
+            item["SR"] = load(self.sr_path[index], self.channels)
         return item
+
+    def get_u8(self, index):
+        """uint8 HWC arrays of an 8-bit dataset (get_raw); a 16-bit dataset has no uint8 form."""
+        if self.max_value is not None:
+            raise ValueError("a 16-bit dataset (max_value set) holds uint16 arrays: use get_raw")
+        return self.get_raw(index)
+
+    def to_tensor(self, img):
+        """(B,H,W,C) stored arrays -> (B,C,H,W) fp32 in [-1,1]: u8_to_tensor, or u16_to_tensor at max_value."""
+        return u8_to_tensor(img) if self.max_value is None else u16_to_tensor(img, self.max_value)
 
     def __getitem__(self, index):
         """The reference's item (fp32 CHW tensors in [-1,1]; 'SR' needs the sr_ folder)."""
-        it = self.get_u8(index)
+        it = self.get_raw(index)
         out = {"Index": index}
         for k in ("HR", "SR", "LR"):
             if k in it:
-                out[k] = u8_to_tensor(torch.from_numpy(it[k])[None])[0]
+                out[k] = self.to_tensor(torch.from_numpy(it[k])[None])[0]
         return out
 
 
 def create_dataset(dataset_opt, phase, channels=3):
-    """data/__init__.py:24-40; `channels`: bands per image (the UNet's out_channel)."""
+    """data/__init__.py:24-40; `channels`: bands per image (the UNet's out_channel); `dataset_opt['max_value']`: the
+    white level of 16-bit data (absent or None: 8-bit data)."""
     return LRHRDataset(dataroot=dataset_opt['dataroot'], datatype=dataset_opt['datatype'],
                        l_resolution=dataset_opt['l_resolution'], r_resolution=dataset_opt['r_resolution'],
                        split=phase, data_len=dataset_opt['data_len'] if dataset_opt['data_len'] is not None else -1,
-                       need_LR=(dataset_opt['mode'] == 'LRHR'), channels=channels)
+                       need_LR=(dataset_opt['mode'] == 'LRHR'), channels=channels,
+                       max_value=dataset_opt.get('max_value'))
 
 
 class BatchLoader:
-    """Iterates `indices` of a dataset in batches of uint8 arrays stacked in pinned host memory, decoding one
-    batch ahead in a background thread.  Yields dicts {'HR','LR'?,'SR'?: pinned uint8 (B,H,W,C), 'Index': list}."""
+    """Iterates `indices` of a dataset in batches of its stored arrays (uint8, or uint16 for 16-bit data) stacked in
+    pinned host memory, decoding one batch ahead in a background thread.  Yields dicts
+    {'HR','LR'?,'SR'?: pinned (B,H,W,C), 'Index': list}."""
 
     def __init__(self, dataset, batch_size, indices=None, prefetch=2, pin=True):
         self.ds = dataset
@@ -207,7 +280,7 @@ class BatchLoader:
         return (len(self.indices) + self.bs - 1) // self.bs
 
     def _assemble(self, idxs):
-        items = [self.ds.get_u8(i) for i in idxs]
+        items = [self.ds.get_raw(i) for i in idxs]
         out = {"Index": list(idxs), "path": [it["path"] for it in items]}
         for k in ("HR", "LR", "SR"):
             if k in items[0]:

@@ -230,6 +230,18 @@ class Engine:
         self._call("fdsr_bicubic_u8", _ptr(lr_u8), B, h, w, H, W, _ptr(o8), _ptr(oc), self._stream())
         return o8, oc
 
+    def bicubic_u16(self, lr_u16, H: int, W: int, max_value: int, want_u16=True, want_cond=True):
+        """lr_u16: (B,h,w,C) torch.uint16 on device -> (u16 (B,H,W,C) | None, cond (B,C,H,W) fp32 | None): each band
+        resized as Pillow resizes an 'I;16' image, cond = (min(v, max_value) / max_value) * 2 - 1 (fdsr_bicubic_u16)."""
+        if lr_u16.dtype != torch.uint16 or lr_u16.dim() != 4 or lr_u16.shape[3] != self.C or lr_u16.device != self.device:
+            raise FdsrError(f"lr must be (B,h,w,{self.C}) uint16 on the engine's device")
+        lr_u16 = lr_u16.contiguous()
+        B, h, w, _ = lr_u16.shape
+        o16 = torch.empty((B, H, W, self.C), dtype=torch.uint16, device=self.device) if want_u16 else None
+        oc = torch.empty((B, self.C, H, W), dtype=torch.float32, device=self.device) if want_cond else None
+        self._call("fdsr_bicubic_u16", _ptr(lr_u16), B, h, w, H, W, int(max_value), _ptr(o16), _ptr(oc), self._stream())
+        return o16, oc
+
     def debug_noise(self, B: int, H: int, W: int, seed: int, stream_id: int, image_offset: int = 0):
         """(B,C,H,W) N(0,1) values of the built-in generator for step stream `stream_id` (T: x_T, t: z of step t)."""
         out = torch.empty((B, self.C, H, W), dtype=torch.float32, device=self.device)
@@ -291,6 +303,16 @@ class Engine:
         B, _, H, W = a.shape
         out = torch.empty((B, 4), dtype=torch.float64, device=self.device)
         self._call("fdsr_metrics_u8", _ptr(a), _ptr(b), B, H, W, float(scale), _ptr(out), self._stream())
+        return out
+
+    def metrics_u16(self, a, b, max_value: int, scale: float = 4.0):
+        """metrics_u8 on images quantised to levels 0..max_value instead of 0..255 (fdsr_metrics_u16): PSNR against
+        max_value^2, SSIM with data_range max_value.  max_value = 255 gives metrics_u8's bits.  Returns (B,4) float64."""
+        a, b = self._img(a, "a"), self._img(b, "b")
+        B, _, H, W = a.shape
+        out = torch.empty((B, 4), dtype=torch.float64, device=self.device)
+        self._call("fdsr_metrics_u16", _ptr(a), _ptr(b), B, H, W, int(max_value), float(scale), _ptr(out),
+                   self._stream())
         return out
 
     # ---- hooks

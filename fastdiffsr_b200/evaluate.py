@@ -3,7 +3,8 @@ batched LR images -> bit-exact bicubic conditioning -> T-step sampling -> device
 ERGAS against HR (for both the bicubic baseline 'INF' and the SR result), averaged like the reference.
 
 Differences, all deliberate: images are processed in batches (the reference feeds one image per step and
-crashes for B>1, SURVEY F2); metrics are computed on the device (`fdsr_metrics_u8`) instead of skimage +
+crashes for B>1, SURVEY F2); metrics are computed on the device (`fdsr_metrics_u8`, or `fdsr_metrics_u16` at the
+white level of 16-bit data) instead of skimage +
 matplotlib on the host; LPIPS (an AlexNet download) and the per-image matplotlib plot are not produced;
 under torchrun the dataset is sharded by image and the sums are all-reduced, or, with `tile_split`, every rank samples
 every image together with the others (each its share of the tiles) and the metrics are counted once.
@@ -18,7 +19,7 @@ import numpy as np
 import torch
 import torch.distributed as dist
 
-from .data import BatchLoader, u8_to_tensor
+from .data import BatchLoader, u16_to_tensor, u8_to_tensor
 from .parallel import reduce_sums, shard_bounds
 
 METRIC_NAMES = ("mse", "psnr", "ssim", "ergas")
@@ -62,6 +63,22 @@ def _save_u8(img_chw, path):
     return path
 
 
+def _save_u16(img_chw, path, max_value):
+    """The 16-bit tensor2img at white level M = max_value, rint(((clamp(x,-1,1) + 1) / 2) * M) in fp32 (ties to even),
+    saved as a single-band I;16 image (PNG / TIFF) for 1 band and as an (H,W,C) uint16 `.npy` array (extension replaced)
+    for any other band count, 3 included.  Returns the path written."""
+    from PIL import Image
+    a = img_chw.detach().float().clamp(-1, 1)
+    a = ((a + 1) / 2).permute(1, 2, 0).cpu().numpy()
+    u16 = (a * np.float32(max_value)).round().astype(np.uint16)
+    if u16.shape[2] == 1:
+        Image.fromarray(u16[:, :, 0]).save(path)  # 2-D uint16: mode I;16
+    else:
+        path = os.path.splitext(path)[0] + ".npy"
+        np.save(path, u16)
+    return path
+
+
 @torch.no_grad()
 def evaluate(netG, dataset, batch_size=16, scale=4, result_path=None, save_ext="tif", seed=0, current_step=0,
              logger=None, max_images=None, tile=None, tile_overlap=32, tile_batch=16, tile_split=False):
@@ -69,7 +86,9 @@ def evaluate(netG, dataset, batch_size=16, scale=4, result_path=None, save_ext="
     `tile`: sample every image as one canvas of overlapping tiles (GaussianDiffusion.super_resolution(tile=...)), one
     image per call (scenes may differ in size; the tiles of one canvas fill the GPU); the HR size is then `scale` x the
     LR size, whatever that size is.  `tile_split` (with `tile`, under torchrun): the ranks split each image's tiles
-    instead of sharding the images (GaussianDiffusion.super_resolution(tile_split=True)); rank 0 writes the images."""
+    instead of sharding the images (GaussianDiffusion.super_resolution(tile_split=True)); rank 0 writes the images.
+    A 16-bit dataset (`dataset.max_value` = M) is conditioned by `fdsr_bicubic_u16` (or its sr_ folder through
+    u16_to_tensor), scored by `fdsr_metrics_u16` at M and saved as 16-bit images; the returned keys are the same."""
     if tile_split and tile is None:
         raise ValueError("tile_split needs tile")
     if tile is not None:
@@ -86,12 +105,19 @@ def evaluate(netG, dataset, batch_size=16, scale=4, result_path=None, save_ext="
     write = result_path and (rank == 0 or not tile_split)
     loader = BatchLoader(dataset, batch_size, indices=range(start, stop))
     acc = torch.zeros(9, dtype=torch.float64, device=dev)       # bic[4], sr[4], n
+    M = getattr(dataset, "max_value", None)                      # None: 8-bit data
+    if M is None:
+        to_tensor, metrics, save = u8_to_tensor, eng.metrics_u8, _save_u8
+    else:
+        to_tensor = lambda x: u16_to_tensor(x, M)                # noqa: E731
+        metrics = lambda a, b, s: eng.metrics_u16(a, b, M, s)    # noqa: E731
+        save = lambda img, path: _save_u16(img, path, M)         # noqa: E731
     if write:                        # every rank writes its own shard's images there (tile_split: rank 0 all of them)
         os.makedirs(result_path, exist_ok=True)
     torch.cuda.synchronize(dev)
     t0 = time.perf_counter()
     for bi, batch in enumerate(loader):
-        hr = u8_to_tensor(batch["HR"].to(dev, non_blocking=True))
+        hr = to_tensor(batch["HR"].to(dev, non_blocking=True))
         H, W = hr.shape[2], hr.shape[3]
         if tile is not None and "LR" in batch:
             H, W = scale * batch["LR"].shape[1], scale * batch["LR"].shape[2]
@@ -99,22 +125,24 @@ def evaluate(netG, dataset, batch_size=16, scale=4, result_path=None, save_ext="
                 raise ValueError(f"image {batch['Index'][0]}: HR is {hr.shape[2]}x{hr.shape[3]}, not {scale} x the LR "
                                  f"size ({H}x{W})")
         if "SR" in batch:                                          # the reference's precomputed bicubic image
-            cond = u8_to_tensor(batch["SR"].to(dev, non_blocking=True)).contiguous()
-        else:
+            cond = to_tensor(batch["SR"].to(dev, non_blocking=True)).contiguous()
+        elif M is None:
             _, cond = eng.bicubic_u8(batch["LR"].to(dev, non_blocking=True), H, W, want_u8=False)
+        else:
+            _, cond = eng.bicubic_u16(batch["LR"].to(dev, non_blocking=True), H, W, M, want_u16=False)
         # one seed for the whole job; the noise of an image depends on its global dataset index only, so the result
         # does not depend on the batch size or the number of ranks
         sr = netG.super_resolution(cond, False, seed=seed, image_offset=start + bi * loader.bs, **tiling)
         if sr.dim() == 3:   # the SR3 baseline returns ret_img[-1] without the batch axis for a single image
             sr = sr[None]
-        m_bic = eng.metrics_u8(cond, hr, scale)
-        m_sr = eng.metrics_u8(sr, hr, scale)
+        m_bic = metrics(cond, hr, scale)
+        m_sr = metrics(sr, hr, scale)
         acc[0:4] += m_bic.sum(0)
         acc[4:8] += m_sr.sum(0)
         acc[8] += hr.shape[0]
         if write:
             for j, idx in enumerate(batch["Index"]):
-                _save_u8(sr[j], '{}/{}_{}_sr.{}'.format(result_path, current_step, idx + 1, save_ext))
+                save(sr[j], '{}/{}_{}_sr.{}'.format(result_path, current_step, idx + 1, save_ext))
     torch.cuda.synchronize(dev)
     dt = time.perf_counter() - t0
     if not tile_split:
@@ -152,12 +180,9 @@ def setup_logger(name="base", log_dir=None, screen=True):
     return lg
 
 
-def main(argv=None, default_config="config/sr_fastdiffsr_test_64_256.json", prog="sr_mfe.py"):
-    """Shared driver of the repo-root `sr_mfe.py` / `infer.py` (same flags as the reference's scripts)."""
+def parse_args(argv=None, default_config="config/sr_fastdiffsr_test_64_256.json", prog="sr_mfe.py"):
+    """The flags of the repo-root `sr_mfe.py` / `infer.py` (the reference's scripts' flags plus the B200 path's)."""
     import argparse
-    from . import config as Cfg
-    from .networks import define_G
-
     ap = argparse.ArgumentParser(prog=prog)
     ap.add_argument('-c', '--config', type=str, default=default_config, help='JSON file for configuration')
     ap.add_argument('-p', '--phase', type=str, choices=['train', 'val'], default='val')
@@ -178,9 +203,36 @@ def main(argv=None, default_config="config/sr_fastdiffsr_test_64_256.json", prog
     ap.add_argument('--tile-split', action='store_true',
                     help='under torchrun, split the tiles of each image over the ranks instead of sharding the images '
                          '(with --tile): one large scene on every GPU, the single-GPU result')
+    ap.add_argument('--max-value', type=int, default=None, metavar='N',
+                    help='16-bit data with white level N (1..65535, e.g. 4095 for 12-bit, 65535 for 16-bit): sets '
+                         'datasets.val.max_value')
     args = ap.parse_args(argv)
     if args.tile_split and args.tile is None:
         ap.error('--tile-split needs --tile')
+    if args.max_value is not None and not 1 <= args.max_value <= 65535:
+        ap.error('--max-value must be 1..65535')
+    return args
+
+
+def load_opt(args):
+    """The run's options: the JSON config (or the programmatic equivalent of a shipped one) with the flags applied."""
+    from . import config as Cfg
+    cfg_path = args.config
+    if os.path.exists(cfg_path) or os.path.basename(cfg_path) in Cfg._ALIASES:
+        opt = Cfg.load_config(cfg_path, phase='val', gpu_ids=args.gpu_ids)
+    else:  # the reference tree (and its JSON files) is absent: programmatic equivalent of the shipped config
+        opt = Cfg.default_config(os.path.basename(cfg_path))
+    opt["model"]["compute_dtype"] = args.dtype
+    if args.max_value is not None:
+        opt['datasets']['val']['max_value'] = args.max_value
+    return opt
+
+
+def main(argv=None, default_config="config/sr_fastdiffsr_test_64_256.json", prog="sr_mfe.py"):
+    """Shared driver of the repo-root `sr_mfe.py` / `infer.py` (same flags as the reference's scripts)."""
+    from .networks import define_G
+
+    args = parse_args(argv, default_config, prog)
     if args.phase == 'train':
         raise NotImplementedError("training is outside the B200 sampling path: train with the reference and point "
                                   "path.resume_state at the checkpoint")
@@ -190,12 +242,7 @@ def main(argv=None, default_config="config/sr_fastdiffsr_test_64_256.json", prog
         os.environ.setdefault("MASTER_ADDR", "127.0.0.1")
         torch.cuda.set_device(local_rank)
         dist.init_process_group("nccl", device_id=torch.device("cuda", local_rank))
-    cfg_path = args.config
-    if os.path.exists(cfg_path) or os.path.basename(cfg_path) in Cfg._ALIASES:
-        opt = Cfg.load_config(cfg_path, phase='val', gpu_ids=args.gpu_ids)
-    else:  # the reference tree (and its JSON files) is absent: programmatic equivalent of the shipped config
-        opt = Cfg.default_config(os.path.basename(cfg_path))
-    opt["model"]["compute_dtype"] = args.dtype
+    opt = load_opt(args)
     paths = opt['path'] or {}
     logger = setup_logger("base", paths.get('log') if isinstance(paths, dict) else None)
     dev = torch.device("cuda", local_rank)

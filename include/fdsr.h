@@ -269,6 +269,29 @@ int fdsr_sse_u8(fdsr_ctx* ctx, const float* a_dev, const float* b_dev, int32_t B
 int fdsr_metrics_u8(fdsr_ctx* ctx, const float* a_dev, const float* b_dev, int32_t B, int32_t H, int32_t W,
                     double ergas_scale, double* out_dev, void* stream);
 
+/* 16-bit imagery.  The white level max_value = M (1..65535) is the sample value that maps to +1: 65535 for 16-bit
+ * data, 4095 for 12-bit, 2047 for 11-bit, 10000 for reflectance scaled by 10^4.
+ *
+ * uint16 (B,h,w,C) dev -> Pillow-exact BICUBIC resize of each band as Pillow resizes an 'I;16' image (Pillow 12.2):
+ * the bounds and normalised double weights of fdsr_bicubic_u8 before its fixed-point step; horizontal pass, then
+ * vertical, with a uint16 intermediate; per sample ss = 0.0, ss = ss + double(p) * k in float64, every multiply and add
+ * rounded on its own; v = ss >= 0 ? floor(ss + 0.5) : -floor(-ss + 0.5); stored byte by byte as Pillow stores I;16,
+ * lo = CLIP8(v % 256), hi = CLIP8(v >> 8).  So v < 0 gives 0, 0..65535 gives v, and v > 65535 gives
+ * 65280 + v % 256, not 65535 (Pillow's store quirk, reproduced so that an sr_ folder written by Pillow and the
+ * conditioning rebuilt here are the same bits).  A uint16 image is always resized this way, even when its values fit
+ * in 8 bits: with M = 255 the result is not fdsr_bicubic_u8's, which uses 22-bit fixed point.
+ *   out_u16_dev (B,H,W,C) the resized levels (not clamped to max_value), or NULL;
+ *   cond_out_dev (B,C,H,W) fp32 = (min(v, max_value) / max_value) * 2 - 1 (fp32, each step rounded to nearest), or NULL.
+ * FDSR_E_INVALID: max_value outside 1..65535, a null lr_dev, both outputs null, B, h, w, H or W < 1. */
+int fdsr_bicubic_u16(fdsr_ctx* ctx, const uint16_t* lr_dev, int32_t B, int32_t h, int32_t w, int32_t H, int32_t W,
+                     int32_t max_value, uint16_t* out_u16_dev, float* cond_out_dev, void* stream);
+/* fdsr_metrics_u8 at white level max_value: both images are quantised to levels 0..M by
+ * rint(((clamp(x, -1, 1) + 1) / 2) * M) in fp32 (ties to even); PSNR = 10 log10(M^2 / mse); SSIM with data_range M
+ * (C1 = (0.01 M)^2, C2 = (0.03 M)^2); ERGAS as in fdsr_metrics_u8.  max_value = 255 gives fdsr_metrics_u8's bits.
+ * FDSR_E_INVALID: max_value outside 1..65535, null pointers, B, H or W < 1. */
+int fdsr_metrics_u16(fdsr_ctx* ctx, const float* a_dev, const float* b_dev, int32_t B, int32_t H, int32_t W,
+                     int32_t max_value, double ergas_scale, double* out_dev, void* stream);
+
 /* ---- test / profiling hooks (not part of the drop-in surface) ---- */
 /* Number of activation tensors of the current plan and their names ("downs.0", "downs.1.h", ...). */
 int32_t fdsr_debug_num_tensors(const fdsr_ctx* ctx);
