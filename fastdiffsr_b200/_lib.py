@@ -82,6 +82,9 @@ _SIGS = {
     "fdsr_sample_tiled_part": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint64, C.c_void_p, C.c_void_p,
                                          C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.c_int32,
                                          C.c_int32, C.c_int32, C.c_void_p, TILE_EXCHANGE_FN, C.c_void_p, C.c_void_p]),
+    "fdsr_sample_tiled_masked": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint64, C.c_void_p,
+                                           C.c_void_p, C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.c_int32,
+                                           C.c_int32, C.c_int32, C.c_void_p]),
     "fdsr_trace_frames": (C.c_int32, [C.c_void_p]),
     "fdsr_super_resolve_u8": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int32, C.c_int32, C.c_int32, C.c_int32,
                                         C.c_int32, C.c_void_p, C.c_uint64, C.c_void_p, C.c_void_p]),
@@ -98,6 +101,8 @@ _SIGS = {
                                    C.c_int32, C.c_void_p, C.c_void_p, C.c_void_p]),
     "fdsr_metrics_u16": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int32, C.c_int32, C.c_int32, C.c_int32,
                                    C.c_double, C.c_void_p, C.c_void_p]),
+    "fdsr_metrics_masked": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int32, C.c_int32,
+                                      C.c_int32, C.c_int32, C.c_double, C.c_void_p, C.c_void_p]),
     "fdsr_debug_num_tensors": (C.c_int32, [C.c_void_p]),
     "fdsr_debug_tensor_name": (C.c_char_p, [C.c_void_p, C.c_int32]),
     "fdsr_debug_read_tensor": (C.c_int, [C.c_void_p, C.c_char_p, C.c_void_p, C.c_int64, C.POINTER(C.c_int32),

@@ -172,7 +172,7 @@ struct fdsr_ctx {
   };
   std::vector<BicTab> bic;
   DevBuf<uint8_t> d_bic_tmp;
-  DevBuf<unsigned long long> d_metric;  // [B][4] integer accumulators of fdsr_metrics_u8 / _u16
+  DevBuf<unsigned long long> d_metric;  // [B][kMetricSlots] integer accumulators of fdsr_metrics_u8 / _u16 / _masked
   // pinned staging for the host-buffer path
   // host-buffer path: two slots so that the copies of one batch overlap the sampling of the next
   struct HostSlot {
@@ -213,6 +213,8 @@ struct fdsr_ctx {
   // fdsr_sample_tiled: [SampleArgs | canvas x_t (B,C,H,W) fp32 | per-tile eps store [slot][C][te_y][te_x] fp32],
   // grow-only, apart from the workspace (which only ever holds one chunk of tiles)
   DevBuf<uint8_t> d_tiled;
+  // fdsr_sample_tiled_masked: [tile flags uint8 | active list int64 | tile -> slot map int32], grow-only
+  DevBuf<uint8_t> d_tile_mask;
 };
 
 namespace {
@@ -1491,9 +1493,11 @@ struct TileOwner {
 // first step, step(t, k) for the k-th step t = T-1 .. 0, a trace frame after every trace_every(T)-th step, and the
 // result sr.  Everything that differs between two calls of the same shape (seed, image offset, noise / trace pointers)
 // is read from the SampleArgs slot in device memory.  owner != nullptr: frames and result at the owner's pixels only.
+// valid != nullptr ((B,H,W) uint8): frames and result are cond where valid is 0.
 template <typename Step>
 int sample_chain(fdsr_ctx* c, const SampleArgs* args, float* x, const float* cond, float* sr, int B, uint32_t HW,
-                 bool has_trace, cudaStream_t st, Step&& step, const TileOwner* owner = nullptr) {
+                 bool has_trace, cudaStream_t st, Step&& step, const TileOwner* owner = nullptr,
+                 const uint8_t* valid = nullptr) {
   const int T = c->T, nfr = fdsr_trace_frames(c), inter = trace_every(T);
   const int64_t per = int64_t(c->bands()) * HW;
   const unsigned gb = unsigned((per * B + 255) / 256);
@@ -1506,7 +1510,8 @@ int sample_chain(fdsr_ctx* c, const SampleArgs* args, float* x, const float* con
     if (owner)
       return launch(c, res2img_owned_kernel, grid, 256, 0, st, src, cond, out, bstride, c->bands(), owner->ay, owner->ax,
                     owner->g0, owner->g1, args, frame_off);
-    return launch(c, res2img_kernel, gb, 256, 0, st, src, cond, out, per, bstride, B, args, frame_off, sr3);
+    return launch(c, res2img_kernel, gb, 256, 0, st, src, cond, out, per, bstride, B, args, frame_off, sr3, valid,
+                  int64_t(HW));
   };
   int rc = launch(c, noise_init_kernel, grid, 256, 0, st, x, HW, c->bands(), args, uint32_t(T));
   if (rc) return rc;
@@ -1571,15 +1576,26 @@ TileChunks tile_chunks(int64_t tiles, int tile_batch) {
   return {n, n ? int((tiles + n - 1) / n) : 0};
 }
 
+// The active tiles of a masked job (fdsr_sample_tiled_masked): valid (B,H,W) uint8; act[s] = global tile of slot s,
+// slot[g] = the slot of tile g or -1
+struct TileMask {
+  const uint8_t* valid;
+  const int64_t* act;
+  const int32_t* slot;
+};
+
 // The T-step tiled loop over the own tiles [g0, g1) of B canvases.  d_tiled holds [SampleArgs | x (B,C,H,W) | ...]; the
 // workspace is reserved for one chunk (bc tiles of te_y x te_x); eps_store is indexed by global tile.  Per step: the
 // own tiles' eps into the store, chunk by chunk, then exchange(user, t, st) when given, then the blend of the pixels the
-// own tiles cover.  fdsr_sample_tiled: [0, n_tiles), no exchange, no owner.  Plain stream launches: a chunk's UNet (~5 ms
-// at bc = 16, 256^2) keeps the device well behind the host's ~0.3 ms of launch calls.
+// own tiles cover.  fdsr_sample_tiled: [0, n_tiles), no exchange, no owner.  mask != nullptr (fdsr_sample_tiled_masked):
+// [g0, g1) = [0, n_active) are slots of the active list, the store is indexed by slot and every pixel is blended.
+// Plain stream launches: a chunk's UNet (~5 ms at bc = 16, 256^2) keeps the device well behind the host's ~0.3 ms of
+// launch calls.
 template <typename T>
 int tiled_enqueue(fdsr_ctx* c, const float* cond, float* sr_out, bool has_trace, int B, const TileAxis& ay,
                   const TileAxis& ax, int64_t g0, int64_t g1, const TileChunks& ch, float* eps_store,
-                  fdsr_tile_exchange_fn exchange, void* user, const TileOwner* owner, cudaStream_t st) {
+                  fdsr_tile_exchange_fn exchange, void* user, const TileOwner* owner, cudaStream_t st,
+                  const TileMask* mask = nullptr) {
   const SampleArgs* args = reinterpret_cast<const SampleArgs*>(c->d_tiled.ptr);
   const uint32_t HW = uint32_t(ay.L) * uint32_t(ax.L);
   const int C = c->bands();
@@ -1593,7 +1609,10 @@ int tiled_enqueue(fdsr_ctx* c, const float* cond, float* sr_out, bool has_trace,
   const int64_t per_canvas = int64_t(ay.n) * ax.n;
   int b0 = 0, nb = B;
   uint32_t p0 = 0, p1 = HW;
-  if (g0 == g1) {
+  int64_t own0 = g0, own1 = g1;
+  if (mask) {
+    own0 = 0, own1 = INT64_MAX;
+  } else if (g0 == g1) {
     nb = 1, p1 = 0;
   } else if (g0 / per_canvas == (g1 - 1) / per_canvas) {
     b0 = int(g0 / per_canvas), nb = 1;
@@ -1608,7 +1627,8 @@ int tiled_enqueue(fdsr_ctx* c, const float* cond, float* sr_out, bool has_trace,
       [&](int t, int k) {
         for (int64_t i = 0; i < ch.n; ++i) {
           const int64_t tile0 = g0 + i * ch.bc, valid = std::min<int64_t>(ch.bc, g1 - tile0);
-          int rc = launch(c, tile_pack_kernel<T>, pack_blocks, 256, 0, st, cond, x, xin, ay, ax, tile0, g1 - 1, ch.bc, C);
+          int rc = launch(c, tile_pack_kernel<T>, pack_blocks, 256, 0, st, cond, x, xin, ay, ax, tile0, g1 - 1, ch.bc, C,
+                          mask ? mask->act : nullptr);
           if (!rc) rc = unet_internal<T>(c, t, st, false, true);
           if (rc) return rc;
           // padding slots repeat the last own tile and stay in the workspace: the store holds other ranks' slots
@@ -1620,9 +1640,10 @@ int tiled_enqueue(fdsr_ctx* c, const float* cond, float* sr_out, bool has_trace,
           if (e) return fail(c, FDSR_E_INVALID, "the tile exchange callback returned %d at step t = %d", e, t);
         }
         return launch(c, tile_blend_posterior_kernel, pgrid, 256, 0, st, x, eps_store, ay, ax, C, c->post[t], args,
-                      int64_t(k + 1), uint32_t(t), t > 0 ? 1 : 0, B, b0, p0, p1, g0, g1);
+                      int64_t(k + 1), uint32_t(t), t > 0 ? 1 : 0, B, b0, p0, p1, own0, own1,
+                      mask ? mask->slot : nullptr);
       },
-      owner);
+      owner, mask ? mask->valid : nullptr);
 }
 
 // The partition and need rule of fdsr_tiled_plan (include/fdsr.h).  Rank r owns [own_lo(r), own_lo(r + 1)).
@@ -1741,17 +1762,18 @@ const fdsr_ctx::BicTab* find_bic(const fdsr_ctx* c, int in, int out) {
   return nullptr;
 }
 
-// fdsr_metrics_u8 / fdsr_metrics_u16: one kernel pair at white level M
-int metrics(fdsr_ctx* c, const float* a, const float* b, int32_t B, int32_t H, int32_t W, int M, double ergas_scale,
-            double* out, cudaStream_t st) {
-  CUDA_TRY(c, c->d_metric.grow(size_t(B) * 32));
-  CUDA_TRY(c, cudaMemsetAsync(c->d_metric, 0, size_t(B) * 32, st));
+// fdsr_metrics_u8 / fdsr_metrics_u16 / fdsr_metrics_masked: one kernel pair at white level M (valid: null = all)
+int metrics(fdsr_ctx* c, const float* a, const float* b, const uint8_t* valid, int32_t B, int32_t H, int32_t W, int M,
+            double ergas_scale, double* out, cudaStream_t st) {
+  const size_t acc_bytes = size_t(B) * kMetricSlots * sizeof(unsigned long long);
+  CUDA_TRY(c, c->d_metric.grow(acc_bytes));
+  CUDA_TRY(c, cudaMemsetAsync(c->d_metric, 0, acc_bytes, st));
   const int C = c->bands();
   const dim3 grid((W + kSsimTile - 1) / kSsimTile, (H + kSsimTile - 1) / kSsimTile, B * C);
-  const int rc = launch(c, metrics_kernel, grid, 256, 0, st, a, b, c->d_metric.ptr, H, W, C, M);
+  const int rc = launch(c, metrics_kernel, grid, 256, 0, st, a, b, c->d_metric.ptr, H, W, C, M, valid);
   if (rc) return rc;
   return launch(c, metrics_finalize_kernel, (B + 127) / 128, 128, 0, st, c->d_metric.ptr, out, B, H, W, C, ergas_scale,
-                M);
+                M, valid != nullptr ? 1 : 0);
 }
 
 // The checks fdsr_sample_tiled, fdsr_sample_tiled_part and fdsr_tiled_plan share (c == nullptr: the global error)
@@ -1787,6 +1809,33 @@ int tiled_prepare(fdsr_ctx* c, const TileChunks& ch, const TileAxis& ay, const T
   CUDA_TRY(c, c->d_tiled.grow(256 + align_up(size_t(B) * c->bands() * ay.L * ax.L * 4, 256) + store_bytes));
   return launch(c, set_args_kernel, 1, 1, 0, st, reinterpret_cast<SampleArgs*>(c->d_tiled.ptr),
                 SampleArgs{seed, c->image0, noise, trace});
+}
+
+// The active tiles of `valid` (B,H,W): tile_active_kernel's flags, read back with the call's one stream synchronise;
+// the active list (global order) and the tile -> slot map go back to d_tile_mask.  *n_active: the number of slots.
+int tile_activity(fdsr_ctx* c, const uint8_t* valid, const TileAxis& ay, const TileAxis& ax, int64_t n_tiles,
+                  TileMask* mask, int64_t* n_active, cudaStream_t st) {
+  const size_t flags_bytes = align_up(size_t(n_tiles), 256), act_bytes = align_up(size_t(n_tiles) * 8, 256);
+  CUDA_TRY(c, c->d_tile_mask.grow(flags_bytes + act_bytes + size_t(n_tiles) * 4));
+  uint8_t* d_flags = c->d_tile_mask;
+  int rc = launch(c, tile_active_kernel, unsigned(n_tiles), 256, 0, st, valid, ay, ax, d_flags);
+  if (rc) return rc;
+  std::vector<uint8_t> flags(n_tiles);
+  CUDA_TRY(c, cudaMemcpyAsync(flags.data(), d_flags, size_t(n_tiles), cudaMemcpyDeviceToHost, st));
+  CUDA_TRY(c, cudaStreamSynchronize(st));
+  std::vector<int64_t> act;
+  std::vector<int32_t> slot(n_tiles, -1);
+  for (int64_t g = 0; g < n_tiles; ++g)
+    if (flags[g]) slot[g] = int32_t(act.size()), act.push_back(g);
+  int64_t* d_act = reinterpret_cast<int64_t*>(c->d_tile_mask + flags_bytes);
+  int32_t* d_slot = reinterpret_cast<int32_t*>(c->d_tile_mask + flags_bytes + act_bytes);
+  // pageable sources: each copy returns once its source is staged, so the vectors may go out of scope
+  if (!act.empty())
+    CUDA_TRY(c, cudaMemcpyAsync(d_act, act.data(), act.size() * 8, cudaMemcpyHostToDevice, st));
+  CUDA_TRY(c, cudaMemcpyAsync(d_slot, slot.data(), slot.size() * 4, cudaMemcpyHostToDevice, st));
+  *mask = TileMask{valid, d_act, d_slot};
+  *n_active = int64_t(act.size());
+  return FDSR_OK;
 }
 }  // namespace
 
@@ -2168,6 +2217,33 @@ int fdsr_sample_tiled(fdsr_ctx* c, const float* cond, const float* noise, uint64
   });
 }
 
+int fdsr_sample_tiled_masked(fdsr_ctx* c, const float* cond, const uint8_t* valid, const float* noise, uint64_t seed,
+                             float* sr_out, float* trace, int32_t B, int32_t H, int32_t W, int32_t tile_h,
+                             int32_t tile_w, int32_t overlap, int32_t tile_batch, void* stream) {
+  if (!c) return FDSR_E_INVALID;
+  int rc = tiled_entry_check(c, cond, sr_out, B, H, W, tile_h, tile_w, overlap, tile_batch);
+  if (rc) return rc;
+  if (!valid) return fail(c, FDSR_E_INVALID, "null argument (valid)");
+  const TileAxis ay = make_axis(H, tile_h, overlap), ax = make_axis(W, tile_w, overlap);
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  const int64_t n_tiles = int64_t(B) * ay.n * ax.n;
+  if (n_tiles > INT32_MAX)  // one block per tile, int32 slots
+    return fail(c, FDSR_E_INVALID, "a masked job has at most 2^31 - 1 tiles (got %lld)", (long long)n_tiles);
+  TileMask mask;
+  int64_t n_active = 0;
+  rc = tile_activity(c, valid, ay, ax, n_tiles, &mask, &n_active, st);
+  if (rc) return rc;
+  const TileChunks ch = tile_chunks(n_active, tile_batch);
+  const size_t store_bytes = size_t(ch.n) * ch.bc * c->bands() * ay.te * ax.te * 4;
+  rc = tiled_prepare(c, ch, ay, ax, B, store_bytes, noise, seed, trace, st);
+  if (rc) return rc;
+  float* eps_store = reinterpret_cast<float*>(c->d_tiled + 256 + align_up(size_t(B) * c->bands() * H * W * 4, 256));
+  return with_dtype(c, [&](auto e) {
+    return tiled_enqueue<typename decltype(e)::type>(c, cond, sr_out, trace != nullptr, B, ay, ax, 0, n_active, ch,
+                                                     eps_store, nullptr, nullptr, nullptr, st, &mask);
+  });
+}
+
 int64_t fdsr_tiled_plan(int32_t B, int32_t H, int32_t W, int32_t tile_h, int32_t tile_w, int32_t overlap, int32_t world,
                         int32_t rank, int64_t* out_host, int64_t cap) {
   int rc = tiled_check(nullptr, B, H, W, tile_h, tile_w, overlap);
@@ -2346,7 +2422,7 @@ int fdsr_sse_u8(fdsr_ctx* c, const float* a, const float* b, int32_t B, int32_t 
 int fdsr_metrics_u8(fdsr_ctx* c, const float* a, const float* b, int32_t B, int32_t H, int32_t W, double ergas_scale,
                     double* out, void* stream) {
   if (!c || !a || !b || !out || B < 1 || H < 1 || W < 1) return fail(c, FDSR_E_INVALID, "bad argument");
-  return metrics(c, a, b, B, H, W, 255, ergas_scale, out, static_cast<cudaStream_t>(stream));
+  return metrics(c, a, b, nullptr, B, H, W, 255, ergas_scale, out, static_cast<cudaStream_t>(stream));
 }
 
 int fdsr_metrics_u16(fdsr_ctx* c, const float* a, const float* b, int32_t B, int32_t H, int32_t W, int32_t max_value,
@@ -2356,7 +2432,18 @@ int fdsr_metrics_u16(fdsr_ctx* c, const float* a, const float* b, int32_t B, int
   if (max_value < 1 || max_value > 65535)
     return fail(c, FDSR_E_INVALID, "max_value must be 1..65535 (got %d)", max_value);
   if (!a || !b || !out) return fail(c, FDSR_E_INVALID, "null argument");
-  return metrics(c, a, b, B, H, W, int(max_value), ergas_scale, out, static_cast<cudaStream_t>(stream));
+  return metrics(c, a, b, nullptr, B, H, W, int(max_value), ergas_scale, out, static_cast<cudaStream_t>(stream));
+}
+
+int fdsr_metrics_masked(fdsr_ctx* c, const float* a, const float* b, const uint8_t* valid, int32_t B, int32_t H,
+                        int32_t W, int32_t max_value, double ergas_scale, double* out, void* stream) {
+  if (!c) return FDSR_E_INVALID;
+  if (B < 1 || H < 1 || W < 1) return fail(c, FDSR_E_INVALID, "B, H and W must be >= 1 (got %d, %dx%d)", B, H, W);
+  if (max_value < 1 || max_value > 65535)
+    return fail(c, FDSR_E_INVALID, "max_value must be 1..65535 (got %d)", max_value);
+  if (!a || !b || !out) return fail(c, FDSR_E_INVALID, "null argument");
+  if (!valid) return fail(c, FDSR_E_INVALID, "null argument (valid)");
+  return metrics(c, a, b, valid, B, H, W, int(max_value), ergas_scale, out, static_cast<cudaStream_t>(stream));
 }
 
 int32_t fdsr_debug_num_tensors(const fdsr_ctx* c) { return c ? int32_t(c->tensors.size()) : 0; }

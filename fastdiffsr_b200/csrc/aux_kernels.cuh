@@ -141,13 +141,19 @@ __global__ void posterior_kernel(const float* __restrict__ x, const float* __res
 // res2img (diffusion.py:275-281): clamp(x,-1,1)/2 + cond.  `out` rows may be strided per sample
 // so the same kernel fills the continous=True trace: out[b*out_bstride + i]; out == nullptr: frame `frame_off`
 // (floats) of args->trace.  raw != 0: plain copy of x (the SR3 baseline's frames are the images themselves).
+// valid != null ((B, hw) uint8, a masked tiled job): cond itself where valid is 0.
 __global__ void res2img_kernel(const float* __restrict__ x, const float* __restrict__ cond,
                                float* __restrict__ out, int64_t per_sample, int64_t out_bstride,
-                               int B, const SampleArgs* __restrict__ args, int64_t frame_off, int raw) {
+                               int B, const SampleArgs* __restrict__ args, int64_t frame_off, int raw,
+                               const uint8_t* __restrict__ valid, int64_t hw) {
   const int64_t i = blockIdx.x * int64_t(blockDim.x) + threadIdx.x;
   if (i >= per_sample * B) return;
   float* o = out != nullptr ? out : args->trace + frame_off;
   const int64_t b = i / per_sample, r = i - b * per_sample;
+  if (valid != nullptr && !valid[b * hw + r % hw]) {
+    o[b * out_bstride + r] = cond[i];
+    return;
+  }
   const float v = fminf(fmaxf(x[i], -1.0f), 1.0f);
   o[b * out_bstride + r] = raw ? x[i] : __fadd_rn(__fdiv_rn(v, 2.0f), cond[i]);
 }
@@ -468,15 +474,20 @@ __global__ void sse_u8_kernel(const float* __restrict__ a, const float* __restri
 // data_range = M, sample covariance (x 49/48), float64, mean over the map cropped by 3 pixels per
 // side, then mean over channels.  Window sums are exact integers (int64: 49 * 65535^2 > 2^31); the map is evaluated
 // in fp64.  M = 255 computes exactly what the uint8 form of this kernel computed.
+// Masked (fdsr_metrics_masked, valid = (B,H,W) uint8): the three sums run over the valid pixels and over the windows
+// whose 49 pixels are all valid, and
+//   acc[b][3] = number of valid values (C |V|),  acc[b][4] = number of SSIM map entries summed (over the C channels).
 // ------------------------------------------------------------------------------------------
 constexpr int kSsimWin = 7, kSsimPad = 3, kSsimTile = 16;
+constexpr int kMetricSlots = 8;  // accumulators per image
 constexpr double kSsimScale = 1099511627776.0;  // 2^40
 
 __global__ void __launch_bounds__(256) metrics_kernel(const float* __restrict__ a, const float* __restrict__ b,
                                                       unsigned long long* __restrict__ acc, int H, int W, int C,
-                                                      int M) {
+                                                      int M, const uint8_t* __restrict__ valid) {
   __shared__ uint16_t sa[kSsimTile + 6][kSsimTile + 6 + 2], sb[kSsimTile + 6][kSsimTile + 6 + 2];
-  __shared__ long long red[8][3];
+  __shared__ uint8_t sv[kSsimTile + 6][kSsimTile + 6 + 2];
+  __shared__ long long red[8][5];
   const int img = blockIdx.z / C, ch = blockIdx.z % C;  // grid z = B * C
   const float* ap = a + (int64_t(img) * C + ch) * H * W;
   const float* bp = b + (int64_t(img) * C + ch) * H * W;
@@ -489,16 +500,26 @@ __global__ void __launch_bounds__(256) metrics_kernel(const float* __restrict__ 
     const bool in = y >= 0 && y < H && x >= 0 && x < W;
     sa[ly][lx] = in ? uint16_t(quant_level(ap[int64_t(y) * W + x], fM)) : 0;
     sb[ly][lx] = in ? uint16_t(quant_level(bp[int64_t(y) * W + x], fM)) : 0;
+    if (valid != nullptr) sv[ly][lx] = in && valid[(int64_t(img) * H + y) * W + x] != 0;
   }
   __syncthreads();
   const int ly = threadIdx.x / kSsimTile, lx = threadIdx.x % kSsimTile;
   const int y = y0 + ly, x = x0 + lx;
-  long long sse = 0, suma = 0, ss = 0;
-  if (y < H && x < W) {
+  long long sse = 0, suma = 0, ss = 0, nv = 0, nw = 0;
+  if (y < H && x < W && (valid == nullptr || sv[ly + kSsimPad][lx + kSsimPad])) {
     const int va = sa[ly + kSsimPad][lx + kSsimPad], vb = sb[ly + kSsimPad][lx + kSsimPad];
     sse = (long long)(va - vb) * (va - vb);
     suma = va;
-    if (y >= kSsimPad && y < H - kSsimPad && x >= kSsimPad && x < W - kSsimPad) {
+    nv = 1;
+    bool win = y >= kSsimPad && y < H - kSsimPad && x >= kSsimPad && x < W - kSsimPad;
+    if (win && valid != nullptr) {
+#pragma unroll
+      for (int dy = 0; dy < kSsimWin; ++dy)
+#pragma unroll
+        for (int dx = 0; dx < kSsimWin; ++dx) win = win && sv[ly + dy][lx + dx];
+    }
+    if (win) {
+      nw = 1;
       int s1 = 0, s2 = 0;
       long long s11 = 0, s22 = 0, s12 = 0;
 #pragma unroll
@@ -526,36 +547,48 @@ __global__ void __launch_bounds__(256) metrics_kernel(const float* __restrict__ 
     sse += __shfl_xor_sync(0xffffffffu, sse, o);
     suma += __shfl_xor_sync(0xffffffffu, suma, o);
     ss += __shfl_xor_sync(0xffffffffu, ss, o);
+    nv += __shfl_xor_sync(0xffffffffu, nv, o);
+    nw += __shfl_xor_sync(0xffffffffu, nw, o);
   }
   const int warp = threadIdx.x >> 5;
   if ((threadIdx.x & 31) == 0) {
     red[warp][0] = sse;
     red[warp][1] = suma;
     red[warp][2] = ss;
+    red[warp][3] = nv;
+    red[warp][4] = nw;
   }
   __syncthreads();
-  if (threadIdx.x < 3) {
+  if (threadIdx.x < 5) {
     long long t = 0;
     for (int w8 = 0; w8 < 8; ++w8) t += red[w8][threadIdx.x];
-    if (t) atomicAdd(&acc[img * 4 + threadIdx.x], static_cast<unsigned long long>(t));  // integer: order-independent
+    if (t) atomicAdd(&acc[img * kMetricSlots + threadIdx.x], static_cast<unsigned long long>(t));  // order-independent
   }
 }
 
 // out[b] = (mse, psnr, ssim, ergas) in float64, exactly as sr_mfe.py derives them from the sums (C bands: n = C H W,
-// SSIM averaged over the C channels, ERGAS divided by C); PSNR = 10 log10(M^2 / mse)
+// SSIM averaged over the C channels, ERGAS divided by C); PSNR = 10 log10(M^2 / mse).  masked: n and the SSIM
+// divisor are the counts acc[b][3] and acc[b][4]; no valid value gives four NaNs, no whole valid window a NaN SSIM.
+// With every pixel valid the counts equal C H W and C (H-6) (W-6), so the result is the unmasked one bit for bit.
 __global__ void metrics_finalize_kernel(const unsigned long long* __restrict__ acc, double* __restrict__ out, int B,
-                                        int H, int W, int C, double scale, int M) {
+                                        int H, int W, int C, double scale, int M, int masked) {
   const int b = blockIdx.x * blockDim.x + threadIdx.x;
   if (b >= B) return;
-  const double n = double(C) * H * W;
-  const double sse = double(static_cast<long long>(acc[b * 4 + 0]));
-  const double mean = double(static_cast<long long>(acc[b * 4 + 1])) / n;
+  const unsigned long long* ab = acc + b * kMetricSlots;
+  const double n = masked ? double(static_cast<long long>(ab[3])) : double(C) * H * W;
+  if (n == 0.0) {
+    out[b * 4 + 0] = out[b * 4 + 1] = out[b * 4 + 2] = out[b * 4 + 3] = NAN;
+    return;
+  }
+  const double sse = double(static_cast<long long>(ab[0]));
+  const double mean = double(static_cast<long long>(ab[1])) / n;
   const double mse = sse / n;
-  const double nss = double(C) * double(H - 2 * kSsimPad) * double(W - 2 * kSsimPad);
+  const double nss = masked ? double(static_cast<long long>(ab[4]))
+                            : double(C) * double(H - 2 * kSsimPad) * double(W - 2 * kSsimPad);
   out[b * 4 + 0] = mse;
   out[b * 4 + 1] = mse > 0.0 ? 10.0 * log10(double(M) * double(M) / mse) : INFINITY;
-  out[b * 4 + 2] = (H > 2 * kSsimPad && W > 2 * kSsimPad)
-                       ? double(static_cast<long long>(acc[b * 4 + 2])) / kSsimScale / nss : NAN;
+  out[b * 4 + 2] = (masked ? nss > 0.0 : (H > 2 * kSsimPad && W > 2 * kSsimPad))
+                       ? double(static_cast<long long>(ab[2])) / kSsimScale / nss : NAN;
   out[b * 4 + 3] = 100.0 * sqrt(mse / (mean * mean) / double(C)) / scale;
 }
 

@@ -42,18 +42,39 @@ __device__ __forceinline__ TileCover tile_cover(const TileAxis& a, int y) {
   return c;
 }
 
+// Tile activity of a masked job (fdsr_sample_tiled_masked): flags[g] = 1 iff the window of global tile g holds a
+// pixel with valid != 0.  valid: (B,H,W) uint8.  grid n_tiles, one block per tile.
+__global__ void __launch_bounds__(256) tile_active_kernel(const uint8_t* __restrict__ valid, TileAxis ay, TileAxis ax,
+                                                          uint8_t* __restrict__ flags) {
+  const int64_t g = blockIdx.x, per_canvas = int64_t(ay.n) * ax.n;
+  const int64_t b = g / per_canvas;
+  const int r = int(g - b * per_canvas);
+  const int y0 = tile_start(ay, r / ax.n), x0 = tile_start(ax, r % ax.n);
+  const uint8_t* v = valid + b * int64_t(ay.L) * ax.L + int64_t(y0) * ax.L + x0;
+  int any = 0;
+  for (int p = threadIdx.x; p < ay.te * ax.te && !any; p += blockDim.x) {
+    const int py = p / ax.te;
+    any = v[int64_t(py) * ax.L + (p - py * ax.te)] != 0;
+  }
+  any = __syncthreads_or(any);
+  if (threadIdx.x == 0) flags[g] = uint8_t(any);
+}
+
 // Packed 16-channel NHWC network input of one chunk of `bc` tiles (x_t and cond of C bands, pack_pixel), read
-// from the canvases at each tile's window.  Chunk slot j holds global tile min(tile0 + j, g_last), g_last = the last
-// tile of the caller's own range: its last chunk is padded with repeats of that tile.  One thread per tile pixel.
+// from the canvases at each tile's window.  Chunk slot j holds tile slot min(tile0 + j, g_last), g_last = the last
+// slot of the caller's own range: its last chunk is padded with repeats of that slot.  Slot s is global tile act[s]
+// (the active tiles of a masked job), or s itself when act is null.  One thread per tile pixel.
 template <typename T>
 __global__ void tile_pack_kernel(const float* __restrict__ cond, const float* __restrict__ x, T* __restrict__ out,
-                                 TileAxis ay, TileAxis ax, int64_t tile0, int64_t g_last, int bc, int C) {
+                                 TileAxis ay, TileAxis ax, int64_t tile0, int64_t g_last, int bc, int C,
+                                 const int64_t* __restrict__ act) {
   const int64_t i = blockIdx.x * int64_t(blockDim.x) + threadIdx.x;
   const int64_t tpx = int64_t(ay.te) * ax.te;
   if (i >= bc * tpx) return;
   const int64_t j = i / tpx;
   const int p = int(i - j * tpx);
-  const int64_t g = min(tile0 + j, g_last);
+  const int64_t s = min(tile0 + j, g_last);
+  const int64_t g = act != nullptr ? act[s] : s;
   const int64_t per_canvas = int64_t(ay.n) * ax.n;
   const int64_t b = g / per_canvas;
   const int r = int(g - b * per_canvas);
@@ -76,14 +97,16 @@ __device__ __forceinline__ int64_t tile_row_base(const TileAxis& ay, const TileA
 // tile order, fp32, round-to-nearest, the sum starting from the first term so that a pixel covered once gets its tile's
 // eps exactly), then x_{t-1} = post1(x_t, eps, z) in place.  z: block z_block of args->noise, else the generator's
 // stream `stream` at (image0 + canvas, pixel index y*W + x); add_noise = 0 (t == 0): z = 0.  No atomics: each thread
-// owns its pixel.  x: (B,C,H,W); eps_store: [tile][C][te_y][te_x], indexed by global tile.
+// owns its pixel.  x: (B,C,H,W); eps_store: [slot][C][te_y][te_x], global tile g in slot slot[g], or in slot g when
+// slot is null.  A masked job's inactive tiles (slot -1) are left out of both sums, so "first" is the first active
+// term; a pixel with no active covering tile is not updated.
 // Own range [g0, g1): a pixel is updated iff one of its covering tiles lies in it (the union of the own tiles' windows,
 // fdsr_sample_tiled_part); [0, n_tiles) updates every pixel.  grid (ceil((p1 - p0) / 256), canvases): canvas
 // b0 + blockIdx.y, pixel indices [p0, p1) of it -- a band that contains every pixel the range updates.
 __global__ void tile_blend_posterior_kernel(float* __restrict__ x, const float* __restrict__ eps_store, TileAxis ay,
                                             TileAxis ax, int C, PostCoef k, const SampleArgs* __restrict__ args,
                                             int64_t z_block, uint32_t stream, int add_noise, int B, int b0, uint32_t p0,
-                                            uint32_t p1, int64_t g0, int64_t g1) {
+                                            uint32_t p1, int64_t g0, int64_t g1, const int32_t* __restrict__ slot) {
   const uint32_t HW = uint32_t(ay.L) * uint32_t(ax.L);
   const uint32_t p = p0 + blockIdx.x * blockDim.x + threadIdx.x;
   if (p >= p1) return;
@@ -98,29 +121,38 @@ __global__ void tile_blend_posterior_kernel(float* __restrict__ x, const float* 
   }
   if (!own) return;
   float wsum = 0.f;
+  bool any = false;
   for (int a = 0; a < ny; ++a) {
     const int ry = tile_ramp(ay, y - tile_start(ay, cy.at(a)));
+    const int64_t r = tile_row_base(ay, ax, b, cy.at(a));
     for (int c = 0; c < nx; ++c) {
+      if (slot != nullptr && slot[r + cx.at(c)] < 0) continue;
       const float w = float(ry * tile_ramp(ax, xx - tile_start(ax, cx.at(c))));
-      wsum = (a | c) ? __fadd_rn(wsum, w) : w;
+      wsum = any ? __fadd_rn(wsum, w) : w;
+      any = true;
     }
   }
+  if (!any) return;
   const int64_t tpx = int64_t(ay.te) * ax.te;
   float e[8] = {0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f};
+  bool first = true;
   for (int a = 0; a < ny; ++a) {
     const int ty = cy.at(a), oy = y - tile_start(ay, ty);
     const int ry = tile_ramp(ay, oy);
     for (int c = 0; c < nx; ++c) {
       const int tx = cx.at(c), ox = xx - tile_start(ax, tx);
-      const float nk = __fdiv_rn(float(ry * tile_ramp(ax, ox)), wsum);
       const int64_t g = tile_row_base(ay, ax, b, ty) + tx;
-      const float* ep = eps_store + g * C * tpx + int64_t(oy) * ax.te + ox;
+      const int64_t sg = slot != nullptr ? int64_t(slot[g]) : g;
+      if (sg < 0) continue;
+      const float nk = __fdiv_rn(float(ry * tile_ramp(ax, ox)), wsum);
+      const float* ep = eps_store + sg * C * tpx + int64_t(oy) * ax.te + ox;
 #pragma unroll
       for (int ch = 0; ch < 8; ++ch) {
         if (ch >= C) continue;
         const float term = __fmul_rn(nk, ep[ch * tpx]);
-        e[ch] = (a | c) ? __fadd_rn(e[ch], term) : term;
+        e[ch] = first ? term : __fadd_rn(e[ch], term);
       }
+      first = false;
     }
   }
   const size_t o = size_t(b) * C * HW + p;

@@ -119,6 +119,21 @@ def u16_to_tensor(img_u16: torch.Tensor, max_value: int):
     return (v / torch.tensor(float(max_value), dtype=torch.float32, device=v.device)) * 2.0 - 1.0
 
 
+def nodata_mask(img: torch.Tensor, nodata: int, H: int, W: int):
+    """The (B,H,W) bool validity mask at the HR size H x W of a (B,h,w,C) uint8 / uint16 image: a source pixel is
+    invalid iff every band equals `nodata`, and HR pixel (Y, X) takes source pixel (((2Y+1) h) // (2H),
+    ((2X+1) w) // (2W)), the one whose area holds the HR pixel's centre (the identity at h = H, w = W).  The bicubic
+    conditioning mixes fill into the valid pixels within two LR pixels of the footprint edge; that halo is scored and
+    sampled as valid, not corrected."""
+    if img.dim() != 4 or img.dtype not in (torch.uint8, torch.uint16):
+        raise ValueError(f"nodata_mask needs a (B,h,w,C) uint8 or uint16 tensor, got {img.dtype} {tuple(img.shape)}")
+    _, h, w, _ = img.shape
+    valid = (img != nodata).any(dim=3)
+    ys = (torch.arange(H, device=img.device) * 2 + 1) * h // (2 * H)
+    xs = (torch.arange(W, device=img.device) * 2 + 1) * w // (2 * W)
+    return valid[:, ys][:, :, xs]
+
+
 def u8_to_tensor(img_u8: torch.Tensor):
     """(B,H,W,C) uint8 -> (B,C,H,W) fp32 in [-1,1]: torchvision ToTensor (/255) then *2-1
     (data/util.py:66-75 with min_max=(-1,1)), same operation order."""
@@ -157,10 +172,12 @@ class LRHRDataset:
     of data/LRHR_dataset.py:17-27, 60-93 (`kv`: any object with get(key: bytes) -> bytes | None; default: the LMDB
     environment at `dataroot`).  `channels`: bands per image (1..8, see the module docstring); 'lmdb' holds
     encoded images and so serves 1 or 3 bands.  `max_value`: None = 8-bit data; an integer M in 1..65535 = 16-bit
-    data with white level M (datatype 'img' only), read by `_load_u16` and normalised by `u16_to_tensor`."""
+    data with white level M (datatype 'img' only), read by `_load_u16` and normalised by `u16_to_tensor`.
+    `nodata`: None, or the sample value V that marks fill (0..255 for 8-bit data, 0..65535 with max_value): a pixel
+    whose bands all equal V is outside the scene's footprint (nodata_mask)."""
 
     def __init__(self, dataroot, datatype="img", l_resolution=64, r_resolution=256, split="val", data_len=-1,
-                 need_LR=True, img_mask="no", kv=None, channels=3, max_value=None):
+                 need_LR=True, img_mask="no", kv=None, channels=3, max_value=None, nodata=None):
         if datatype not in ("img", "lmdb"):
             raise NotImplementedError('data_type [{:s}] is not recognized.'.format(str(datatype)))
         if max_value is not None:
@@ -171,6 +188,13 @@ class LRHRDataset:
                 raise ValueError(f"max_value: 16-bit data is read from image folders (datatype 'img'); datatype "
                                  f"'{datatype}' stores encoded 8-bit images")
         self.max_value = max_value
+        if nodata is not None:
+            top = 255 if max_value is None else 65535
+            if isinstance(nodata, bool) or int(nodata) != nodata or not 0 <= int(nodata) <= top:
+                raise ValueError(f"nodata must be an integer 0..{top} for {'8' if max_value is None else '16'}-bit data "
+                                 f"(got {nodata!r})")
+            nodata = int(nodata)
+        self.nodata = nodata
         if not 1 <= int(channels) <= 8:
             raise ValueError(f"channels must be 1..8 (got {channels})")
         if datatype == "lmdb" and channels not in (1, 3):
@@ -256,12 +280,13 @@ class LRHRDataset:
 
 def create_dataset(dataset_opt, phase, channels=3):
     """data/__init__.py:24-40; `channels`: bands per image (the UNet's out_channel); `dataset_opt['max_value']`: the
-    white level of 16-bit data (absent or None: 8-bit data)."""
+    white level of 16-bit data (absent or None: 8-bit data); `dataset_opt['nodata']`: the fill value (absent or None:
+    every pixel is valid)."""
     return LRHRDataset(dataroot=dataset_opt['dataroot'], datatype=dataset_opt['datatype'],
                        l_resolution=dataset_opt['l_resolution'], r_resolution=dataset_opt['r_resolution'],
                        split=phase, data_len=dataset_opt['data_len'] if dataset_opt['data_len'] is not None else -1,
                        need_LR=(dataset_opt['mode'] == 'LRHR'), channels=channels,
-                       max_value=dataset_opt.get('max_value'))
+                       max_value=dataset_opt.get('max_value'), nodata=dataset_opt.get('nodata'))
 
 
 class BatchLoader:

@@ -175,20 +175,26 @@ class GaussianDiffusion(nn.Module):
 
     @torch.no_grad()
     def p_sample_loop(self, x_in, continous=False, noise=None, seed=None, image_offset=0, *, tile=None, tile_overlap=32,
-                      tile_batch=16, tile_split=False):
+                      tile_batch=16, tile_split=False, valid=None):
         """`tile` (int or (th, tw), multiples of 8): sample canvases of any size (H, W >= 8) as overlapping tiles blended
         at every step (Engine.sample_tiled; `tile_overlap` pixels, `tile_batch` tiles per UNet call).  None: one piece.
         `tile_split` (with `tile`): every rank of the default process group samples the same canvases together, each
-        its share of the tiles (parallel.split_sample_tiled), and returns the whole, single-GPU result."""
+        its share of the tiles (parallel.split_sample_tiled), and returns the whole, single-GPU result.
+        `valid` (with `tile`, not with `tile_split`): a (B,H,W) bool / uint8 nodata mask, nonzero = valid: tiles with
+        no valid pixel are skipped and invalid pixels are returned as x_in (Engine.sample_tiled(valid=...))."""
         if not self.conditional:
             raise NotImplementedError("unconditional sampling is not on the SR path (unused by every config)")
         if tile is not None and self.sr3:
             raise NotImplementedError("tiled sampling is implemented for the FastDiffSR model only, not the SR3 baseline")
         if tile_split and tile is None:
             raise ValueError("tile_split splits the tiles of a canvas: it needs tile=")
+        if valid is not None and tile is None:
+            raise ValueError("valid masks the tiles of a canvas: it needs tile=")
+        if valid is not None and tile_split:
+            raise NotImplementedError("a nodata mask with tile_split is not implemented: sample masked canvases on one GPU")
         dist = torch.distributed
         split = tile_split and dist.is_available() and dist.is_initialized() and dist.get_world_size() > 1
-        tiling = None if tile is None else (tile, tile_overlap, tile_batch, split)
+        tiling = None if tile is None else (tile, tile_overlap, tile_batch, split, valid)
         if seed is None:   # unseeded like the reference (SURVEY F7); ranks seeded alike must still draw different noise
             seed = int(torch.randint(0, 2 ** 62, (1,)).item())
             if split:      # ... unless they sample the same canvases together: then every rank takes rank 0's seed
@@ -219,7 +225,7 @@ class GaussianDiffusion(nn.Module):
                           seed=seed, image_offset=image_offset)
         else:
             run = partial(eng.sample_tiled, x_in, tiling[0], overlap=tiling[1], tile_batch=tiling[2], noise=noise,
-                          seed=seed, image_offset=image_offset)
+                          seed=seed, image_offset=image_offset, valid=tiling[4])
         if not continous:
             sr = run()
             eng.check_overflow()
@@ -230,12 +236,12 @@ class GaussianDiffusion(nn.Module):
 
     @torch.no_grad()
     def super_resolution(self, x_in, continous=False, noise=None, seed=None, image_offset=0, *, tile=None,
-                         tile_overlap=32, tile_batch=16, tile_split=False):
+                         tile_overlap=32, tile_batch=16, tile_split=False, valid=None):
         """`image_offset`: global index of x_in[0] in a job sharded over batches / ranks (see Engine.sample).
         `tile`, `tile_overlap`, `tile_batch`: tiled sampling of large canvases (see p_sample_loop); `tile_split`: split
-        each canvas's tiles over the ranks of the default process group."""
+        each canvas's tiles over the ranks of the default process group; `valid`: the nodata mask of tiled sampling."""
         return self.p_sample_loop(x_in, continous, noise=noise, seed=seed, image_offset=image_offset, tile=tile,
-                                  tile_overlap=tile_overlap, tile_batch=tile_batch, tile_split=tile_split)
+                                  tile_overlap=tile_overlap, tile_batch=tile_batch, tile_split=tile_split, valid=valid)
 
     @torch.no_grad()
     def sample(self, batch_size=1, continous=False):

@@ -160,16 +160,31 @@ class Engine:
         self._call("fdsr_sample", _ptr(cond), _ptr(noise), seed, _ptr(out), _ptr(tr), B, H, W, self._stream())
         return (out, tr) if trace else out
 
+    def _valid(self, valid, B, H, W):
+        """A (B,H,W) bool or uint8 validity mask on this engine's device (nonzero = valid), as contiguous uint8."""
+        if (not isinstance(valid, torch.Tensor) or valid.dtype not in (torch.bool, torch.uint8)
+                or tuple(valid.shape) != (B, H, W) or valid.device != self.device):
+            raise FdsrError(f"valid must be a ({B},{H},{W}) bool or uint8 tensor on {self.device}")
+        valid = valid.contiguous()
+        return valid.view(torch.uint8) if valid.dtype == torch.bool else valid
+
     def sample_tiled(self, cond, tile, overlap: int = 32, tile_batch: int = 16, noise=None, seed: int = 0,
-                     trace: bool = False, image_offset: int = 0):
+                     trace: bool = False, image_offset: int = 0, valid=None):
         """T-step sampling of (B,C,H,W) canvases of any size (H, W >= 8) as overlapping tiles blended at every step
         (fdsr_sample_tiled).  `tile`: int or (th, tw), multiples of 8; `tile_batch`: tiles per UNet call (the activation
-        workspace scales with it, not with the canvas).  Noise, seed, image_offset and the trace are as in `sample`."""
+        workspace scales with it, not with the canvas).  Noise, seed, image_offset and the trace are as in `sample`.
+        `valid`: a (B,H,W) bool / uint8 mask, nonzero = valid (fdsr_sample_tiled_masked): only the tiles that hold a
+        valid pixel go through the UNet, and invalid pixels of the result and trace are cond itself."""
         th, tw = (tile, tile) if isinstance(tile, int) else (int(tile[0]), int(tile[1]))
         cond, noise, out, tr = self._sample_io(cond, noise, trace, image_offset)
         B, _, H, W = cond.shape
-        self._call("fdsr_sample_tiled", _ptr(cond), _ptr(noise), seed, _ptr(out), _ptr(tr), B, H, W, th, tw,
-                   int(overlap), int(tile_batch), self._stream())
+        if valid is None:
+            self._call("fdsr_sample_tiled", _ptr(cond), _ptr(noise), seed, _ptr(out), _ptr(tr), B, H, W, th, tw,
+                       int(overlap), int(tile_batch), self._stream())
+        else:
+            valid = self._valid(valid, B, H, W)
+            self._call("fdsr_sample_tiled_masked", _ptr(cond), _ptr(valid), _ptr(noise), seed, _ptr(out), _ptr(tr), B,
+                       H, W, th, tw, int(overlap), int(tile_batch), self._stream())
         return (out, tr) if trace else out
 
     @staticmethod
@@ -296,23 +311,33 @@ class Engine:
         self._call("fdsr_sse_u8", _ptr(a), _ptr(b), B, H, W, _ptr(out), self._stream())
         return out
 
-    def metrics_u8(self, a, b, scale: float = 4.0):
+    def metrics_u8(self, a, b, scale: float = 4.0, valid=None):
         """Per-image (mse, psnr, ssim, ergas) of `a` (SR or bicubic image) against `b` (HR), both (B,C,H,W) fp32
-        in [-1,1]: the reference's evaluation block (sr_mfe.py:315-345) on the device.  Returns (B,4) float64."""
+        in [-1,1]: the reference's evaluation block (sr_mfe.py:315-345) on the device.  Returns (B,4) float64.
+        `valid`: a (B,H,W) bool / uint8 mask: score the valid pixels only (fdsr_metrics_masked at 255)."""
+        if valid is not None:
+            return self.metrics_u16(a, b, 255, scale, valid=valid)
         a, b = self._img(a, "a"), self._img(b, "b")
         B, _, H, W = a.shape
         out = torch.empty((B, 4), dtype=torch.float64, device=self.device)
         self._call("fdsr_metrics_u8", _ptr(a), _ptr(b), B, H, W, float(scale), _ptr(out), self._stream())
         return out
 
-    def metrics_u16(self, a, b, max_value: int, scale: float = 4.0):
+    def metrics_u16(self, a, b, max_value: int, scale: float = 4.0, valid=None):
         """metrics_u8 on images quantised to levels 0..max_value instead of 0..255 (fdsr_metrics_u16): PSNR against
-        max_value^2, SSIM with data_range max_value.  max_value = 255 gives metrics_u8's bits.  Returns (B,4) float64."""
+        max_value^2, SSIM with data_range max_value.  max_value = 255 gives metrics_u8's bits.  Returns (B,4) float64.
+        `valid`: a (B,H,W) bool / uint8 mask: MSE, PSNR and ERGAS over the valid pixels, SSIM over the windows that
+        are wholly valid, NaN where nothing qualifies (fdsr_metrics_masked)."""
         a, b = self._img(a, "a"), self._img(b, "b")
         B, _, H, W = a.shape
         out = torch.empty((B, 4), dtype=torch.float64, device=self.device)
-        self._call("fdsr_metrics_u16", _ptr(a), _ptr(b), B, H, W, int(max_value), float(scale), _ptr(out),
-                   self._stream())
+        if valid is None:
+            self._call("fdsr_metrics_u16", _ptr(a), _ptr(b), B, H, W, int(max_value), float(scale), _ptr(out),
+                       self._stream())
+        else:
+            valid = self._valid(valid, B, H, W)
+            self._call("fdsr_metrics_masked", _ptr(a), _ptr(b), _ptr(valid), B, H, W, int(max_value), float(scale),
+                       _ptr(out), self._stream())
         return out
 
     # ---- hooks

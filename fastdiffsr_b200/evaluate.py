@@ -19,7 +19,7 @@ import numpy as np
 import torch
 import torch.distributed as dist
 
-from .data import BatchLoader, u16_to_tensor, u8_to_tensor
+from .data import BatchLoader, nodata_mask, u16_to_tensor, u8_to_tensor
 from .parallel import reduce_sums, shard_bounds
 
 METRIC_NAMES = ("mse", "psnr", "ssim", "ergas")
@@ -46,13 +46,20 @@ def load_network(netG, opt, logger=None):
     return True
 
 
-def _save_u8(img_chw, path):
+def _fill(img_hwc, fill):
+    """fill = (valid (H,W) bool tensor, V): every band of the invalid pixels set to V, in place."""
+    if fill is not None:
+        img_hwc[~fill[0].cpu().numpy()] = fill[1]
+    return img_hwc
+
+
+def _save_u8(img_chw, path, fill=None):
     """RGB for 3 bands, a single-band 'L' image for 1, an (H,W,C) uint8 `.npy` array (extension replaced) otherwise.
-    Returns the path written."""
+    `fill` = (valid, V): the invalid pixels are written as V in every band.  Returns the path written."""
     from PIL import Image
     a = img_chw.detach().float().clamp(-1, 1)
     a = ((a + 1) / 2).permute(1, 2, 0).cpu().numpy()
-    u8 = (a * 255.0).round().astype(np.uint8)
+    u8 = _fill((a * 255.0).round().astype(np.uint8), fill)
     if u8.shape[2] == 3:
         Image.fromarray(u8).save(path)
     elif u8.shape[2] == 1:
@@ -63,14 +70,15 @@ def _save_u8(img_chw, path):
     return path
 
 
-def _save_u16(img_chw, path, max_value):
+def _save_u16(img_chw, path, max_value, fill=None):
     """The 16-bit tensor2img at white level M = max_value, rint(((clamp(x,-1,1) + 1) / 2) * M) in fp32 (ties to even),
     saved as a single-band I;16 image (PNG / TIFF) for 1 band and as an (H,W,C) uint16 `.npy` array (extension replaced)
-    for any other band count, 3 included.  Returns the path written."""
+    for any other band count, 3 included.  `fill` = (valid, V): the invalid pixels are written as V in every band.
+    Returns the path written."""
     from PIL import Image
     a = img_chw.detach().float().clamp(-1, 1)
     a = ((a + 1) / 2).permute(1, 2, 0).cpu().numpy()
-    u16 = (a * np.float32(max_value)).round().astype(np.uint16)
+    u16 = _fill((a * np.float32(max_value)).round().astype(np.uint16), fill)
     if u16.shape[2] == 1:
         Image.fromarray(u16[:, :, 0]).save(path)  # 2-D uint16: mode I;16
     else:
@@ -88,7 +96,11 @@ def evaluate(netG, dataset, batch_size=16, scale=4, result_path=None, save_ext="
     LR size, whatever that size is.  `tile_split` (with `tile`, under torchrun): the ranks split each image's tiles
     instead of sharding the images (GaussianDiffusion.super_resolution(tile_split=True)); rank 0 writes the images.
     A 16-bit dataset (`dataset.max_value` = M) is conditioned by `fdsr_bicubic_u16` (or its sr_ folder through
-    u16_to_tensor), scored by `fdsr_metrics_u16` at M and saved as 16-bit images; the returned keys are the same."""
+    u16_to_tensor), scored by `fdsr_metrics_u16` at M and saved as 16-bit images; the returned keys are the same.
+    A dataset with a fill value (`dataset.nodata` = V) is scored on its valid pixels (nodata_mask of the LR image, or
+    of the sr_ image without LR; fdsr_metrics_masked), tiled sampling skips the tiles with no valid pixel, every band of
+    an invalid pixel is written as V, and an image whose eight metrics are not all finite (no valid pixel, or no wholly
+    valid SSIM window) is left out of the averages; 'n_excluded' counts those."""
     if tile_split and tile is None:
         raise ValueError("tile_split needs tile")
     if tile is not None:
@@ -104,14 +116,15 @@ def evaluate(netG, dataset, batch_size=16, scale=4, result_path=None, save_ext="
     start, stop, _ = (0, n_total, n_total) if tile_split else shard_bounds(n_total, rank, world)
     write = result_path and (rank == 0 or not tile_split)
     loader = BatchLoader(dataset, batch_size, indices=range(start, stop))
-    acc = torch.zeros(9, dtype=torch.float64, device=dev)       # bic[4], sr[4], n
+    acc = torch.zeros(10, dtype=torch.float64, device=dev)      # bic[4], sr[4], n averaged, n excluded
     M = getattr(dataset, "max_value", None)                      # None: 8-bit data
+    nodata = getattr(dataset, "nodata", None)                    # None: every pixel is valid
     if M is None:
         to_tensor, metrics, save = u8_to_tensor, eng.metrics_u8, _save_u8
     else:
-        to_tensor = lambda x: u16_to_tensor(x, M)                # noqa: E731
-        metrics = lambda a, b, s: eng.metrics_u16(a, b, M, s)    # noqa: E731
-        save = lambda img, path: _save_u16(img, path, M)         # noqa: E731
+        to_tensor = lambda x: u16_to_tensor(x, M)                                  # noqa: E731
+        metrics = lambda a, b, s, valid=None: eng.metrics_u16(a, b, M, s, valid)   # noqa: E731
+        save = lambda img, path, fill=None: _save_u16(img, path, M, fill)          # noqa: E731
     if write:                        # every rank writes its own shard's images there (tile_split: rank 0 all of them)
         os.makedirs(result_path, exist_ok=True)
     torch.cuda.synchronize(dev)
@@ -124,6 +137,9 @@ def evaluate(netG, dataset, batch_size=16, scale=4, result_path=None, save_ext="
             if (hr.shape[2], hr.shape[3]) != (H, W):
                 raise ValueError(f"image {batch['Index'][0]}: HR is {hr.shape[2]}x{hr.shape[3]}, not {scale} x the LR "
                                  f"size ({H}x{W})")
+        valid = None
+        if nodata is not None:                                     # the footprint: from LR, else from the sr_ image
+            valid = nodata_mask(batch["LR" if "LR" in batch else "SR"].to(dev, non_blocking=True), nodata, H, W)
         if "SR" in batch:                                          # the reference's precomputed bicubic image
             cond = to_tensor(batch["SR"].to(dev, non_blocking=True)).contiguous()
         elif M is None:
@@ -132,23 +148,37 @@ def evaluate(netG, dataset, batch_size=16, scale=4, result_path=None, save_ext="
             _, cond = eng.bicubic_u16(batch["LR"].to(dev, non_blocking=True), H, W, M, want_u16=False)
         # one seed for the whole job; the noise of an image depends on its global dataset index only, so the result
         # does not depend on the batch size or the number of ranks
-        sr = netG.super_resolution(cond, False, seed=seed, image_offset=start + bi * loader.bs, **tiling)
+        masked = {} if valid is None or tile is None else {"valid": valid}   # untiled: every pixel is sampled
+        sr = netG.super_resolution(cond, False, seed=seed, image_offset=start + bi * loader.bs, **tiling, **masked)
         if sr.dim() == 3:   # the SR3 baseline returns ret_img[-1] without the batch axis for a single image
             sr = sr[None]
-        m_bic = metrics(cond, hr, scale)
-        m_sr = metrics(sr, hr, scale)
-        acc[0:4] += m_bic.sum(0)
-        acc[4:8] += m_sr.sum(0)
-        acc[8] += hr.shape[0]
+        if valid is None:
+            m_bic = metrics(cond, hr, scale)
+            m_sr = metrics(sr, hr, scale)
+            acc[0:4] += m_bic.sum(0)
+            acc[4:8] += m_sr.sum(0)
+            acc[8] += hr.shape[0]
+        else:
+            m_bic = metrics(cond, hr, scale, valid=valid)
+            m_sr = metrics(sr, hr, scale, valid=valid)
+            keep = torch.isfinite(m_bic).all(1) & torch.isfinite(m_sr).all(1)
+            acc[0:4] += m_bic[keep].sum(0)
+            acc[4:8] += m_sr[keep].sum(0)
+            acc[8] += keep.sum()
+            acc[9] += (~keep).sum()
         if write:
             for j, idx in enumerate(batch["Index"]):
-                save(sr[j], '{}/{}_{}_sr.{}'.format(result_path, current_step, idx + 1, save_ext))
+                fill = None if valid is None else (valid[j], nodata)
+                save(sr[j], '{}/{}_{}_sr.{}'.format(result_path, current_step, idx + 1, save_ext), fill=fill)
     torch.cuda.synchronize(dev)
     dt = time.perf_counter() - t0
     if not tile_split:
         reduce_sums(acc)
     n = max(acc[8].item(), 1.0)
-    out = {"n": int(acc[8].item()), "seconds": dt, "images_per_s": acc[8].item() / dt if dt > 0 else float("nan")}
+    n_all = acc[8].item() + acc[9].item()
+    out = {"n": int(n_all), "seconds": dt, "images_per_s": n_all / dt if dt > 0 else float("nan")}
+    if nodata is not None:
+        out["n_excluded"] = int(acc[9].item())
     for i, k in enumerate(METRIC_NAMES):
         out["bic_" + k] = acc[i].item() / n
         out["sr_" + k] = acc[4 + i].item() / n
@@ -159,6 +189,9 @@ def evaluate(netG, dataset, batch_size=16, scale=4, result_path=None, save_ext="
             out["sr_mse"], out["sr_psnr"], out["sr_ssim"], out["sr_ergas"]))
         logger.info('{} images in {:.3f} s ({:.1f} images/s, batch {} x {} rank(s))'.format(
             out["n"], dt, out["images_per_s"], batch_size, world))
+        if nodata is not None:
+            logger.info('nodata {}: {} image(s) without a finite score left out of the averages'.format(
+                nodata, out["n_excluded"]))
     return out
 
 
@@ -206,11 +239,19 @@ def parse_args(argv=None, default_config="config/sr_fastdiffsr_test_64_256.json"
     ap.add_argument('--max-value', type=int, default=None, metavar='N',
                     help='16-bit data with white level N (1..65535, e.g. 4095 for 12-bit, 65535 for 16-bit): sets '
                          'datasets.val.max_value')
+    ap.add_argument('--nodata', type=int, default=None, metavar='V',
+                    help='fill value of the scenes (0..255, or 0..65535 for 16-bit data): pixels whose bands all equal '
+                         'V are not scored, are written as V and, with --tile, skip the UNet; sets datasets.val.nodata')
     args = ap.parse_args(argv)
     if args.tile_split and args.tile is None:
         ap.error('--tile-split needs --tile')
     if args.max_value is not None and not 1 <= args.max_value <= 65535:
         ap.error('--max-value must be 1..65535')
+    if args.nodata is not None:
+        if not 0 <= args.nodata <= 65535:
+            ap.error('--nodata must be 0..65535')
+        if args.tile_split:
+            ap.error('--nodata cannot be combined with --tile-split (masked tiles are sampled on one GPU)')
     return args
 
 
@@ -225,6 +266,8 @@ def load_opt(args):
     opt["model"]["compute_dtype"] = args.dtype
     if args.max_value is not None:
         opt['datasets']['val']['max_value'] = args.max_value
+    if args.nodata is not None:
+        opt['datasets']['val']['nodata'] = args.nodata
     return opt
 
 

@@ -214,6 +214,30 @@ int fdsr_sample_tiled_part(fdsr_ctx* ctx, const float* cond_dev, const float* no
                            int32_t tile_w, int32_t overlap, int32_t tile_batch, int32_t rank, int32_t world,
                            float* eps_store_dev, fdsr_tile_exchange_fn exchange, void* user, void* stream);
 
+/* Tiled sampling of scenes with nodata: fdsr_sample_tiled (same arguments and checks) with a validity mask
+ * valid_dev, a (B,H,W) uint8 array at the canvas resolution, nonzero = valid; all bands of a pixel share it.
+ *   Active tile: a tile of fdsr_sample_tiled's grid (same t_e, o_e, starts and global order) whose window holds at
+ *     least one valid pixel.  Only active tiles go through the UNet.
+ *   Chunking over the n_active active tiles in global order: n_chunks = ceil(n_active / tile_batch) UNet calls of
+ *     Bc = ceil(n_active / n_chunks) tiles (the last one padded with repeats); the eps store holds active tiles only.
+ *   Blend and update: per pixel over its *active* covering tiles in global order, with fdsr_sample_tiled's weights,
+ *     normalisation and fp32 round-to-nearest, the sums starting from the first active term.  A pixel with no active
+ *     covering tile is not updated; such a pixel is always invalid (every tile covering a valid pixel is active).
+ *   Noise: unchanged, drawn per canvas pixel from the same generator or noise_dev.
+ *   Output: valid pixels get fdsr_sample_tiled's res2img(x); invalid pixels get cond_dev, bit for bit.  Trace frames
+ *     follow the same rule.
+ *   Hence: when every tile is active (an all-valid mask among others) the valid pixels are fdsr_sample_tiled's bits;
+ *   with overlap 0 on a canvas the tiles partition and a mask invalid exactly on whole tiles, the valid pixels equal
+ *   fdsr_sample of the remaining crops (noise cropped alike); tile_batch does not change the result.
+ *   The tile flags are computed on the device (one block per tile) and read back once: the call synchronises `stream`
+ *   once, before it enqueues the sampling.  Launches: 1 + fdsr_sample_tiled's count with n_tiles replaced by n_active,
+ *   i.e. 3 + T * (n_chunks * (1 + UNet launches) + 1) + trace frames.  A canvas with no active tile runs no UNet and
+ *   returns cond (trace frames too).  FDSR_E_INVALID: everything fdsr_sample_tiled rejects, a null valid_dev, more than
+ *   2^31 - 1 tiles. */
+int fdsr_sample_tiled_masked(fdsr_ctx* ctx, const float* cond_dev, const uint8_t* valid_dev, const float* noise_dev,
+                             uint64_t seed, float* sr_out_dev, float* trace_out_dev, int32_t B, int32_t H, int32_t W,
+                             int32_t tile_h, int32_t tile_w, int32_t overlap, int32_t tile_batch, void* stream);
+
 /* fp16 mode only (always FDSR_OK otherwise): synchronises `stream`, then returns FDSR_E_OVERFLOW if any activation
  * stored since the last check had left the fp16 range (it was stored saturated, so nothing downstream is inf / NaN,
  * but the image is not the network's output), and clears the flag.  fdsr_super_resolve_u8 performs this check itself;
@@ -291,6 +315,15 @@ int fdsr_bicubic_u16(fdsr_ctx* ctx, const uint16_t* lr_dev, int32_t B, int32_t h
  * FDSR_E_INVALID: max_value outside 1..65535, null pointers, B, H or W < 1. */
 int fdsr_metrics_u16(fdsr_ctx* ctx, const float* a_dev, const float* b_dev, int32_t B, int32_t H, int32_t W,
                      int32_t max_value, double ergas_scale, double* out_dev, void* stream);
+/* fdsr_metrics_u16 over the valid pixels only: valid_dev (B,H,W) uint8, nonzero = valid (all bands share it).
+ *   MSE and the ERGAS mean run over the C |V| values of the valid pixels V; PSNR = 10 log10(M^2 / MSE);
+ *   SSIM = the mean, over the C channels and the cropped-interior positions whose whole 7x7 window is valid, of
+ *   fdsr_metrics_u16's SSIM map.  No such window: SSIM is NaN.  |V| = 0: all four are NaN.
+ *   An all-valid mask gives fdsr_metrics_u16's bits (fdsr_metrics_u8's at max_value = 255).  The SSIM accumulator
+ *   limit of fdsr_metrics_u16 (about 8.4 M band-pixels, DESIGN 4.6) applies unchanged.
+ * FDSR_E_INVALID: as fdsr_metrics_u16, and a null valid_dev. */
+int fdsr_metrics_masked(fdsr_ctx* ctx, const float* a_dev, const float* b_dev, const uint8_t* valid_dev, int32_t B,
+                        int32_t H, int32_t W, int32_t max_value, double ergas_scale, double* out_dev, void* stream);
 
 /* ---- test / profiling hooks (not part of the drop-in surface) ---- */
 /* Number of activation tensors of the current plan and their names ("downs.0", "downs.1.h", ...). */
